@@ -2,7 +2,7 @@
 """bench.py -- 6-view scenes/sec of the RoadMapBCE training step on B200 (BASELINE.json config 2:
 bf16 activations, batch 32 scenes per GPU, views 6x3x256x306, hidden 256 / latent 128).
 
-    python bench.py [--gpus N --steps K --warmup W] [--impl reference]
+    python bench.py [--gpus N --steps K --warmup W] [--impl reference] [--dump-outputs DIR]
 
 One "step" = zero_grad + stitch/conv encoder/dense blocks/800x800 head + fused BCE/threat score +
 backward + Adam on one batch of synthetic scenes; for N>1 the gradient exchange, the Adam update of each rank's
@@ -53,9 +53,16 @@ def parse():
     ap.add_argument("--no-defer-join", action="store_true", help="A/B: join the overlapped weight exchange inside step()")
     ap.add_argument("--multicast", default="auto", choices=["auto", "on", "off"],
                     help="A/B: NVLink multicast (multimem) vs peer loads in the sharded update; auto = peer loads")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (float32 / "
+                         "float64, at most 64 MB: larger tensors as a fixed seeded sample), to compare two builds")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     if a.mode == "inference":
         a.config = "inference"
+    if a.dump_outputs and (a.impl != "ours" or a.config == "inference"):
+        ap.error("--dump-outputs covers the training step of --impl ours (configs roadmap, ae, bb)")
     if a.batch is None:
         a.batch = 64 if a.config == "ae" else (256 if a.config == "inference" else 32)
     return a
@@ -443,7 +450,7 @@ def run_inference(args):
         for b in sizes:
             if name == "fp32" and b > 64:
                 continue                                  # the fp32 SIMT parity path is not the throughput path
-            iters = max(3, min(args.steps * 4, 256 // b))
+            iters = args.steps
             row = {"dtype": name, "batch": b}
             out_h = torch.empty(b, MAP, MAP, dtype=torch.uint8).pin_memory()
             for mode, src in (("resident", views_d[:b]), ("e2e", views_h[:b])):
@@ -541,6 +548,39 @@ def inference_parity(loaders, state_dict, n):
     return res
 
 
+DUMP_MAX_BYTES = 64 << 20
+DUMP_SAMPLE = 1 << 20          # elements written of a tensor larger than this
+
+
+def step_outputs(model, loss):
+    """What one training step hands its caller: the loss, the model state it leaves behind (parameters after the optimizer
+    step, BatchNorm statistics) and, where the model keeps them (RoadMapBCE), the step's threat scores and binary map."""
+    out = {"loss": loss}
+    out.update(("state." + k, v) for k, v in model.state_dict().items())
+    out.update(("metrics." + k, v) for k, v in (getattr(model, "last_metrics", None) or {}).items())
+    return out
+
+
+def dump_outputs(tensors, path):
+    """Each tensor as <path>/<name>.npy: float32, or float64 for 64-bit floats and integers (exact counts).  A tensor of
+    more than DUMP_SAMPLE elements is written flat as its elements at DUMP_SAMPLE indices drawn with a fixed seed, so two
+    runs, or two builds, write the same positions."""
+    import numpy as np
+    arrays = {}
+    for name, t in tensors.items():
+        t = t.detach()
+        if t.numel() > DUMP_SAMPLE:
+            idx = torch.randint(t.numel(), (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(0)).sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        wide = t.dtype in (torch.float64, torch.int64, torch.int32)
+        arrays[name] = t.to(torch.float64 if wide else torch.float32).cpu().numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit(f"bench.py: --dump-outputs would write {total} bytes (limit {DUMP_MAX_BYTES})")
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
 
 def run_ours(args):
     rank = int(os.environ.get("RANK", "0"))
@@ -600,6 +640,8 @@ def run_ours(args):
     sec = e0.elapsed_time(e1) * 1e-3
     clocks = sampler.stop() if sampler else None
     final_loss = float(loss.detach())
+    if args.dump_outputs and rank == 0:      # now: the end-to-end steps below train the model further
+        dump_outputs(step_outputs(model, loss), args.dump_outputs)
 
     # ---- end to end: host buffers in, loss out, every step -------------------------------------
     copy_stream = torch.cuda.Stream()

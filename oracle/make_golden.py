@@ -233,7 +233,7 @@ def binarise_case():
 
 if __name__ == "__main__":
     os.makedirs(GOLD, exist_ok=True)
-    torch.set_num_threads(os.cpu_count())
+    torch.set_num_threads(so.GOLDEN_THREADS)
     if len(sys.argv) > 1 and sys.argv[1] == "bb":
         bb_case("bb_full_b1", batch=1, hidden=8, latent=8)
         sys.exit(0)

@@ -26,6 +26,9 @@ import torch
 import torch.nn.functional as F
 
 VIEW_ORDER = (0, 1, 2, 5, 4, 3)  # roadmap_bce_v2.py:58, autoencoder.py:55, spatial_w_rm.py:58
+# intra-op threads of torch's CPU ops when the golden files were written: conv / linear split their reductions by
+# thread count, so a bit-for-bit comparison with those files has to run with the same count on any machine
+GOLDEN_THREADS = 8
 BINARISE_THRESHOLD_BITS = 0x33C00000  # sigmoid(x).round()==1  <=>  x > 1.5*2**-24 (see binarise)
 
 

@@ -52,6 +52,54 @@ def test_clock_sampler_reports_only_samples_of_the_timed_region():
     assert r["reasons"] == ["sw_power_cap"]
 
 
+def test_dump_outputs_writes_a_fixed_sample(tmp_path):
+    """--dump-outputs: float32 (float64 for 64-bit types), shapes kept below the sample size, larger tensors as the same
+    seeded sample on every call, and the size cap enforced before anything is written."""
+    import numpy as np
+    import pytest
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    big = torch.arange(bench.DUMP_SAMPLE * 3, dtype=torch.float32)
+    tensors = {"loss": torch.tensor(0.5, dtype=torch.bfloat16), "counts": torch.tensor([3, 1 << 40]),
+               "binary": torch.ones(2, 3, dtype=torch.uint8), "big": big}
+    for d in ("a", "b"):
+        bench.dump_outputs(tensors, str(tmp_path / d))
+    a = {n: np.load(tmp_path / "a" / (n + ".npy")) for n in tensors}
+    assert a["loss"].dtype == np.float32 and a["loss"].shape == () and float(a["loss"]) == 0.5
+    assert a["counts"].dtype == np.float64 and a["counts"].tolist() == [3, 1 << 40]
+    assert a["binary"].dtype == np.float32 and a["binary"].shape == (2, 3)
+    s = a["big"]
+    assert s.shape == (bench.DUMP_SAMPLE,) and np.all(np.diff(s) >= 0) and s.max() > 2 * bench.DUMP_SAMPLE
+    assert np.array_equal(s, np.load(tmp_path / "b" / "big.npy"))
+    many = {f"t{i}": big for i in range(17)}                       # 17 x 4 MB samples > 64 MB
+    with pytest.raises(SystemExit):
+        bench.dump_outputs(many, str(tmp_path / "c"))
+    assert not (tmp_path / "c").exists()
+
+
+def test_step_outputs_of_the_roadmap_step():
+    """What a training step hands its caller: loss, the state left behind, RoadMapBCE's metrics."""
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    from driving_dirty_b200.synthetic import random_roadmap_model
+    model = random_roadmap_model(16, 8, 16, 20, dtype="fp32", device="cpu", map_size=8)
+    model.last_metrics = {"ts": torch.tensor(0.25), "binary": torch.zeros(1, 8, 8, dtype=torch.uint8)}
+    out = bench.step_outputs(model, torch.tensor(0.75))
+    assert float(out["loss"]) == 0.75 and float(out["metrics.ts"]) == 0.25
+    assert torch.equal(out["metrics.binary"], model.last_metrics["binary"])
+    assert {k[len("state."):] for k in out if k.startswith("state.")} == set(model.state_dict())
+    assert torch.equal(out["state.fc1.weight"], model.fc1.weight)
+
+
+def test_bench_rejects_zero_steps_and_unsupported_dumps():
+    for extra in (["--steps", "0"], ["--config", "inference", "--dump-outputs", "x"], ["--impl", "reference", "--dump-outputs", "x"]):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + extra, capture_output=True, text=True,
+                             timeout=300, cwd=ROOT)
+        assert out.returncode == 2 and out.stdout == "", (extra, out.stderr[-500:])
+
+
 def test_clock_sampler_without_nvidia_smi():
     sys.path.insert(0, ROOT)
     import bench

@@ -35,6 +35,15 @@ def q(x, dtype):
     return x.to(dtype).float()
 
 
+def init_from(mod, g):
+    """torch's default Conv2d / ConvTranspose2d initialisation (uniform in +-1/sqrt(fan_in)) drawn from the test's own
+    generator: with the global RNG the layer would depend on which tests ran before it in the same process."""
+    bound = mod.weight[0].numel() ** -0.5
+    with torch.no_grad():
+        for t in (mod.weight, mod.bias):
+            t.copy_((torch.rand(t.shape, generator=g) * 2 - 1) * bound)
+
+
 # ------------------------------------------------------------------------------- stitch ------
 @pytest.mark.parametrize("B,H,W", [(1, 4, 6), (3, 16, 20), (2, 5, 7), (2, 256, 306)])
 def test_stitch_bit_exact(dd, B, H, W):
@@ -547,6 +556,7 @@ def test_conv2d_generic_fwd_dgrad_wgrad(dd, layer, dtype, tol, relu):
     g = torch.Generator().manual_seed(sum(map(ord, layer)))
     mod_cls = torch.nn.ConvTranspose2d if L["t"] else torch.nn.Conv2d
     mod = mod_cls(L["cin"], L["cout"], kernel_size=L["k"], stride=L["s"], padding=L["p"], dilation=L["d"])
+    init_from(mod, g)
     with torch.no_grad():
         # bf16 path: the tensor-core layers read their weights as bf16 operands; give the reference the same operands, or
         # outputs within rounding of zero flip their ReLU mask and the comparison measures the flips, not the kernel
@@ -596,6 +606,7 @@ def test_conv2d_tcgen05_layers(dd, layer):
     g = torch.Generator().manual_seed(sum(map(ord, layer)))
     mod_cls = torch.nn.ConvTranspose2d if t else torch.nn.Conv2d
     mod = mod_cls(cin, cout, kernel_size=k, stride=1, padding=p, dilation=d)
+    init_from(mod, g)
     with torch.no_grad():
         mod.weight.copy_(q(mod.weight, dtype))            # the kernel reads the weights as bf16 operands
     x = q(F.relu(torch.randn(B, cin, *hw, generator=g)), dtype).requires_grad_(True)

@@ -9,6 +9,15 @@ import torch
 from oracle import scene_oracle as so
 
 
+@pytest.fixture(autouse=True)
+def golden_thread_count():
+    """The goldens are compared bit for bit: run torch's CPU ops with the thread count they were written with."""
+    n = torch.get_num_threads()
+    torch.set_num_threads(so.GOLDEN_THREADS)
+    yield
+    torch.set_num_threads(n)
+
+
 def sha(t):
     return hashlib.sha256(np.ascontiguousarray(t.detach().cpu().numpy()).tobytes()).hexdigest()
 
