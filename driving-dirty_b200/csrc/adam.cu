@@ -12,16 +12,16 @@
 //   The caller brackets the launch with cross-rank barriers (grads complete before / weights landed after).
 //
 // HBM-bound when local (28 B per element), NVLink-bound when sharded.
+#include "adam.cuh"
 #include "dd_common.cuh"
 
 namespace {
 
+using dd::AdamHyper;
+using dd::adam_one;
+
 constexpr int kMaxRanks = 16;
 constexpr int kThreads = 256;   // 256 threads x <= 96 registers: one update CTA fits on an SM beside any persistent conv CTA
-
-struct AdamHyper {
-  float beta1, beta2, eps, step_size, inv_sqrt_bc2, weight_decay, grad_scale;
-};
 
 struct PeerPtrs {
   const float* grad[kMaxRanks];   // every rank's gradient replica (index = rank), full length
@@ -37,15 +37,6 @@ __device__ __forceinline__ float4 ld_reduce_add(const float* mc) {
 __device__ __forceinline__ void mc_store(float* mc, float4 v) {
   asm volatile("multimem.st.relaxed.sys.global.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(mc), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w)
                : "memory");
-}
-
-__device__ __forceinline__ float adam_one(float p, float g, float& m, float& v, const AdamHyper& h) {
-  g = g * h.grad_scale;
-  if (h.weight_decay != 0.f) g = fmaf(h.weight_decay, p, g);          // torch.optim.Adam: L2 term added to the gradient
-  m = m + (1.f - h.beta1) * (g - m);                                   // lerp, as torch's fused kernel
-  v = h.beta2 * v + (1.f - h.beta2) * g * g;
-  const float denom = sqrtf(v) * h.inv_sqrt_bc2 + h.eps;
-  return p - h.step_size * (m / denom);
 }
 
 // MODE 0: local (grad / param = one pointer each).  MODE 1: peer pointers.  MODE 2: multicast pointers.
@@ -139,15 +130,6 @@ int grid_for(long long n4) {
   return (int)(want < cap ? (want < 1 ? 1 : want) : cap);
 }
 
-AdamHyper hyper(float lr, float beta1, float beta2, float eps, float weight_decay, long long step, float grad_scale) {
-  const double bc1 = 1.0 - pow((double)beta1, (double)step), bc2 = 1.0 - pow((double)beta2, (double)step);
-  AdamHyper h;
-  h.beta1 = beta1; h.beta2 = beta2; h.eps = eps; h.weight_decay = weight_decay; h.grad_scale = grad_scale;
-  h.step_size = (float)((double)lr / bc1);
-  h.inv_sqrt_bc2 = (float)(1.0 / sqrt(bc2));
-  return h;
-}
-
 }  // namespace
 
 extern "C" int dd_adam_step(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, long long n, float lr,
@@ -156,7 +138,7 @@ extern "C" int dd_adam_step(float* param, const float* grad, float* exp_avg, flo
   DD_REQUIRE(param && grad && exp_avg && exp_avg_sq, DD_ERR_BAD_ARG, "dd_adam_step: null pointer");
   DD_REQUIRE(n >= 0 && step >= 1, DD_ERR_BAD_ARG, "dd_adam_step: n %lld step %lld", n, step);
   if (n == 0) return 0;
-  const AdamHyper h = hyper(lr, beta1, beta2, eps, weight_decay, step, grad_scale);
+  const AdamHyper h = dd::adam_hyper(lr, beta1, beta2, eps, weight_decay, step, grad_scale);
   cudaStream_t st = dd::as_stream(stream);
   const bool aligned = ((((uintptr_t)param) | ((uintptr_t)grad) | ((uintptr_t)exp_avg) | ((uintptr_t)exp_avg_sq)) & 15) == 0;
   const long long nvec = aligned ? (n & ~3LL) : 0;
@@ -192,7 +174,7 @@ extern "C" int dd_adam_step_sharded(const void* const* grad_replicas, void* cons
     DD_REQUIRE(((((uintptr_t)pp.grad[k]) | ((uintptr_t)pp.param[k])) & 15) == 0, DD_ERR_ALIGNMENT,
                "dd_adam_step_sharded: replica %d is not 16-byte aligned", k);
   }
-  const AdamHyper h = hyper(lr, beta1, beta2, eps, weight_decay, step, grad_scale);
+  const AdamHyper h = dd::adam_hyper(lr, beta1, beta2, eps, weight_decay, step, grad_scale);
   cudaStream_t st = dd::as_stream(stream);
   // ctas_per_sm = 1 leaves room for a persistent conv CTA beside each update CTA (update overlapped with the backward pass)
   const long long want = ((shard_numel >> 2) + kThreads - 1) / kThreads;

@@ -5,6 +5,7 @@
 // fp32 weights / accumulation: this is the fp32 parity path and the on-device check for the
 // tensor-core weight-streaming kernels in linear_tc.cu.  All three passes stream W exactly once
 // per 32 batch rows; reductions over split K / split N go through ordered partial buffers.
+#include "adam.cuh"
 #include "dd_common.cuh"
 
 namespace {
@@ -378,8 +379,9 @@ int linear_fwd_tc(const float* x, const float* w, const float* bias, float* y, v
                   long long K, cudaStream_t st);
 int linear_dgrad_tc(const float* dy, const float* w, void* dx, int dx_dtype, void* ws, size_t ws_bytes, int B, int N,
                     long long K, cudaStream_t st);
-int linear_wgrad_tc(const float* dy, const float* x, float* dw, int B, int N, long long K, int accumulate, cudaStream_t st,
-                    float* const* adam_pmv = nullptr, const float* hyper = nullptr);
+int linear_wgrad_tc(const float* dy, const float* x, float* dw, int B, int N, long long K, int accumulate, cudaStream_t st);
+int linear_bwd_adam_tc(const float* dy, const float* x, float* w, float* m, float* v, void* dx, int dx_dtype, void* ws,
+                       size_t ws_bytes, int B, int N, long long K, const AdamHyper& h, cudaStream_t st);
 }  // namespace dd
 
 // tcgen05 path: only on explicit request (DD_IMPL_TCGEN05) -- fp32 callers under DD_IMPL_AUTO keep the
@@ -497,21 +499,22 @@ extern "C" int dd_linear_wgrad(const float* dy, const void* x, int x_dtype, floa
   return 0;
 }
 
-// Weight gradient of a wide linear layer with the Adam update folded into its epilogue (world size 1): see
-// include/dd_b200.h.  tcgen05 path only (fp32 x, B <= 32, dd_linear_tc_supported); the bias gradient is written as usual.
-extern "C" int dd_linear_wgrad_adam(const float* dy, const float* x, float* weight, float* exp_avg, float* exp_avg_sq, float* db,
-                                    int B, int N, long long K, float lr, float beta1, float beta2, float eps, float weight_decay,
-                                    long long step, void* stream) {
-  DD_REQUIRE(dy && x && weight && exp_avg && exp_avg_sq, DD_ERR_BAD_ARG, "dd_linear_wgrad_adam: null pointer");
-  DD_REQUIRE(B > 0 && B <= 32 && N > 0 && K > 0 && step >= 1, DD_ERR_BAD_ARG, "dd_linear_wgrad_adam: B=%d (<= 32) N=%d K=%lld step=%lld", B, N, K, step);
-  DD_REQUIRE(dd::linear_tc_supported(B, N, K), DD_ERR_UNSUPPORTED, "dd_linear_wgrad_adam: needs the tcgen05 path (N %% 4 == K %% 4 == 0, N*K >= 2^22)");
-  DD_REQUIRE((((uintptr_t)weight | (uintptr_t)exp_avg | (uintptr_t)exp_avg_sq) & 15) == 0, DD_ERR_ALIGNMENT,
-             "dd_linear_wgrad_adam: weight / moments must be 16-byte aligned");
+// Backward pass of a wide linear layer with the Adam update of its weight folded in (world size 1): see include/dd_b200.h.
+// tcgen05 path only (fp32 x, B <= 32, dd_linear_tc_supported); the bias gradient is written as by dd_linear_wgrad.
+extern "C" int dd_linear_bwd_adam(const float* dy, const float* x, float* weight, float* exp_avg, float* exp_avg_sq, void* dx,
+                                  int dx_dtype, float* db, void* workspace, size_t ws_bytes, int B, int N, long long K, float lr,
+                                  float beta1, float beta2, float eps, float weight_decay, long long step, void* stream) {
+  DD_REQUIRE(dy && x && weight && exp_avg && exp_avg_sq, DD_ERR_BAD_ARG, "dd_linear_bwd_adam: null pointer");
+  DD_REQUIRE(B > 0 && B <= 32 && N > 0 && K > 0 && step >= 1, DD_ERR_BAD_ARG, "dd_linear_bwd_adam: B=%d (<= 32) N=%d K=%lld step=%lld", B, N, K, step);
+  DD_REQUIRE(!dx || dx_dtype == DD_F32 || dx_dtype == DD_BF16, DD_ERR_UNSUPPORTED, "dd_linear_bwd_adam: dtype %d", dx_dtype);
+  DD_REQUIRE(dd::linear_tc_supported(B, N, K), DD_ERR_UNSUPPORTED, "dd_linear_bwd_adam: needs the tcgen05 path (N %% 4 == K %% 4 == 0, N*K >= 2^22)");
+  DD_REQUIRE((((uintptr_t)weight | (uintptr_t)exp_avg | (uintptr_t)exp_avg_sq | (uintptr_t)dy | (uintptr_t)x) & 15) == 0, DD_ERR_ALIGNMENT,
+             "dd_linear_bwd_adam: dy / x / weight / moments must be 16-byte aligned");
+  DD_REQUIRE(!dx || (workspace && ws_bytes >= dd_linear_workspace_bytes(B, N, K)), DD_ERR_WORKSPACE,
+             "dd_linear_bwd_adam: workspace %zu < %zu", ws_bytes, dd_linear_workspace_bytes(B, N, K));
   cudaStream_t st = dd::as_stream(stream);
-  const double bc1 = 1.0 - pow((double)beta1, (double)step), bc2 = 1.0 - pow((double)beta2, (double)step);
-  const float hyper[6] = {beta1, beta2, eps, (float)((double)lr / bc1), (float)(1.0 / sqrt(bc2)), weight_decay};
-  float* pmv[3] = {weight, exp_avg, exp_avg_sq};
-  if (int e = dd::linear_wgrad_tc(dy, x, nullptr, B, N, K, 0, st, pmv, hyper)) return e;
+  const dd::AdamHyper h = dd::adam_hyper(lr, beta1, beta2, eps, weight_decay, step, 1.f);
+  if (int e = dd::linear_bwd_adam_tc(dy, x, weight, exp_avg, exp_avg_sq, dx, dx_dtype, workspace, ws_bytes, B, N, K, h, st)) return e;
   if (db) {
     colsum_kernel<<<ceil_div(N, 256), 256, 0, st>>>(dy, db, B, N, 0);
     if (int e2 = dd::check_launch("colsum")) return e2;

@@ -12,12 +12,15 @@
 //   dgrad dx[b][k] = sum_n dy[b][n] W[n][k]    D[128 k x 32 b]:  A = W^T tile, MN-major -- for tf32 that
 //                                              is SWIZZLE_128B_BASE32B (TMA ..._ATOM_32B);  B = dy, K-major
 //   wgrad dW[n][k] = sum_b dy[b][n] x[b][k]    D[128 n x 256 k]: A = dy^T, B = x, both MN-major
+//   bwd + Adam (world size 1): dgrad as above and G^T[k][n] = sum_b x[b][k] dy[b][n] (A = x, B = dy, both MN-major) per
+//                              weight tile, whose Adam update is applied on chip: one pass over W, m and v
 // Operand descriptors were verified on hardware with tools/umma_tf32_probe.cu
 // (profiles/r1_umma_tf32_tma_probe.txt).
 //
 // Warp roles (192 threads): warp 0 = TMA producer (one lane), warp 1 = MMA issuer + TMEM owner,
 // warps 2..5 = epilogue (TMEM -> registers -> global).  Persistent CTAs walk (tile, split) work items;
 // split contractions go to ordered partial buffers folded by a second kernel (deterministic).
+#include "adam.cuh"
 #include "dd_common.cuh"
 #include "tma_host.h"
 #include "umma.cuh"
@@ -215,26 +218,9 @@ __global__ void split_fold_kernel(const float* __restrict__ partial, const float
 constexpr int W_STAGES = 3;
 constexpr int W_STAGE_BYTES = 4 * BOX + 8 * BOX;     // dy^T: 4 boxes of 32 n; x: up to 8 boxes of 32 k
 constexpr int W_TPAD = 36;                           // floats per row of a warp's 32 x 32 transpose block
-// epilogue warps: 4 for the plain weight gradient (192 threads x ~118 registers: co-resides with the data-parallel update CTA
-// of csrc/adam.cu), 8 for the form with Adam folded in (two per TMEM lane quarter, alternate 32-column chunks: it needs
-// the bytes in flight)
-template <bool ADAM> struct WCfg { static constexpr int EPI = ADAM ? 8 : 4; static constexpr int THREADS = 32 * (2 + EPI); };
-constexpr int W_SMEM = W_STAGES * W_STAGE_BYTES + 8 * 32 * W_TPAD * 4 + 2048;
-
-// Adam folded into the weight-gradient epilogue (world size 1): the gradient tile never goes to HBM -- the epilogue reads
-// the weight and its two moments where it would have written dW, and writes them back updated: 24 bytes per parameter
-// instead of 4 (dW write) + 28 (a separate Adam pass).  Same arithmetic as csrc/adam.cu (torch.optim.Adam, amsgrad off).
-struct AdamFuse {
-  float* p; float* m; float* v;          // weight [N][K], exp_avg, exp_avg_sq (same layout); p == nullptr: plain weight gradient
-  float beta1, beta2, eps, step_size, inv_sqrt_bc2, weight_decay;
-};
-__device__ __forceinline__ float adam_fused_one(float p, float g, float& m, float& v, const AdamFuse& h) {
-  if (h.weight_decay != 0.f) g = fmaf(h.weight_decay, p, g);
-  m = m + (1.f - h.beta1) * (g - m);
-  v = h.beta2 * v + (1.f - h.beta2) * g * g;
-  const float denom = sqrtf(v) * h.inv_sqrt_bc2 + h.eps;
-  return p - h.step_size * (m / denom);
-}
+constexpr int W_EPI = 4;                             // epilogue warps (192 threads x ~118 registers: co-resides with the
+constexpr int W_THREADS = 32 * (2 + W_EPI);          // data-parallel update CTA of csrc/adam.cu)
+constexpr int W_SMEM = W_STAGES * W_STAGE_BYTES + W_EPI * 32 * W_TPAD * 4 + 2048;
 
 struct WgradBars {
   uint64_t full[W_STAGES], empty[W_STAGES], acc_full[2], acc_empty[2];
@@ -246,18 +232,15 @@ struct WgradGeo {
   long long K;
   int n_tiles, k_tiles, KT;      // KT = 128 or 256 columns per tile
   int accumulate;
-  AdamFuse adam;
 };
 
-template <bool ADAM>
-__global__ void __launch_bounds__(WCfg<ADAM>::THREADS, 1) linear_wgrad_tc_kernel(const __grid_constant__ CUtensorMap map_dy,
-                                                                                 const __grid_constant__ CUtensorMap map_x,
-                                                                                 float* __restrict__ dw, const WgradGeo g) {
-  constexpr int W_EPI = WCfg<ADAM>::EPI;
+__global__ void __launch_bounds__(W_THREADS, 1) linear_wgrad_tc_kernel(const __grid_constant__ CUtensorMap map_dy,
+                                                                       const __grid_constant__ CUtensorMap map_x,
+                                                                       float* __restrict__ dw, const WgradGeo g) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = align1024(smem_raw);
   float* stage_out = reinterpret_cast<float*>(smem + W_STAGES * W_STAGE_BYTES);
-  WgradBars* bars = reinterpret_cast<WgradBars*>(smem + W_STAGES * W_STAGE_BYTES + 8 * 32 * W_TPAD * 4);
+  WgradBars* bars = reinterpret_cast<WgradBars*>(smem + W_STAGES * W_STAGE_BYTES + W_EPI * 32 * W_TPAD * 4);
   const int tid = threadIdx.x, lane = tid & 31;
   const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);
   const long long items = (long long)g.n_tiles * g.k_tiles;
@@ -313,7 +296,6 @@ __global__ void __launch_bounds__(WCfg<ADAM>::THREADS, 1) linear_wgrad_tc_kernel
     }
   } else {
     const int quarter = warp & 3;
-    const int sub = (warp - 2) >> 2;               // ADAM: which of the quarter's two warps (takes the 32-column chunks of its parity)
     uint32_t c = 0;
     for (long long it = blockIdx.x; it < items; it += gridDim.x, ++c) {
       const int ni = (int)(it / g.k_tiles), ki = (int)(it % g.k_tiles);
@@ -323,7 +305,7 @@ __global__ void __launch_bounds__(WCfg<ADAM>::THREADS, 1) linear_wgrad_tc_kernel
       const int n0 = ni * 128 + quarter * 32;
       const long long k0 = (long long)ki * g.KT;
       float* blk = stage_out + (warp - 2) * (32 * W_TPAD);
-      for (int cb = 32 * sub; cb < g.KT; cb += 32 * (W_EPI / 4)) {
+      for (int cb = 0; cb < g.KT; cb += 32) {
         uint32_t v[32];
         umma::tmem_ld_32x32(tmem + ((uint32_t)(quarter * 32) << 16) + a * 256 + cb, v);
         umma::tmem_ld_wait();
@@ -337,43 +319,8 @@ __global__ void __launch_bounds__(WCfg<ADAM>::THREADS, 1) linear_wgrad_tc_kernel
                           __uint_as_float(v[4 * q + 3]));
         __syncwarp();
         const int cq = lane & 7;
-        if (ADAM) {
-          // fused Adam: all eight rows of the chunk at once -> 24 independent 16-byte loads per thread in flight (with
-          // four rows per batch the kernel sat at 4.1 TB/s: ~49 KB in flight per SM do not cover the loaded-DRAM latency)
-          {
-            float4 pp[8], mm[8], vv[8];
-            bool ok[8];
 #pragma unroll
-            for (int q = 0; q < 8; ++q) {
-              const int r = (lane >> 3) + 4 * q;
-              const int n = n0 + r;
-              const long long k = k0 + cb + 4 * cq;
-              ok[q] = n < g.N && k < g.K;
-              if (ok[q]) {
-                const size_t e = (size_t)n * g.K + k;
-                pp[q] = *reinterpret_cast<const float4*>(g.adam.p + e);
-                mm[q] = __ldcs(reinterpret_cast<const float4*>(g.adam.m + e));
-                vv[q] = __ldcs(reinterpret_cast<const float4*>(g.adam.v + e));
-              }
-            }
-#pragma unroll
-            for (int q = 0; q < 8; ++q) {
-              if (!ok[q]) continue;
-              const int r = (lane >> 3) + 4 * q;
-              const size_t e = (size_t)(n0 + r) * g.K + (k0 + cb + 4 * cq);
-              const float4 gr = *reinterpret_cast<const float4*>(blk + r * W_TPAD + 4 * cq);
-              pp[q].x = adam_fused_one(pp[q].x, gr.x, mm[q].x, vv[q].x, g.adam);
-              pp[q].y = adam_fused_one(pp[q].y, gr.y, mm[q].y, vv[q].y, g.adam);
-              pp[q].z = adam_fused_one(pp[q].z, gr.z, mm[q].z, vv[q].z, g.adam);
-              pp[q].w = adam_fused_one(pp[q].w, gr.w, mm[q].w, vv[q].w, g.adam);
-              *reinterpret_cast<float4*>(g.adam.p + e) = pp[q];
-              __stcs(reinterpret_cast<float4*>(g.adam.m + e), mm[q]);
-              __stcs(reinterpret_cast<float4*>(g.adam.v + e), vv[q]);
-            }
-          }
-        }
-#pragma unroll
-        for (int itr = 0; itr < (ADAM ? 0 : 8); ++itr) {
+        for (int itr = 0; itr < 8; ++itr) {
           const int r = (lane >> 3) + 4 * itr;
           const int n = n0 + r;
           const long long k = k0 + cb + 4 * cq;
@@ -393,6 +340,236 @@ __global__ void __launch_bounds__(WCfg<ADAM>::THREADS, 1) linear_wgrad_tc_kernel
   umma::tc_fence_before_sync();
   __syncthreads();
   if (warp == 1) umma::tmem_dealloc(tmem, 512);
+}
+
+// ------------------------------------------------------------------------------------------------
+// backward + Adam (world size 1): per 32 n x 128 k weight tile, ONE pass over W and its two moments
+//   dgrad  dx[b][k] += sum_n dy[b][n] W[n][k]    the MMAs of MODE 1 above, same order (bit-identical dx)
+//   wgrad  G^T[k][n] = sum_b x[b][k] dy[b][n]    D[128 k x 32 n]: A = x tile, B = dy chunk, both MN-major
+//   Adam   W, m, v tiles updated in shared memory from G^T (TMEM), then stored by TMA in place
+// The W tile is loaded once and serves as the dgrad operand and the Adam input; the weight gradient never reaches HBM:
+// 24 bytes per parameter instead of 4 (dgrad) + 4 (wgrad) + 28 (Adam) + 4 (dW read back).
+// Work decomposition, split plan and split partials are those of the dgrad kernel.  Warp roles (352 threads): warp 0 = TMA
+// producer, warp 1 = MMA issuer + TMEM owner, warps 2..9 = epilogue (two per TMEM lane quarter, 16 n rows each), warp 10 =
+// TMA stores of the updated tiles (a stage goes back to the producer as soon as its stores have read it).
+// The W / m / v boxes use the SWIZZLE_128B_ATOM_32B layout of the MN-major dgrad operand for the load AND the store
+// (tools/tma_store_atom32_probe.cu): element (row r, column c) of a 32 x 32 box sits in 32-byte atom (c / 8) ^ (r % 4)
+// of its 128-byte row.
+// ------------------------------------------------------------------------------------------------
+constexpr int BA_STAGES = 3;
+constexpr int BA_TILE = 4 * BOX;                      // W, m or v: [32 n][128 k] as 4 boxes of 32 k
+constexpr int BA_STAGE_BYTES = 3 * BA_TILE + 2 * BOX;  // W, m, v; dy chunk K-major (dgrad) and MN-major (wgrad)
+constexpr int BA_EPI = 8;
+constexpr int BA_THREADS = 32 * (3 + BA_EPI);
+constexpr int BA_SMEM = BA_STAGES * BA_STAGE_BYTES + 2 * BA_TILE + 2048;   // + x [32 b][128 k], double-buffered per item
+
+struct BwdAdamBars {
+  uint64_t full[BA_STAGES], empty[BA_STAGES], tile_ready[BA_STAGES], x_full[2], x_empty[2], g_full[2], g_empty[2], acc_full[2], acc_empty[2];
+  uint32_t tmem_base;
+};
+
+// shared-memory accesses by address (the tile pointer went through align1024: plain C++ would compile to generic LD / ST)
+__device__ __forceinline__ float lds_f32(uint32_t a) {
+  float v;
+  asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v) : "r"(a) : "memory");
+  return v;
+}
+__device__ __forceinline__ void sts_f32(uint32_t a, float v) { asm volatile("st.shared.f32 [%0], %1;" ::"r"(a), "f"(v) : "memory"); }
+// TMEM columns: [0, 64) dgrad accumulator of the item (x 2), [64, 128) G^T of the chunk (x 2)
+template <typename TOUT>
+__global__ void __launch_bounds__(BA_THREADS, 1) linear_bwd_adam_tc_kernel(
+    const __grid_constant__ CUtensorMap map_w, const __grid_constant__ CUtensorMap map_m, const __grid_constant__ CUtensorMap map_v,
+    const __grid_constant__ CUtensorMap map_dy, const __grid_constant__ CUtensorMap map_dyt, const __grid_constant__ CUtensorMap map_x,
+    TOUT* __restrict__ dx, float* __restrict__ partial, StreamGeo g, const dd::AdamHyper h) {
+  extern __shared__ uint8_t smem_raw[];
+  uint8_t* smem = align1024(smem_raw);
+  uint8_t* xbuf = smem + BA_STAGES * BA_STAGE_BYTES;
+  BwdAdamBars* bars = reinterpret_cast<BwdAdamBars*>(xbuf + 2 * BA_TILE);
+  const int tid = threadIdx.x, lane = tid & 31;
+  const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);
+  const int items = g.tiles * g.splits;
+  const bool has_dx = dx != nullptr;
+
+  if (tid == 0) {
+    for (int i = 0; i < BA_STAGES; ++i) {
+      umma::mbar_init(&bars->full[i], 1); umma::mbar_init(&bars->empty[i], 1); umma::mbar_init(&bars->tile_ready[i], BA_EPI);
+    }
+    for (int i = 0; i < 2; ++i) {
+      umma::mbar_init(&bars->x_full[i], 1); umma::mbar_init(&bars->x_empty[i], 1);
+      umma::mbar_init(&bars->g_full[i], 1); umma::mbar_init(&bars->g_empty[i], BA_EPI);
+      umma::mbar_init(&bars->acc_full[i], 1); umma::mbar_init(&bars->acc_empty[i], BA_EPI);
+    }
+    umma::fence_mbar_init();
+    umma::tma_prefetch_desc(&map_w); umma::tma_prefetch_desc(&map_m); umma::tma_prefetch_desc(&map_v);
+    umma::tma_prefetch_desc(&map_dy); umma::tma_prefetch_desc(&map_dyt); umma::tma_prefetch_desc(&map_x);
+  }
+  if (warp == 1) umma::tmem_alloc(&bars->tmem_base, 128);
+  umma::tc_fence_before_sync();
+  __syncthreads();
+  umma::tc_fence_after_sync();
+  const uint32_t tmem = __shfl_sync(0xffffffffu, bars->tmem_base, 0);
+
+  if (warp == 0) {
+    // =========================== TMA producer ===================================================
+    if (umma::elect_one()) {
+      const uint32_t stage_tx = has_dx ? BA_STAGE_BYTES : BA_STAGE_BYTES - BOX;
+      uint32_t c = 0, n_item = 0;
+      for (int it = blockIdx.x; it < items; it += gridDim.x, ++n_item) {
+        const int ti = it % g.tiles, si = it / g.tiles;
+        const int c0 = si * g.chunks_per_split;
+        const int c1 = min(c0 + g.chunks_per_split, g.chunks);
+        const uint32_t xb = n_item & 1;
+        umma::mbar_wait(&bars->x_empty[xb], ((n_item >> 1) & 1) ^ 1);
+        umma::mbar_expect_tx(&bars->x_full[xb], BA_TILE);
+#pragma unroll
+        for (int i = 0; i < 4; ++i)                                                           // x[b][k tile], 4 x 32 k
+          umma::tma_load_2d(umma::smem_u32(xbuf + xb * BA_TILE + i * BOX), &map_x, ti * 128 + 32 * i, 0, &bars->x_full[xb]);
+        for (int ch = c0; ch < c1; ++ch, ++c) {
+          const uint32_t s = c % BA_STAGES;
+          umma::mbar_wait(&bars->empty[s], ((c / BA_STAGES) & 1) ^ 1);
+          const uint32_t dst = umma::smem_u32(smem + s * BA_STAGE_BYTES);
+          umma::mbar_expect_tx(&bars->full[s], stage_tx);
+#pragma unroll
+          for (int i = 0; i < 4; ++i) {                                                       // [n chunk][k tile], 4 x 32 k
+            umma::tma_load_2d(dst + i * BOX, &map_w, ti * 128 + 32 * i, ch * kChunk, &bars->full[s]);
+            umma::tma_load_2d(dst + BA_TILE + i * BOX, &map_m, ti * 128 + 32 * i, ch * kChunk, &bars->full[s]);
+            umma::tma_load_2d(dst + 2 * BA_TILE + i * BOX, &map_v, ti * 128 + 32 * i, ch * kChunk, &bars->full[s]);
+          }
+          umma::tma_load_2d(dst + 3 * BA_TILE, &map_dyt, ch * kChunk, 0, &bars->full[s]);             // dy[b][chunk], MN-major
+          if (has_dx) umma::tma_load_2d(dst + 3 * BA_TILE + BOX, &map_dy, ch * kChunk, 0, &bars->full[s]);  // ... K-major
+        }
+      }
+    }
+  } else if (warp == 1) {
+    // =========================== MMA issuer =======================================================
+    constexpr uint32_t idesc_d = umma::make_idesc_tf32(128, NB, true, false);   // dgrad, as MODE 1
+    constexpr uint32_t idesc_g = umma::make_idesc_tf32(128, NB, true, true);    // G^T = x^T dy
+    uint32_t c = 0, n_item = 0;
+    for (int it = blockIdx.x; it < items; it += gridDim.x, ++n_item) {
+      const int si = it / g.tiles;
+      const int c0 = si * g.chunks_per_split;
+      const int c1 = min(c0 + g.chunks_per_split, g.chunks);
+      const uint32_t a = n_item & 1;
+      if (has_dx) umma::mbar_wait(&bars->acc_empty[a], ((n_item >> 1) & 1) ^ 1);
+      umma::mbar_wait(&bars->x_full[a], (n_item >> 1) & 1);
+      const uint32_t xbase = umma::smem_u32(xbuf + a * BA_TILE);
+      for (int ch = c0; ch < c1; ++ch, ++c) {
+        const uint32_t s = c % BA_STAGES, ga = c & 1;
+        umma::mbar_wait(&bars->full[s], (c / BA_STAGES) & 1);
+        umma::mbar_wait(&bars->g_empty[ga], ((c >> 1) & 1) ^ 1);
+        umma::tc_fence_after_sync();
+        const uint32_t base = umma::smem_u32(smem + s * BA_STAGE_BYTES);
+        if (umma::elect_one()) {
+          if (has_dx) {
+#pragma unroll
+            for (int k = 0; k < 4; ++k)
+              umma::mma_tf32_lohi(tmem + a * NB, umma::desc_lo(base + k * 1024, BOX), umma::desc_hi_sw128_base32(512),
+                                  umma::desc_lo(base + 3 * BA_TILE + BOX + k * 32, 16), umma::desc_hi_sw128(1024), idesc_d,
+                                  (ch > c0 || k > 0) ? 1u : 0u);
+          }
+#pragma unroll
+          for (int k = 0; k < 4; ++k)
+            umma::mma_tf32_lohi(tmem + 2 * NB + ga * NB, umma::desc_lo(xbase + k * 1024, BOX), umma::desc_hi_sw128_base32(512),
+                                umma::desc_lo(base + 3 * BA_TILE + k * 1024, BOX), umma::desc_hi_sw128_base32(512), idesc_g,
+                                k > 0 ? 1u : 0u);
+          umma::mma_commit(&bars->g_full[ga]);          // also: the dgrad MMAs are done reading the old W tile
+          if (ch == c1 - 1) {
+            if (has_dx) umma::mma_commit(&bars->acc_full[a]);
+            umma::mma_commit(&bars->x_empty[a]);
+          }
+        }
+        __syncwarp();
+      }
+    }
+  } else if (warp == 2 + BA_EPI) {
+    // =========================== TMA stores of the updated W / m / v tiles ===========================
+    if (umma::elect_one()) {
+      uint32_t c = 0;
+      for (int it = blockIdx.x; it < items; it += gridDim.x) {
+        const int ti = it % g.tiles, si = it / g.tiles;
+        const int c0 = si * g.chunks_per_split;
+        const int c1 = min(c0 + g.chunks_per_split, g.chunks);
+        for (int ch = c0; ch < c1; ++ch, ++c) {
+          const uint32_t s = c % BA_STAGES;
+          mbar_wait_relaxed(&bars->tile_ready[s], (c / BA_STAGES) & 1);
+          const uint32_t src = umma::smem_u32(smem + s * BA_STAGE_BYTES);
+#pragma unroll
+          for (int i = 0; i < 4; ++i) {
+            umma::tma_store_2d(&map_w, src + i * BOX, ti * 128 + 32 * i, ch * kChunk);
+            umma::tma_store_2d(&map_m, src + BA_TILE + i * BOX, ti * 128 + 32 * i, ch * kChunk);
+            umma::tma_store_2d(&map_v, src + 2 * BA_TILE + i * BOX, ti * 128 + 32 * i, ch * kChunk);
+          }
+          umma::bulk_commit_group();
+          umma::bulk_wait_group_read<0>();
+          umma::mbar_arrive(&bars->empty[s]);
+        }
+      }
+      umma::bulk_wait_group<0>();
+    }
+  } else {
+    // =========================== epilogue (warps 2..9) =============================================
+    // thread = k lane (quarter * 32 + lane of the tile: box `quarter`, column `lane`), 16 n rows (half `sub` of the chunk)
+    const int quarter = warp & 3, sub = (warp - 2) >> 2;
+    uint32_t c = 0, n_item = 0;
+    for (int it = blockIdx.x; it < items; it += gridDim.x, ++n_item) {
+      const int ti = it % g.tiles, si = it / g.tiles;
+      const int c0 = si * g.chunks_per_split;
+      const int c1 = min(c0 + g.chunks_per_split, g.chunks);
+      for (int ch = c0; ch < c1; ++ch, ++c) {
+        const uint32_t s = c % BA_STAGES, ga = c & 1;
+        mbar_wait_relaxed(&bars->g_full[ga], (c >> 1) & 1);
+        umma::tc_fence_after_sync();
+        uint32_t gv[16];
+        umma::tmem_ld_32x16(tmem + ((uint32_t)(quarter * 32) << 16) + 2 * NB + ga * NB + sub * 16, gv);
+        umma::tmem_ld_wait();
+        umma::tc_fence_before_sync();
+        __syncwarp();
+        if (lane == 0) umma::mbar_arrive(&bars->g_empty[ga]);
+        const uint32_t wt = umma::smem_u32(smem + s * BA_STAGE_BYTES + quarter * BOX);
+#pragma unroll
+        for (int j = 0; j < 16; ++j) {
+          const int r = sub * 16 + j;
+          const uint32_t e = wt + 4 * (r * 32 + ((((lane >> 3) ^ (r & 3)) << 3) | (lane & 7)));
+          float m = lds_f32(e + BA_TILE), v = lds_f32(e + 2 * BA_TILE);
+          const float p = dd::adam_one(lds_f32(e), __uint_as_float(gv[j]), m, v, h);
+          sts_f32(e, p);
+          sts_f32(e + BA_TILE, m);
+          sts_f32(e + 2 * BA_TILE, v);
+        }
+        umma::fence_proxy_async_smem();             // the writes above, then the TMA stores of warp 2 + BA_EPI
+        __syncwarp();
+        if (lane == 0) umma::mbar_arrive(&bars->tile_ready[s]);
+        if (has_dx && ch == c1 - 1) {
+          // the item's input gradient, as the dgrad kernel writes it (this warp: 16 of the 32 batch rows)
+          const uint32_t a = n_item & 1;
+          mbar_wait_relaxed(&bars->acc_full[a], (n_item >> 1) & 1);
+          umma::tc_fence_after_sync();
+          uint32_t v[16];
+          umma::tmem_ld_32x16(tmem + ((uint32_t)(quarter * 32) << 16) + a * NB + sub * 16, v);
+          umma::tmem_ld_wait();
+          umma::tc_fence_before_sync();
+          __syncwarp();
+          if (lane == 0) umma::mbar_arrive(&bars->acc_empty[a]);
+          const int r = ti * 128 + quarter * 32 + lane;
+          if (r < g.LD) {
+            if (g.splits == 1) {
+#pragma unroll
+              for (int b = 0; b < 16; ++b)       // + 0.f as the dgrad kernel adds its (absent) bias: -0 is written as +0
+                if (sub * 16 + b < g.B) dd::st<TOUT>(dx + (size_t)(sub * 16 + b) * g.LD + r, __uint_as_float(v[b]) + 0.f);
+            } else {
+              float* p = partial + (size_t)si * g.B * g.LD + r;
+#pragma unroll
+              for (int b = 0; b < 16; ++b)
+                if (sub * 16 + b < g.B) p[(size_t)(sub * 16 + b) * g.LD] = __uint_as_float(v[b]);
+            }
+          }
+        }
+      }
+    }
+  }
+  umma::tc_fence_before_sync();
+  __syncthreads();
+  if (warp == 1) umma::tmem_dealloc(tmem, 128);
 }
 
 int ceil_div_ll(long long a, long long b) { return (int)((a + b - 1) / b); }
@@ -513,18 +690,50 @@ int linear_dgrad_tc(const float* dy, const float* w, void* dx, int dx_dtype, voi
   return g.splits > 1 ? check_launch("linear_dgrad_fold") : 0;
 }
 
-// dy fp32 [B][N], x fp32 [B][K] -> dW fp32 [N][K] (overwritten, or accumulated into); with adam_pmv != nullptr the epilogue
-// applies the Adam update to {weight, exp_avg, exp_avg_sq} = adam_pmv[0..2] instead of writing dW (hyper: beta1, beta2,
-// eps, step_size = lr / (1 - beta1^t), inv_sqrt_bc2 = 1 / sqrt(1 - beta2^t), weight_decay)
-int linear_wgrad_tc(const float* dy, const float* x, float* dw, int B, int N, long long K, int accumulate, cudaStream_t st,
-                    float* const* adam_pmv = nullptr, const float* hyper = nullptr) {
+// dy fp32 [B][N], x fp32 [B][K], W / m / v fp32 [N][K] updated in place; dx [B][K] fp32 or bf16 from the old W, or nullptr
+int linear_bwd_adam_tc(const float* dy, const float* x, float* w, float* m, float* v, void* dx, int dx_dtype, void* ws,
+                       size_t ws_bytes, int B, int N, long long K, const AdamHyper& h, cudaStream_t st) {
+  StreamGeo g;
+  g.B = B; g.LD = (int)K;
+  g.tiles = ceil_div_ll(K, 128);
+  g.chunks = ceil_div_ll(N, kChunk);
+  plan_stream(g.tiles, g.chunks, g.splits, g.chunks_per_split);
+  if (dx && g.splits > 1 && ws_bytes < (size_t)g.splits * B * K * sizeof(float))
+    return fail(DD_ERR_WORKSPACE, "linear_bwd_adam_tc: workspace %zu too small for %d splits", ws_bytes, g.splits);
+  CUtensorMap mw, mm, mv, mdy, mdyt, mx;
+  char msg[256];
+  if (tma_map_2d_checked(&mw, w, 4, N, K, K, 32, 32, true, msg, sizeof msg) ||
+      tma_map_2d_checked(&mm, m, 4, N, K, K, 32, 32, true, msg, sizeof msg) ||
+      tma_map_2d_checked(&mv, v, 4, N, K, K, 32, 32, true, msg, sizeof msg) ||
+      tma_map_2d_checked(&mdy, dy, 4, B, N, N, 32, 32, false, msg, sizeof msg) ||
+      tma_map_2d_checked(&mdyt, dy, 4, B, N, N, 32, 32, true, msg, sizeof msg) ||
+      tma_map_2d_checked(&mx, x, 4, B, K, K, 32, 32, true, msg, sizeof msg))
+    return fail(DD_ERR_UNSUPPORTED, "linear_bwd_adam_tc: %s", msg);
+  const int items = g.tiles * g.splits;
+  const int grid = items < kSMs ? items : kSMs;
+  const long long n = (long long)B * K;
+  if (dx_dtype == DD_BF16 && dx) {
+    auto k = linear_bwd_adam_tc_kernel<__nv_bfloat16>;
+    if (int e = set_smem(k, BA_SMEM)) return e;
+    k<<<grid, BA_THREADS, BA_SMEM, st>>>(mw, mm, mv, mdy, mdyt, mx, (__nv_bfloat16*)dx, (float*)ws, g, h);
+    if (int e = check_launch("linear_bwd_adam_tc")) return e;
+    if (g.splits > 1)
+      split_fold_kernel<__nv_bfloat16><<<ceil_div_ll(n, 256), 256, 0, st>>>((const float*)ws, nullptr, (__nv_bfloat16*)dx, g.splits, n, (int)K);
+  } else {
+    auto k = linear_bwd_adam_tc_kernel<float>;
+    if (int e = set_smem(k, BA_SMEM)) return e;
+    k<<<grid, BA_THREADS, BA_SMEM, st>>>(mw, mm, mv, mdy, mdyt, mx, (float*)dx, (float*)ws, g, h);
+    if (int e = check_launch("linear_bwd_adam_tc")) return e;
+    if (dx && g.splits > 1)
+      split_fold_kernel<float><<<ceil_div_ll(n, 256), 256, 0, st>>>((const float*)ws, nullptr, (float*)dx, g.splits, n, (int)K);
+  }
+  return dx && g.splits > 1 ? check_launch("linear_bwd_adam_fold") : 0;
+}
+
+// dy fp32 [B][N], x fp32 [B][K] -> dW fp32 [N][K] (overwritten, or accumulated into)
+int linear_wgrad_tc(const float* dy, const float* x, float* dw, int B, int N, long long K, int accumulate, cudaStream_t st) {
   WgradGeo g = {};
   g.B = B; g.N = N; g.K = K;
-  if (adam_pmv) {
-    g.adam.p = adam_pmv[0]; g.adam.m = adam_pmv[1]; g.adam.v = adam_pmv[2];
-    g.adam.beta1 = hyper[0]; g.adam.beta2 = hyper[1]; g.adam.eps = hyper[2]; g.adam.step_size = hyper[3];
-    g.adam.inv_sqrt_bc2 = hyper[4]; g.adam.weight_decay = hyper[5];
-  }
   g.KT = K >= 256 ? 256 : 128;
   g.n_tiles = ceil_div_ll(N, 128);
   g.k_tiles = ceil_div_ll(K, g.KT);
@@ -536,13 +745,8 @@ int linear_wgrad_tc(const float* dy, const float* x, float* dw, int B, int N, lo
     return fail(DD_ERR_UNSUPPORTED, "linear_wgrad_tc: %s", msg);
   const long long items = (long long)g.n_tiles * g.k_tiles;
   const int grid = (int)(items < kSMs ? items : kSMs);
-  if (adam_pmv) {
-    if (int e = set_smem(linear_wgrad_tc_kernel<true>, W_SMEM)) return e;
-    linear_wgrad_tc_kernel<true><<<grid, WCfg<true>::THREADS, W_SMEM, st>>>(mdy, mx, dw, g);
-  } else {
-    if (int e = set_smem(linear_wgrad_tc_kernel<false>, W_SMEM)) return e;
-    linear_wgrad_tc_kernel<false><<<grid, WCfg<false>::THREADS, W_SMEM, st>>>(mdy, mx, dw, g);
-  }
+  if (int e = set_smem(linear_wgrad_tc_kernel, W_SMEM)) return e;
+  linear_wgrad_tc_kernel<<<grid, W_THREADS, W_SMEM, st>>>(mdy, mx, dw, g);
   return check_launch("linear_wgrad_tc");
 }
 

@@ -98,6 +98,16 @@ __device__ __forceinline__ void tmem_ld_32x32(uint32_t taddr, uint32_t (&r)[32])
       : "r"(taddr)
       : "memory");
 }
+// 32 lanes x 16 columns of fp32
+__device__ __forceinline__ void tmem_ld_32x16(uint32_t taddr, uint32_t (&r)[16]) {
+  asm volatile(
+      "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
+      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
+      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
+        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
+      : "r"(taddr)
+      : "memory");
+}
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 
 // ---------------------------------------------------------------- descriptors -------------
@@ -261,6 +271,24 @@ __device__ __forceinline__ void tma_load_4d(uint32_t dst_smem, const void* tmap,
 }
 __device__ __forceinline__ void tma_prefetch_desc(const void* tmap) {
   asm volatile("prefetch.tensormap [%0];" ::"l"(tmap) : "memory");
+}
+// TMA: 2-D tile shared -> global (out-of-range elements are not written).  The writers of the tile must have run
+// fence_proxy_async_smem() and synchronised with the issuing thread first.
+__device__ __forceinline__ void tma_store_2d(const void* tmap, uint32_t src_smem, int c0, int c1) {
+  asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];"
+               ::"l"(tmap), "r"(src_smem), "r"(c0), "r"(c1)
+               : "memory");
+}
+__device__ __forceinline__ void bulk_commit_group() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
+// at most N committed bulk groups of this thread still READ their shared-memory source (the source may then be reused)
+template <int N>
+__device__ __forceinline__ void bulk_wait_group_read() {
+  asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory");
+}
+// at most N committed bulk groups of this thread are still incomplete (writes visible in global memory)
+template <int N>
+__device__ __forceinline__ void bulk_wait_group() {
+  asm volatile("cp.async.bulk.wait_group %0;" ::"n"(N) : "memory");
 }
 
 }  // namespace umma

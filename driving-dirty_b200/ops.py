@@ -279,18 +279,21 @@ class SkinnyLinear(torch.autograd.Function):
         dy = _c(dy.float())
         st = stream_ptr()
         dx = dw = db = None
+        if ctx.needs_input_grad[1] and ctx.fused_update is not None and ctx.impl == _lib.IMPL_TCGEN05 and B <= 32 \
+                and x.dtype == torch.float32:
+            # optim.FusedAdam (world size 1) folds this weight's Adam step into the backward pass: one kernel computes the
+            # input gradient from the old weight and updates the weight and its moments in place; the weight gradient never
+            # exists in HBM (dd_linear_bwd_adam)
+            dx = torch.empty(B, K, dtype=ctx.x_dtype, device=x.device) if ctx.needs_input_grad[0] else None
+            ws, n = _linear_ws(B, N, K, x.device)
+            db = torch.empty(N, dtype=torch.float32, device=x.device) if ctx.has_bias else None
+            ctx.fused_update(dy, x, dx, db, ws, n)
+            return dx, None, db, None, None, None, None
         if ctx.needs_input_grad[0]:
             dx = torch.empty(B, K, dtype=ctx.x_dtype, device=x.device)
             ws, n = _linear_ws(B, N, K, x.device)
             call("dd_linear_dgrad", dy.data_ptr(), w.data_ptr(), dx.data_ptr(), dtype_code(ctx.x_dtype), ws.data_ptr(), n,
                  B, N, K, ctx.impl, st)
-        if ctx.needs_input_grad[1] and ctx.fused_update is not None and ctx.impl == _lib.IMPL_TCGEN05 and B <= 32 \
-                and x.dtype == torch.float32:
-            # optim.FusedAdam (world size 1) folds this weight's Adam step into the weight-gradient kernel's epilogue: the
-            # gradient never exists in HBM (dd_linear_wgrad_adam); the input gradient above was computed from the old weight
-            db = torch.empty(N, dtype=torch.float32, device=x.device) if ctx.has_bias else None
-            ctx.fused_update(dy, x, db)
-            return dx, None, db, None, None, None, None
         if ctx.needs_input_grad[1]:
             # a parameter claimed by optim.FusedAdam's sharded update owns a persistent (peer-mapped) gradient
             # buffer: the kernel writes there and autograd gets no tensor to clone or accumulate

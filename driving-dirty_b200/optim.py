@@ -1,7 +1,9 @@
 """Fused Adam for the scene pipeline (reference: ``torch.optim.Adam(self.parameters(), lr)`` at
 roadmap_bce_v2.py:155 / autoencoder.py:120, stepped by Lightning after ddp's gradient all-reduce).
 
-One process per GPU.  With world size 1 every tensor is updated by one ``dd_adam_step`` launch.
+One process per GPU.  With world size 1 every tensor is updated by one ``dd_adam_step`` launch; with
+``overlap_backward=True`` the wide FC weights instead take their step inside the backward pass, in the same kernel that
+computes their layer's input gradient (``dd_linear_bwd_adam``).
 With world size N the parameters are *sharded across ranks for the update only*: gradient and
 weight replicas live in one symmetric-memory buffer per rank
 (``torch.distributed._symmetric_memory``: every replica is peer-mapped into every process, plus an
@@ -89,7 +91,7 @@ class FusedAdam(torch.optim.Optimizer):
         self._fused = {}            # id(param) -> True once its step ran inside the backward pass (world size 1)
         if self.world > 1:
             self._setup_sharding(shard_min_numel, multicast, broadcast_init)
-        elif fuse_into_backward:
+        elif overlap_backward or fuse_into_backward:
             self._setup_fused_backward(shard_min_numel)
 
     # The two places where the device is touched outside `_launch_sharded`; tests/test_optim.py overrides them (and the
@@ -192,30 +194,32 @@ class FusedAdam(torch.optim.Optimizer):
         hdl.barrier()
 
     def _setup_fused_backward(self, min_numel):
-        """World size 1: the wide 2-D weights (the FC layers: > 99.9 % of the parameters) get their Adam step INSIDE the
-        backward pass, in the epilogue of ops.linear's weight-gradient kernel (dd_linear_wgrad_adam): the gradient tile is
-        consumed where it is produced and never written to HBM (24 bytes per parameter instead of 32, and no gradient
-        buffers: 1.3 GB less for RoadMapBCE).  Measured at the bench shape the step time is the same as the unfused pair of
-        kernels (5.94 ms both: the epilogue's scattered 128-byte accesses to three arrays reach 4.4 TB/s against the
-        streaming Adam kernel's 6.2), so it is opt-in (``fuse_into_backward=True``).  step() then skips them.  Like the sharded form's
-        overlap_backward this is for loops that step after every backward (the reference's); ops.linear falls back to a
-        stored gradient whenever the fused kernel does not apply (batch > 32, CUDA-core path), and step() handles that."""
+        """World size 1, ``overlap_backward=True`` (``fuse_into_backward=True`` names the same form): the wide 2-D weights
+        (the FC layers: > 99.9 % of the parameters) get their Adam step INSIDE the backward pass.  ops.linear's backward
+        then runs one kernel per layer (dd_linear_bwd_adam) that streams each weight tile and its two moments through shared
+        memory once: the input gradient is computed from the old weight, the weight gradient is consumed on chip where it is
+        produced, and the updated weight and moments are written back -- 24 bytes per parameter instead of the 40 of the
+        input-gradient, weight-gradient and Adam kernels, and no gradient buffers (1.3 GB less for RoadMapBCE).  Results are
+        those of the unfused form.  step() then skips these weights.  Like the sharded form's overlap_backward this is for
+        loops that step after every backward (the reference's); ops.linear falls back to a stored gradient whenever the fused
+        kernel does not apply (batch > 32, CUDA-core path), and step() handles that."""
         for g in self.param_groups:
             for p in g["params"]:
                 if p.dim() == 2 and p.numel() >= min_numel and p.is_cuda:
-                    p._dd_fused_update = (lambda q, grp: (lambda dy, x, db: self._fused_step(grp, q, dy, x, db)))(p, g)
+                    p._dd_fused_update = (lambda q, grp: (lambda dy, x, dx, db, ws, n: self._fused_step(grp, q, dy, x, dx, db, ws, n)))(p, g)
 
     @torch.no_grad()
-    def _fused_step(self, g, p, dy, x, db):
+    def _fused_step(self, g, p, dy, x, dx, db, ws, ws_bytes):
         if id(p) in self._fused:
             raise RuntimeError("FusedAdam: two backward passes reached a weight whose Adam step is folded into its backward, "
                                "without a step() in between")
         st = self._state(p, p.numel(), p.device)
         st["step"] += 1
         B, K = x.shape
-        call("dd_linear_wgrad_adam", dy.data_ptr(), x.data_ptr(), p.data_ptr(), st["exp_avg"].data_ptr(), st["exp_avg_sq"].data_ptr(),
-             db.data_ptr() if db is not None else None, B, p.shape[0], K, float(g["lr"]), float(g["betas"][0]), float(g["betas"][1]),
-             float(g["eps"]), float(g["weight_decay"]), st["step"], stream_ptr())
+        call("dd_linear_bwd_adam", dy.data_ptr(), x.data_ptr(), p.data_ptr(), st["exp_avg"].data_ptr(), st["exp_avg_sq"].data_ptr(),
+             dx.data_ptr() if dx is not None else None, _lib.dtype_code(dx.dtype) if dx is not None else _lib.DD_F32,
+             db.data_ptr() if db is not None else None, ws.data_ptr(), ws_bytes, B, p.shape[0], K, float(g["lr"]),
+             float(g["betas"][0]), float(g["betas"][1]), float(g["eps"]), float(g["weight_decay"]), st["step"], stream_ptr())
         self._fused[id(p)] = True
 
     @property

@@ -126,13 +126,16 @@ int dd_linear_dgrad(const float* dy, const float* w, void* dx, int dx_dtype, voi
                     size_t ws_bytes, int B, int N, long long K, int impl, void* stream);
 int dd_linear_wgrad(const float* dy, const void* x, int x_dtype, float* dw, float* db, int B,
                     int N, long long K, int impl, void* stream);
-/* dd_linear_wgrad with torch.optim.Adam's update (roadmap_bce_v2.py:155) folded into the epilogue, for world size 1: the
- * gradient tile dy^T x never goes to HBM -- the epilogue reads {weight, exp_avg, exp_avg_sq} where it would have written dW
- * and writes them back updated (24 bytes per parameter instead of 4 + 28).  `step` = t >= 1; db (may be NULL) is written
- * as usual.  tcgen05 path only: fp32 x, B <= 32, dd_linear_tc_supported(B, N, K). */
-int dd_linear_wgrad_adam(const float* dy, const float* x, float* weight, float* exp_avg, float* exp_avg_sq, float* db, int B,
-                         int N, long long K, float lr, float beta1, float beta2, float eps, float weight_decay, long long step,
-                         void* stream);
+/* The backward pass of a wide linear layer with torch.optim.Adam's update of W (roadmap_bce_v2.py:155) folded in, for world
+ * size 1.  ONE pass over each weight tile: the tile of W, exp_avg and exp_avg_sq is loaded once, the input gradient dx is
+ * computed from the OLD W (bit-identical to dd_linear_dgrad), the weight gradient dy^T x is formed on chip and never reaches
+ * HBM, and W, exp_avg, exp_avg_sq are written back updated (24 bytes per parameter).  Same arithmetic as dd_adam_step
+ * (grad_scale 1); `step` = t >= 1.  dx (x_dtype dx_dtype) may be NULL: no input gradient, and the workspace is then unused;
+ * db (may be NULL) is written as by dd_linear_wgrad.  tcgen05 path only: fp32 x, B <= 32, dd_linear_tc_supported(B, N, K),
+ * dy, x, W and the moments 16-byte aligned; workspace as for dd_linear_dgrad. */
+int dd_linear_bwd_adam(const float* dy, const float* x, float* weight, float* exp_avg, float* exp_avg_sq, void* dx,
+                       int dx_dtype, float* db, void* workspace, size_t ws_bytes, int B, int N, long long K, float lr,
+                       float beta1, float beta2, float eps, float weight_decay, long long step, void* stream);
 size_t dd_linear_workspace_bytes(int B, int N, long long K);
 /* impl = DD_IMPL_TCGEN05 runs the weight-streaming tensor-core kernels (fp32 operands read as tf32 through
  * TMA; x must be fp32): allowed when this returns 1 (N, K multiples of 4, N*K >= 2^22).  DD_IMPL_AUTO
