@@ -60,14 +60,6 @@ struct DilBars {
   uint32_t tmem_base;
 };
 
-__device__ __forceinline__ void wait_backoff(uint64_t* bar, uint32_t parity) {
-  uint32_t spins = 0;
-  while (!umma::mbar_try_wait(bar, parity)) {
-    __nanosleep(64);
-    if (++spins > (1u << 22)) __trap();
-  }
-}
-
 // item -> (b, class rho, first class row t0, strip); strips vary fastest so that neighbouring CTAs share input rows in L2
 struct Item { int b, rho, t0, w0, nrows; };
 __device__ __forceinline__ Item decode(const DilGeo& g, int it, int G_) {
@@ -111,10 +103,7 @@ __global__ void __launch_bounds__(DT_THREADS, 1) conv_dil_tc_kernel(const __grid
     umma::fence_mbar_init();
   }
   if (warp == 2) umma::tmem_alloc(&bars->tmem_base, T::COLS);
-  umma::tc_fence_before_sync();
-  __syncthreads();
-  umma::tc_fence_after_sync();
-  const uint32_t tmem = __shfl_sync(0xffffffffu, bars->tmem_base, 0);
+  const uint32_t tmem = umma::tmem_publish(&bars->tmem_base);
 
   if (warp == 0) {
     // =========================== producer: input rows (one thread, TMA) ============================
@@ -225,7 +214,7 @@ __global__ void __launch_bounds__(DT_THREADS, 1) conv_dil_tc_kernel(const __grid
       const Item im = decode(g, it, G);
       if (im.nrows <= 0) continue;
       const uint32_t buf = T::NBUF == 2 ? (ic & 1) : 0;
-      wait_backoff(&bars->acc_full[buf], (ic / T::NBUF) & 1);
+      umma::mbar_wait_sleep(&bars->acc_full[buf], (ic / T::NBUF) & 1);
       umma::tc_fence_after_sync();
       const int w = im.w0 + quarter * 32 + lane;
       for (int i = half; i < G; i += 2) {
@@ -308,30 +297,13 @@ int launch_dil(const void* in, const __nv_bfloat16* wp, const float* bias, const
   g.groups_max = (Tmax + G - 1) / G;
   g.items = g.B * g.D * g.groups_max * g.strips;
   auto k = conv_dil_tc_kernel<KC, N, G>;
-  cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, T::SMEM);
-  dd::prefer_max_smem(k);
-  if (e != cudaSuccess) return dd::fail((int)e, "conv_dil_tc: cudaFuncSetAttribute(%d): %s", T::SMEM, cudaGetErrorString(e));
+  if (int e = dd::set_smem(k, T::SMEM, dd::Carveout::kMaxShared, "conv_dil_tc")) return e;
   CUtensorMap min_, mw;
-  {
-    dd::EncodeTiledFn enc = dd::tma_encoder();
-    if (!enc) return dd::fail(DD_ERR_UNSUPPORTED, "conv_dil_tc: cuTensorMapEncodeTiled unavailable");
-    static thread_local bool ctx_bound = false;
-    if (!ctx_bound) { cudaFree(nullptr); ctx_bound = true; }
-    const cuuint64_t dims[4] = {(cuuint64_t)K, (cuuint64_t)g.Wi, (cuuint64_t)g.Hi, (cuuint64_t)g.B};
-    const cuuint64_t strides[3] = {(cuuint64_t)K * 2, (cuuint64_t)g.Wi * K * 2, (cuuint64_t)g.Hi * g.Wi * K * 2};
-    const cuuint32_t box[4] = {32, TILE_PX, 1, 1};
-    const cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = enc(&min_, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(in), dims, strides, box, estr,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return dd::fail(DD_ERR_UNSUPPORTED, "conv_dil_tc: cuTensorMapEncodeTiled(in) -> %d", (int)r);
-    const cuuint64_t wdims[2] = {32, (cuuint64_t)KC * g.KT * g.KT * N};
-    const cuuint64_t wstr[1] = {64};
-    const cuuint32_t wbox[2] = {32, (cuuint32_t)N};
-    r = enc(&mw, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<__nv_bfloat16*>(wp), wdims, wstr, wbox, estr,
-            CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return dd::fail(DD_ERR_UNSUPPORTED, "conv_dil_tc: cuTensorMapEncodeTiled(w) -> %d", (int)r);
-  }
+  char msg[256];
+  if (dd::tma_map_nhwc_sw64(&min_, in, g.B, g.Hi, g.Wi, K, TILE_PX, 1, msg, sizeof msg))
+    return dd::fail(DD_ERR_UNSUPPORTED, "conv_dil_tc: in: %s", msg);
+  if (dd::tma_map_2d(&mw, wp, 2, (uint64_t)KC * g.KT * g.KT * N, 32, 32, 32, N, CU_TENSOR_MAP_SWIZZLE_64B, msg, sizeof msg))
+    return dd::fail(DD_ERR_UNSUPPORTED, "conv_dil_tc: w: %s", msg);
   const int grid = g.items < dd::kSMs ? g.items : dd::kSMs;
   k<<<grid, DT_THREADS, T::SMEM, st>>>(min_, mw, bias, (const __nv_bfloat16*)mask, (__nv_bfloat16*)out, g);
   return dd::check_launch("conv_dil_tc");

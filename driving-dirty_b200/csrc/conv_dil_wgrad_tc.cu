@@ -41,14 +41,6 @@ struct WgdBars {
   uint32_t tmem_base;
 };
 
-__device__ __forceinline__ void wait_backoff2(uint64_t* bar, uint32_t parity) {
-  uint32_t spins = 0;
-  while (!umma::mbar_try_wait(bar, parity)) {
-    __nanosleep(64);
-    if (++spins > (1u << 22)) __trap();
-  }
-}
-
 struct WItem { int b, rho, ta, tb, w0; };
 __device__ __forceinline__ WItem wdecode(const WgdGeo& g, int it) {
   WItem o;
@@ -87,10 +79,7 @@ __global__ void __launch_bounds__(WGD_THREADS, 1) conv_dil_wgrad_tc_kernel(const
     umma::fence_mbar_init();
   }
   if (warp == 4) umma::tmem_alloc(&bars->tmem_base, 512);
-  umma::tc_fence_before_sync();
-  __syncthreads();
-  umma::tc_fence_after_sync();
-  const uint32_t tmem = __shfl_sync(0xffffffffu, bars->tmem_base, 0);
+  const uint32_t tmem = umma::tmem_publish(&bars->tmem_base);
 
   if (warp == 0) {
     // =========================== producer (one thread): stage = {one `in` class row, one dout class row} ==========
@@ -168,7 +157,7 @@ __global__ void __launch_bounds__(WGD_THREADS, 1) conv_dil_wgrad_tc_kernel(const
   // =========================== epilogue: TMEM -> this CTA's partials [kw][kh][k 32][n] ===================================
   __syncwarp();
   if (warp < 4) {
-    wait_backoff2(&bars->fin, 0);
+    umma::mbar_wait_sleep(&bars->fin, 0);
     umma::tc_fence_after_sync();
     const int r = warp;                                    // TMEM lane quarter = row r of the group; lane = channel k
     float* outp = partial + (size_t)blockIdx.x * (g.kws * KT * 32 * N);
@@ -218,21 +207,6 @@ __global__ void wgd_fold_kernel(const float* __restrict__ partial, float* __rest
     }
     dw[n * sn + k * sk + (long long)kh * g.KT + kw] = s;
   }
-}
-
-int encode_nhwc(CUtensorMap* map, const void* base, int C, int W, int H, int B, int box_px) {
-  dd::EncodeTiledFn enc = dd::tma_encoder();
-  if (!enc) return -1;
-  static thread_local bool ctx_bound = false;
-  if (!ctx_bound) { cudaFree(nullptr); ctx_bound = true; }
-  const cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)B};
-  const cuuint64_t strides[3] = {(cuuint64_t)C * 2, (cuuint64_t)W * C * 2, (cuuint64_t)H * W * C * 2};
-  const cuuint32_t box[4] = {32, (cuuint32_t)box_px, 1, 1};
-  const cuuint32_t estr[4] = {1, 1, 1, 1};
-  const CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(base), dims, strides, box, estr,
-                         CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  return r == CUDA_SUCCESS ? 0 : (int)r;
 }
 
 WgdGeo make_geo(int B, int Ho, int Wo, int K, int N, int KT, int D, int sign, int off) {
@@ -289,19 +263,15 @@ int conv_dil_wgrad_tc(const void* in, const void* dout, float* dw, long long sn,
   const size_t need = (size_t)grid * g.kws * KT * 32 * N * sizeof(float);
   if (ws_bytes < need) return fail(DD_ERR_WORKSPACE, "conv_dil_wgrad_tc: workspace %zu < %zu", ws_bytes, need);
   CUtensorMap mx, md;
-  if (int r = encode_nhwc(&mx, in, K, Wi, Hi, B, XTILE_PX)) return fail(DD_ERR_UNSUPPORTED, "conv_dil_wgrad_tc: cuTensorMapEncodeTiled(in) -> %d", r);
-  if (int r = encode_nhwc(&md, dout, N, Wo, Ho, B, KPX)) return fail(DD_ERR_UNSUPPORTED, "conv_dil_wgrad_tc: cuTensorMapEncodeTiled(dout) -> %d", r);
+  char msg[256];
+  if (tma_map_nhwc_sw64(&mx, in, B, Hi, Wi, K, XTILE_PX, 1, msg, sizeof msg)) return fail(DD_ERR_UNSUPPORTED, "conv_dil_wgrad_tc: in: %s", msg);
+  if (tma_map_nhwc_sw64(&md, dout, B, Ho, Wo, N, KPX, 1, msg, sizeof msg)) return fail(DD_ERR_UNSUPPORTED, "conv_dil_wgrad_tc: dout: %s", msg);
   const int smem = (g.RX + 3) * XS + g.RD * (N / 32) * DHALF + 256;
-  cudaError_t e;
   if (N == 64) {
-    e = cudaFuncSetAttribute(conv_dil_wgrad_tc_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-    dd::prefer_max_smem(conv_dil_wgrad_tc_kernel<64>);
-    if (e != cudaSuccess) return fail((int)e, "conv_dil_wgrad_tc: cudaFuncSetAttribute(%d): %s", smem, cudaGetErrorString(e));
+    if (int e = set_smem(conv_dil_wgrad_tc_kernel<64>, smem, Carveout::kMaxShared, "conv_dil_wgrad_tc")) return e;
     conv_dil_wgrad_tc_kernel<64><<<grid, WGD_THREADS, smem, st>>>(mx, md, (float*)ws, g);
   } else {
-    e = cudaFuncSetAttribute(conv_dil_wgrad_tc_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-    dd::prefer_max_smem(conv_dil_wgrad_tc_kernel<32>);
-    if (e != cudaSuccess) return fail((int)e, "conv_dil_wgrad_tc: cudaFuncSetAttribute(%d): %s", smem, cudaGetErrorString(e));
+    if (int e = set_smem(conv_dil_wgrad_tc_kernel<32>, smem, Carveout::kMaxShared, "conv_dil_wgrad_tc")) return e;
     conv_dil_wgrad_tc_kernel<32><<<grid, WGD_THREADS, smem, st>>>(mx, md, (float*)ws, g);
   }
   if (int err = check_launch("conv_dil_wgrad_tc")) return err;

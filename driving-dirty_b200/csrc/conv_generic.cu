@@ -436,8 +436,7 @@ int launch_wgrad_tile(const T* P, const T* Q, float* partial, const WGeo& g, int
 #define DD_WT(a, b, q)                                                                                             \
   if (TT == a && TP == b && TQ == q) {                                                                             \
     auto k = conv2d_wgrad_tile_kernel<T, a, b, q>;                                                                 \
-    cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);               \
-    if (e != cudaSuccess) return dd::fail((int)e, "conv2d wgrad tile: cudaFuncSetAttribute: %s", cudaGetErrorString(e)); \
+    if (int e = dd::set_smem(k, smem, dd::Carveout::kDefault, "conv2d wgrad tile")) return e;                      \
     k<<<grid, 256, smem, st>>>(P, Q, partial, g, c);                                                               \
     return dd::check_launch("conv2d_wgrad_tile");                                                                  \
   }

@@ -433,13 +433,6 @@ __global__ void relu_mask_kernel(const T* __restrict__ g, const T* __restrict__ 
 constexpr int kWgradBlocks = dd::kSMs * 2;
 constexpr size_t kWgradWsBytes = (size_t)12 << 20;   // >= SIMT partials (296 x 9248 floats) and tcgen05 partials (148 x 18432 + 592 x 32)
 
-template <typename K>
-int set_smem(K kernel, size_t bytes) {
-  cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
-  if (e != cudaSuccess) return dd::fail((int)e, "cudaFuncSetAttribute(smem=%zu): %s", bytes, cudaGetErrorString(e));
-  return 0;
-}
-
 template <typename T>
 int conv_fwd_simt(const T* in, const float* w, const float* bias, T* out, int B, int H, int W, int stride,
                   cudaStream_t st) {
@@ -448,13 +441,13 @@ int conv_fwd_simt(const T* in, const float* w, const float* bias, T* out, int B,
     constexpr int TH = 8, TW = 32;
     const size_t smem = (9 * C * C + (TH + 2) * (TW + 2) * PADC) * sizeof(float);
     auto k = conv3x3_c32_simt<T, 1, 0, TH, TW>;
-    if (int e = set_smem(k, smem)) return e;
+    if (int e = dd::set_smem(k, smem, dd::Carveout::kDefault, "conv3x3_c32_fwd_simt")) return e;
     k<<<dim3((Wo + TW - 1) / TW, (Ho + TH - 1) / TH, B), TH * TW, smem, st>>>(in, w, bias, nullptr, out, H, W, Ho, Wo);
   } else {
     constexpr int TH = 8, TW = 16;
     const size_t smem = (9 * C * C + (2 * TH + 1) * (2 * TW + 1) * PADC) * sizeof(float);
     auto k = conv3x3_c32_simt<T, 2, 0, TH, TW>;
-    if (int e = set_smem(k, smem)) return e;
+    if (int e = dd::set_smem(k, smem, dd::Carveout::kDefault, "conv3x3_c32_fwd_simt")) return e;
     k<<<dim3((Wo + TW - 1) / TW, (Ho + TH - 1) / TH, B), TH * TW, smem, st>>>(in, w, bias, nullptr, out, H, W, Ho, Wo);
   }
   return dd::check_launch("conv3x3_c32_fwd_simt");
@@ -467,13 +460,13 @@ int conv_dgrad_simt(const T* dy, const float* w, const T* x, T* dx, int B, int H
     constexpr int TH = 8, TW = 32;
     const size_t smem = (9 * C * C + (TH + 2) * (TW + 2) * PADC) * sizeof(float);
     auto k = conv3x3_c32_simt<T, 1, 1, TH, TW>;
-    if (int e = set_smem(k, smem)) return e;
+    if (int e = dd::set_smem(k, smem, dd::Carveout::kDefault, "conv3x3_c32_dgrad_simt")) return e;
     k<<<dim3((W + TW - 1) / TW, (H + TH - 1) / TH, B), TH * TW, smem, st>>>(dy, w, nullptr, x, dx, H, W, H, W);
   } else {
     const int Ho = (H - 1) / 2 + 1, Wo = (W - 1) / 2 + 1;
     const size_t smem = (9 * C * C + 5 * 33 * PADC) * sizeof(float);
     auto k = conv3x3_c32_dgrad_s2_simt<T>;
-    if (int e = set_smem(k, smem)) return e;
+    if (int e = dd::set_smem(k, smem, dd::Carveout::kDefault, "conv3x3_c32_dgrad_simt")) return e;
     k<<<dim3((W + 63) / 64, (H + 7) / 8, B), 256, smem, st>>>(dy, w, x, dx, H, W, Ho, Wo);
   }
   return dd::check_launch("conv3x3_c32_dgrad_simt");
@@ -490,7 +483,7 @@ int conv_wgrad_simt(const T* x, const T* dy, float* dw, float* db, float* ws, in
     nblk = tiles < kWgradBlocks ? tiles : kWgradBlocks;
     const size_t smem = (TH * TW * C + (TH + 2) * (TW + 2) * PADC) * sizeof(float);
     auto k = conv3x3_c32_wgrad_simt<T, 1, TH, TW>;
-    if (int e = set_smem(k, smem)) return e;
+    if (int e = dd::set_smem(k, smem, dd::Carveout::kDefault, "conv3x3_c32_wgrad_simt")) return e;
     k<<<nblk, 288, smem, st>>>(x, dy, ws, B, H, W, Ho, Wo);
   } else {
     constexpr int TH = 8, TW = 16;
@@ -498,7 +491,7 @@ int conv_wgrad_simt(const T* x, const T* dy, float* dw, float* db, float* ws, in
     nblk = tiles < kWgradBlocks ? tiles : kWgradBlocks;
     const size_t smem = (TH * TW * C + (2 * TH + 1) * (2 * TW + 1) * PADC) * sizeof(float);
     auto k = conv3x3_c32_wgrad_simt<T, 2, TH, TW>;
-    if (int e = set_smem(k, smem)) return e;
+    if (int e = dd::set_smem(k, smem, dd::Carveout::kDefault, "conv3x3_c32_wgrad_simt")) return e;
     k<<<nblk, 288, smem, st>>>(x, dy, ws, B, H, W, Ho, Wo);
   }
   if (int e = dd::check_launch("conv3x3_c32_wgrad_simt")) return e;

@@ -39,16 +39,6 @@ constexpr int NPROD = 4;             // producer warps (0..3); warp 4 issues MMA
 constexpr int MMA_WARP = NPROD;
 constexpr int NTHREADS = 32 * (NPROD + 1 + 4);
 
-// Epilogue-side wait: back off between polls so the spinning warps do not take issue slots from the
-// producer / MMA warps that share their schedulers.
-__device__ __forceinline__ void mbar_wait_relaxed(uint64_t* bar, uint32_t parity) {
-  uint32_t spins = 0;
-  while (!umma::mbar_try_wait(bar, parity)) {
-    __nanosleep(64);
-    if (++spins > (1u << 22)) __trap();
-  }
-}
-
 // one pixel's 32 channels (fp32 in registers) -> bf16 -> two 32-byte stores (64-byte aligned destination): whole sectors
 // per lane instead of four half-sector 16-byte stores
 __device__ __forceinline__ void store_pixel32(__nv_bfloat16* dst, const float (&v)[C]) {
@@ -115,10 +105,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) conv3x3_c32_s2_tc_kernel(const __
   }
   if (warp == MMA_WARP) umma::tmem_alloc(&bars->tmem_base, NACC * 32);
   umma::fence_proxy_async_smem();      // weights were written with generic stores
-  umma::tc_fence_before_sync();
-  __syncthreads();
-  umma::tc_fence_after_sync();
-  const uint32_t tmem = __shfl_sync(0xffffffffu, bars->tmem_base, 0);
+  const uint32_t tmem = umma::tmem_publish(&bars->tmem_base);
 
   if (warp == 0) {
     // =========================== producer: one thread, TMA =====================================
@@ -199,7 +186,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) conv3x3_c32_s2_tc_kernel(const __
       for (int j = 0; j < rows; ++j, ++row_ctr) {
         const uint32_t buf = row_ctr % NACC;
         const size_t off = (((size_t)b * Ho + ho0 + j) * Wo + (wo < Wo ? wo : 0)) * C;
-        mbar_wait_relaxed(&bars->acc_full[buf], (row_ctr / NACC) & 1);
+        umma::mbar_wait_sleep(&bars->acc_full[buf], (row_ctr / NACC) & 1);
         umma::tc_fence_after_sync();
         uint32_t r[32];
         umma::tmem_ld_32x32(tmem + ((uint32_t)(quarter * 32) << 16) + buf * 32, r);
@@ -225,13 +212,12 @@ __global__ void __launch_bounds__(NTHREADS, 1) conv3x3_c32_s2_tc_kernel(const __
 int launch_s2_fwd(const void* in, const float* w, const float* bias, void* out, int B, int H, int W, cudaStream_t st) {
   const int Ho = (H - 1) / 2 + 1, Wo = (W - 1) / 2 + 1;
   const int items = B * ((Wo + TILE_M - 1) / TILE_M) * ((Ho + ROWS - 1) / ROWS);
-  cudaError_t e = cudaFuncSetAttribute(conv3x3_c32_s2_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, S2_SMEM);
-  dd::prefer_max_smem(conv3x3_c32_s2_tc_kernel);
-  if (e != cudaSuccess) return dd::fail((int)e, "conv_tc s2: cudaFuncSetAttribute(%d): %s", S2_SMEM, cudaGetErrorString(e));
+  if (int e = dd::set_smem(conv3x3_c32_s2_tc_kernel, S2_SMEM, dd::Carveout::kMaxShared, "conv_tc s2")) return e;
   CUtensorMap m2, m1;
-  int r = dd::tma_map_nhwc_sw64(&m2, in, (uint64_t)B, (uint64_t)H, (uint64_t)W, 255, 2);      // 255 source pixels -> 128 loaded
-  if (!r) r = dd::tma_map_nhwc_sw64(&m1, in, (uint64_t)B, (uint64_t)H, (uint64_t)W, 1, 1);
-  if (r) return dd::fail(DD_ERR_UNSUPPORTED, "conv_tc s2: cuTensorMapEncodeTiled -> %d (B %d H %d W %d)", r, B, H, W);
+  char msg[256];
+  if (dd::tma_map_nhwc_sw64(&m2, in, B, H, W, C, 255, 2, msg, sizeof msg) ||      // 255 source pixels -> 128 loaded
+      dd::tma_map_nhwc_sw64(&m1, in, B, H, W, C, 1, 1, msg, sizeof msg))
+    return dd::fail(DD_ERR_UNSUPPORTED, "conv_tc s2: %s", msg);
   const int grid = items < dd::kSMs ? items : dd::kSMs;
   conv3x3_c32_s2_tc_kernel<<<grid, NTHREADS, S2_SMEM, st>>>(m2, m1, w, bias, (__nv_bfloat16*)out, B, H, W, Ho, Wo);
   return dd::check_launch("conv3x3_c32_s2_tc");
@@ -317,10 +303,7 @@ __global__ void __launch_bounds__(S1_THREADS, 1) conv3x3_c32_s1_tc_kernel(const 
   }
   if (warp == MMA_WARP) umma::tmem_alloc(&bars->tmem_base, S1_NACC * 32);
   umma::fence_proxy_async_smem();
-  umma::tc_fence_before_sync();
-  __syncthreads();
-  umma::tc_fence_after_sync();
-  const uint32_t tmem = __shfl_sync(0xffffffffu, bars->tmem_base, 0);
+  const uint32_t tmem = umma::tmem_publish(&bars->tmem_base);
 
   if (warp < NPROD) {
     // =========================== producer: one thread of warp 0, TMA (warps 1..3 idle) ============
@@ -519,14 +502,12 @@ int launch_s1(const void* in, const float* w, const float* bias, const void* mas
               cudaStream_t st) {
   const int items = B * ((W + TILE_M - 1) / TILE_M) * ((H + S1_ROWS - 1) / S1_ROWS);
   auto k = conv3x3_c32_s1_tc_kernel<MODE>;
-  cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, S1_SMEM);
-  dd::prefer_max_smem(k);
-  if (e != cudaSuccess) return dd::fail((int)e, "conv_tc s1: cudaFuncSetAttribute(%d): %s", S1_SMEM, cudaGetErrorString(e));
+  if (int e = dd::set_smem(k, S1_SMEM, dd::Carveout::kMaxShared, "conv_tc s1")) return e;
   const int grid = items < dd::kSMs ? items : dd::kSMs;
   if ((reinterpret_cast<uintptr_t>(in) & 15) != 0) return dd::fail(DD_ERR_ALIGNMENT, "conv_tc s1: input is not 16-byte aligned");
   CUtensorMap map;
-  if (int r = dd::tma_map_nhwc_sw64(&map, in, (uint64_t)B, (uint64_t)H, (uint64_t)W, 130))
-    return dd::fail(DD_ERR_UNSUPPORTED, "conv_tc s1: cuTensorMapEncodeTiled -> %d (B %d H %d W %d)", r, B, H, W);
+  char msg[256];
+  if (dd::tma_map_nhwc_sw64(&map, in, B, H, W, C, 130, 1, msg, sizeof msg)) return dd::fail(DD_ERR_UNSUPPORTED, "conv_tc s1: %s", msg);
   k<<<grid, S1_THREADS, S1_SMEM, st>>>(map, w, bias, (const __nv_bfloat16*)mask, (__nv_bfloat16*)out, B, H, W);
   return dd::check_launch("conv3x3_c32_s1_tc");
 }
@@ -581,10 +562,7 @@ __global__ void __maxnreg__(96) conv3x3_c32_dgrad_s2_tc_kernel(const __grid_cons
   }
   if (warp == MMA_WARP) umma::tmem_alloc(&bars->tmem_base, 256);
   umma::fence_proxy_async_smem();
-  umma::tc_fence_before_sync();
-  __syncthreads();
-  umma::tc_fence_after_sync();
-  const uint32_t tmem = __shfl_sync(0xffffffffu, bars->tmem_base, 0);
+  const uint32_t tmem = umma::tmem_publish(&bars->tmem_base);
 
   if (warp < NPROD) {
     // =========================== producer: dy rows m0 .. m0+rows, one thread, TMA ===============
@@ -674,7 +652,7 @@ __global__ void __maxnreg__(96) conv3x3_c32_dgrad_s2_tc_kernel(const __grid_cons
             for (int gq = 0; gq < 4; ++gq) mk[aa][gq] = __ldg(reinterpret_cast<const uint4*>(mask + moff) + gq);
           }
         }
-        mbar_wait_relaxed(&bars->acc_full[set], (mctr >> 1) & 1);
+        umma::mbar_wait_sleep(&bars->acc_full[set], (mctr >> 1) & 1);
         umma::tc_fence_after_sync();
 #pragma unroll
         for (int aa = 0; aa < 2; ++aa) {
@@ -739,16 +717,6 @@ struct C1Bars {
 };
 
 // pointer to channel 0 of (b, mosaic row h, mosaic column wm); channel stride returned in cstride
-// torchvision ToTensor (data_helper.py:109-114): byte -> float32, divided by 255.  The IEEE division (bit-identical to
-// x.float() / 255) is done ONCE per CTA for the 256 possible bytes into a shared-memory table; a division per pixel
-// made the raw-byte kernels instruction-bound (the c1 forward + weight gradient pair ran 1.6 ms slower per step).
-template <typename TIN> __device__ __forceinline__ float c1_cvt(TIN x, const float* lut);
-template <> __device__ __forceinline__ float c1_cvt<float>(float x, const float*) { return x; }
-template <> __device__ __forceinline__ float c1_cvt<uint8_t>(uint8_t x, const float* lut) { return lut[x]; }
-__device__ __forceinline__ void c1_fill_lut(float* lut) {
-  for (int i = threadIdx.x; i < 256; i += blockDim.x) lut[i] = __fdiv_rn((float)i, 255.0f);
-}
-
 template <bool IS_VIEWS, typename TIN>
 __device__ __forceinline__ const TIN* c1_src(const TIN* __restrict__ in, int b, int h, int wm, int H, int Wm,
                                              size_t& cstride) {
@@ -786,7 +754,7 @@ __device__ __forceinline__ void c1_load_row(uint8_t* __restrict__ slab, const TI
 #pragma unroll
   for (int k = 0; k < 5; ++k) {
 #pragma unroll
-    for (int c = 0; c < 3; ++c) v[k][c] = ok[k] ? c1_cvt<TIN>(raw[k][c], lut) : 0.f;
+    for (int c = 0; c < 3; ++c) v[k][c] = ok[k] ? dd::c1_cvt<TIN>(raw[k][c], lut) : 0.f;
   }
 #pragma unroll
   for (int k = 0; k < 5; ++k) {
@@ -812,7 +780,7 @@ __global__ void __launch_bounds__(C1_THREADS, 1) conv_c1_tc_kernel(const TIN* __
   C1Bars* bars = reinterpret_cast<C1Bars*>(smem + C1_WBYTES + C1_RING * PS);
   __shared__ float s_bias[C];
   __shared__ float s_lut[256];
-  c1_fill_lut(s_lut);
+  dd::c1_fill_lut(s_lut);
   const int tid = threadIdx.x, lane = tid & 31;
   const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);
   const int wtiles = (Wm + TILE_M - 1) / TILE_M;
@@ -835,10 +803,7 @@ __global__ void __launch_bounds__(C1_THREADS, 1) conv_c1_tc_kernel(const TIN* __
   }
   if (warp == C1_MMA_WARP) umma::tmem_alloc(&bars->tmem_base, NACC * 32);
   umma::fence_proxy_async_smem();
-  umma::tc_fence_before_sync();
-  __syncthreads();
-  umma::tc_fence_after_sync();
-  const uint32_t tmem = __shfl_sync(0xffffffffu, bars->tmem_base, 0);
+  const uint32_t tmem = umma::tmem_publish(&bars->tmem_base);
 
   if (warp < C1_NPROD) {
     // =========================== producers: slab g -> warp g % C1_NPROD =========================
@@ -901,7 +866,7 @@ __global__ void __launch_bounds__(C1_THREADS, 1) conv_c1_tc_kernel(const TIN* __
       const int wo = wt * TILE_M + quarter * 32 + lane;
       for (int j = 0; j < rows; ++j, ++row_ctr) {
         const uint32_t buf = row_ctr % NACC;
-        mbar_wait_relaxed(&bars->acc_full[buf], (row_ctr / NACC) & 1);
+        umma::mbar_wait_sleep(&bars->acc_full[buf], (row_ctr / NACC) & 1);
         umma::tc_fence_after_sync();
         uint32_t r[32];
         umma::tmem_ld_32x32(tmem + ((uint32_t)(quarter * 32) << 16) + buf * 32, r);
@@ -983,7 +948,7 @@ __global__ void __maxnreg__(80) enc_c1c2_fused_kernel(const TIN* __restrict__ in
   EBars* bars = reinterpret_cast<EBars*>(smem + E_OFF_BARS);
   __shared__ float s_b1[C], s_b2[C];
   __shared__ float s_lut[256];
-  c1_fill_lut(s_lut);
+  dd::c1_fill_lut(s_lut);
   const int tid = threadIdx.x, lane = tid & 31;
   const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);
   const int wtiles = (Wm + E_STRIP - 1) / E_STRIP;
@@ -1017,10 +982,7 @@ __global__ void __maxnreg__(80) enc_c1c2_fused_kernel(const TIN* __restrict__ in
   }
   if (warp == E_MMA_WARP) umma::tmem_alloc(&bars->tmem_base, 512);
   umma::fence_proxy_async_smem();
-  umma::tc_fence_before_sync();
-  __syncthreads();
-  umma::tc_fence_after_sync();
-  const uint32_t tmem = __shfl_sync(0xffffffffu, bars->tmem_base, 0);
+  const uint32_t tmem = umma::tmem_publish(&bars->tmem_base);
   const uint32_t tmem2 = tmem + E_NACC1 * 32;
 
   if (warp < E_NCONV) {
@@ -1249,7 +1211,7 @@ __global__ void __maxnreg__(80) enc_c1c2_fused_kernel(const TIN* __restrict__ in
       const bool ok = m < E_STRIP && wo < Wm;
       for (int j = (int)((grb ^ half) & 1); j < rows; j += 2) {
         const uint32_t rr = grb + j, slot = rr % E_NACC2, d = gab + j + 2;
-        mbar_wait_relaxed(&bars->c2_done[d % E_DONE], (d / E_DONE) & 1);
+        umma::mbar_wait_sleep(&bars->c2_done[d % E_DONE], (d / E_DONE) & 1);
         umma::tc_fence_after_sync();
         uint32_t r[32];
         umma::tmem_ld_32x32(tmem2 + ((uint32_t)(quarter * 32) << 16) + slot * 32, r);
@@ -1303,13 +1265,11 @@ int conv3x3_c32_fwd_tc(const void* in, const float* w, const float* bias, void* 
     // here `in` = dy [B,Ho,Wo,32], `out` = dx [B,H,W,32]
     const int Ho = (H - 1) / 2 + 1, Wo = (W - 1) / 2 + 1;
     const int items = B * (((W + 1) / 2 + TILE_M - 1) / TILE_M) * (((H + 1) / 2 + DG_MROWS - 1) / DG_MROWS);
-    cudaError_t e = cudaFuncSetAttribute(conv3x3_c32_dgrad_s2_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, DG_SMEM);
-    dd::prefer_max_smem(conv3x3_c32_dgrad_s2_tc_kernel);
-    if (e != cudaSuccess) return fail((int)e, "dgrad_s2_tc: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
+    if (int e = set_smem(conv3x3_c32_dgrad_s2_tc_kernel, DG_SMEM, Carveout::kMaxShared, "dgrad_s2_tc")) return e;
     if ((reinterpret_cast<uintptr_t>(in) & 15) != 0) return fail(DD_ERR_ALIGNMENT, "dgrad_s2_tc: dy is not 16-byte aligned");
     CUtensorMap mdy;
-    if (int r = tma_map_nhwc_sw64(&mdy, in, (uint64_t)B, (uint64_t)Ho, (uint64_t)Wo, 129))
-      return fail(DD_ERR_UNSUPPORTED, "dgrad_s2_tc: cuTensorMapEncodeTiled -> %d", r);
+    char msg[256];
+    if (tma_map_nhwc_sw64(&mdy, in, B, Ho, Wo, C, 129, 1, msg, sizeof msg)) return fail(DD_ERR_UNSUPPORTED, "dgrad_s2_tc: %s", msg);
     conv3x3_c32_dgrad_s2_tc_kernel<<<items < kSMs ? items : kSMs, DG_THREADS, DG_SMEM, st>>>(
         mdy, w, (const __nv_bfloat16*)mask, (__nv_bfloat16*)out, B, H, W, Ho, Wo);
     return check_launch("conv3x3_c32_dgrad_s2_tc");
@@ -1324,9 +1284,7 @@ int conv_c1_fwd_tc(const void* in, int in_flags, const float* w, const float* bi
   const int items = B * ((Wm + TILE_M - 1) / TILE_M) * ((H + ROWS - 1) / ROWS);
   const int grid = items < kSMs ? items : kSMs;
   auto launch1 = [&](auto k, auto* typed_in) {
-    cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, C1_SMEM);
-    dd::prefer_max_smem(k);
-    if (e != cudaSuccess) return fail((int)e, "conv_c1_tc: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
+    if (int e = set_smem(k, C1_SMEM, Carveout::kMaxShared, "conv_c1_tc")) return e;
     k<<<grid, C1_THREADS, C1_SMEM, st>>>(typed_in, w, bias, (__nv_bfloat16*)out, B, H, Wm);
     return check_launch("conv_c1_tc");
   };
@@ -1342,9 +1300,7 @@ int enc_c1c2_fused_fwd_tc(const void* in, int in_flags, const float* w1, const f
   const int items = B * ((Wm + E_STRIP - 1) / E_STRIP) * ((H + E_ROWS - 1) / E_ROWS);
   const int grid = items < kSMs ? items : kSMs;
   auto launch1 = [&](auto k, auto* typed_in) {
-    cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, E_SMEM);
-    dd::prefer_max_smem(k);
-    if (e != cudaSuccess) return fail((int)e, "enc_c1c2_fused: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
+    if (int e = set_smem(k, E_SMEM, Carveout::kMaxShared, "enc_c1c2_fused")) return e;
     k<<<grid, E_THREADS, E_SMEM, st>>>(typed_in, w1, b1, w2, b2, (__nv_bfloat16*)out, B, H, Wm);
     return check_launch("enc_c1c2_fused");
   };

@@ -56,14 +56,6 @@ struct RingBars {
   uint32_t tmem_base;
 };
 
-__device__ __forceinline__ void mbar_wait_backoff(uint64_t* bar, uint32_t parity) {
-  uint32_t spins = 0;
-  while (!umma::mbar_try_wait(bar, parity)) {
-    __nanosleep(64);
-    if (++spins > (1u << 22)) __trap();
-  }
-}
-
 template <int STRIDE>
 __global__ void __launch_bounds__(WGT_THREADS, 1) conv3x3_c32_wgrad_ring_kernel(const __grid_constant__ CUtensorMap map_x,
                                                                                 const __grid_constant__ CUtensorMap map_x1,
@@ -89,10 +81,7 @@ __global__ void __launch_bounds__(WGT_THREADS, 1) conv3x3_c32_wgrad_ring_kernel(
     umma::fence_mbar_init();
   }
   if (warp == 4) umma::tmem_alloc(&bars->tmem_base, 256);
-  umma::tc_fence_before_sync();
-  __syncthreads();
-  umma::tc_fence_after_sync();
-  const uint32_t tmem = __shfl_sync(0xffffffffu, bars->tmem_base, 0);
+  const uint32_t tmem = umma::tmem_publish(&bars->tmem_base);
 
   if (warp == 0) {
     // =========================== producer: one thread, TMA ========================================
@@ -154,7 +143,7 @@ __global__ void __launch_bounds__(WGT_THREADS, 1) conv3x3_c32_wgrad_ring_kernel(
       const int P = (rows + G::NQ - 1) / G::NQ;
       for (int i = 0; i <= P; ++i, ++g) {
         const uint32_t s = g % G::NS;
-        mbar_wait_backoff(&bars->full[s], (g / G::NS) & 1);
+        umma::mbar_wait_sleep(&bars->full[s], (g / G::NS) & 1);
         if (i < P) {
           const uint32_t base = umma::smem_u32(s_d) + s * G::NQ * DROW;
 #pragma unroll
@@ -228,7 +217,7 @@ __global__ void __launch_bounds__(WGT_THREADS, 1) conv3x3_c32_wgrad_ring_kernel(
   // =========================== epilogue: TMEM -> per-CTA partials (warps 0..3) ========================
   __syncwarp();
   if (warp < 4) {
-    mbar_wait_backoff(&bars->done, 0);
+    umma::mbar_wait_sleep(&bars->done, 0);
     umma::tc_fence_after_sync();
     const int r = warp;                      // TMEM lane quarter = x row r of the group; lane = ci
     float* out = partial + (size_t)blockIdx.x * G::PARTIAL;
@@ -300,18 +289,6 @@ constexpr int C1_PARTIAL = C1_RB * 3 * 10 * C;  // floats per CTA: [q][kh][j][co
 constexpr int C1_THREADS = 192;
 static_assert(C1_SMEM <= 227 * 1024, "shared memory");
 
-// torchvision ToTensor (data_helper.py:109-114): byte -> float32, divided by 255.  The IEEE division (bit-identical to
-// x.float() / 255) is done ONCE per CTA for the 256 possible bytes into a shared-memory table; a division per pixel
-// made the raw-byte kernels instruction-bound (the c1 forward + weight gradient pair ran 1.6 ms slower per step).
-// byte -> float through the table AFTER the prefetch distance: a look-up at load time would make every prefetched global
-// load wait for its own round trip (the raw-byte kernel ran 0.37 ms against 0.25 for fp32 views)
-template <typename TIN> __device__ __forceinline__ float c1_cvt(TIN x, const float* lut);
-template <> __device__ __forceinline__ float c1_cvt<float>(float x, const float*) { return x; }
-template <> __device__ __forceinline__ float c1_cvt<uint8_t>(uint8_t x, const float* lut) { return lut[x]; }
-__device__ __forceinline__ void c1_fill_lut(float* lut) {
-  for (int i = threadIdx.x; i < 256; i += blockDim.x) lut[i] = __fdiv_rn((float)i, 255.0f);
-}
-
 template <bool IS_VIEWS, typename TIN>
 __global__ void __launch_bounds__(C1_THREADS, 1) conv_c1_wgrad_ring_kernel(const TIN* __restrict__ in,
                                                                            const __grid_constant__ CUtensorMap map_dy,
@@ -321,7 +298,7 @@ __global__ void __launch_bounds__(C1_THREADS, 1) conv_c1_wgrad_ring_kernel(const
   uint8_t* s_d = smem + C1_XBYTES;
   RingBars* bars = reinterpret_cast<RingBars*>(smem + C1_XBYTES + C1_DBYTES);
   __shared__ float s_lut[256];
-  c1_fill_lut(s_lut);
+  dd::c1_fill_lut(s_lut);
   const int tid = threadIdx.x, lane = tid & 31;
   const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);
   const int wtiles = (Wm + KP - 1) / KP;
@@ -335,10 +312,7 @@ __global__ void __launch_bounds__(C1_THREADS, 1) conv_c1_wgrad_ring_kernel(const
     umma::fence_mbar_init();
   }
   if (warp == 4) umma::tmem_alloc(&bars->tmem_base, 128);
-  umma::tc_fence_before_sync();
-  __syncthreads();
-  umma::tc_fence_after_sync();
-  const uint32_t tmem = __shfl_sync(0xffffffffu, bars->tmem_base, 0);
+  const uint32_t tmem = umma::tmem_publish(&bars->tmem_base);
 
   if (warp < 4) {
     // =========================== converters: thread = pixel column of the strip ====================
@@ -404,7 +378,7 @@ __global__ void __launch_bounds__(C1_THREADS, 1) conv_c1_wgrad_ring_kernel(const
 #pragma unroll
       for (int r = 0; r < C1_RB; ++r)
 #pragma unroll
-        for (int c = 0; c < 3; ++c) { v[r][c] = c1_cvt<TIN>(rv[r][c], s_lut); e[r][c] = c1_cvt<TIN>(re[r][c], s_lut); }
+        for (int c = 0; c < 3; ++c) { v[r][c] = dd::c1_cvt<TIN>(rv[r][c], s_lut); e[r][c] = dd::c1_cvt<TIN>(re[r][c], s_lut); }
 #pragma unroll
       for (int r = 0; r < C1_RB; ++r) {
         float lf[3], rt[3];
@@ -501,7 +475,7 @@ __global__ void __launch_bounds__(C1_THREADS, 1) conv_c1_wgrad_ring_kernel(const
   // =========================== epilogue: TMEM -> per-CTA partials (warps 0..3) ==========================
   __syncwarp();
   if (warp < 4) {
-    mbar_wait_backoff(&bars->done, 0);
+    umma::mbar_wait_sleep(&bars->done, 0);
     umma::tc_fence_after_sync();
     const int r = 2 * warp + (lane >> 4), j = lane & 15;     // TMEM lane = r*16 + j
     float* out = partial + (size_t)blockIdx.x * C1_PARTIAL;
@@ -558,20 +532,19 @@ int wgrad_ring_launch(const void* x, const void* dy, float* dw, float* db, void*
   float* partial = (float*)ws;
   float* dbp = partial + (size_t)grid * G::PARTIAL;
   auto k = conv3x3_c32_wgrad_ring_kernel<STRIDE>;
-  cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, G::SMEM);
-  dd::prefer_max_smem(k);
-  if (e != cudaSuccess) return dd::fail((int)e, "wgrad_tc: cudaFuncSetAttribute(%d): %s", G::SMEM, cudaGetErrorString(e));
+  if (int e = dd::set_smem(k, G::SMEM, dd::Carveout::kMaxShared, "wgrad_tc")) return e;
   CUtensorMap mx = {}, mx1 = {}, mdy = {};
+  char msg[256];
   int r;
   if (STRIDE == 1) {
-    r = dd::tma_map_nhwc_sw64(&mx, x, (uint64_t)B, (uint64_t)H, (uint64_t)W, 130, 1);
+    r = dd::tma_map_nhwc_sw64(&mx, x, B, H, W, C, 130, 1, msg, sizeof msg);
   } else {
-    r = dd::tma_map_nhwc_sw64(&mx, x, (uint64_t)B, (uint64_t)H, (uint64_t)W, 255, 2);          // 255 source pixels -> 128 loaded
-    if (!r) r = dd::tma_map_nhwc_sw64(&mx1, x, (uint64_t)B, (uint64_t)H, (uint64_t)W, 1, 1);
+    r = dd::tma_map_nhwc_sw64(&mx, x, B, H, W, C, 255, 2, msg, sizeof msg);          // 255 source pixels -> 128 loaded
+    if (!r) r = dd::tma_map_nhwc_sw64(&mx1, x, B, H, W, C, 1, 1, msg, sizeof msg);
   }
-  if (r) return dd::fail(DD_ERR_UNSUPPORTED, "tcgen05 wgrad: cuTensorMapEncodeTiled(x) -> %d", r);
-  if ((r = dd::tma_map_nhwc_sw64(&mdy, dy, (uint64_t)B, (uint64_t)Ho, (uint64_t)Wo, KP, 1)))
-    return dd::fail(DD_ERR_UNSUPPORTED, "tcgen05 wgrad: cuTensorMapEncodeTiled(dy) -> %d", r);
+  if (r) return dd::fail(DD_ERR_UNSUPPORTED, "tcgen05 wgrad: x: %s", msg);
+  if (dd::tma_map_nhwc_sw64(&mdy, dy, B, Ho, Wo, C, KP, 1, msg, sizeof msg))
+    return dd::fail(DD_ERR_UNSUPPORTED, "tcgen05 wgrad: dy: %s", msg);
   k<<<grid, WGT_THREADS, G::SMEM, st>>>(mx, mx1, mdy, partial, dbp, B, Ho, Wo);
   if (int err = dd::check_launch("conv3x3_c32_wgrad_ring")) return err;
   wgrad_ring_reduce_kernel<<<(9 * C * C + C + 255) / 256, 256, 0, st>>>(partial, grid * G::NQ, dbp, grid, dw, db);
@@ -599,12 +572,10 @@ int conv_c1_wgrad_tc(const void* in, int in_flags, const void* dy, float* dw, fl
   if (ws_bytes < need) return fail(DD_ERR_WORKSPACE, "tcgen05 c1 wgrad: workspace %zu < %zu", ws_bytes, need);
   if ((reinterpret_cast<uintptr_t>(dy) & 15) != 0) return fail(DD_ERR_ALIGNMENT, "tcgen05 c1 wgrad: dy is not 16-byte aligned");
   CUtensorMap mdy;
-  if (int r = dd::tma_map_nhwc_sw64(&mdy, dy, (uint64_t)B, (uint64_t)H, (uint64_t)Wm, KP, 1))
-    return fail(DD_ERR_UNSUPPORTED, "tcgen05 c1 wgrad: cuTensorMapEncodeTiled(dy) -> %d", r);
+  char msg[256];
+  if (tma_map_nhwc_sw64(&mdy, dy, B, H, Wm, C, KP, 1, msg, sizeof msg)) return fail(DD_ERR_UNSUPPORTED, "tcgen05 c1 wgrad: dy: %s", msg);
   auto launch1 = [&](auto k, auto* typed_in) {
-    cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, C1_SMEM);
-    dd::prefer_max_smem(k);
-    if (e != cudaSuccess) return fail((int)e, "conv_c1_wgrad_tc: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
+    if (int e = set_smem(k, C1_SMEM, Carveout::kMaxShared, "conv_c1_wgrad_tc")) return e;
     k<<<grid, C1_THREADS, C1_SMEM, st>>>(typed_in, mdy, (float*)ws, B, H, Wm);
     return check_launch("conv_c1_wgrad_ring");
   };

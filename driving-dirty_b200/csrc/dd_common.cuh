@@ -1,4 +1,4 @@
-// Shared helpers for libdd_b200: error text, launch accounting, dtype load/store.
+// Shared helpers for libdd_b200: error text, launch accounting and attributes, dtype load/store.
 #pragma once
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
@@ -18,17 +18,21 @@ int check_launch(const char* what);  // cudaGetLastError -> return code, counts 
 
 inline cudaStream_t as_stream(void* s) { return reinterpret_cast<cudaStream_t>(s); }
 
-// Persistent kernels that live on big dynamic shared memory ask for the maximum shared-memory carveout: an SM changes its
-// L1 / shared split only when idle, so a kernel that needs more shared memory than the split chosen for the previous one
-// cannot join an SM that the overlapped optimizer update keeps busy (it queued behind the whole update at N > 1).
+// Raises a kernel's dynamic shared-memory limit to `bytes`; reports a failure through fail(), naming `what`.
+// Persistent kernels that live on big dynamic shared memory also ask for the maximum shared-memory carveout: an SM changes
+// its L1 / shared split only when idle, so a kernel that needs more shared memory than the split chosen for the previous
+// one cannot join an SM that the overlapped optimizer update keeps busy (it queued behind the whole update at N > 1).
+enum class Carveout { kDefault, kMaxShared };
 template <class K>
-inline void prefer_max_smem(K kernel) {
-#ifndef DD_NO_CARVEOUT_PREFERENCE
-  cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-#else
-  (void)kernel;
-#endif
+inline int set_smem(K kernel, size_t bytes, Carveout carveout, const char* what) {
+  const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+  if (carveout == Carveout::kMaxShared)
+    cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+  if (e != cudaSuccess) return fail((int)e, "%s: cudaFuncSetAttribute(%zu): %s", what, bytes, cudaGetErrorString(e));
+  return 0;
 }
+
+inline int ceil_div(long long a, long long b) { return (int)((a + b - 1) / b); }
 
 #define DD_REQUIRE(cond, code, ...) \
   do {                              \
@@ -92,6 +96,18 @@ __device__ __forceinline__ long long warp_sum(long long v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
   return v;
+}
+
+// torchvision ToTensor (data_helper.py:109-114): byte -> float32, divided by 255.  The IEEE division (bit-identical to
+// x.float() / 255) is done ONCE per CTA for the 256 possible bytes into a shared-memory table; a division per pixel
+// made the raw-byte kernels instruction-bound (the c1 forward + weight gradient pair ran 1.6 ms slower per step).
+// Callers look a byte up only after its global load and the loads issued behind it: a look-up at load time makes every
+// prefetched load wait for its own round trip (the raw-byte c1 weight gradient ran 0.37 ms against 0.25 for fp32 views).
+template <typename TIN> __device__ __forceinline__ float c1_cvt(TIN x, const float* lut);
+template <> __device__ __forceinline__ float c1_cvt<float>(float x, const float*) { return x; }
+template <> __device__ __forceinline__ float c1_cvt<uint8_t>(uint8_t x, const float* lut) { return lut[x]; }
+__device__ __forceinline__ void c1_fill_lut(float* lut) {
+  for (int i = threadIdx.x; i < 256; i += blockDim.x) lut[i] = __fdiv_rn((float)i, 255.0f);
 }
 
 // mosaic slot j shows dataset view kViewOrder[j] (roadmap_bce_v2.py:58)

@@ -275,32 +275,30 @@ __global__ void colsum_kernel(const float* __restrict__ dy, float* __restrict__ 
   db[n] = s;
 }
 
-int ceil_div(long long a, long long b) { return (int)((a + b - 1) / b); }
-
 // choose split counts so that ~4 CTAs per SM exist without oversizing the partial buffers
 struct FwdPlan { int row_blocks, ksplits; long long kchunk; };
 FwdPlan plan_fwd(int N, long long K) {
   FwdPlan p;
-  p.row_blocks = ceil_div(N, 8 * NR);
-  int want = ceil_div(dd::kSMs * 4, p.row_blocks);
+  p.row_blocks = dd::ceil_div(N, 8 * NR);
+  int want = dd::ceil_div(dd::kSMs * 4, p.row_blocks);
   long long maxsplit = (K + KC - 1) / KC;
   if (want > maxsplit) want = (int)maxsplit;
   if (want < 1) want = 1;
   p.kchunk = ((K + want - 1) / want + KC - 1) / KC * KC;
-  p.ksplits = ceil_div(K, p.kchunk);
+  p.ksplits = dd::ceil_div(K, p.kchunk);
   return p;
 }
 struct DgradPlan { int kt, kblocks, nsplits, nchunk; };
 DgradPlan plan_dgrad(int N, long long K) {
   DgradPlan p;
   p.kt = (K / 4 >= 256) ? 256 : 32;
-  p.kblocks = ceil_div(K / 4, p.kt);
-  int want = ceil_div(dd::kSMs * 2, p.kblocks);
-  int maxsplit = ceil_div(N, NCH);
+  p.kblocks = dd::ceil_div(K / 4, p.kt);
+  int want = dd::ceil_div(dd::kSMs * 2, p.kblocks);
+  int maxsplit = dd::ceil_div(N, NCH);
   if (want > maxsplit) want = maxsplit;
   if (want < 1) want = 1;
-  p.nchunk = ceil_div(ceil_div(N, want), NCH) * NCH;
-  p.nsplits = ceil_div(N, p.nchunk);
+  p.nchunk = dd::ceil_div(dd::ceil_div(N, want), NCH) * NCH;
+  p.nsplits = dd::ceil_div(N, p.nchunk);
   return p;
 }
 
@@ -310,12 +308,12 @@ int fwd_launch(const T* x, const float* w, const float* bias, float* y, float* w
   const FwdPlan p = plan_fwd(N, K);
   const size_t smem = (size_t)BT * KC * sizeof(float);
   auto kern = linear_fwd_simt<T, BT>;
-  cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (int e = dd::set_smem(kern, smem, dd::Carveout::kDefault, "linear_fwd_simt")) return e;
   kern<<<dim3(p.row_blocks, p.ksplits), NTHREADS, smem, st>>>(x, w, bias, y, ws, B, N, K, p.kchunk);
   if (int e = dd::check_launch("linear_fwd_simt")) return e;
   if (p.ksplits > 1) {
     const long long bn = (long long)B * N;
-    splitk_reduce_kernel<<<ceil_div(bn, 256), 256, 0, st>>>(ws, bias, y, p.ksplits, bn, N);
+    splitk_reduce_kernel<<<dd::ceil_div(bn, 256), 256, 0, st>>>(ws, bias, y, p.ksplits, bn, N);
     return dd::check_launch("splitk_reduce");
   }
   return 0;
@@ -333,13 +331,13 @@ int dgrad_launch(const float* dy, const float* w, T* dx, float* ws, int B, int N
     const size_t fold = (size_t)8 * BT * 32 * 4 * sizeof(float);
     if (fold > smem) smem = fold;
     auto k = linear_dgrad_simt<T, BT, 32>;
-    cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (int e = dd::set_smem(k, smem, dd::Carveout::kDefault, "linear_dgrad_simt")) return e;
     k<<<grid, NTHREADS, smem, st>>>(dy, w, dx, ws, B, N, K, p.nchunk);
   }
   if (int e = dd::check_launch("linear_dgrad_simt")) return e;
   if (p.nsplits > 1) {
     const long long bk = (long long)B * K;
-    splitn_reduce_kernel<T><<<ceil_div(bk, 256), 256, 0, st>>>(ws, dx, p.nsplits, bk);
+    splitn_reduce_kernel<T><<<dd::ceil_div(bk, 256), 256, 0, st>>>(ws, dx, p.nsplits, bk);
     return dd::check_launch("splitn_reduce");
   }
   return 0;
@@ -348,13 +346,13 @@ int dgrad_launch(const float* dy, const float* w, T* dx, float* ws, int B, int N
 template <typename T, int BT>
 int wgrad_launch(const float* dy, const T* x, float* dw, int B, int N, long long K, int accumulate, cudaStream_t st) {
   const int kt = (K / 4 >= 256) ? 256 : 32;
-  const int kblocks = ceil_div(K / 4, kt);
-  int want = ceil_div(dd::kSMs * 4, kblocks);
-  int maxsplit = ceil_div(N, NCH);
+  const int kblocks = dd::ceil_div(K / 4, kt);
+  int want = dd::ceil_div(dd::kSMs * 4, kblocks);
+  int maxsplit = dd::ceil_div(N, NCH);
   if (want > maxsplit) want = maxsplit;
   if (want < 1) want = 1;
-  const int nchunk = ceil_div(ceil_div(N, want), NCH) * NCH;
-  dim3 grid(kblocks, ceil_div(N, nchunk));
+  const int nchunk = dd::ceil_div(dd::ceil_div(N, want), NCH) * NCH;
+  dim3 grid(kblocks, dd::ceil_div(N, nchunk));
   const size_t smem = (size_t)NCH * BT * sizeof(float);
   if (kt == 256) linear_wgrad_simt<T, BT, 256><<<grid, NTHREADS, smem, st>>>(dy, x, dw, B, N, K, nchunk, accumulate);
   else linear_wgrad_simt<T, BT, 32><<<grid, NTHREADS, smem, st>>>(dy, x, dw, B, N, K, nchunk, accumulate);
@@ -492,7 +490,7 @@ extern "C" int dd_linear_wgrad(const float* dy, const void* x, int x_dtype, floa
                   : wgrad_launch<__nv_bfloat16, 32>(dyp, (const __nv_bfloat16*)xp, dw, bc, N, K, accumulate, st);
     if (e) return e;
     if (db) {
-      colsum_kernel<<<ceil_div(N, 256), 256, 0, st>>>(dyp, db, bc, N, accumulate);
+      colsum_kernel<<<dd::ceil_div(N, 256), 256, 0, st>>>(dyp, db, bc, N, accumulate);
       if (int e2 = dd::check_launch("colsum")) return e2;
     }
   }
@@ -516,7 +514,7 @@ extern "C" int dd_linear_bwd_adam(const float* dy, const float* x, float* weight
   const dd::AdamHyper h = dd::adam_hyper(lr, beta1, beta2, eps, weight_decay, step, 1.f);
   if (int e = dd::linear_bwd_adam_tc(dy, x, weight, exp_avg, exp_avg_sq, dx, dx_dtype, workspace, ws_bytes, B, N, K, h, st)) return e;
   if (db) {
-    colsum_kernel<<<ceil_div(N, 256), 256, 0, st>>>(dy, db, B, N, 0);
+    colsum_kernel<<<dd::ceil_div(N, 256), 256, 0, st>>>(dy, db, B, N, 0);
     if (int e2 = dd::check_launch("colsum")) return e2;
   }
   return 0;

@@ -36,14 +36,6 @@ constexpr int kChunk = 32;                // contraction elements per stage (one
 __device__ __forceinline__ uint8_t* align1024(uint8_t* p) {
   return reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(p) + 1023) & ~static_cast<uintptr_t>(1023));
 }
-__device__ __forceinline__ void mbar_wait_relaxed(uint64_t* bar, uint32_t parity) {
-  uint32_t spins = 0;
-  while (!umma::mbar_try_wait(bar, parity)) {
-    __nanosleep(64);
-    if (++spins > (1u << 22)) __trap();
-  }
-}
-
 // ------------------------------------------------------------------------------------------------
 // fwd (MODE 0) and dgrad (MODE 1): out[b * LD + r] = sum over the contraction, r = row of the 128-row tile
 // ------------------------------------------------------------------------------------------------
@@ -90,10 +82,7 @@ __global__ void __launch_bounds__(THREADS, 1) linear_stream_tc_kernel(const __gr
     umma::tma_prefetch_desc(&map_v);
   }
   if (warp == 1) umma::tmem_alloc(&bars->tmem_base, 2 * NBT);
-  umma::tc_fence_before_sync();
-  __syncthreads();
-  umma::tc_fence_after_sync();
-  const uint32_t tmem = __shfl_sync(0xffffffffu, bars->tmem_base, 0);
+  const uint32_t tmem = umma::tmem_publish(&bars->tmem_base);
 
   if (warp == 0) {
     // =========================== TMA producer ===================================================
@@ -157,7 +146,7 @@ __global__ void __launch_bounds__(THREADS, 1) linear_stream_tc_kernel(const __gr
     for (int it = blockIdx.x; it < items; it += gridDim.x, ++n_item) {
       const int ti = it % g.tiles, si = it / g.tiles;
       const uint32_t a = n_item & 1;
-      mbar_wait_relaxed(&bars->acc_full[a], (n_item >> 1) & 1);
+      umma::mbar_wait_sleep(&bars->acc_full[a], (n_item >> 1) & 1);
       umma::tc_fence_after_sync();
       const int r = ti * 128 + quarter * 32 + lane;
       const float bv = (g.splits == 1 && bias && r < g.LD) ? __ldg(bias + r) : 0.f;
@@ -255,10 +244,7 @@ __global__ void __launch_bounds__(W_THREADS, 1) linear_wgrad_tc_kernel(const __g
     umma::tma_prefetch_desc(&map_x);
   }
   if (warp == 1) umma::tmem_alloc(&bars->tmem_base, 512);
-  umma::tc_fence_before_sync();
-  __syncthreads();
-  umma::tc_fence_after_sync();
-  const uint32_t tmem = __shfl_sync(0xffffffffu, bars->tmem_base, 0);
+  const uint32_t tmem = umma::tmem_publish(&bars->tmem_base);
 
   // item -> (n tile, k tile): consecutive items of a CTA share the n tile (its dy^T boxes stay in L2)
   if (warp == 0) {
@@ -300,7 +286,7 @@ __global__ void __launch_bounds__(W_THREADS, 1) linear_wgrad_tc_kernel(const __g
     for (long long it = blockIdx.x; it < items; it += gridDim.x, ++c) {
       const int ni = (int)(it / g.k_tiles), ki = (int)(it % g.k_tiles);
       const uint32_t a = c & 1;
-      mbar_wait_relaxed(&bars->acc_full[a], (c >> 1) & 1);
+      umma::mbar_wait_sleep(&bars->acc_full[a], (c >> 1) & 1);
       umma::tc_fence_after_sync();
       const int n0 = ni * 128 + quarter * 32;
       const long long k0 = (long long)ki * g.KT;
@@ -404,10 +390,7 @@ __global__ void __launch_bounds__(BA_THREADS, 1) linear_bwd_adam_tc_kernel(
     umma::tma_prefetch_desc(&map_dy); umma::tma_prefetch_desc(&map_dyt); umma::tma_prefetch_desc(&map_x);
   }
   if (warp == 1) umma::tmem_alloc(&bars->tmem_base, 128);
-  umma::tc_fence_before_sync();
-  __syncthreads();
-  umma::tc_fence_after_sync();
-  const uint32_t tmem = __shfl_sync(0xffffffffu, bars->tmem_base, 0);
+  const uint32_t tmem = umma::tmem_publish(&bars->tmem_base);
 
   if (warp == 0) {
     // =========================== TMA producer ===================================================
@@ -491,7 +474,7 @@ __global__ void __launch_bounds__(BA_THREADS, 1) linear_bwd_adam_tc_kernel(
         const int c1 = min(c0 + g.chunks_per_split, g.chunks);
         for (int ch = c0; ch < c1; ++ch, ++c) {
           const uint32_t s = c % BA_STAGES;
-          mbar_wait_relaxed(&bars->tile_ready[s], (c / BA_STAGES) & 1);
+          umma::mbar_wait_sleep(&bars->tile_ready[s], (c / BA_STAGES) & 1);
           const uint32_t src = umma::smem_u32(smem + s * BA_STAGE_BYTES);
 #pragma unroll
           for (int i = 0; i < 4; ++i) {
@@ -517,7 +500,7 @@ __global__ void __launch_bounds__(BA_THREADS, 1) linear_bwd_adam_tc_kernel(
       const int c1 = min(c0 + g.chunks_per_split, g.chunks);
       for (int ch = c0; ch < c1; ++ch, ++c) {
         const uint32_t s = c % BA_STAGES, ga = c & 1;
-        mbar_wait_relaxed(&bars->g_full[ga], (c >> 1) & 1);
+        umma::mbar_wait_sleep(&bars->g_full[ga], (c >> 1) & 1);
         umma::tc_fence_after_sync();
         uint32_t gv[16];
         umma::tmem_ld_32x16(tmem + ((uint32_t)(quarter * 32) << 16) + 2 * NB + ga * NB + sub * 16, gv);
@@ -542,7 +525,7 @@ __global__ void __launch_bounds__(BA_THREADS, 1) linear_bwd_adam_tc_kernel(
         if (has_dx && ch == c1 - 1) {
           // the item's input gradient, as the dgrad kernel writes it (this warp: 16 of the 32 batch rows)
           const uint32_t a = n_item & 1;
-          mbar_wait_relaxed(&bars->acc_full[a], (n_item >> 1) & 1);
+          umma::mbar_wait_sleep(&bars->acc_full[a], (n_item >> 1) & 1);
           umma::tc_fence_after_sync();
           uint32_t v[16];
           umma::tmem_ld_32x16(tmem + ((uint32_t)(quarter * 32) << 16) + a * NB + sub * 16, v);
@@ -572,16 +555,6 @@ __global__ void __launch_bounds__(BA_THREADS, 1) linear_bwd_adam_tc_kernel(
   if (warp == 1) umma::tmem_dealloc(tmem, 128);
 }
 
-int ceil_div_ll(long long a, long long b) { return (int)((a + b - 1) / b); }
-
-template <typename K>
-int set_smem(K kernel, int bytes) {
-  cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
-  dd::prefer_max_smem(kernel);
-  if (e != cudaSuccess) return dd::fail((int)e, "linear_tc: cudaFuncSetAttribute(%d): %s", bytes, cudaGetErrorString(e));
-  return 0;
-}
-
 // split the contraction so that ~kSMs work items exist; rows = 128-row output tiles
 void plan_stream(int tiles, int chunks, int& splits, int& cps) {
   splits = 1;
@@ -601,15 +574,15 @@ namespace dd {
 
 bool linear_tc_supported(int B, int N, long long K) {
   // TMA needs 16-byte row pitches; the streaming design pays off only for wide layers
-  return B >= 1 && N % 4 == 0 && K % 4 == 0 && (long long)N * K >= (1ll << 22) && tma_encoder() != nullptr;
+  return B >= 1 && N % 4 == 0 && K % 4 == 0 && (long long)N * K >= (1ll << 22) && tma_available();
 }
 
 size_t linear_tc_workspace_bytes(int B, int N, long long K) {
   const int Bf = B < kLinearTcMaxRows ? B : kLinearTcMaxRows;     // forward: up to 256 rows per pass
   const int Bd = B < NB ? B : NB;                                 // input gradient: 32
   int s1, c1, s2, c2;
-  plan_stream(ceil_div_ll(N, 128), ceil_div_ll(K, kChunk), s1, c1);      // fwd: tiles over N, contraction K
-  plan_stream(ceil_div_ll(K, 128), ceil_div_ll(N, kChunk), s2, c2);      // dgrad: tiles over K, contraction N
+  plan_stream(ceil_div(N, 128), ceil_div(K, kChunk), s1, c1);      // fwd: tiles over N, contraction K
+  plan_stream(ceil_div(K, 128), ceil_div(N, kChunk), s2, c2);      // dgrad: tiles over K, contraction N
   const size_t a = s1 > 1 ? (size_t)s1 * Bf * N * sizeof(float) : 0;
   const size_t b = s2 > 1 ? (size_t)s2 * Bd * K * sizeof(float) : 0;
   return (a > b ? a : b) + 256;
@@ -619,7 +592,7 @@ template <int NBT>
 int launch_fwd(const CUtensorMap& mw, const CUtensorMap& mx, const float* bias, float* y, float* ws, const StreamGeo& g,
                cudaStream_t st) {
   auto k = linear_stream_tc_kernel<0, float, NBT>;
-  if (int e = set_smem(k, SCfg<NBT>::SMEM)) return e;
+  if (int e = set_smem(k, SCfg<NBT>::SMEM, Carveout::kMaxShared, "linear_tc")) return e;
   const int items = g.tiles * g.splits;
   k<<<items < kSMs ? items : kSMs, THREADS, SCfg<NBT>::SMEM, st>>>(mw, mx, bias, y, ws, g);
   return check_launch("linear_fwd_tc");
@@ -631,16 +604,16 @@ int linear_fwd_tc(const float* x, const float* w, const float* bias, float* y, v
   if (B > kLinearTcMaxRows) return fail(DD_ERR_UNSUPPORTED, "linear_fwd_tc: %d rows per pass (max %d)", B, kLinearTcMaxRows);
   StreamGeo g;
   g.B = B; g.LD = N;
-  g.tiles = ceil_div_ll(N, 128);
-  g.chunks = ceil_div_ll(K, kChunk);
+  g.tiles = ceil_div(N, 128);
+  g.chunks = ceil_div(K, kChunk);
   plan_stream(g.tiles, g.chunks, g.splits, g.chunks_per_split);
   if (g.splits > 1 && ws_bytes < (size_t)g.splits * B * N * sizeof(float))
     return fail(DD_ERR_WORKSPACE, "linear_fwd_tc: workspace %zu too small for %d splits", ws_bytes, g.splits);
   const int nbt = B <= 32 ? 32 : B <= 64 ? 64 : B <= 128 ? 128 : 256;
   CUtensorMap mw, mx;
   char msg[256];
-  if (tma_map_2d_checked(&mw, w, 4, N, K, K, 32, 128, false, msg, sizeof msg) ||
-      tma_map_2d_checked(&mx, x, 4, B, K, K, 32, nbt, false, msg, sizeof msg))
+  if (tma_map_2d(&mw, w, 4, N, K, K, 32, 128, CU_TENSOR_MAP_SWIZZLE_128B, msg, sizeof msg) ||
+      tma_map_2d(&mx, x, 4, B, K, K, 32, nbt, CU_TENSOR_MAP_SWIZZLE_128B, msg, sizeof msg))
     return fail(DD_ERR_UNSUPPORTED, "linear_fwd_tc: %s", msg);
   int e = nbt == 32 ? launch_fwd<32>(mw, mx, bias, y, (float*)ws, g, st)
         : nbt == 64 ? launch_fwd<64>(mw, mx, bias, y, (float*)ws, g, st)
@@ -649,7 +622,7 @@ int linear_fwd_tc(const float* x, const float* w, const float* bias, float* y, v
   if (e) return e;
   if (g.splits > 1) {
     const long long n = (long long)B * N;
-    split_fold_kernel<float><<<ceil_div_ll(n, 256), 256, 0, st>>>((const float*)ws, bias, y, g.splits, n, N);
+    split_fold_kernel<float><<<ceil_div(n, 256), 256, 0, st>>>((const float*)ws, bias, y, g.splits, n, N);
     return check_launch("linear_fwd_fold");
   }
   return 0;
@@ -660,32 +633,32 @@ int linear_dgrad_tc(const float* dy, const float* w, void* dx, int dx_dtype, voi
                     long long K, cudaStream_t st) {
   StreamGeo g;
   g.B = B; g.LD = (int)K;
-  g.tiles = ceil_div_ll(K, 128);
-  g.chunks = ceil_div_ll(N, kChunk);
+  g.tiles = ceil_div(K, 128);
+  g.chunks = ceil_div(N, kChunk);
   plan_stream(g.tiles, g.chunks, g.splits, g.chunks_per_split);
   if (g.splits > 1 && ws_bytes < (size_t)g.splits * B * K * sizeof(float))
     return fail(DD_ERR_WORKSPACE, "linear_dgrad_tc: workspace %zu too small for %d splits", ws_bytes, g.splits);
   CUtensorMap mw, mdy;
   char msg[256];
-  if (tma_map_2d_checked(&mw, w, 4, N, K, K, 32, 32, /*atom32=*/true, msg, sizeof msg) ||
-      tma_map_2d_checked(&mdy, dy, 4, B, N, N, 32, 32, false, msg, sizeof msg))
+  if (tma_map_2d(&mw, w, 4, N, K, K, 32, 32, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, msg, sizeof msg) ||
+      tma_map_2d(&mdy, dy, 4, B, N, N, 32, 32, CU_TENSOR_MAP_SWIZZLE_128B, msg, sizeof msg))
     return fail(DD_ERR_UNSUPPORTED, "linear_dgrad_tc: %s", msg);
   const int items = g.tiles * g.splits;
   const int grid = items < kSMs ? items : kSMs;
   const long long n = (long long)B * K;
   if (dx_dtype == DD_F32) {
     auto k = linear_stream_tc_kernel<1, float>;
-    if (int e = set_smem(k, SCfg<NB>::SMEM)) return e;
+    if (int e = set_smem(k, SCfg<NB>::SMEM, Carveout::kMaxShared, "linear_tc")) return e;
     k<<<grid, THREADS, SCfg<NB>::SMEM, st>>>(mw, mdy, nullptr, (float*)dx, (float*)ws, g);
     if (int e = check_launch("linear_dgrad_tc")) return e;
-    if (g.splits > 1) split_fold_kernel<float><<<ceil_div_ll(n, 256), 256, 0, st>>>((const float*)ws, nullptr, (float*)dx, g.splits, n, (int)K);
+    if (g.splits > 1) split_fold_kernel<float><<<ceil_div(n, 256), 256, 0, st>>>((const float*)ws, nullptr, (float*)dx, g.splits, n, (int)K);
   } else {
     auto k = linear_stream_tc_kernel<1, __nv_bfloat16>;
-    if (int e = set_smem(k, SCfg<NB>::SMEM)) return e;
+    if (int e = set_smem(k, SCfg<NB>::SMEM, Carveout::kMaxShared, "linear_tc")) return e;
     k<<<grid, THREADS, SCfg<NB>::SMEM, st>>>(mw, mdy, nullptr, (__nv_bfloat16*)dx, (float*)ws, g);
     if (int e = check_launch("linear_dgrad_tc")) return e;
     if (g.splits > 1)
-      split_fold_kernel<__nv_bfloat16><<<ceil_div_ll(n, 256), 256, 0, st>>>((const float*)ws, nullptr, (__nv_bfloat16*)dx, g.splits, n, (int)K);
+      split_fold_kernel<__nv_bfloat16><<<ceil_div(n, 256), 256, 0, st>>>((const float*)ws, nullptr, (__nv_bfloat16*)dx, g.splits, n, (int)K);
   }
   return g.splits > 1 ? check_launch("linear_dgrad_fold") : 0;
 }
@@ -695,37 +668,37 @@ int linear_bwd_adam_tc(const float* dy, const float* x, float* w, float* m, floa
                        size_t ws_bytes, int B, int N, long long K, const AdamHyper& h, cudaStream_t st) {
   StreamGeo g;
   g.B = B; g.LD = (int)K;
-  g.tiles = ceil_div_ll(K, 128);
-  g.chunks = ceil_div_ll(N, kChunk);
+  g.tiles = ceil_div(K, 128);
+  g.chunks = ceil_div(N, kChunk);
   plan_stream(g.tiles, g.chunks, g.splits, g.chunks_per_split);
   if (dx && g.splits > 1 && ws_bytes < (size_t)g.splits * B * K * sizeof(float))
     return fail(DD_ERR_WORKSPACE, "linear_bwd_adam_tc: workspace %zu too small for %d splits", ws_bytes, g.splits);
   CUtensorMap mw, mm, mv, mdy, mdyt, mx;
   char msg[256];
-  if (tma_map_2d_checked(&mw, w, 4, N, K, K, 32, 32, true, msg, sizeof msg) ||
-      tma_map_2d_checked(&mm, m, 4, N, K, K, 32, 32, true, msg, sizeof msg) ||
-      tma_map_2d_checked(&mv, v, 4, N, K, K, 32, 32, true, msg, sizeof msg) ||
-      tma_map_2d_checked(&mdy, dy, 4, B, N, N, 32, 32, false, msg, sizeof msg) ||
-      tma_map_2d_checked(&mdyt, dy, 4, B, N, N, 32, 32, true, msg, sizeof msg) ||
-      tma_map_2d_checked(&mx, x, 4, B, K, K, 32, 32, true, msg, sizeof msg))
+  if (tma_map_2d(&mw, w, 4, N, K, K, 32, 32, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, msg, sizeof msg) ||
+      tma_map_2d(&mm, m, 4, N, K, K, 32, 32, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, msg, sizeof msg) ||
+      tma_map_2d(&mv, v, 4, N, K, K, 32, 32, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, msg, sizeof msg) ||
+      tma_map_2d(&mdy, dy, 4, B, N, N, 32, 32, CU_TENSOR_MAP_SWIZZLE_128B, msg, sizeof msg) ||
+      tma_map_2d(&mdyt, dy, 4, B, N, N, 32, 32, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, msg, sizeof msg) ||
+      tma_map_2d(&mx, x, 4, B, K, K, 32, 32, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, msg, sizeof msg))
     return fail(DD_ERR_UNSUPPORTED, "linear_bwd_adam_tc: %s", msg);
   const int items = g.tiles * g.splits;
   const int grid = items < kSMs ? items : kSMs;
   const long long n = (long long)B * K;
   if (dx_dtype == DD_BF16 && dx) {
     auto k = linear_bwd_adam_tc_kernel<__nv_bfloat16>;
-    if (int e = set_smem(k, BA_SMEM)) return e;
+    if (int e = set_smem(k, BA_SMEM, Carveout::kMaxShared, "linear_tc")) return e;
     k<<<grid, BA_THREADS, BA_SMEM, st>>>(mw, mm, mv, mdy, mdyt, mx, (__nv_bfloat16*)dx, (float*)ws, g, h);
     if (int e = check_launch("linear_bwd_adam_tc")) return e;
     if (g.splits > 1)
-      split_fold_kernel<__nv_bfloat16><<<ceil_div_ll(n, 256), 256, 0, st>>>((const float*)ws, nullptr, (__nv_bfloat16*)dx, g.splits, n, (int)K);
+      split_fold_kernel<__nv_bfloat16><<<ceil_div(n, 256), 256, 0, st>>>((const float*)ws, nullptr, (__nv_bfloat16*)dx, g.splits, n, (int)K);
   } else {
     auto k = linear_bwd_adam_tc_kernel<float>;
-    if (int e = set_smem(k, BA_SMEM)) return e;
+    if (int e = set_smem(k, BA_SMEM, Carveout::kMaxShared, "linear_tc")) return e;
     k<<<grid, BA_THREADS, BA_SMEM, st>>>(mw, mm, mv, mdy, mdyt, mx, (float*)dx, (float*)ws, g, h);
     if (int e = check_launch("linear_bwd_adam_tc")) return e;
     if (dx && g.splits > 1)
-      split_fold_kernel<float><<<ceil_div_ll(n, 256), 256, 0, st>>>((const float*)ws, nullptr, (float*)dx, g.splits, n, (int)K);
+      split_fold_kernel<float><<<ceil_div(n, 256), 256, 0, st>>>((const float*)ws, nullptr, (float*)dx, g.splits, n, (int)K);
   }
   return dx && g.splits > 1 ? check_launch("linear_bwd_adam_fold") : 0;
 }
@@ -735,17 +708,17 @@ int linear_wgrad_tc(const float* dy, const float* x, float* dw, int B, int N, lo
   WgradGeo g = {};
   g.B = B; g.N = N; g.K = K;
   g.KT = K >= 256 ? 256 : 128;
-  g.n_tiles = ceil_div_ll(N, 128);
-  g.k_tiles = ceil_div_ll(K, g.KT);
+  g.n_tiles = ceil_div(N, 128);
+  g.k_tiles = ceil_div(K, g.KT);
   g.accumulate = accumulate;
   CUtensorMap mdy, mx;
   char msg[256];
-  if (tma_map_2d_checked(&mdy, dy, 4, B, N, N, 32, 32, true, msg, sizeof msg) ||
-      tma_map_2d_checked(&mx, x, 4, B, K, K, 32, 32, true, msg, sizeof msg))
+  if (tma_map_2d(&mdy, dy, 4, B, N, N, 32, 32, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, msg, sizeof msg) ||
+      tma_map_2d(&mx, x, 4, B, K, K, 32, 32, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, msg, sizeof msg))
     return fail(DD_ERR_UNSUPPORTED, "linear_wgrad_tc: %s", msg);
   const long long items = (long long)g.n_tiles * g.k_tiles;
   const int grid = (int)(items < kSMs ? items : kSMs);
-  if (int e = set_smem(linear_wgrad_tc_kernel, W_SMEM)) return e;
+  if (int e = set_smem(linear_wgrad_tc_kernel, W_SMEM, Carveout::kMaxShared, "linear_tc")) return e;
   linear_wgrad_tc_kernel<<<grid, W_THREADS, W_SMEM, st>>>(mdy, mx, dw, g);
   return check_launch("linear_wgrad_tc");
 }

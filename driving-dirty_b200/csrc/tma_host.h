@@ -1,5 +1,6 @@
 // Host-side TMA descriptor (CUtensorMap) construction without linking libcuda: the driver entry point
-// cuTensorMapEncodeTiled is fetched through the runtime (cudaGetDriverEntryPoint).
+// cuTensorMapEncodeTiled is fetched through the runtime (cudaGetDriverEntryPoint).  Every tensor map of the library is
+// encoded here.
 #pragma once
 #include <cuda.h>
 #include <cuda_runtime.h>
@@ -24,77 +25,62 @@ inline EncodeTiledFn tma_encoder() {
   return fn;
 }
 
-// Row-major 2-D matrix [rows][cols] of 4-byte (fp32) or 2-byte (bf16) elements, row pitch in elements;
-// box = box_cols x box_rows, 128-byte swizzle (box_cols * elem_bytes must be 128; atom32: the 32-byte-atom
-// variant that MN-major tf32 operands need), out-of-range = 0.
-// Returns 0 on success.
+inline bool tma_available() { return tma_encoder() != nullptr; }
+
+// Tiled map of 2 to 4 dimensions (dims / box innermost first, strides in bytes), out-of-range elements = 0.
+// Returns 0 on success, else the driver's error (-1: no encoder) and, if msg is given, a description of the map in msg.
+inline int tma_encode(CUtensorMap* map, CUtensorMapDataType dtype, int rank, const void* base, const cuuint64_t* dims,
+                      const cuuint64_t* strides, const cuuint32_t* box, const cuuint32_t* estr, CUtensorMapSwizzle swizzle,
+                      char* msg, size_t msg_len) {
+  int r = -1;
+  if (EncodeTiledFn enc = tma_encoder()) {
+    // cuTensorMapEncodeTiled is a DRIVER call: it needs a current context on the calling thread.  PyTorch's
+    // autograd worker threads may not have one yet (the runtime binds it lazily; seen as error 201 =
+    // CUDA_ERROR_INVALID_CONTEXT from backward passes) -- a runtime no-op binds the primary context.
+    static thread_local bool ctx_bound = false;
+    if (!ctx_bound) { cudaFree(nullptr); ctx_bound = true; }
+    const CUresult e = enc(map, dtype, (cuuint32_t)rank, const_cast<void*>(base), dims, strides, box, estr,
+                           CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    r = e == CUDA_SUCCESS ? 0 : (int)e;
+  }
+  if (r != 0 && msg) {
+    unsigned long long d[4] = {1, 1, 1, 1};
+    unsigned b[4] = {1, 1, 1, 1};
+    for (int i = 0; i < rank && i < 4; ++i) { d[i] = dims[i]; b[i] = box[i]; }
+    snprintf(msg, msg_len, "cuTensorMapEncodeTiled -> %d (base %p, dims %llux%llux%llux%llu, pitch %llu B, box %ux%ux%ux%u, swizzle %d)",
+             r, base, d[0], d[1], d[2], d[3], (unsigned long long)strides[0], b[0], b[1], b[2], b[3], (int)swizzle);
+  }
+  return r;
+}
+
+// Row-major 2-D matrix [rows][cols] of 4-byte (fp32) or 2-byte (bf16) elements, row pitch in elements; box = box_cols x
+// box_rows with box_cols * elem_bytes = the swizzle span: 128 B for CU_TENSOR_MAP_SWIZZLE_128B and _128B_ATOM_32B (the
+// 32-byte-atom variant that MN-major tf32 operands need), 64 B for CU_TENSOR_MAP_SWIZZLE_64B.
 inline int tma_map_2d(CUtensorMap* map, const void* base, int elem_bytes, uint64_t rows, uint64_t cols, uint64_t pitch_elems,
-                      uint32_t box_cols, uint32_t box_rows, bool atom32 = false) {
-  EncodeTiledFn enc = tma_encoder();
-  if (!enc) return -1;
-  // cuTensorMapEncodeTiled is a DRIVER call: it needs a current context on the calling thread.  PyTorch's
-  // autograd worker threads may not have one yet (the runtime binds it lazily; seen as error 201 =
-  // CUDA_ERROR_INVALID_CONTEXT from backward passes) -- a runtime no-op binds the primary context.
-  static thread_local bool ctx_bound = false;
-  if (!ctx_bound) { cudaFree(nullptr); ctx_bound = true; }
+                      uint32_t box_cols, uint32_t box_rows, CUtensorMapSwizzle swizzle, char* msg, size_t msg_len) {
   const cuuint64_t dims[2] = {cols, rows};
   const cuuint64_t strides[1] = {pitch_elems * (uint64_t)elem_bytes};
   const cuuint32_t box[2] = {box_cols, box_rows};
   const cuuint32_t estr[2] = {1, 1};
-  const CUresult r = enc(map, elem_bytes == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2,
-                         const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                         atom32 ? CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B : CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  return r == CUDA_SUCCESS ? 0 : (int)r;
+  return tma_encode(map, elem_bytes == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, base, dims,
+                    strides, box, estr, swizzle, msg, msg_len);
 }
 
-// NHWC bf16 activation [B][H][W][32] seen as a 4-D tensor (channel, w, h, b) with a box of 8 channels x box_w pixels of one
-// row: a load at (8*cg, w0, h, b) lands as the [pixel][8 ch] plane of channel group cg that the SWIZZLE_NONE K-major UMMA
-// operands use, and every out-of-image pixel (w0 = -1, h = -1, h = H, the right edge) is zero-filled = the conv padding.
-inline int tma_map_nhwc_c8(CUtensorMap* map, const void* base, uint64_t B, uint64_t H, uint64_t W, uint32_t box_w) {
-  EncodeTiledFn enc = tma_encoder();
-  if (!enc) return -1;
-  static thread_local bool ctx_bound = false;
-  if (!ctx_bound) { cudaFree(nullptr); ctx_bound = true; }
-  const cuuint64_t dims[4] = {32, W, H, B};
-  const cuuint64_t strides[3] = {64, W * 64, H * W * 64};
-  const cuuint32_t box[4] = {8, box_w, 1, 1};
-  const cuuint32_t estr[4] = {1, 1, 1, 1};
-  const CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(base), dims, strides, box, estr,
-                         CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  return r == CUDA_SUCCESS ? 0 : (int)r;
-}
-
-// NHWC bf16 activation [B][H][W][32] as a 4-D tensor (c, w, h, b) with a box of WHOLE pixels: 32 channels x box_w SOURCE
-// pixels of one row, taking every estride-th pixel (box_w <= 256; estride 2 -> ceil(box_w / 2) pixels land), 64-byte
-// swizzle (inner extent = one 64-byte pixel).  The tile that lands is at once the K-major SWIZZLE_64B operand of a forward
-// conv (rows = pixels, K = channels) and the MN-major one of a weight gradient (K = pixels); a tap is a shift of the
-// operand's start address by whole pixels (tools/tma_layout_probe.cu, tools/tma_sw64_mn_probe.cu).  Full 32-byte
-// sectors from L2 and one request per row, against half sectors and four requests with tma_map_nhwc_c8.
-inline int tma_map_nhwc_sw64(CUtensorMap* map, const void* base, uint64_t B, uint64_t H, uint64_t W, uint32_t box_w,
-                             uint32_t estride = 1) {
-  EncodeTiledFn enc = tma_encoder();
-  if (!enc) return -1;
-  static thread_local bool ctx_bound = false;
-  if (!ctx_bound) { cudaFree(nullptr); ctx_bound = true; }
-  const cuuint64_t dims[4] = {32, W, H, B};
-  const cuuint64_t strides[3] = {64, W * 64, H * W * 64};
+// NHWC bf16 activation [B][H][W][C] as a 4-D tensor (c, w, h, b) with a box of 32 channels x box_w SOURCE pixels of one
+// row, taking every estride-th pixel (box_w <= 256; estride 2 -> ceil(box_w / 2) pixels land), 64-byte swizzle (inner
+// extent = 64 bytes: a whole pixel when C = 32).  The tile that lands is at once the K-major SWIZZLE_64B operand of a
+// forward conv (rows = pixels, K = channels) and the MN-major one of a weight gradient (K = pixels); a tap is a shift of
+// the operand's start address by whole pixels (tools/tma_layout_probe.cu, tools/tma_sw64_mn_probe.cu).  Full 32-byte
+// sectors from L2 and one request per row, against half sectors and four requests with 8-channel boxes.
+inline int tma_map_nhwc_sw64(CUtensorMap* map, const void* base, uint64_t B, uint64_t H, uint64_t W, uint64_t C, uint32_t box_w,
+                             uint32_t estride, char* msg, size_t msg_len) {
+  const cuuint64_t dims[4] = {C, W, H, B};
+  const cuuint64_t strides[3] = {C * 2, W * C * 2, H * W * C * 2};
   const cuuint32_t box[4] = {32, box_w, 1, 1};
   const cuuint32_t estr[4] = {1, estride, 1, 1};
-  const CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(base), dims, strides, box, estr,
-                         CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  return r == CUDA_SUCCESS ? 0 : (int)r;
-}
-
-// last failing encode, for error texts
-inline int tma_map_2d_checked(CUtensorMap* map, const void* base, int elem_bytes, uint64_t rows, uint64_t cols,
-                              uint64_t pitch_elems, uint32_t box_cols, uint32_t box_rows, bool atom32, char* msg, size_t msg_len) {
-  const int r = tma_map_2d(map, base, elem_bytes, rows, cols, pitch_elems, box_cols, box_rows, atom32);
-  if (r != 0 && msg)
-    snprintf(msg, msg_len, "cuTensorMapEncodeTiled -> %d (base %p, rows %llu, cols %llu, pitch %llu, box %ux%u, atom32 %d)", r, base,
-             (unsigned long long)rows, (unsigned long long)cols, (unsigned long long)pitch_elems, box_cols, box_rows, (int)atom32);
-  return r;
+  return tma_encode(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, base, dims, strides, box, estr, CU_TENSOR_MAP_SWIZZLE_64B, msg,
+                    msg_len);
 }
 
 }  // namespace dd

@@ -1,6 +1,7 @@
-// Minimal sm_100a tcgen05 / TMEM / mbarrier wrappers (inline PTX) used by conv_tc.cu and
-// linear_tc.cu.  Descriptor bit layouts follow the PTX ISA "matrix descriptor" / "instruction
-// descriptor" tables (same fields as cute::UMMA::SmemDescriptor / InstrDescriptor).
+// Minimal sm_100a tcgen05 / TMEM / mbarrier / TMA wrappers (inline PTX) shared by every tensor-core kernel of the
+// library (conv_tc.cu, conv_wgrad_tc.cu, conv_dil_tc.cu, conv_dil_wgrad_tc.cu, linear_tc.cu) and the probes in tools/.
+// This is the only place that waits on an mbarrier.  Descriptor bit layouts follow the PTX ISA "matrix descriptor" /
+// "instruction descriptor" tables (same fields as cute::UMMA::SmemDescriptor / InstrDescriptor).
 #pragma once
 #include <cuda_bf16.h>
 #include <stdint.h>
@@ -61,6 +62,15 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
     if (++spins > (1u << 22)) __trap();
   }
 }
+// The same bound, backing off between polls: for waiters (epilogue and store warps) that would otherwise take issue
+// slots from the producer / MMA warps sharing their schedulers.
+__device__ __forceinline__ void mbar_wait_sleep(uint64_t* bar, uint32_t parity) {
+  uint32_t spins = 0;
+  while (!mbar_try_wait(bar, parity)) {
+    __nanosleep(64);
+    if (++spins > (1u << 22)) __trap();
+  }
+}
 
 // ---------------------------------------------------------------- proxies / fences --------
 // generic-proxy smem writes (st.shared, cp.async) -> visible to the async proxy (UMMA, TMA)
@@ -83,6 +93,13 @@ __device__ __forceinline__ void tmem_alloc(uint32_t* dst, uint32_t ncols) {
 }
 __device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {
   asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
+}
+// whole CTA, after one warp's tmem_alloc(slot, ...): returns the allocated base to every thread
+__device__ __forceinline__ uint32_t tmem_publish(uint32_t* slot) {
+  tc_fence_before_sync();
+  __syncthreads();
+  tc_fence_after_sync();
+  return __shfl_sync(0xffffffffu, *slot, 0);
 }
 
 // 32 lanes x 32 columns of fp32: thread i of the warp gets lane (base_lane + i), columns c..c+31
@@ -166,16 +183,6 @@ __device__ __forceinline__ void mma_bf16_lohi(uint32_t tmem_d, uint32_t a_lo, ui
       ::"r"(tmem_d), "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(accumulate)
       : "memory");
 }
-// kind::tf32: fp32 operands in smem read as tf32
-__device__ __forceinline__ void mma_tf32(uint32_t tmem_d, uint64_t a_desc, uint64_t b_desc, uint32_t idesc,
-                                         uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
 // arrive on an mbarrier when all tcgen05.mma issued so far by this thread have completed
 __device__ __forceinline__ void mma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
@@ -193,22 +200,6 @@ __device__ __forceinline__ void stg256(void* p, const uint32_t* v) {
   asm volatile("st.global.v8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"l"(p), "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]),
                "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7])
                : "memory");
-}
-
-// ---------------------------------------------------------------- cp.async ----------------
-// 16-byte global -> shared copy; src_bytes = 0 zero-fills (used for the conv padding)
-__device__ __forceinline__ void cp_async16(uint32_t dst_smem, const void* src, uint32_t src_bytes) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst_smem), "l"(src), "r"(src_bytes) : "memory");
-}
-// the mbarrier receives one arrival from this thread once all of its earlier cp.async have landed
-// (".noinc": the barrier's expected count must already include this thread)
-__device__ __forceinline__ void cp_async_mbar_arrive_noinc(uint64_t* bar) {
-  asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() {
-  asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory");
 }
 
 }  // namespace umma

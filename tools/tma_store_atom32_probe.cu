@@ -60,8 +60,8 @@ int main() {
     cudaMemset(bad, 0, 4);
     CUtensorMap tin, tout;
     char msg[256];
-    if (dd::tma_map_2d_checked(&tin, in, 4, R, C, C, 32, 32, true, msg, sizeof msg) ||
-        dd::tma_map_2d_checked(&tout, out, 4, R, C, C, 32, 32, true, msg, sizeof msg)) {
+    if (dd::tma_map_2d(&tin, in, 4, R, C, C, 32, 32, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, msg, sizeof msg) ||
+        dd::tma_map_2d(&tout, out, 4, R, C, C, 32, 32, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, msg, sizeof msg)) {
       printf("encode failed: %s\n", msg);
       return 1;
     }

@@ -82,9 +82,12 @@ static int run(const char* name, const std::vector<float>& A, int a_rows, int a_
   cudaMemcpy(dB, B.data(), B.size() * 4, cudaMemcpyHostToDevice);
   cudaMemset(dD, 0xff, 128 * 256 * 4);
   CUtensorMap ta, tb;
-  if (dd::tma_map_2d(&ta, dA, 4, a_rows, a_cols, a_cols, 32, a_box_rows, p.a_base32) ||
-      dd::tma_map_2d(&tb, dB, 4, b_rows, b_cols, b_cols, 32, b_box_rows, p.b_base32)) {
-    printf("%-52s tensor map encode failed\n", name);
+  char msg[256];
+  const CUtensorMapSwizzle a_sw = p.a_base32 ? CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B : CU_TENSOR_MAP_SWIZZLE_128B;
+  const CUtensorMapSwizzle b_sw = p.b_base32 ? CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B : CU_TENSOR_MAP_SWIZZLE_128B;
+  if (dd::tma_map_2d(&ta, dA, 4, a_rows, a_cols, a_cols, 32, a_box_rows, a_sw, msg, sizeof msg) ||
+      dd::tma_map_2d(&tb, dB, 4, b_rows, b_cols, b_cols, 32, b_box_rows, b_sw, msg, sizeof msg)) {
+    printf("%-52s %s\n", name, msg);
     return 1;
   }
   p.a_box_bytes = a_box_rows * 128; p.b_box_bytes = b_box_rows * 128;
