@@ -64,6 +64,7 @@ SIGNATURES = {
     "dd_bce_prob_bwd": (_I, [_P, _P, _P, _P, _L, _P]),
     "dd_bce_prob_workspace_bytes": (_Z, []),
     "dd_ats_bounding_boxes": (_I, [_P, _I, _P, _I, _P, _P, _P]),
+    "dd_boxes_to_map": (_I, [_P, _I, _P, _I, _P, _P]),
     "dd_mse_fwd": (_I, [_P, _P, _P, _P, _Z, _L, _P]),
     "dd_mse_bwd": (_I, [_P, _P, _P, _P, _L, _P]),
     "dd_adam_step": (_I, [_P, _P, _P, _P, _L, _F, _F, _F, _F, _F, _L, _F, _P]),

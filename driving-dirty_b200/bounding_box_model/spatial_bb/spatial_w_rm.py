@@ -12,7 +12,6 @@ from ... import ops
 from ...autoencoder.autoencoder import BasicAE
 from ...autoencoder.components import resolve_dtype
 from ...lightning_compat import LightningModule
-from ...utils.bb_to_img import boxes_to_binary_map
 from .components import RoadMapBoxesMergingCNN, SpatialMappingCNN
 
 random.seed(20200505)
@@ -54,13 +53,14 @@ class BBSpatialRoadMap(LightningModule):
         return yhat.float().reshape(yhat.shape[0], yhat.shape[1], yhat.shape[2])
 
     def bb_coord_to_map(self, target):
-        """tuple of B dicts with 'bounding_box' [N,2,4] -> [B,800,800] raster (:85-95, host side)."""
-        return torch.from_numpy(np.stack([boxes_to_binary_map(s["bounding_box"]).copy() for s in target]))
+        """tuple of B dicts with 'bounding_box' [N,2,4] -> [B,800,800] raster (:85-95) on the model's device: the
+        reference's boxes_to_binary_map per scene, bit for bit, rasterised by the device kernel (ops.boxes_to_map)."""
+        return ops.boxes_to_map([s["bounding_box"] for s in target], next(self.parameters()).device)
 
     def _run_step(self, batch, batch_idx, step_name):
         sample, target, road_image = batch
         sample = ops.as_view_batch(sample)
-        # `target`: the dataloader's tuple of dicts (rasterised here on the host like the reference, :85-95), or -- an
+        # `target`: the dataloader's tuple of dicts (rasterised here, on the device, :85-95), or -- an
         # extension for loaders that rasterise ahead of time -- the [B,800,800] raster itself
         target_bb_img = (target if torch.is_tensor(target) else self.bb_coord_to_map(target)).to(device=sample.device,
                                                                                               dtype=torch.float32)

@@ -7,6 +7,8 @@
 // convex hull of 4 points (monotone chain), Sutherland-Hodgman clipping of one hull by the other, shoelace areas, all in
 // float64 like shapely; the union is area1 + area2 - intersection.  The final score repeats the reference's float32
 // arithmetic step by step (tensor ops on a 0-dim float32 tensor).  One CTA: box counts are tens, not thousands.
+// Also the training target's rasteriser, box_raster_kernel (below).
+#include "box_raster.cuh"
 #include "dd_common.cuh"
 
 namespace {
@@ -126,4 +128,88 @@ extern "C" int dd_ats_bounding_boxes(const float* boxes1, int n1, const float* b
              "dd_ats_bounding_boxes: box counts %d x %d", n1, n2);
   ats_kernel<<<1, 256, (size_t)n2 * sizeof(unsigned int), dd::as_stream(stream)>>>(boxes1, n1, boxes2, n2, iou_matrix, ats);
   return dd::check_launch("ats_bounding_boxes");
+}
+
+// ---- box rasteriser: boxes_to_binary_map (src/utils/bb_to_img.py:5-21) for a batch of scenes -------------------------
+// One CTA per (scene, band of kBand image rows).  The CTA converts its scene's boxes (in chunks of kChunk) to Pillow's
+// integer corners and edge records in shared memory, ORs every (box, row) span into a bit row per image row (a union of
+// ones: the result does not depend on the order), then writes the band's rows at their flipped positions as 16-byte
+// stores of 0. / 1.  The corner arithmetic is the reference's own: metre * 10 + 400 in the boxes' dtype, each
+// operation rounded separately (no FMA), truncated to int like Pillow.
+namespace {
+
+constexpr int kBand = 16;                            // image rows per CTA
+constexpr int kChunk = 128;                          // boxes per shared-memory chunk
+constexpr int kWords = box_raster::kMap / 32;        // 25 words of bits per row
+constexpr int kRasterThreads = 256;
+
+template <typename T>
+__device__ __forceinline__ int to_pixel(T metre);
+template <>
+__device__ __forceinline__ int to_pixel<float>(float m) { return __float2int_rz(__fadd_rn(__fmul_rn(m, 10.f), 400.f)); }
+template <>
+__device__ __forceinline__ int to_pixel<double>(double m) { return __double2int_rz(__dadd_rn(__dmul_rn(m, 10.0), 400.0)); }
+
+template <typename T>
+__global__ void __launch_bounds__(kRasterThreads) box_raster_kernel(const T* __restrict__ boxes, const int* __restrict__ offsets,
+                                                                    float* __restrict__ out) {
+  using namespace box_raster;
+  __shared__ Poly s_poly[kChunk];
+  __shared__ unsigned int s_bits[kBand][kWords];
+  __shared__ float s_xx[kMaxCross][kRasterThreads];
+  constexpr int kBands = kMap / kBand;
+  const int scene = blockIdx.x / kBands, y0 = (blockIdx.x % kBands) * kBand;
+  for (int i = threadIdx.x; i < kBand * kWords; i += blockDim.x) (&s_bits[0][0])[i] = 0u;
+  const int begin = offsets[scene], end = offsets[scene + 1];
+  for (int c = begin; c < end; c += kChunk) {
+    const int n = min(kChunk, end - c);
+    __syncthreads();                                   // the previous chunk's rows are done (and the bits are zeroed)
+    if (threadIdx.x < n) {
+      const T* b = boxes + (size_t)(c + threadIdx.x) * 8;   // [2][4]: x row, y row; columns fl, fr, bl, br
+      int x[4], y[4];
+      const int col[4] = {0, 1, 3, 2};                 // drawn as fl, fr, br, bl
+#pragma unroll
+      for (int k = 0; k < 4; ++k) { x[k] = to_pixel<T>(b[col[k]]); y[k] = to_pixel<T>(b[4 + col[k]]); }
+      build(s_poly[threadIdx.x], x, y);
+    }
+    __syncthreads();
+    for (int p = threadIdx.x; p < n * kBand; p += blockDim.x) {
+      const int r = p / n, box = p - r * n;
+      row_spans(s_poly[box], y0 + r, &s_xx[0][threadIdx.x], kRasterThreads, [&](int a, int e) {
+        for (int w = a >> 5; w <= (e >> 5); ++w) {
+          const int lo = max(a - w * 32, 0), hi = min(e - w * 32, 31);
+          const unsigned int m = (hi == 31 ? ~0u : ((1u << (hi + 1)) - 1u)) & (~0u << lo);
+          atomicOr(&s_bits[r][w], m);
+        }
+      });
+    }
+  }
+  __syncthreads();
+  float* dst = out + (size_t)scene * kMap * kMap;
+  for (int i = threadIdx.x; i < kBand * (kMap / 4); i += blockDim.x) {
+    const int r = i / (kMap / 4), q = i - r * (kMap / 4);
+    const unsigned int bits = s_bits[r][q >> 3] >> ((q & 7) * 4);
+    const float4 v = make_float4((float)(bits & 1u), (float)((bits >> 1) & 1u), (float)((bits >> 2) & 1u),
+                                 (float)((bits >> 3) & 1u));
+    reinterpret_cast<float4*>(dst + (size_t)(kMap - 1 - (y0 + r)) * kMap)[q] = v;   // image row y -> output row 799 - y
+  }
+}
+
+}  // namespace
+
+extern "C" int dd_boxes_to_map(const void* boxes, int boxes_f64, const int* offsets, int B, float* out, void* stream) {
+  DD_REQUIRE(B >= 0, DD_ERR_BAD_ARG, "dd_boxes_to_map: B = %d < 0", B);
+  if (B == 0) return DD_OK;
+  DD_REQUIRE(boxes && offsets && out, DD_ERR_BAD_ARG, "dd_boxes_to_map: null pointer (boxes %p, offsets %p, out %p)", boxes,
+             (const void*)offsets, (void*)out);
+  DD_REQUIRE(((uintptr_t)out & 15) == 0, DD_ERR_ALIGNMENT, "dd_boxes_to_map: out must be 16-byte aligned");
+  const long long grid = (long long)B * (box_raster::kMap / kBand);
+  DD_REQUIRE(grid <= 0x7fffffffLL, DD_ERR_BAD_ARG, "dd_boxes_to_map: B = %d is too large", B);
+  if (boxes_f64)
+    box_raster_kernel<double><<<(unsigned)grid, kRasterThreads, 0, dd::as_stream(stream)>>>(
+        static_cast<const double*>(boxes), offsets, out);
+  else
+    box_raster_kernel<float><<<(unsigned)grid, kRasterThreads, 0, dd::as_stream(stream)>>>(
+        static_cast<const float*>(boxes), offsets, out);
+  return dd::check_launch("boxes_to_map");
 }

@@ -701,3 +701,95 @@ class BceProb(torch.autograd.Function):
 
 def bce_prob(pred, target):
     return BceProb.apply(pred, target)
+
+
+# --------------------------------------------------------------------------------------------
+# training target of the box model: boxes_to_binary_map (utils/bb_to_img.py:5-21) on the device
+MAP_SIZE = 800
+
+
+class _BoxStaging:
+    """Per-device ring of two staging slots for ``boxes_to_map``'s inputs (offsets, then boxes), so host boxes cross in
+    one asynchronous copy.  A slot is (pinned host buffer, device buffer, event); the event is recorded after the kernel
+    that reads the slot's device buffer.  Before a slot is reused, waiting on its event guarantees that the copy out of
+    the pinned buffer and the kernel reading the device buffer have both finished, whichever stream they ran on.  With
+    two slots the host waits for the call before last, not the last one, so it can run a step ahead of the device.
+    Buffers grow to the next power of two, so slowly growing batches do not re-pin memory on every call."""
+
+    SLOTS = 2
+
+    def __init__(self):
+        self._rings = {}
+
+    def get(self, nbytes: int, device):
+        ring = self._rings.setdefault(device.index, {"next": 0, "slots": [None] * self.SLOTS})
+        i = ring["next"]
+        ring["next"] = (i + 1) % self.SLOTS
+        slot = ring["slots"][i]
+        if slot is None or slot[0].numel() < nbytes:
+            if slot is not None:
+                slot[2].synchronize()                        # the old buffers' last copy and reader have finished
+            n = 1 << max(12, (nbytes - 1).bit_length())
+            slot = (torch.empty(n, dtype=torch.uint8).pin_memory(), torch.empty(n, dtype=torch.uint8, device=device),
+                    torch.cuda.Event())
+            ring["slots"][i] = slot
+        return slot
+
+
+_box_staging = _BoxStaging()
+
+
+def boxes_to_map(boxes: Sequence[torch.Tensor], device) -> torch.Tensor:
+    """The dataloader's per-scene boxes ([N,2,4]: metres; rows x / y; columns fl, fr, bl, br; N may be 0), all float32 or
+    all float64, on the host or on ``device`` -> float32 [B,800,800] of 0./1. on ``device``: exactly
+    ``boxes_to_binary_map`` of each scene (the reference's Pillow fill, arithmetic in the boxes' own dtype).
+    Host boxes travel with their offsets through reused pinned buffers (_BoxStaging) in one asynchronous copy."""
+    device = torch.device(device)
+    if device.type != "cuda":
+        raise RuntimeError("boxes_to_map runs on CUDA (sm_100a) only; there is no CPU fallback on this path.")
+    if device.index is None:
+        device = torch.device("cuda", torch.cuda.current_device())
+    boxes = list(boxes)
+    dtypes = set()
+    for b in boxes:
+        if not torch.is_tensor(b) or b.dim() != 3 or tuple(b.shape[1:]) != (2, 4):
+            raise ValueError(f"boxes_to_map: every scene's boxes must have shape [N,2,4], got "
+                             f"{tuple(b.shape) if torch.is_tensor(b) else type(b).__name__}")
+        if b.dtype not in (torch.float32, torch.float64):
+            raise ValueError(f"boxes_to_map: boxes dtype must be float32 or float64, got {b.dtype}")
+        dtypes.add(b.dtype)
+    if len(dtypes) > 1:
+        raise ValueError("boxes_to_map: the batch mixes float32 and float64 boxes (dtype); the fill's arithmetic "
+                         "differs per dtype, so convert them explicitly")
+    B = len(boxes)
+    out = torch.empty(B, MAP_SIZE, MAP_SIZE, dtype=torch.float32, device=device)
+    if B == 0:
+        return out
+    dtype = dtypes.pop()
+    counts = [int(b.shape[0]) for b in boxes]
+    offsets = [0]
+    for c in counts:
+        offsets.append(offsets[-1] + c)
+    total = offsets[-1]
+    on_device = all(b.is_cuda and b.device == device for b in boxes)
+    box_at = (4 * (B + 1) + 15) // 16 * 16
+    nbytes = box_at + (0 if on_device else total * 8 * dtype.itemsize)
+    with torch.cuda.device(device):
+        host, dev, done = _box_staging.get(nbytes, device)
+        done.synchronize()                                   # this slot's last copy and kernel have finished
+        host[:4 * (B + 1)].view(torch.int32).copy_(torch.tensor(offsets, dtype=torch.int32))
+        if not on_device and total:
+            torch.cat([b.detach().reshape(-1, 8).cpu() for b in boxes],
+                      out=host[box_at:nbytes].view(dtype).view(total, 8))
+        cur = torch.cuda.current_stream(device)
+        dev[:nbytes].copy_(host[:nbytes], non_blocking=True)
+        if on_device and total:
+            src = _c(torch.cat([b.detach().reshape(-1, 8) for b in boxes]))
+        else:
+            src = dev[box_at:]
+        call("dd_boxes_to_map", src.data_ptr(), int(dtype == torch.float64), dev.data_ptr(), B, out.data_ptr(),
+             cur.cuda_stream)
+        done.record(cur)
+        if on_device and total:
+            src.record_stream(cur)
+    return out

@@ -208,6 +208,16 @@ int dd_bce_prob_bwd(const float* probs, const float* target, const float* grad_o
                     long long n, void* stream);
 size_t dd_bce_prob_workspace_bytes(void);
 
+/* dd_boxes_to_map: the training target of the box model, boxes_to_binary_map (utils/bb_to_img.py:5-21) per scene as
+ * BBSpatialRoadMap.bb_coord_to_map uses it (spatial_w_rm.py:85-95), bit for bit with the reference's Pillow fill.
+ *   boxes: [total,2,4] on the device (metres; rows x / y; columns fl, fr, bl, br), float32 (boxes_f64 = 0) or float64 (1);
+ *   pixel = metre * 10 + 400 in that dtype, polygon fl, fr, br, bl, filled as ImageDraw.polygon(fill=1) does.
+ *   offsets: int32 [B+1] on the device, scene b owns boxes [offsets[b], offsets[b+1]).
+ *   out: f32 [B,800,800] of 0./1., vertically flipped like the reference; every element is written.
+ * B < 0 or a null pointer with B > 0: DD_ERR_BAD_ARG.  B == 0 enqueues nothing.  out not 16-byte aligned:
+ * DD_ERR_ALIGNMENT. */
+int dd_boxes_to_map(const void* boxes, int boxes_f64, const int* offsets, int B, float* out, void* stream);
+
 /* ---- 8(f)3: bounding-box evaluation ------------------------------------------------------------------
  * compute_ats_bounding_boxes (helper.py:33-72, with compute_iou :79-83): boxes1 [n1,2,4], boxes2 [n2,2,4] fp32
  * (metres; rows x / y; columns fl, fr, bl, br) -> ats f32[1], the IoU-thresholded average threat score.
