@@ -30,10 +30,13 @@ SIGNATURES = {
     "dd_stitch_u8": (_I, [_P, _P, _I, _I, _I, _P]),
     "dd_u8_to_f32": (_I, [_P, _P, _L, _P]),
     "dd_conv_c1_fwd": (_I, [_P, _I, _P, _P, _P, _I, _I, _I, _I, _I, _P]),
+    "dd_conv_c1_fwd_bits": (_I, [_P, _I, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P]),
     "dd_encoder_c1c2_fused_fwd": (_I, [_P, _I, _P, _P, _P, _P, _P, _I, _I, _I, _P]),
     "dd_conv_c1_wgrad": (_I, [_P, _I, _P, _I, _P, _P, _P, _Z, _I, _I, _I, _I, _P]),
     "dd_conv3x3_c32_fwd": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _P]),
     "dd_conv3x3_c32_dgrad": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _P]),
+    "dd_conv3x3_c32_fwd_bits": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _P]),
+    "dd_conv3x3_c32_dgrad_bits": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _P]),
     "dd_conv3x3_c32_wgrad": (_I, [_P, _P, _P, _P, _P, _Z, _I, _I, _I, _I, _I, _I, _P]),
     "dd_conv_wgrad_workspace_bytes": (_Z, []),
     "dd_pool4_fwd": (_I, [_P, _P, _I, _I, _I, _I, _P]),

@@ -504,12 +504,12 @@ int conv_wgrad_simt(const T* x, const T* dy, float* dw, float* db, float* ws, in
 // tcgen05 implementations live in conv_tc.cu
 namespace dd {
 int conv3x3_c32_fwd_tc(const void* in, const float* w, const float* bias, void* out, int B, int H, int W,
-                       int stride, int mode, const void* mask, cudaStream_t st);
+                       int stride, int mode, const void* mask, uint32_t* bits, cudaStream_t st);
 int conv3x3_c32_wgrad_tc(const void* x, const void* dy, float* dw, float* db, void* ws, size_t ws_bytes, int B,
                          int H, int W, int stride, cudaStream_t st);
 bool conv_tc_supported(int H, int W, int stride, int mode);
-int conv_c1_fwd_tc(const void* in, int in_flags, const float* w, const float* bias, void* out, int B, int H, int Wm,
-                   cudaStream_t st);
+int conv_c1_fwd_tc(const void* in, int in_flags, const float* w, const float* bias, void* out, uint32_t* bits, int B, int H,
+                   int Wm, cudaStream_t st);
 int enc_c1c2_fused_fwd_tc(const void* in, int in_flags, const float* w1, const float* b1, const float* w2, const float* b2,
                           void* out, int B, int H, int Wm, cudaStream_t st);
 int conv_c1_wgrad_tc(const void* in, int in_flags, const void* dy, float* dw, float* db, void* ws, size_t ws_bytes,
@@ -528,7 +528,7 @@ extern "C" int dd_conv3x3_c32_fwd(const void* in, const float* w_oihw, const flo
   cudaStream_t st = dd::as_stream(stream);
   if (dtype == DD_BF16 && impl != DD_IMPL_SIMT) {
     if (dd::conv_tc_supported(H, W, stride, 0))
-      return dd::conv3x3_c32_fwd_tc(in, w_oihw, bias, out, B, H, W, stride, 0, nullptr, st);
+      return dd::conv3x3_c32_fwd_tc(in, w_oihw, bias, out, B, H, W, stride, 0, nullptr, nullptr, st);
     DD_REQUIRE(impl != DD_IMPL_TCGEN05, DD_ERR_UNSUPPORTED, "dd_conv3x3_c32_fwd: tcgen05 path unsupported for H=%d W=%d stride=%d", H, W, stride);
   }
   DD_REQUIRE(!(dtype == DD_F32 && impl == DD_IMPL_TCGEN05), DD_ERR_UNSUPPORTED, "tcgen05 conv is bf16 only");
@@ -547,7 +547,7 @@ extern "C" int dd_conv3x3_c32_dgrad(const void* dy, const float* w_oihw, const v
   cudaStream_t st = dd::as_stream(stream);
   if (dtype == DD_BF16 && impl != DD_IMPL_SIMT) {
     if (dd::conv_tc_supported(H, W, stride, 1))
-      return dd::conv3x3_c32_fwd_tc(dy, w_oihw, nullptr, dx, B, H, W, stride, 1, x, st);
+      return dd::conv3x3_c32_fwd_tc(dy, w_oihw, nullptr, dx, B, H, W, stride, 1, x, nullptr, st);
     DD_REQUIRE(impl != DD_IMPL_TCGEN05, DD_ERR_UNSUPPORTED, "dd_conv3x3_c32_dgrad: tcgen05 path unsupported here");
   }
   DD_REQUIRE(!(dtype == DD_F32 && impl == DD_IMPL_TCGEN05), DD_ERR_UNSUPPORTED, "tcgen05 conv is bf16 only");
@@ -557,6 +557,32 @@ extern "C" int dd_conv3x3_c32_dgrad(const void* dy, const float* w_oihw, const v
     return conv_dgrad_simt<__nv_bfloat16>((const __nv_bfloat16*)dy, w_oihw, (const __nv_bfloat16*)x,
                                           (__nv_bfloat16*)dx, B, H, W, stride, st);
   return dd::fail(DD_ERR_UNSUPPORTED, "dd_conv3x3_c32_dgrad: dtype %d", dtype);
+}
+
+// the ReLU sign-word forms (conv_tc.cu, relu_bits): bf16 tensor-core kernels only; every check runs before the launch
+extern "C" int dd_conv3x3_c32_fwd_bits(const void* in, const float* w_oihw, const float* bias, void* out, uint32_t* bits,
+                                       int dtype, int B, int H, int W, int stride, int impl, void* stream) {
+  DD_REQUIRE(in && w_oihw && bias && out && bits, DD_ERR_BAD_ARG, "dd_conv3x3_c32_fwd_bits: null pointer");
+  DD_REQUIRE(B >= 0 && H > 0 && W > 0, DD_ERR_BAD_ARG, "dd_conv3x3_c32_fwd_bits: bad shape");
+  DD_REQUIRE(stride == 1, DD_ERR_UNSUPPORTED, "dd_conv3x3_c32_fwd_bits: stride %d (sign words are kept for stride 1 only)", stride);
+  DD_REQUIRE(dtype == DD_BF16 && impl != DD_IMPL_SIMT && dd::conv_tc_supported(H, W, stride, 0), DD_ERR_UNSUPPORTED,
+             "dd_conv3x3_c32_fwd_bits: sign words come from the bf16 tensor-core kernel only (dtype %d, impl %d, H=%d W=%d)",
+             dtype, impl, H, W);
+  if (B == 0) return 0;
+  return dd::conv3x3_c32_fwd_tc(in, w_oihw, bias, out, B, H, W, stride, 0, nullptr, bits, dd::as_stream(stream));
+}
+
+extern "C" int dd_conv3x3_c32_dgrad_bits(const void* dy, const float* w_oihw, const uint32_t* x_bits, void* dx, int dtype,
+                                         int B, int H, int W, int stride, int impl, void* stream) {
+  DD_REQUIRE(dy && w_oihw && x_bits && dx, DD_ERR_BAD_ARG, "dd_conv3x3_c32_dgrad_bits: null pointer");
+  DD_REQUIRE(B >= 0 && H > 0 && W > 0, DD_ERR_BAD_ARG, "dd_conv3x3_c32_dgrad_bits: bad shape");
+  DD_REQUIRE(stride == 1 || stride == 2, DD_ERR_UNSUPPORTED, "dd_conv3x3_c32_dgrad_bits: stride %d", stride);
+  DD_REQUIRE(dtype == DD_BF16 && impl != DD_IMPL_SIMT && dd::conv_tc_supported(H, W, stride, 1), DD_ERR_UNSUPPORTED,
+             "dd_conv3x3_c32_dgrad_bits: sign words are read by the bf16 tensor-core kernels only (dtype %d, impl %d, H=%d W=%d)",
+             dtype, impl, H, W);
+  if (B == 0) return 0;
+  return dd::conv3x3_c32_fwd_tc(dy, w_oihw, nullptr, dx, B, H, W, stride, 1, nullptr, const_cast<uint32_t*>(x_bits),
+                                dd::as_stream(stream));
 }
 
 extern "C" int dd_conv3x3_c32_wgrad(const void* x, const void* dy, float* dw, float* db, void* workspace,
@@ -602,7 +628,7 @@ extern "C" int dd_conv_c1_fwd(const void* in_, int in_flags, const float* w_oihw
   if (B == 0) return 0;
   cudaStream_t st = dd::as_stream(stream);
   DD_REQUIRE(!(out_dtype == DD_F32 && impl == DD_IMPL_TCGEN05), DD_ERR_UNSUPPORTED, "tcgen05 conv is bf16 only");
-  if (out_dtype == DD_BF16 && impl != DD_IMPL_SIMT) return dd::conv_c1_fwd_tc(in_, in_flags, w_oihw, bias, out, B, H, Wm, st);
+  if (out_dtype == DD_BF16 && impl != DD_IMPL_SIMT) return dd::conv_c1_fwd_tc(in_, in_flags, w_oihw, bias, out, nullptr, B, H, Wm, st);
   DD_REQUIRE(!(in_flags & DD_IN_U8), DD_ERR_UNSUPPORTED, "dd_conv_c1_fwd: raw-byte input runs on the bf16 tensor-core path only "
              "(fp32 parity path: dd_stitch_u8 first)");
   const float* in = (const float*)in_;
@@ -617,6 +643,18 @@ extern "C" int dd_conv_c1_fwd(const void* in_, int in_flags, const float* w_oihw
     return dd::fail(DD_ERR_UNSUPPORTED, "dd_conv_c1_fwd: dtype %d", out_dtype);
   }
   return dd::check_launch("conv_c1_fwd");
+}
+
+extern "C" int dd_conv_c1_fwd_bits(const void* in_, int in_flags, const float* w_oihw, const float* bias, void* out,
+                                   uint32_t* bits, int out_dtype, int B, int H, int Wm, int impl, void* stream) {
+  DD_REQUIRE(in_ && w_oihw && bias && out && bits, DD_ERR_BAD_ARG, "dd_conv_c1_fwd_bits: null pointer");
+  DD_REQUIRE(B >= 0 && H > 0 && Wm > 0, DD_ERR_BAD_ARG, "dd_conv_c1_fwd_bits: bad shape");
+  DD_REQUIRE((in_flags & ~3) == 0, DD_ERR_BAD_ARG, "dd_conv_c1_fwd_bits: in_flags %d", in_flags);
+  DD_REQUIRE(!(in_flags & DD_IN_VIEWS) || Wm % 6 == 0, DD_ERR_BAD_ARG, "dd_conv_c1_fwd_bits: mosaic width %d not a multiple of 6", Wm);
+  DD_REQUIRE(out_dtype == DD_BF16 && impl != DD_IMPL_SIMT, DD_ERR_UNSUPPORTED,
+             "dd_conv_c1_fwd_bits: sign words come from the bf16 tensor-core kernel only (dtype %d, impl %d)", out_dtype, impl);
+  if (B == 0) return 0;
+  return dd::conv_c1_fwd_tc(in_, in_flags, w_oihw, bias, out, bits, B, H, Wm, dd::as_stream(stream));
 }
 
 extern "C" int dd_conv_c1_wgrad(const void* in_, int in_flags, const void* dy, int dtype, float* dw, float* db,

@@ -39,9 +39,47 @@ constexpr int NPROD = 4;             // producer warps (0..3); warp 4 issues MMA
 constexpr int MMA_WARP = NPROD;
 constexpr int NTHREADS = 32 * (NPROD + 1 + 4);
 
+// ReLU sign words: the ReLU mask of a1 / a2 as the c2 / c3 input gradients need it, 4 bytes per pixel instead of the
+// 64-byte activation.  One uint32 per pixel, NHWC pixel order [B][H][W]; bit c is 1 exactly when the STORED bf16
+// activation of channel c is > 0 -- the comparison the input-gradient epilogues apply to the activation itself, so a
+// positive fp32 value that rounds to bf16 zero and a -0 both give 0, and either form of the mask yields the same bits.
+// Written by the c1 and stride-1 forward epilogues beside the activation (thread = pixel: a warp stores 128 contiguous
+// bytes), read by the stride-1 and stride-2 input-gradient epilogues.
+// (c1's four epilogue warps are one per scheduler, so every instruction and dependent step here is time of that kernel:
+// one masked OR per half, in four independent chains, instead of shifting each bit into place)
+__device__ __forceinline__ uint32_t relu_bits(const uint32_t (&pk)[16]) {
+  const __nv_bfloat162 zero = __floats2bfloat162_rn(0.f, 0.f);
+  uint32_t a[2] = {0u, 0u}, r[2] = {0u, 0u};
+#pragma unroll
+  for (int k = 0; k < 16; ++k) {
+    // m: 0xffff in the half of each channel (2k low, 2k+1 high) that is > 0.  Of bits 2k and 2k+1 one lies in its own
+    // channel's half and is taken in place (a); the other is taken 16 places away (r), and r is rotated by 16 at the end
+    const uint32_t m = __hgt2_mask(*reinterpret_cast<const __nv_bfloat162*>(&pk[k]), zero);
+    if (k < 8) { a[k & 1] |= m & (1u << (2 * k)); r[k & 1] |= m & (1u << (2 * k + 17)); }
+    else { a[k & 1] |= m & (1u << (2 * k + 1)); r[k & 1] |= m & (1u << (2 * k - 16)); }
+  }
+  const uint32_t rr = r[0] | r[1];
+  return a[0] | a[1] | __funnelshift_l(rr, rr, 16);
+}
+
+// Sign word -> masks of channel pairs (0xffff per half whose bit is set, as __hgt2_mask gives).  r[s] = bits << s puts
+// channel c at the top bit of byte c / 8 of r[7 - c % 8]; a byte permute with sign replication (prmt selector bit 3)
+// spreads that bit over two bytes, so a pair costs one prmt.
+__device__ __forceinline__ void relu_mask_prep(uint32_t bits, uint32_t (&r)[8]) {
+#pragma unroll
+  for (int s = 0; s < 8; ++s) r[s] = bits << s;
+}
+__device__ __forceinline__ uint32_t relu_mask2(const uint32_t (&r)[8], int k) {
+  const int j = k >> 2, sa = 7 - ((2 * k) & 7);           // channel 2k: top of byte j of r[sa]; 2k+1: of r[sa - 1]
+  const uint32_t sel = (8u | j) * 0x11u | ((8u | (4 + j)) * 0x11u) << 8;
+  uint32_t m;
+  asm("prmt.b32 %0, %1, %2, %3;" : "=r"(m) : "r"(r[sa]), "r"(r[sa - 1]), "r"(sel));
+  return m;
+}
+
 // one pixel's 32 channels (fp32 in registers) -> bf16 -> two 32-byte stores (64-byte aligned destination): whole sectors
-// per lane instead of four half-sector 16-byte stores
-__device__ __forceinline__ void store_pixel32(__nv_bfloat16* dst, const float (&v)[C]) {
+// per lane instead of four half-sector 16-byte stores.  Returns the stored pixel's sign word (compiled away where unused).
+__device__ __forceinline__ uint32_t store_pixel32(__nv_bfloat16* dst, const float (&v)[C]) {
   uint32_t pk[16];
 #pragma unroll
   for (int k = 0; k < 16; ++k) {
@@ -50,6 +88,7 @@ __device__ __forceinline__ void store_pixel32(__nv_bfloat16* dst, const float (&
   }
   umma::stg256(dst, pk);
   umma::stg256(dst + 16, pk + 8);
+  return relu_bits(pk);
 }
 
 struct Bars {
@@ -266,13 +305,15 @@ struct S1Bars {
   uint32_t tmem_base;
 };
 
-template <int MODE>
+// BITS: MODE 0 also writes the output's ReLU sign words to `bits`; MODE 1 takes the ReLU mask from the sign words in `bits`
+// instead of the activation `mask`
+template <int MODE, bool BITS>
 __global__ void __launch_bounds__(S1_THREADS, 1) conv3x3_c32_s1_tc_kernel(const __grid_constant__ CUtensorMap map_in,
                                                                            const float* __restrict__ w_oihw,
                                                                            const float* __restrict__ bias,
                                                                            const __nv_bfloat16* __restrict__ mask,
                                                                            __nv_bfloat16* __restrict__ out, int B, int H,
-                                                                           int W) {
+                                                                           int W, uint32_t* __restrict__ bits) {
   extern __shared__ __align__(1024) uint8_t smem[];
   uint8_t* s_w = smem;
   uint8_t* s_slab = smem + W_BYTES;
@@ -448,13 +489,19 @@ __global__ void __launch_bounds__(S1_THREADS, 1) conv3x3_c32_s1_tc_kernel(const 
       const int rows = min(S1_ROWS, H - h0);
       const int wo = wt * TILE_M + quarter * 32 + lane;
       const bool ok = wo < W;
-      for (int j = (int)((rc0 ^ half) & 1); j < rows; j += 2) {
+      const int j0 = (int)((rc0 ^ half) & 1);
+      // sign words: this warp's next row is loaded while the current one is processed -- one 4-byte load issued just before
+      // the wait for the MMAs leaves its DRAM round trip exposed on every row
+      uint32_t mb_next = 0;
+      if (MODE == 1 && BITS && ok && j0 < rows) mb_next = __ldg(bits + ((size_t)b * H + h0 + j0) * W + wo);
+      for (int j = j0; j < rows; j += 2) {
         const uint32_t rc = rc0 + j;
         const uint32_t buf = rc % S1_NACC;
         const uint32_t grp = rc >> 2;
         const size_t off = (((size_t)b * H + h0 + j) * W + (ok ? wo : 0)) * C;
-        uint32_t mk[16];
-        if (MODE == 1 && mask != nullptr && ok) {      // in flight while this warp waits for the MMAs
+        uint32_t mk[16], mb = mb_next;
+        if (MODE == 1 && BITS && ok && j + 2 < rows) mb_next = __ldg(bits + off / C + 2 * (size_t)W);
+        if (MODE == 1 && !BITS && mask != nullptr && ok) {
           umma::ldg256(mask + off, mk);
           umma::ldg256(mask + off + 16, mk + 8);
         }
@@ -472,20 +519,24 @@ __global__ void __launch_bounds__(S1_THREADS, 1) conv3x3_c32_s1_tc_kernel(const 
         umma::tmem_ld_32x32(tmem + ((uint32_t)(quarter * 32) << 16) + buf * 32, r);
         umma::tmem_ld_wait();
         if (ok) {
-          uint32_t pk[16];
+          uint32_t pk[16], mr[8];
+          if (MODE == 1 && BITS) relu_mask_prep(mb, mr);
 #pragma unroll
           for (int k = 0; k < 16; ++k) {
             float x0 = __uint_as_float(r[2 * k]), x1 = __uint_as_float(r[2 * k + 1]);
             if (MODE == 0) { x0 = fmaxf(x0 + bs[2 * k], 0.f); x1 = fmaxf(x1 + bs[2 * k + 1], 0.f); }
             __nv_bfloat162 h = __floats2bfloat162_rn(x0, x1);
             pk[k] = *reinterpret_cast<uint32_t*>(&h);
-            if (MODE == 1 && mask != nullptr) {
+            if (MODE == 1 && BITS) {
+              pk[k] &= relu_mask2(mr, k);
+            } else if (MODE == 1 && mask != nullptr) {
               const __nv_bfloat162 zero = __floats2bfloat162_rn(0.f, 0.f);
               pk[k] &= __hgt2_mask(*reinterpret_cast<const __nv_bfloat162*>(&mk[k]), zero);
             }
           }
           umma::stg256(out + off, pk);
           umma::stg256(out + off + 16, pk + 8);
+          if (MODE == 0 && BITS) bits[off / C] = relu_bits(pk);
         }
       }
       rc0 += rows;
@@ -497,18 +548,18 @@ __global__ void __launch_bounds__(S1_THREADS, 1) conv3x3_c32_s1_tc_kernel(const 
   if (warp == MMA_WARP) umma::tmem_dealloc(tmem, S1_NACC * 32);
 }
 
-template <int MODE>
+template <int MODE, bool BITS>
 int launch_s1(const void* in, const float* w, const float* bias, const void* mask, void* out, int B, int H, int W,
-              cudaStream_t st) {
+              uint32_t* bits, cudaStream_t st) {
   const int items = B * ((W + TILE_M - 1) / TILE_M) * ((H + S1_ROWS - 1) / S1_ROWS);
-  auto k = conv3x3_c32_s1_tc_kernel<MODE>;
+  auto k = conv3x3_c32_s1_tc_kernel<MODE, BITS>;
   if (int e = dd::set_smem(k, S1_SMEM, dd::Carveout::kMaxShared, "conv_tc s1")) return e;
   const int grid = items < dd::kSMs ? items : dd::kSMs;
   if ((reinterpret_cast<uintptr_t>(in) & 15) != 0) return dd::fail(DD_ERR_ALIGNMENT, "conv_tc s1: input is not 16-byte aligned");
   CUtensorMap map;
   char msg[256];
   if (dd::tma_map_nhwc_sw64(&map, in, B, H, W, C, 130, 1, msg, sizeof msg)) return dd::fail(DD_ERR_UNSUPPORTED, "conv_tc s1: %s", msg);
-  k<<<grid, S1_THREADS, S1_SMEM, st>>>(map, w, bias, (const __nv_bfloat16*)mask, (__nv_bfloat16*)out, B, H, W);
+  k<<<grid, S1_THREADS, S1_SMEM, st>>>(map, w, bias, (const __nv_bfloat16*)mask, (__nv_bfloat16*)out, B, H, W, bits);
   return dd::check_launch("conv3x3_c32_s1_tc");
 }
 
@@ -532,11 +583,14 @@ struct DgBars {
 
 // (96 registers x 416 threads + the optimizer's 96 x 256 update CTA = 64.5 K: both fit one SM's register file, which the
 // overlapped data-parallel update needs -- see csrc/adam.cu)
+// BITS: the ReLU mask comes from the sign words in `bits` (8-byte aligned) instead of the activation `mask`
+template <bool BITS>
 __global__ void __maxnreg__(96) conv3x3_c32_dgrad_s2_tc_kernel(const __grid_constant__ CUtensorMap map_dy,
                                                                                const float* __restrict__ w_oihw,
                                                                                const __nv_bfloat16* __restrict__ mask,
                                                                                __nv_bfloat16* __restrict__ dx, int B,
-                                                                               int H, int W, int Ho, int Wo) {
+                                                                               int H, int W, int Ho, int Wo,
+                                                                               const uint32_t* __restrict__ bits) {
   constexpr int SLAB = 4 * PS;
   extern __shared__ __align__(1024) uint8_t smem[];
   uint8_t* s_w = smem;
@@ -642,7 +696,20 @@ __global__ void __maxnreg__(96) conv3x3_c32_dgrad_s2_tc_kernel(const __grid_cons
       for (int j = 0; j < rows; ++j, ++mctr) {
         const uint32_t set = mctr & 1;
         uint4 mk[2][4];
-        if (mask != nullptr) {
+        uint32_t mb[2];
+        if (BITS) {
+          // this warp's dx row, pixels 2i and 2i+1: one 8-byte load where W is even (the pair is 8-byte aligned), two 4-byte
+          // loads where it is odd; the odd-W edge and out-of-image pixels are clamped as below and never stored
+          const int h = 2 * (m0 + j) + half, w = 2 * i;
+          const size_t p = ((size_t)b * H + (h < H ? h : 0)) * W + (w < W ? w : 0);
+          if ((W & 1) == 0) {
+            const uint2 q = __ldg(reinterpret_cast<const uint2*>(bits + p));
+            mb[0] = q.x; mb[1] = q.y;
+          } else {
+            mb[0] = __ldg(bits + p);
+            mb[1] = __ldg(bits + p + (w + 1 < W ? 1 : 0));
+          }
+        } else if (mask != nullptr) {
 #pragma unroll
           for (int aa = 0; aa < 2; ++aa) {
             const int a = 2 * half + aa;
@@ -671,7 +738,10 @@ __global__ void __maxnreg__(96) conv3x3_c32_dgrad_s2_tc_kernel(const __grid_cons
             float v[C];
 #pragma unroll
             for (int k = 0; k < C; ++k) v[k] = __uint_as_float(r[k]);
-            if (mask) {
+            if (BITS) {
+#pragma unroll
+              for (int k = 0; k < C; ++k) v[k] = (mb[aa] >> k) & 1u ? v[k] : 0.f;
+            } else if (mask) {
 #pragma unroll
               for (int gq = 0; gq < 4; ++gq) {
                 const __nv_bfloat162* h2 = reinterpret_cast<const __nv_bfloat162*>(&mk[aa][gq]);
@@ -769,11 +839,13 @@ __device__ __forceinline__ void c1_load_row(uint8_t* __restrict__ slab, const TI
   }
 }
 
-template <bool IS_VIEWS, typename TIN>
+// BITS: also write the output's ReLU sign words to `bits`
+template <bool IS_VIEWS, typename TIN, bool BITS>
 __global__ void __launch_bounds__(C1_THREADS, 1) conv_c1_tc_kernel(const TIN* __restrict__ in,
                                                                     const float* __restrict__ w_oihw,
                                                                     const float* __restrict__ bias,
-                                                                    __nv_bfloat16* __restrict__ out, int B, int H, int Wm) {
+                                                                    __nv_bfloat16* __restrict__ out, int B, int H, int Wm,
+                                                                    uint32_t* __restrict__ bits) {
   extern __shared__ __align__(1024) uint8_t smem[];
   uint8_t* s_w = smem;
   uint8_t* s_slab = smem + C1_WBYTES;
@@ -879,7 +951,8 @@ __global__ void __launch_bounds__(C1_THREADS, 1) conv_c1_tc_kernel(const TIN* __
           float v[C];
 #pragma unroll
           for (int k = 0; k < C; ++k) v[k] = fmaxf(__uint_as_float(r[k]) + s_bias[k], 0.f);
-          store_pixel32(dst, v);
+          const uint32_t sign = store_pixel32(dst, v);
+          if (BITS) bits[((size_t)b * H + h0 + j) * Wm + wo] = sign;
         }
       }
     }
@@ -1253,44 +1326,58 @@ bool conv_tc_supported(int H, int W, int stride, int mode) {
   return mode >= 0 && mode <= 2 && (stride == 1 || stride == 2);
 }
 
+// bits (may be NULL): the ReLU sign words (see relu_bits), written by mode 0 stride 1, read instead of `mask` by mode 1
 int conv3x3_c32_fwd_tc(const void* in, const float* w, const float* bias, void* out, int B, int H, int W, int stride,
-                       int mode, const void* mask, cudaStream_t st) {
+                       int mode, const void* mask, uint32_t* bits, cudaStream_t st) {
   // the epilogues store (and read the ReLU mask) in 32-byte pieces; the producers read 16-byte pieces
   if (((reinterpret_cast<uintptr_t>(out) | reinterpret_cast<uintptr_t>(mask)) & 31) != 0 || (reinterpret_cast<uintptr_t>(in) & 15) != 0)
     return fail(DD_ERR_ALIGNMENT, "conv_tc: activations must be 32-byte aligned (in %p, out %p, mask %p)", in, out, mask);
-  if (mode == 0 && stride == 1) return launch_s1<0>(in, w, bias, nullptr, out, B, H, W, st);
+  if ((reinterpret_cast<uintptr_t>(bits) & 7) != 0) return fail(DD_ERR_ALIGNMENT, "conv_tc: sign words %p are not 8-byte aligned", bits);
+  if (bits && mode == 0 && stride != 1) return fail(DD_ERR_UNSUPPORTED, "conv_tc: sign words are written by the stride-1 forward only");
+  if (mode == 0 && stride == 1)
+    return bits ? launch_s1<0, true>(in, w, bias, nullptr, out, B, H, W, bits, st) : launch_s1<0, false>(in, w, bias, nullptr, out, B, H, W, nullptr, st);
   if (mode == 0 && stride == 2) return launch_s2_fwd(in, w, bias, out, B, H, W, st);
-  if (mode == 1 && stride == 1) return launch_s1<1>(in, w, nullptr, mask, out, B, H, W, st);
+  if (mode == 1 && stride == 1)
+    return bits ? launch_s1<1, true>(in, w, nullptr, nullptr, out, B, H, W, bits, st) : launch_s1<1, false>(in, w, nullptr, mask, out, B, H, W, nullptr, st);
   if (mode == 1 && stride == 2) {
     // here `in` = dy [B,Ho,Wo,32], `out` = dx [B,H,W,32]
     const int Ho = (H - 1) / 2 + 1, Wo = (W - 1) / 2 + 1;
     const int items = B * (((W + 1) / 2 + TILE_M - 1) / TILE_M) * (((H + 1) / 2 + DG_MROWS - 1) / DG_MROWS);
-    if (int e = set_smem(conv3x3_c32_dgrad_s2_tc_kernel, DG_SMEM, Carveout::kMaxShared, "dgrad_s2_tc")) return e;
+    auto k = bits ? conv3x3_c32_dgrad_s2_tc_kernel<true> : conv3x3_c32_dgrad_s2_tc_kernel<false>;
+    if (int e = set_smem(k, DG_SMEM, Carveout::kMaxShared, "dgrad_s2_tc")) return e;
     if ((reinterpret_cast<uintptr_t>(in) & 15) != 0) return fail(DD_ERR_ALIGNMENT, "dgrad_s2_tc: dy is not 16-byte aligned");
     CUtensorMap mdy;
     char msg[256];
     if (tma_map_nhwc_sw64(&mdy, in, B, Ho, Wo, C, 129, 1, msg, sizeof msg)) return fail(DD_ERR_UNSUPPORTED, "dgrad_s2_tc: %s", msg);
-    conv3x3_c32_dgrad_s2_tc_kernel<<<items < kSMs ? items : kSMs, DG_THREADS, DG_SMEM, st>>>(
-        mdy, w, (const __nv_bfloat16*)mask, (__nv_bfloat16*)out, B, H, W, Ho, Wo);
+    k<<<items < kSMs ? items : kSMs, DG_THREADS, DG_SMEM, st>>>(mdy, w, bits ? nullptr : (const __nv_bfloat16*)mask,
+                                                                 (__nv_bfloat16*)out, B, H, W, Ho, Wo, bits);
     return check_launch("conv3x3_c32_dgrad_s2_tc");
   }
   return fail(DD_ERR_UNSUPPORTED, "conv_tc: mode %d stride %d", mode, stride);
 }
 
 // in_flags: bit 0 = six views [B,6,3,H,W] (stitch folded in), else a mosaic [B,3,H,Wm]; bit 1 = raw camera bytes (u8, /255 folded in)
-int conv_c1_fwd_tc(const void* in, int in_flags, const float* w, const float* bias, void* out, int B, int H, int Wm,
-                   cudaStream_t st) {
+// bits (may be NULL): also write a1's ReLU sign words (see relu_bits)
+int conv_c1_fwd_tc(const void* in, int in_flags, const float* w, const float* bias, void* out, uint32_t* bits, int B, int H,
+                   int Wm, cudaStream_t st) {
   if ((reinterpret_cast<uintptr_t>(out) & 31) != 0) return fail(DD_ERR_ALIGNMENT, "conv_c1_tc: out %p is not 32-byte aligned", out);
+  if ((reinterpret_cast<uintptr_t>(bits) & 7) != 0) return fail(DD_ERR_ALIGNMENT, "conv_c1_tc: sign words %p are not 8-byte aligned", bits);
   const int items = B * ((Wm + TILE_M - 1) / TILE_M) * ((H + ROWS - 1) / ROWS);
   const int grid = items < kSMs ? items : kSMs;
   auto launch1 = [&](auto k, auto* typed_in) {
     if (int e = set_smem(k, C1_SMEM, Carveout::kMaxShared, "conv_c1_tc")) return e;
-    k<<<grid, C1_THREADS, C1_SMEM, st>>>(typed_in, w, bias, (__nv_bfloat16*)out, B, H, Wm);
+    k<<<grid, C1_THREADS, C1_SMEM, st>>>(typed_in, w, bias, (__nv_bfloat16*)out, B, H, Wm, bits);
     return check_launch("conv_c1_tc");
   };
+  auto launch = [&](auto typed_in, auto k_plain, auto k_bits) { return bits ? launch1(k_bits, typed_in) : launch1(k_plain, typed_in); };
   const bool views = in_flags & 1, u8 = in_flags & 2;
-  if (u8) return views ? launch1(conv_c1_tc_kernel<true, uint8_t>, (const uint8_t*)in) : launch1(conv_c1_tc_kernel<false, uint8_t>, (const uint8_t*)in);
-  return views ? launch1(conv_c1_tc_kernel<true, float>, (const float*)in) : launch1(conv_c1_tc_kernel<false, float>, (const float*)in);
+  const uint8_t* in8 = (const uint8_t*)in;
+  const float* in32 = (const float*)in;
+  if (u8)
+    return views ? launch(in8, conv_c1_tc_kernel<true, uint8_t, false>, conv_c1_tc_kernel<true, uint8_t, true>)
+                 : launch(in8, conv_c1_tc_kernel<false, uint8_t, false>, conv_c1_tc_kernel<false, uint8_t, true>);
+  return views ? launch(in32, conv_c1_tc_kernel<true, float, false>, conv_c1_tc_kernel<true, float, true>)
+               : launch(in32, conv_c1_tc_kernel<false, float, false>, conv_c1_tc_kernel<false, float, true>);
 }
 
 // relu(c1) -> relu(c2) of the encoder in one kernel (inference: the first activation is not kept); out = a2, bf16 NHWC

@@ -118,6 +118,12 @@ def stitch_mask(views: torch.Tensor, slot: int):
 # --------------------------------------------------------------------------------------------
 # encoder conv stack (c1 -> c2 -> c3 [-> flat max-pool]) as ONE autograd node
 # --------------------------------------------------------------------------------------------
+# On the bf16 tensor-core training path the c2 / c3 input gradients take the ReLU masks of a1 / a2 as sign words (4 bytes
+# per pixel, written by the c1 / c2 forward kernels) instead of re-reading the 64-byte activations; the gradients are
+# bit-identical either way.  False selects the activation-mask form (kept so that the two can be compared in one process).
+RELU_MASK_BITS = True
+
+
 def _conv_ws(device):
     n = int(_lib.load().dd_conv_wgrad_workspace_bytes())
     return _ws.get("conv_wgrad", n, device), n
@@ -153,6 +159,7 @@ class EncoderConvStack(torch.autograd.Function):
         H3, W3 = (H - 1) // 2 + 1, (Wm - 1) // 2 + 1
         w1, b1, w2, b2, w3, b3 = (_c(t.detach().float()) for t in (w1, b1, w2, b2, w3, b3))
         in_flags = (_lib.IN_VIEWS if is_views else 0) | (_lib.IN_U8 if inp.dtype == torch.uint8 else 0)
+        bits1 = bits2 = None
         if fused_front:
             # no backward pass will ask for the first activation: c1 -> c2 in one kernel, a1 stays in shared memory / TMEM
             # (same bits as the two kernels below)
@@ -160,6 +167,16 @@ class EncoderConvStack(torch.autograd.Function):
             a2 = torch.empty(B, H, Wm, 32, dtype=act_dtype, device=dev)
             call("dd_encoder_c1c2_fused_fwd", inp.data_ptr(), in_flags, w1.data_ptr(), b1.data_ptr(), w2.data_ptr(),
                  b2.data_ptr(), a2.data_ptr(), B, H, Wm, st)
+        elif tensor_core and RELU_MASK_BITS:
+            # training: a1 / a2 are kept for the weight gradients, their ReLU masks as sign words for the input gradients
+            a1 = torch.empty(B, H, Wm, 32, dtype=act_dtype, device=dev)
+            bits1 = torch.empty(B, H, Wm, dtype=torch.int32, device=dev)
+            call("dd_conv_c1_fwd_bits", inp.data_ptr(), in_flags, w1.data_ptr(), b1.data_ptr(), a1.data_ptr(),
+                 bits1.data_ptr(), code, B, H, Wm, impl, st)
+            a2 = torch.empty_like(a1)
+            bits2 = torch.empty_like(bits1)
+            call("dd_conv3x3_c32_fwd_bits", a1.data_ptr(), w2.data_ptr(), b2.data_ptr(), a2.data_ptr(), bits2.data_ptr(),
+                 code, B, H, Wm, 1, impl, st)
         else:
             a1 = torch.empty(B, H, Wm, 32, dtype=act_dtype, device=dev)
             call("dd_conv_c1_fwd", inp.data_ptr(), in_flags, w1.data_ptr(), b1.data_ptr(), a1.data_ptr(), code,
@@ -184,7 +201,7 @@ class EncoderConvStack(torch.autograd.Function):
             call("dd_pool4_fwd", a3.data_ptr(), out.data_ptr(), code, B, H3, W3, st)
         ctx.geom = (B, H, Wm, H3, W3, in_flags, code, c3_only, impl, act_dtype)
         if not inference:
-            ctx.save_for_backward(inp, w2, w3, a1, a2, a3)
+            ctx.save_for_backward(inp, w2, w3, a1, a2, a3, bits1, bits2)
         return out
 
     @staticmethod
@@ -194,7 +211,7 @@ class EncoderConvStack(torch.autograd.Function):
             # (the reference never asks for one: the views come from the dataloader) -- fail loudly, not with zeros
             raise NotImplementedError("encoder_conv_stack: the camera views / mosaic require grad, but the scene pipeline "
                                       "has no input gradient for the first conv")
-        inp, w2, w3, a1, a2, a3 = ctx.saved_tensors
+        inp, w2, w3, a1, a2, a3, bits1, bits2 = ctx.saved_tensors
         B, H, Wm, H3, W3, in_flags, code, c3_only, impl, act_dtype = ctx.geom
         dev, st = g.device, stream_ptr()
         ws, ws_n = _conv_ws(dev)
@@ -214,15 +231,23 @@ class EncoderConvStack(torch.autograd.Function):
         call("dd_conv3x3_c32_wgrad", a2.data_ptr(), da3.data_ptr(), dw3.data_ptr(), db3.data_ptr(), ws.data_ptr(),
              ws_n, code, B, H, Wm, 2, impl, st)
         da2 = torch.empty_like(a2)
-        call("dd_conv3x3_c32_dgrad", da3.data_ptr(), w3.data_ptr(), a2.data_ptr(), da2.data_ptr(), code, B, H, Wm, 2,
-             impl, st)
+        if bits2 is not None:
+            call("dd_conv3x3_c32_dgrad_bits", da3.data_ptr(), w3.data_ptr(), bits2.data_ptr(), da2.data_ptr(), code, B, H,
+                 Wm, 2, impl, st)
+        else:
+            call("dd_conv3x3_c32_dgrad", da3.data_ptr(), w3.data_ptr(), a2.data_ptr(), da2.data_ptr(), code, B, H, Wm, 2,
+                 impl, st)
         del da3
         dw2, db2 = torch.empty(32, 32, 3, 3, **f32), torch.empty(32, **f32)
         call("dd_conv3x3_c32_wgrad", a1.data_ptr(), da2.data_ptr(), dw2.data_ptr(), db2.data_ptr(), ws.data_ptr(),
              ws_n, code, B, H, Wm, 1, impl, st)
         da1 = torch.empty_like(a1)
-        call("dd_conv3x3_c32_dgrad", da2.data_ptr(), w2.data_ptr(), a1.data_ptr(), da1.data_ptr(), code, B, H, Wm, 1,
-             impl, st)
+        if bits1 is not None:
+            call("dd_conv3x3_c32_dgrad_bits", da2.data_ptr(), w2.data_ptr(), bits1.data_ptr(), da1.data_ptr(), code, B, H,
+                 Wm, 1, impl, st)
+        else:
+            call("dd_conv3x3_c32_dgrad", da2.data_ptr(), w2.data_ptr(), a1.data_ptr(), da1.data_ptr(), code, B, H, Wm, 1,
+                 impl, st)
         del da2
         dw1, db1 = torch.empty(32, 3, 3, 3, **f32), torch.empty(32, **f32)
         call("dd_conv_c1_wgrad", inp.data_ptr(), in_flags, da1.data_ptr(), code, dw1.data_ptr(), db1.data_ptr(),

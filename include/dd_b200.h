@@ -70,6 +70,13 @@ int dd_u8_to_f32(const uint8_t* in, float* out, long long n, void* stream);
 enum { DD_IN_VIEWS = 1, DD_IN_U8 = 2 };
 int dd_conv_c1_fwd(const void* in, int in_flags, const float* w_oihw, const float* bias,
                    void* out, int out_dtype, int B, int H, int Wm, int impl, void* stream);
+/* ReLU sign words: the ReLU mask of a1 / a2 for the input gradients of c2 / c3, 4 bytes per pixel instead of the
+ * 64-byte activation.  One uint32 per pixel [B,H,W] (NHWC pixel order); bit c is 1 exactly when the stored bf16
+ * activation of channel c is > 0.  `bits` must be 8-byte aligned.  The *_bits entry points run on the bf16 tensor-core
+ * kernels only: fp32, DD_IMPL_SIMT or a shape those kernels do not take return DD_ERR_UNSUPPORTED before anything runs.
+ * dd_conv_c1_fwd_bits = dd_conv_c1_fwd (same out) that also writes out's sign words. */
+int dd_conv_c1_fwd_bits(const void* in, int in_flags, const float* w_oihw, const float* bias, void* out,
+                        uint32_t* bits, int out_dtype, int B, int H, int Wm, int impl, void* stream);
 /* Inference front of the encoder in one kernel: a2 = relu(c2(relu(c1(x)))) (components.py:41-43), bf16 NHWC [B,H,Wm,32];
  * the first activation stays in shared memory / TMEM (halo recompute per 126-pixel x 64-row strip).  Same bits as
  * dd_conv_c1_fwd + dd_conv3x3_c32_fwd on the bf16 tensor-core path.  in / in_flags as for dd_conv_c1_fwd. */
@@ -92,6 +99,12 @@ int dd_conv3x3_c32_fwd(const void* in, const float* w_oihw, const float* bias, v
  * layer's post-ReLU output; pass x = NULL for no mask).  dy must already be masked. */
 int dd_conv3x3_c32_dgrad(const void* dy, const float* w_oihw, const void* x, void* dx,
                          int dtype, int B, int H, int W, int stride, int impl, void* stream);
+/* Sign-word forms (see dd_conv_c1_fwd_bits): the stride-1 forward also writes out's sign words; the input gradient
+ * takes the mask from x's sign words (x_bits [B,H,W]) instead of x, bit-identical to passing x. */
+int dd_conv3x3_c32_fwd_bits(const void* in, const float* w_oihw, const float* bias, void* out, uint32_t* bits,
+                            int dtype, int B, int H, int W, int stride, int impl, void* stream);
+int dd_conv3x3_c32_dgrad_bits(const void* dy, const float* w_oihw, const uint32_t* x_bits, void* dx,
+                              int dtype, int B, int H, int W, int stride, int impl, void* stream);
 /* dW [32,32,3,3] f32, db [32] f32 (overwritten, deterministic reduction order). */
 int dd_conv3x3_c32_wgrad(const void* x, const void* dy, float* dw, float* db, void* workspace,
                          size_t ws_bytes, int dtype, int B, int H, int W, int stride, int impl,
