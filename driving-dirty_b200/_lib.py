@@ -28,11 +28,13 @@ SIGNATURES = {
     "dd_stitch_f32": (_I, [_P, _P, _I, _I, _I, _P]),
     "dd_stitch_mask_f32": (_I, [_P, _P, _P, _I, _I, _I, _I, _P]),
     "dd_stitch_u8": (_I, [_P, _P, _I, _I, _I, _P]),
+    "dd_unstitch_f32": (_I, [_P, _P, _P, _I, _I, _I, _I, _P]),
     "dd_u8_to_f32": (_I, [_P, _P, _L, _P]),
     "dd_conv_c1_fwd": (_I, [_P, _I, _P, _P, _P, _I, _I, _I, _I, _I, _P]),
     "dd_conv_c1_fwd_bits": (_I, [_P, _I, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P]),
     "dd_encoder_c1c2_fused_fwd": (_I, [_P, _I, _P, _P, _P, _P, _P, _I, _I, _I, _P]),
     "dd_conv_c1_wgrad": (_I, [_P, _I, _P, _I, _P, _P, _P, _Z, _I, _I, _I, _I, _P]),
+    "dd_conv_c1_dgrad": (_I, [_P, _I, _P, _P, _I, _I, _I, _I, _I, _P]),
     "dd_conv3x3_c32_fwd": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _P]),
     "dd_conv3x3_c32_dgrad": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _P]),
     "dd_conv3x3_c32_fwd_bits": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _P]),
@@ -61,6 +63,7 @@ SIGNATURES = {
     "dd_conv2d_workspace_bytes": (_Z, [_P]),
     "dd_conv2d_tc_supported": (_I, [_P, _I, _I]),
     "dd_view_extract": (_I, [_P, _P, _I, _I, _I, _I, _I, _I, _P]),
+    "dd_view_extract_bwd": (_I, [_P, _I, _P, _I, _I, _I, _I, _I, _P]),
     "dd_nhwc_place": (_I, [_P, _P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _P]),
     "dd_sigmoid_bwd": (_I, [_P, _P, _P, _I, _L, _P]),
     "dd_bce_prob_fwd": (_I, [_P, _P, _P, _P, _Z, _L, _P]),

@@ -33,8 +33,8 @@ class SpatialMappingCNN(nn.Module):
     def forward_nhwc(self, x):
         views = ops.as_view_batch(x)
         cells, offsets = [], []
-        for name, cam, mode, (r, c) in _STRIPS:
-            img = ops.view_extract(views, cam, mode, self.compute_dtype)
+        imgs = ops.view_extract_all(views, [(cam, mode) for _, cam, mode, _ in _STRIPS], self.compute_dtype)
+        for (name, cam, mode, (r, c)), img in zip(_STRIPS, imgs):
             cells.append((r, c, ops.conv2d_nhwc(img, getattr(self, name), relu=True)))
         hs = [max(t.shape[1] for rr, _, t in cells if rr == r) for r in range(3)]
         w0 = max(t.shape[2] for _, cc, t in cells if cc == 0)

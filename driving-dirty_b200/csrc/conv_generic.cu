@@ -789,6 +789,26 @@ __global__ void view_extract_kernel(const float* __restrict__ views, T* __restri
   }
 }
 
+// backward of view_extract_kernel: thread = element of view `view` of the views gradient (each written once; the other
+// five views are not touched); it reads the extracted image's gradient at the transformed position
+template <typename T>
+__global__ void view_extract_bwd_kernel(const T* __restrict__ dout, float* __restrict__ dviews, int B, int H, int W,
+                                        int view, int mode, int Ho, int Wo) {
+  const long long total = (long long)B * 3 * H * W;
+  for (long long idx = blockIdx.x * (long long)blockDim.x + threadIdx.x; idx < total; idx += (long long)gridDim.x * blockDim.x) {
+    const int w = (int)(idx % W);
+    const int h = (int)((idx / W) % H);
+    const int c = (int)((idx / ((long long)W * H)) % 3);
+    const long long b = idx / (3LL * W * H);
+    int i, j;
+    if (mode == 0) { i = h; j = w; }
+    else if (mode == 1) { i = W - 1 - w; j = h; }
+    else if (mode == 2) { i = w; j = H - 1 - h; }
+    else { i = H - 1 - h; j = W - 1 - w; }
+    dviews[(((b * 6 + view) * 3 + c) * H + h) * (size_t)W + w] = dd::ld<T>(dout + ((b * Ho + i) * Wo + j) * 3 + c);
+  }
+}
+
 // dir 0: big[b, oy+i, ox+j, oc+k] = small[b,i,j,k];  dir 1: small[b,i,j,k] = big[b, oy+i, ox+j, oc+k]
 template <typename T>
 __global__ void nhwc_place_kernel(T* __restrict__ small_, T* __restrict__ big, int B, int h, int w, int c, int H, int W,
@@ -878,6 +898,25 @@ extern "C" int dd_view_extract(const float* views, void* out, int out_dtype, int
     view_extract_kernel<__nv_bfloat16><<<grid_elems(total), 256, 0, st>>>(views, (__nv_bfloat16*)out, B, H, W, view, mode, Ho, Wo);
   else return dd::fail(DD_ERR_UNSUPPORTED, "dd_view_extract: dtype %d", out_dtype);
   return dd::check_launch("view_extract");
+}
+
+extern "C" int dd_view_extract_bwd(const void* dout, int dtype, float* dviews, int B, int H, int W, int view, int mode,
+                                   void* stream) {
+  DD_REQUIRE(B >= 0 && H > 0 && W > 0, DD_ERR_BAD_ARG, "dd_view_extract_bwd: bad shape");
+  DD_REQUIRE(view >= 0 && view < 6 && mode >= 0 && mode <= 3, DD_ERR_BAD_ARG, "dd_view_extract_bwd: view %d mode %d", view, mode);
+  if (B == 0) return 0;
+  DD_REQUIRE(dout && dviews, DD_ERR_BAD_ARG, "dd_view_extract_bwd: null pointer");
+  const bool rot = mode == 1 || mode == 2;
+  const int Ho = rot ? W : H, Wo = rot ? H : W;
+  const long long total = (long long)B * 3 * H * W;
+  cudaStream_t st = dd::as_stream(stream);
+  if (dtype == DD_F32)
+    view_extract_bwd_kernel<float><<<grid_elems(total), 256, 0, st>>>((const float*)dout, dviews, B, H, W, view, mode, Ho, Wo);
+  else if (dtype == DD_BF16)
+    view_extract_bwd_kernel<__nv_bfloat16><<<grid_elems(total), 256, 0, st>>>((const __nv_bfloat16*)dout, dviews, B, H, W, view,
+                                                                                mode, Ho, Wo);
+  else return dd::fail(DD_ERR_UNSUPPORTED, "dd_view_extract_bwd: dtype %d", dtype);
+  return dd::check_launch("view_extract_bwd");
 }
 
 extern "C" int dd_nhwc_place(void* small_, void* big, int dtype, int B, int h, int w, int c, int H, int W, int C, int oy,

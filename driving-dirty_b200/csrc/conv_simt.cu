@@ -337,6 +337,56 @@ __global__ void __launch_bounds__(256) conv_c1_fwd_simt(const float* __restrict_
   }
 }
 
+// c1 input gradient on the CUDA cores (the fp32 parity path; bf16 with DD_IMPL_SIMT): thread = image pixel, reading the
+// whole 32-channel da1 pixel of each of its 9 taps; fp32 dx stored into the NCHW mosaic or, IS_VIEWS, the views
+// (mosaic column w of slot j = w / Wv lands in view dd::view_of_slot(j)).  Fixed summation order: kh, kw, o.
+template <typename T, bool IS_VIEWS>
+__global__ void __launch_bounds__(256) conv_c1_dgrad_simt(const T* __restrict__ dy, const float* __restrict__ w_oihw,
+                                                          float* __restrict__ dx, int H, int Wm) {
+  constexpr int TH = 8, TW = 32;
+  __shared__ float s_w[9 * C * 3];                 // [tap][o][c]
+  const int tid = threadIdx.x, b = blockIdx.z;
+  for (int i = tid; i < 9 * C * 3; i += 256) {
+    const int c = i % 3, o = (i / 3) % C, tap = i / (3 * C);
+    s_w[i] = w_oihw[(o * 3 + c) * 9 + tap];
+  }
+  __syncthreads();
+  const int h = blockIdx.y * TH + tid / TW, w = blockIdx.x * TW + tid % TW;
+  if (h >= H || w >= Wm) return;
+  float acc[3] = {0.f, 0.f, 0.f};
+  for (int kh = 0; kh < 3; ++kh) {
+    const int y = h + 1 - kh;
+    if (y < 0 || y >= H) continue;
+    for (int kw = 0; kw < 3; ++kw) {
+      const int x = w + 1 - kw;
+      if (x < 0 || x >= Wm) continue;
+      const T* p = dy + (((size_t)b * H + y) * Wm + x) * C;
+      const float* wt = s_w + (kh * 3 + kw) * C * 3;
+#pragma unroll
+      for (int g = 0; g < C / 8; ++g) {
+        float v[8];
+        dd::ld8<T>(p + 8 * g, v);
+#pragma unroll
+        for (int k = 0; k < 8; ++k)
+#pragma unroll
+          for (int c = 0; c < 3; ++c) acc[c] = fmaf(v[k], wt[(8 * g + k) * 3 + c], acc[c]);
+      }
+    }
+  }
+  float* dst;
+  size_t cs;
+  if (IS_VIEWS) {
+    const int Wv = Wm / 6, j = w / Wv;
+    dst = dx + ((size_t)(6 * b + dd::view_of_slot(j)) * 3 * H + h) * Wv + (w - j * Wv);
+    cs = (size_t)H * Wv;
+  } else {
+    dst = dx + ((size_t)3 * b * H + h) * Wm + w;
+    cs = (size_t)H * Wm;
+  }
+#pragma unroll
+  for (int c = 0; c < 3; ++c) dst[c * cs] = acc[c];
+}
+
 // c1 wgrad: lane k<27 owns filter tap k = ci*9+tap for all 32 co; the 8 warps split the tile's
 // pixels; CTA partial [27][32] + db[32] to the workspace (persistent tile loop).
 template <typename T, bool IS_VIEWS>
@@ -514,6 +564,7 @@ int enc_c1c2_fused_fwd_tc(const void* in, int in_flags, const float* w1, const f
                           void* out, int B, int H, int Wm, cudaStream_t st);
 int conv_c1_wgrad_tc(const void* in, int in_flags, const void* dy, float* dw, float* db, void* ws, size_t ws_bytes,
                      int B, int H, int Wm, cudaStream_t st);
+int conv_c1_dgrad_tc(const void* dy, const float* w, float* dx, bool views, int B, int H, int Wm, cudaStream_t st);
 }  // namespace dd
 
 extern "C" size_t dd_conv_wgrad_workspace_bytes(void) { return kWgradWsBytes; }
@@ -686,6 +737,32 @@ extern "C" int dd_conv_c1_wgrad(const void* in_, int in_flags, const void* dy, i
   if (int e = dd::check_launch("conv_c1_wgrad")) return e;
   c1_wgrad_reduce_kernel<<<4, 256, 0, st>>>(ws, nblk, dw, db);
   return dd::check_launch("c1_wgrad_reduce");
+}
+
+extern "C" int dd_conv_c1_dgrad(const void* dy, int dtype, const float* w_oihw, float* dx, int out_flags, int B, int H,
+                                int Wm, int impl, void* stream) {
+  DD_REQUIRE(B >= 0 && H > 0 && Wm > 0, DD_ERR_BAD_ARG, "dd_conv_c1_dgrad: bad shape");
+  DD_REQUIRE((out_flags & ~3) == 0, DD_ERR_BAD_ARG, "dd_conv_c1_dgrad: out_flags %d", out_flags);
+  DD_REQUIRE(!(out_flags & DD_IN_U8), DD_ERR_UNSUPPORTED, "dd_conv_c1_dgrad: raw camera bytes have no gradient");
+  const bool views = out_flags & DD_IN_VIEWS;
+  DD_REQUIRE(!views || Wm % 6 == 0, DD_ERR_BAD_ARG, "dd_conv_c1_dgrad: mosaic width %d not a multiple of 6", Wm);
+  DD_REQUIRE(dtype == DD_F32 || dtype == DD_BF16, DD_ERR_UNSUPPORTED, "dd_conv_c1_dgrad: dtype %d", dtype);
+  DD_REQUIRE(!(dtype == DD_F32 && impl == DD_IMPL_TCGEN05), DD_ERR_UNSUPPORTED, "tcgen05 conv is bf16 only");
+  if (B == 0) return 0;
+  DD_REQUIRE(dy && w_oihw && dx, DD_ERR_BAD_ARG, "dd_conv_c1_dgrad: null pointer");
+  DD_REQUIRE((uintptr_t)dy % 16 == 0 && (uintptr_t)dx % 4 == 0, DD_ERR_ALIGNMENT,
+             "dd_conv_c1_dgrad: dy %p must be 16-byte aligned, dx %p 4-byte aligned", dy, dx);
+  cudaStream_t st = dd::as_stream(stream);
+  if (dtype == DD_BF16 && impl != DD_IMPL_SIMT) return dd::conv_c1_dgrad_tc(dy, w_oihw, dx, views, B, H, Wm, st);
+  dim3 grid((Wm + 31) / 32, (H + 7) / 8, B);
+  if (dtype == DD_F32) {
+    if (views) conv_c1_dgrad_simt<float, true><<<grid, 256, 0, st>>>((const float*)dy, w_oihw, dx, H, Wm);
+    else conv_c1_dgrad_simt<float, false><<<grid, 256, 0, st>>>((const float*)dy, w_oihw, dx, H, Wm);
+  } else {
+    if (views) conv_c1_dgrad_simt<__nv_bfloat16, true><<<grid, 256, 0, st>>>((const __nv_bfloat16*)dy, w_oihw, dx, H, Wm);
+    else conv_c1_dgrad_simt<__nv_bfloat16, false><<<grid, 256, 0, st>>>((const __nv_bfloat16*)dy, w_oihw, dx, H, Wm);
+  }
+  return dd::check_launch("conv_c1_dgrad");
 }
 
 extern "C" int dd_relu_mask(const void* g, const void* act, void* out, int dtype, long long n, void* stream) {

@@ -264,7 +264,8 @@ int launch_s2_fwd(const void* in, const float* w, const float* bias, void* out, 
 
 
 // ================================================================================================
-// Stride-1 32->32 3x3 conv (c2 forward, c2 input gradient), "row scatter" formulation.
+// Stride-1 32->32 3x3 conv (c2 forward, c2 input gradient), "row scatter" formulation; also the image gradient of c1
+// (MODE 2, see below).
 //
 // An SS tcgen05.mma with N = 32 is bound by the shared-memory reads of its operands, not by the tensor
 // pipe (tools/umma_rate2.cu: 40 cycles per M128 N32 K16 against a 16-cycle tensor floor; the 4 KB A
@@ -305,6 +306,12 @@ struct S1Bars {
   uint32_t tmem_base;
 };
 
+// MODE 0: forward (bias + ReLU), MODE 1: input gradient (ReLU mask of the layer input), MODE 2: input gradient of c1
+// (components.py:19,41), dx[c,h,w] = sum over o, kh, kw of da1[o, h+1-kh, w+1-kw] * W1[o,c,kh,kw].  MODE 2 reads the same
+// operand as MODE 1 (da1, a [B,H,W,32] bf16 gradient) and issues the same MMAs: the B operand is W1 flipped, its 3 image
+// channels zero-padded to the 32-column slot (as conv_generic.cu pads narrow layers).  Only the epilogue differs: 3 of the
+// 32 accumulator columns, no mask (the images have no activation), fp32 stores into the NCHW mosaic [B,3,H,W] or, with
+// Wv > 0, straight into the views [B,6,3,H,Wv] (W = 6 Wv; mosaic slot j -> view dd::view_of_slot(j)), `out` then being float*.
 // BITS: MODE 0 also writes the output's ReLU sign words to `bits`; MODE 1 takes the ReLU mask from the sign words in `bits`
 // instead of the activation `mask`
 template <int MODE, bool BITS>
@@ -313,7 +320,7 @@ __global__ void __launch_bounds__(S1_THREADS, 1) conv3x3_c32_s1_tc_kernel(const 
                                                                            const float* __restrict__ bias,
                                                                            const __nv_bfloat16* __restrict__ mask,
                                                                            __nv_bfloat16* __restrict__ out, int B, int H,
-                                                                           int W, uint32_t* __restrict__ bits) {
+                                                                           int W, uint32_t* __restrict__ bits, int Wv) {
   extern __shared__ __align__(1024) uint8_t smem[];
   uint8_t* s_w = smem;
   uint8_t* s_slab = smem + W_BYTES;
@@ -332,7 +339,8 @@ __global__ void __launch_bounds__(S1_THREADS, 1) conv3x3_c32_s1_tc_kernel(const 
     const int kh = tap / 3, kw = tap - 3 * kh;
     float v;
     if (MODE == 0) v = w_oihw[(co * C + ci) * 9 + tap];
-    else v = w_oihw[(ci * C + co) * 9 + (8 - tap)];               // dgrad: W[co=in][ci=out][flipped tap]
+    else if (MODE == 1) v = w_oihw[(ci * C + co) * 9 + (8 - tap)];  // dgrad: W[co=in][ci=out][flipped tap]
+    else v = co < 3 ? w_oihw[(ci * 3 + co) * 9 + (8 - tap)] : 0.f;   // c1 dgrad: W1 [32 out][3 in], columns 3..31 zero
     *reinterpret_cast<__nv_bfloat16*>(s_w + (kw * 4 + (ci >> 3)) * S1_WN + ((2 - kh) * 32 + co) * 16 + (ci & 7) * 2) =
         __float2bfloat16_rn(v);
   }
@@ -490,6 +498,19 @@ __global__ void __launch_bounds__(S1_THREADS, 1) conv3x3_c32_s1_tc_kernel(const 
       const int wo = wt * TILE_M + quarter * 32 + lane;
       const bool ok = wo < W;
       const int j0 = (int)((rc0 ^ half) & 1);
+      // MODE 2: this pixel's channel-0 element in row h0 of the image gradient; row and channel strides
+      float* dx = nullptr;
+      const int Wr = Wv > 0 ? Wv : W;
+      const size_t cstride = (size_t)H * Wr;
+      if (MODE == 2 && ok) {
+        int img = 3 * b, col = wo;
+        if (Wv > 0) {
+          const int sj = wo / Wv;
+          img = 3 * (6 * b + dd::view_of_slot(sj));
+          col = wo - sj * Wv;
+        }
+        dx = reinterpret_cast<float*>(out) + ((size_t)img * H + h0) * Wr + col;
+      }
       // sign words: this warp's next row is loaded while the current one is processed -- one 4-byte load issued just before
       // the wait for the MMAs leaves its DRAM round trip exposed on every row
       uint32_t mb_next = 0;
@@ -514,6 +535,17 @@ __global__ void __launch_bounds__(S1_THREADS, 1) conv3x3_c32_s1_tc_kernel(const 
           umma::mbar_wait(&bars->acc_full[grp % S1_NGRP], (grp / S1_NGRP) & 1);
           umma::tc_fence_after_sync();
           cur_grp = grp;
+        }
+        if (MODE == 2) {
+          uint32_t r[4];
+          umma::tmem_ld_32x4(tmem + ((uint32_t)(quarter * 32) << 16) + buf * 32, r);
+          umma::tmem_ld_wait();
+          if (ok) {
+            float* d = dx + (size_t)j * Wr;
+#pragma unroll
+            for (int c = 0; c < 3; ++c) d[c * cstride] = __uint_as_float(r[c]);
+          }
+          continue;
         }
         uint32_t r[32];
         umma::tmem_ld_32x32(tmem + ((uint32_t)(quarter * 32) << 16) + buf * 32, r);
@@ -550,7 +582,7 @@ __global__ void __launch_bounds__(S1_THREADS, 1) conv3x3_c32_s1_tc_kernel(const 
 
 template <int MODE, bool BITS>
 int launch_s1(const void* in, const float* w, const float* bias, const void* mask, void* out, int B, int H, int W,
-              uint32_t* bits, cudaStream_t st) {
+              uint32_t* bits, cudaStream_t st, int Wv = 0) {
   const int items = B * ((W + TILE_M - 1) / TILE_M) * ((H + S1_ROWS - 1) / S1_ROWS);
   auto k = conv3x3_c32_s1_tc_kernel<MODE, BITS>;
   if (int e = dd::set_smem(k, S1_SMEM, dd::Carveout::kMaxShared, "conv_tc s1")) return e;
@@ -559,7 +591,7 @@ int launch_s1(const void* in, const float* w, const float* bias, const void* mas
   CUtensorMap map;
   char msg[256];
   if (dd::tma_map_nhwc_sw64(&map, in, B, H, W, C, 130, 1, msg, sizeof msg)) return dd::fail(DD_ERR_UNSUPPORTED, "conv_tc s1: %s", msg);
-  k<<<grid, S1_THREADS, S1_SMEM, st>>>(map, w, bias, (const __nv_bfloat16*)mask, (__nv_bfloat16*)out, B, H, W, bits);
+  k<<<grid, S1_THREADS, S1_SMEM, st>>>(map, w, bias, (const __nv_bfloat16*)mask, (__nv_bfloat16*)out, B, H, W, bits, Wv);
   return dd::check_launch("conv3x3_c32_s1_tc");
 }
 
@@ -1354,6 +1386,12 @@ int conv3x3_c32_fwd_tc(const void* in, const float* w, const float* bias, void* 
     return check_launch("conv3x3_c32_dgrad_s2_tc");
   }
   return fail(DD_ERR_UNSUPPORTED, "conv_tc: mode %d stride %d", mode, stride);
+}
+
+// image gradient of c1 from da1 (bf16 NHWC [B,H,Wm,32]) -> fp32 dx: the views [B,6,3,H,Wm/6] when `views`, else the
+// mosaic [B,3,H,Wm]
+int conv_c1_dgrad_tc(const void* dy, const float* w, float* dx, bool views, int B, int H, int Wm, cudaStream_t st) {
+  return launch_s1<2, false>(dy, w, nullptr, nullptr, dx, B, H, Wm, nullptr, st, views ? Wm / 6 : 0);
 }
 
 // in_flags: bit 0 = six views [B,6,3,H,W] (stitch folded in), else a mosaic [B,3,H,Wm]; bit 1 = raw camera bytes (u8, /255 folded in)

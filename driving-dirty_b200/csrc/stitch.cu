@@ -96,6 +96,30 @@ __global__ void __launch_bounds__(256) u8_to_f32_kernel(const uint8_t* __restric
   for (long long i = (n16 << 4) + (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) out[i] = lut[in[i]];
 }
 
+// Backward of the stitch (and of the mask variant, slot >= 0): dviews[b,v,c,h,w] = dmosaic[b,c,h,j*W+w] with j the slot
+// showing view v (the order is its own inverse), except that the masked slot's view takes dy[b,c,h,w] (0 for dy == NULL):
+// its block of x was zeroed and passes nothing back.  Thread = views element, so every element is written once.
+__global__ void __launch_bounds__(256) unstitch_kernel(const float* __restrict__ dmosaic, const float* __restrict__ dy,
+                                                       float* __restrict__ dviews, int B, int H, int W, int slot) {
+  const long long total = (long long)B * 18 * H * W;
+  for (long long idx = blockIdx.x * (long long)blockDim.x + threadIdx.x; idx < total;
+       idx += (long long)gridDim.x * blockDim.x) {
+    const int w = (int)(idx % W);
+    long long r = idx / W;
+    const int h = (int)(r % H);
+    r /= H;
+    const int c = (int)(r % 3);
+    r /= 3;
+    const int j = dd::view_of_slot((int)(r % 6));
+    const long long b = r / 6;
+    const size_t row = ((size_t)b * 3 + c) * H + h;
+    float g;
+    if (j == slot) g = dy ? dy[row * W + w] : 0.f;
+    else g = dmosaic[row * 6 * W + (size_t)j * W + w];
+    dviews[idx] = g;
+  }
+}
+
 int launch_stitch(const float* views, float* x, float* y, int B, int H, int W, int slot, int mode,
                   cudaStream_t st) {
   const int rows = B * 3 * H;
@@ -129,6 +153,18 @@ extern "C" int dd_stitch_mask_f32(const float* views, float* x, float* y, int B,
   DD_REQUIRE(slot >= 0 && slot < 6, DD_ERR_BAD_ARG, "dd_stitch_mask_f32: slot %d outside [0,6)", slot);
   if (B == 0) return 0;
   return launch_stitch(views, x, y, B, H, W, slot, 1, dd::as_stream(stream));
+}
+
+extern "C" int dd_unstitch_f32(const float* dmosaic, const float* dy, float* dviews, int B, int H, int W, int slot,
+                               void* stream) {
+  DD_REQUIRE(B >= 0 && H > 0 && W > 0, DD_ERR_BAD_ARG, "dd_unstitch_f32: bad shape B=%d H=%d W=%d", B, H, W);
+  DD_REQUIRE(slot >= -1 && slot < 6, DD_ERR_BAD_ARG, "dd_unstitch_f32: slot %d outside [-1,6)", slot);
+  if (B == 0) return 0;
+  DD_REQUIRE(dmosaic && dviews, DD_ERR_BAD_ARG, "dd_unstitch_f32: null pointer");
+  const long long total = (long long)B * 18 * H * W;
+  const int grid = (int)((total + 255) / 256 < dd::kSMs * 8 ? (total + 255) / 256 : dd::kSMs * 8);
+  unstitch_kernel<<<grid, 256, 0, dd::as_stream(stream)>>>(dmosaic, dy, dviews, B, H, W, slot);
+  return dd::check_launch("unstitch");
 }
 
 extern "C" int dd_stitch_u8(const uint8_t* views, float* mosaic, int B, int H, int W, void* stream) {

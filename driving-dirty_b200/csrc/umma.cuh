@@ -125,6 +125,13 @@ __device__ __forceinline__ void tmem_ld_32x16(uint32_t taddr, uint32_t (&r)[16])
       : "r"(taddr)
       : "memory");
 }
+// 32 lanes x 4 columns of fp32
+__device__ __forceinline__ void tmem_ld_32x4(uint32_t taddr, uint32_t (&r)[4]) {
+  asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0, %1, %2, %3}, [%4];"
+               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3])
+               : "r"(taddr)
+               : "memory");
+}
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 
 // ---------------------------------------------------------------- descriptors -------------

@@ -84,15 +84,31 @@ def bytes_to_float(x_u8: torch.Tensor) -> torch.Tensor:
     return out
 
 
+class _Stitch(torch.autograd.Function):
+    """wide_stitch_six_images on fp32 views; backward: the inverse permutation (dd_unstitch_f32)."""
+
+    @staticmethod
+    def forward(ctx, views):
+        B, _, _, H, W = views.shape
+        out = torch.empty(B, 3, H, 6 * W, dtype=torch.float32, device=views.device)
+        call("dd_stitch_f32", views.data_ptr(), out.data_ptr(), B, H, W, stream_ptr())
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        g = _c(g)
+        B, _, H, Wm = g.shape
+        d = torch.empty(B, 6, 3, H, Wm // 6, dtype=torch.float32, device=g.device)
+        call("dd_unstitch_f32", g.data_ptr(), None, d.data_ptr(), B, H, Wm // 6, -1, stream_ptr())
+        return d
+
+
 def stitch(views: torch.Tensor) -> torch.Tensor:
-    """wide_stitch_six_images (roadmap_bce_v2.py:53-64): [B,6,3,H,W] -> [B,3,H,6W] (raw bytes: with ToTensor's /255)."""
+    """wide_stitch_six_images (roadmap_bce_v2.py:53-64): [B,6,3,H,W] -> [B,3,H,6W] (raw bytes: with ToTensor's /255).
+    Differentiable for float views: the mosaic's gradient goes back to the views."""
     if torch.is_tensor(views) and views.dtype == torch.uint8:
         return stitch_u8(views)
-    views = as_view_batch(views)
-    B, _, _, H, W = views.shape
-    out = torch.empty(B, 3, H, 6 * W, dtype=torch.float32, device=views.device)
-    call("dd_stitch_f32", views.data_ptr(), out.data_ptr(), B, H, W, stream_ptr())
-    return out
+    return _Stitch.apply(as_view_batch(views))
 
 
 def stitch_u8(views_u8: torch.Tensor) -> torch.Tensor:
@@ -105,14 +121,30 @@ def stitch_u8(views_u8: torch.Tensor) -> torch.Tensor:
     return out
 
 
+class _StitchMask(torch.autograd.Function):
+    """six_to_one_task on fp32 views.  Backward: the zeroed block of x passes no gradient, the slot's view takes y's."""
+
+    @staticmethod
+    def forward(ctx, views, slot):
+        B, _, _, H, W = views.shape
+        x = torch.empty(B, 3, H, 6 * W, dtype=torch.float32, device=views.device)
+        y = torch.empty(B, 3, H, W, dtype=torch.float32, device=views.device)
+        call("dd_stitch_mask_f32", views.data_ptr(), x.data_ptr(), y.data_ptr(), B, H, W, slot, stream_ptr())
+        ctx.slot = slot
+        return x, y
+
+    @staticmethod
+    def backward(ctx, gx, gy):
+        gx, gy = _c(gx), _c(gy)
+        B, _, H, W = gy.shape
+        d = torch.empty(B, 6, 3, H, W, dtype=torch.float32, device=gx.device)
+        call("dd_unstitch_f32", gx.data_ptr(), gy.data_ptr(), d.data_ptr(), B, H, W, ctx.slot, stream_ptr())
+        return d, None
+
+
 def stitch_mask(views: torch.Tensor, slot: int):
-    """six_to_one_task (autoencoder.py:53-73) for an already drawn slot: (x, y)."""
-    views = as_view_batch(views)
-    B, _, _, H, W = views.shape
-    x = torch.empty(B, 3, H, 6 * W, dtype=torch.float32, device=views.device)
-    y = torch.empty(B, 3, H, W, dtype=torch.float32, device=views.device)
-    call("dd_stitch_mask_f32", views.data_ptr(), x.data_ptr(), y.data_ptr(), B, H, W, int(slot), stream_ptr())
-    return x, y
+    """six_to_one_task (autoencoder.py:53-73) for an already drawn slot: (x, y), both differentiable in the views."""
+    return _StitchMask.apply(as_view_batch(views), int(slot))
 
 
 # --------------------------------------------------------------------------------------------
@@ -134,13 +166,18 @@ class EncoderConvStack(torch.autograd.Function):
     (components.py:41-47).  ``inp`` is the views batch [B,6,3,H,W] (stitch folded into c1's loads)
     or a mosaic / NCHW image [B,3,H,Wm].  Activations are NHWC in ``act_dtype``.  Returns the
     pooled features [B, 8*H3*W3] (act_dtype; fp32 copies of the same values when nothing requires grad) or, with ``c3_only``, the c3 activation as NCHW fp32
-    (components.py:44-45; ``c3_only == 2``: as the NHWC activation itself)."""
+    (components.py:44-45; ``c3_only == 2``: as the NHWC activation itself).
+
+    An fp32 ``inp`` that requires grad gets the image gradient of c1 (dd_conv_c1_dgrad), in its own layout: views or
+    mosaic.  When no conv weight requires grad (a frozen model under attribution) the backward runs the input-gradient
+    chain alone, and on the sign-word path a1 / a2 are not kept: that chain reads only a3 and the sign words."""
 
     @staticmethod
     def forward(ctx, inp, w1, b1, w2, b2, w3, b3, act_dtype, c3_only, impl):
         _require_cuda(inp, w1, w2, w3)
         inp = _c(inp)
         inference = not any(ctx.needs_input_grad)
+        want_dw = any(ctx.needs_input_grad[1:7])
         tensor_core = act_dtype == torch.bfloat16 and impl != _lib.IMPL_SIMT
         fused_front = inference and tensor_core
         if inp.dtype == torch.uint8 and not tensor_core:
@@ -201,18 +238,17 @@ class EncoderConvStack(torch.autograd.Function):
             call("dd_pool4_fwd", a3.data_ptr(), out.data_ptr(), code, B, H3, W3, st)
         ctx.geom = (B, H, Wm, H3, W3, in_flags, code, c3_only, impl, act_dtype)
         if not inference:
-            ctx.save_for_backward(inp, w2, w3, a1, a2, a3, bits1, bits2)
+            keep = want_dw or bits1 is None     # the activation-mask form reads a1 / a2 as the ReLU masks
+            ctx.save_for_backward(inp if want_dw else None, w1, w2, w3, a1 if keep else None, a2 if keep else None, a3,
+                                  bits1, bits2)
         return out
 
     @staticmethod
     def backward(ctx, g):
-        if ctx.needs_input_grad[0]:
-            # nn.Conv2d would propagate a gradient to the images; there is no c1 input-gradient kernel on this path
-            # (the reference never asks for one: the views come from the dataloader) -- fail loudly, not with zeros
-            raise NotImplementedError("encoder_conv_stack: the camera views / mosaic require grad, but the scene pipeline "
-                                      "has no input gradient for the first conv")
-        inp, w2, w3, a1, a2, a3, bits1, bits2 = ctx.saved_tensors
+        inp, w1, w2, w3, a1, a2, a3, bits1, bits2 = ctx.saved_tensors
         B, H, Wm, H3, W3, in_flags, code, c3_only, impl, act_dtype = ctx.geom
+        want_dx, want_dw = ctx.needs_input_grad[0], any(ctx.needs_input_grad[1:7])
+        dw1 = db1 = dw2 = db2 = dw3 = db3 = dx = None
         dev, st = g.device, stream_ptr()
         ws, ws_n = _conv_ws(dev)
         da3 = torch.empty_like(a3)
@@ -227,10 +263,11 @@ class EncoderConvStack(torch.autograd.Function):
             g = _c(g.to(act_dtype))
             call("dd_pool4_bwd", a3.data_ptr(), g.data_ptr(), da3.data_ptr(), code, B, H3, W3, st)
         f32 = dict(dtype=torch.float32, device=dev)
-        dw3, db3 = torch.empty(32, 32, 3, 3, **f32), torch.empty(32, **f32)
-        call("dd_conv3x3_c32_wgrad", a2.data_ptr(), da3.data_ptr(), dw3.data_ptr(), db3.data_ptr(), ws.data_ptr(),
-             ws_n, code, B, H, Wm, 2, impl, st)
-        da2 = torch.empty_like(a2)
+        if want_dw:
+            dw3, db3 = torch.empty(32, 32, 3, 3, **f32), torch.empty(32, **f32)
+            call("dd_conv3x3_c32_wgrad", a2.data_ptr(), da3.data_ptr(), dw3.data_ptr(), db3.data_ptr(), ws.data_ptr(),
+                 ws_n, code, B, H, Wm, 2, impl, st)
+        da2 = torch.empty(B, H, Wm, 32, dtype=act_dtype, device=dev)     # (a1 / a2 are not kept for a frozen stack)
         if bits2 is not None:
             call("dd_conv3x3_c32_dgrad_bits", da3.data_ptr(), w3.data_ptr(), bits2.data_ptr(), da2.data_ptr(), code, B, H,
                  Wm, 2, impl, st)
@@ -238,10 +275,11 @@ class EncoderConvStack(torch.autograd.Function):
             call("dd_conv3x3_c32_dgrad", da3.data_ptr(), w3.data_ptr(), a2.data_ptr(), da2.data_ptr(), code, B, H, Wm, 2,
                  impl, st)
         del da3
-        dw2, db2 = torch.empty(32, 32, 3, 3, **f32), torch.empty(32, **f32)
-        call("dd_conv3x3_c32_wgrad", a1.data_ptr(), da2.data_ptr(), dw2.data_ptr(), db2.data_ptr(), ws.data_ptr(),
-             ws_n, code, B, H, Wm, 1, impl, st)
-        da1 = torch.empty_like(a1)
+        if want_dw:
+            dw2, db2 = torch.empty(32, 32, 3, 3, **f32), torch.empty(32, **f32)
+            call("dd_conv3x3_c32_wgrad", a1.data_ptr(), da2.data_ptr(), dw2.data_ptr(), db2.data_ptr(), ws.data_ptr(),
+                 ws_n, code, B, H, Wm, 1, impl, st)
+        da1 = torch.empty(B, H, Wm, 32, dtype=act_dtype, device=dev)
         if bits1 is not None:
             call("dd_conv3x3_c32_dgrad_bits", da2.data_ptr(), w2.data_ptr(), bits1.data_ptr(), da1.data_ptr(), code, B, H,
                  Wm, 1, impl, st)
@@ -249,10 +287,15 @@ class EncoderConvStack(torch.autograd.Function):
             call("dd_conv3x3_c32_dgrad", da2.data_ptr(), w2.data_ptr(), a1.data_ptr(), da1.data_ptr(), code, B, H, Wm, 1,
                  impl, st)
         del da2
-        dw1, db1 = torch.empty(32, 3, 3, 3, **f32), torch.empty(32, **f32)
-        call("dd_conv_c1_wgrad", inp.data_ptr(), in_flags, da1.data_ptr(), code, dw1.data_ptr(), db1.data_ptr(),
-             ws.data_ptr(), ws_n, B, H, Wm, impl, st)
-        return None, dw1, db1, dw2, db2, dw3, db3, None, None, None
+        if want_dw:
+            dw1, db1 = torch.empty(32, 3, 3, 3, **f32), torch.empty(32, **f32)
+            call("dd_conv_c1_wgrad", inp.data_ptr(), in_flags, da1.data_ptr(), code, dw1.data_ptr(), db1.data_ptr(),
+                 ws.data_ptr(), ws_n, B, H, Wm, impl, st)
+        if want_dx:
+            views = in_flags & _lib.IN_VIEWS
+            dx = torch.empty((B, 6, 3, H, Wm // 6) if views else (B, 3, H, Wm), **f32)
+            call("dd_conv_c1_dgrad", da1.data_ptr(), code, w1.data_ptr(), dx.data_ptr(), views, B, H, Wm, impl, st)
+        return dx, dw1, db1, dw2, db2, dw3, db3, None, None, None
 
 
 def encoder_conv_stack(inp, c1, c2, c3, act_dtype=torch.float32, c3_only=False, impl=IMPL_AUTO):
@@ -650,15 +693,47 @@ def decoder_deconv_stack(x, dc1, dc2, dc3, dc4, act_dtype=torch.float32):
 # --------------------------------------------------------------------------------------------
 # bounding-box model plumbing: camera extraction, tiling / concatenation, prob-space BCE
 # --------------------------------------------------------------------------------------------
-def view_extract(views, view: int, mode: int, dtype=torch.float32):
-    """One camera of every scene as an NHWC image with SpatialMappingCNN's rot90 / flip folded in
-    (spatial_bb/components.py:34-62).  mode 0 as is, 1 rot90(1,[2,3]), 2 rot90(1,[3,2]), 3 flip([2,3])."""
+class ViewExtract(torch.autograd.Function):
+    """Cameras of every scene as NHWC images, ``specs`` = ((view, mode), ...) with each view at most once.  Backward writes
+    ONE views-shaped gradient: every extracted view's slice by dd_view_extract_bwd, the others zero."""
+
+    @staticmethod
+    def forward(ctx, views, specs, dtype):
+        B, _, _, H, W = views.shape
+        outs = []
+        for view, mode in specs:
+            Ho, Wo = (W, H) if mode in (1, 2) else (H, W)
+            out = torch.empty(B, Ho, Wo, 3, dtype=dtype, device=views.device)
+            call("dd_view_extract", views.data_ptr(), out.data_ptr(), dtype_code(dtype), B, H, W, view, mode, stream_ptr())
+            outs.append(out)
+        ctx.specs, ctx.shape = specs, tuple(views.shape)
+        return tuple(outs)
+
+    @staticmethod
+    def backward(ctx, *grads):
+        B, _, _, H, W = ctx.shape
+        every_view = len(ctx.specs) == 6
+        d = (torch.empty if every_view else torch.zeros)(ctx.shape, dtype=torch.float32, device=grads[0].device)
+        for (view, mode), g in zip(ctx.specs, grads):
+            g = _c(g)
+            call("dd_view_extract_bwd", g.data_ptr(), dtype_code(g.dtype), d.data_ptr(), B, H, W, view, mode, stream_ptr())
+        return d, None, None
+
+
+def view_extract_all(views, specs, dtype=torch.float32):
+    """The cameras ``specs`` = ((view, mode), ...) of every scene as NHWC images with SpatialMappingCNN's rot90 / flip
+    folded in (spatial_bb/components.py:34-62); mode 0 as is, 1 rot90(1,[2,3]), 2 rot90(1,[3,2]), 3 flip([2,3]).
+    Differentiable in the views; each view may be extracted once."""
     views = as_view_batch(views)
-    B, _, _, H, W = views.shape
-    Ho, Wo = (W, H) if mode in (1, 2) else (H, W)
-    out = torch.empty(B, Ho, Wo, 3, dtype=dtype, device=views.device)
-    call("dd_view_extract", views.data_ptr(), out.data_ptr(), dtype_code(dtype), B, H, W, int(view), int(mode), stream_ptr())
-    return out
+    specs = tuple((int(v), int(m)) for v, m in specs)
+    if len({v for v, _ in specs}) != len(specs):
+        raise ValueError(f"view_extract_all: a view is extracted more than once in {specs}")
+    return ViewExtract.apply(views, specs, dtype)
+
+
+def view_extract(views, view: int, mode: int, dtype=torch.float32):
+    """One camera of every scene as an NHWC image (see view_extract_all)."""
+    return view_extract_all(views, ((view, mode),), dtype)[0]
 
 
 class TileNHWC(torch.autograd.Function):

@@ -58,6 +58,12 @@ int dd_stitch_mask_f32(const float* views, float* x, float* y, int B, int H, int
 /* Front-end for raw camera bytes (data_helper.py:109-114 ToTensor): views u8 [B,6,3,H,W] ->
  * mosaic f32 with value/255 (bit-identical to x.float()/255). */
 int dd_stitch_u8(const uint8_t* views, float* mosaic, int B, int H, int W, void* stream);
+/* Backward of the two stitches (autograd through wide_stitch_six_images / six_to_one_task):
+ * dviews [B,6,3,H,W] f32 = the inverse permutation of dmosaic [B,3,H,6W].  slot = -1: dd_stitch_f32's
+ * backward.  slot in [0,6): dd_stitch_mask_f32's -- the zeroed block of x passes no gradient, and
+ * view DD_VIEW_ORDER[slot] takes dy [B,3,H,W], the gradient of y (dy may be NULL: zero). */
+int dd_unstitch_f32(const float* dmosaic, const float* dy, float* dviews, int B, int H, int W, int slot,
+                    void* stream);
 /* ToTensor alone (data_helper.py:113): out[i] = float(in[i]) / 255, bit-identical, n elements of any layout. */
 int dd_u8_to_f32(const uint8_t* in, float* out, long long n, void* stream);
 
@@ -86,6 +92,16 @@ int dd_encoder_c1c2_fused_fwd(const void* in, int in_flags, const float* w1_oihw
 int dd_conv_c1_wgrad(const void* in, int in_flags, const void* dy, int dtype, float* dw,
                      float* db, void* workspace, size_t ws_bytes, int B, int H, int Wm, int impl,
                      void* stream);
+
+/* Image gradient of c1 (components.py:41, roadmap_bce_v2.py:53-64): what loss.backward() hands
+ * the camera views or the mosaic.  dx[c,h,w] = sum over o, kh, kw of dy[o, h+1-kh, w+1-kw] *
+ * w[o,c,kh,kw], zero outside the image; dy = dL/d(pre-activation of c1) (ReLU mask applied), NHWC
+ * [B,H,Wm,32] of `dtype`, 16-byte aligned.  dx fp32: with out_flags & DD_IN_VIEWS the views
+ * [B,6,3,H,Wm/6] (the inverse stitch folded into the stores), else the NCHW mosaic [B,3,H,Wm].
+ * DD_IN_U8: DD_ERR_UNSUPPORTED (bytes have no gradient).  bf16 with AUTO / TCGEN05: tensor cores
+ * (w read as bf16, as c1's forward reads it); fp32, or DD_IMPL_SIMT: CUDA cores, fp32 weights. */
+int dd_conv_c1_dgrad(const void* dy, int dtype, const float* w_oihw, float* dx, int out_flags, int B,
+                     int H, int Wm, int impl, void* stream);
 
 /* c2 / c3: 32->32, 3x3, pad 1, stride 1 or 2, + bias + ReLU; NHWC in [B,H,W,32] ->
  * NHWC out [B,Ho,Wo,32], Ho = (H-1)/stride+1.  The bf16 tensor-core kernels read their activations
@@ -212,6 +228,10 @@ int dd_conv2d_tc_supported(const dd_conv_desc* d, int dtype, int pass);
  *   (spatial_w_rm.py:131); bwd = g * (p - t) / max((1-p) p, 1e-12) / n. */
 int dd_view_extract(const float* views, void* out, int out_dtype, int B, int H, int W, int view, int mode,
                     void* stream);
+/* dd_view_extract_bwd: the backward of dd_view_extract.  dout NHWC [B,H',W',3] of dtype -> view
+ * `view` of the fp32 views gradient dviews [B,6,3,H,W]; only that view's elements are written. */
+int dd_view_extract_bwd(const void* dout, int dtype, float* dviews, int B, int H, int W, int view, int mode,
+                        void* stream);
 int dd_nhwc_place(void* small_, void* big, int dtype, int B, int h, int w, int c, int H, int W, int C,
                   int oy, int ox, int oc, int dir, void* stream);
 int dd_sigmoid_bwd(const void* dy, const void* y, void* out, int dtype, long long n, void* stream);
