@@ -321,16 +321,12 @@ bool conv_dil_tc_supported(int K, int N, int KT, int D) {
          (K == 32 && N == 64);
 }
 
-size_t conv_dil_tc_pack_bytes(int K, int N, int KT) { return (size_t)((K + 31) / 32) * KT * KT * N * 32 * 2; }
-
 // w: torch-layout fp32 weights; (sn, sk): strides of the produced / gathered channel index in it; flip: kh = KT-1-kappa
 int conv_dil_tc(const void* in, const float* w, long long sn, long long sk, int flip, const float* bias, const void* mask, void* out,
                 void* pack_ws, int B, int Hi, int Wi, int Ho, int Wo, int K, int N, int KT, int D, int sign, int off, int relu,
                 cudaStream_t st, int Kreal, int Nreal) {
   // Kreal < K: `in` carries K channels per pixel of which only the first Kreal exist in the weights (zero-padded pixels);
   // Nreal < N: the weights have Nreal produced channels, `out` / bias / mask carry N (the caller drops the padding)
-  if (Kreal <= 0 || Kreal > K) Kreal = K;
-  if (Nreal <= 0 || Nreal > N) Nreal = N;
   if (((reinterpret_cast<uintptr_t>(in) | reinterpret_cast<uintptr_t>(out) | reinterpret_cast<uintptr_t>(mask) |
         reinterpret_cast<uintptr_t>(pack_ws)) & 31) != 0)
     return fail(DD_ERR_ALIGNMENT, "conv_dil_tc: pointers must be 32-byte aligned");

@@ -254,8 +254,6 @@ int conv_dil_wgrad_tc(const void* in, const void* dout, float* dw, long long sn,
                       int Hi, int Wi, int Ho, int Wo, int K, int N, int KT, int D, int sign, int off, cudaStream_t st, int Kreal,
                       int Nreal) {
   // Kreal < K / Nreal < N: zero-padded pixels; only dw[n < Nreal][k < Kreal] exists
-  if (Kreal <= 0 || Kreal > K) Kreal = K;
-  if (Nreal <= 0 || Nreal > N) Nreal = N;
   if (((reinterpret_cast<uintptr_t>(in) | reinterpret_cast<uintptr_t>(dout)) & 15) != 0)
     return fail(DD_ERR_ALIGNMENT, "conv_dil_wgrad_tc: operands must be 16-byte aligned");
   WgdGeo g = make_geo(B, Ho, Wo, K, N, KT, D, sign, off);

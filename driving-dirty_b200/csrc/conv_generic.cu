@@ -331,7 +331,7 @@ static bool wtile_config(const WGeo& g, int taps, int& TT, int& TP, int& TQ, WTi
   TQ = g.cQ % 4 == 0 ? 4 : (g.cQ == 3 ? 3 : (g.cQ == 1 ? 1 : 0));
   if (TQ == 0) return false;
   TT = taps % 7 == 0 ? 7 : (taps <= 4 ? 4 : (taps % 8 == 0 ? 8 : 7));
-  if (TQ == 4 && TT == 8 && false) return false;
+  if (TT == 4 && TQ == 3) return false;     // not instantiated (launch_wgrad_cc): e.g. the decoder's dc4, 32 -> 3, 1 tap
   c.ntg = (taps + TT - 1) / TT; c.npg = (g.cP + TP - 1) / TP; c.nqg = (g.cQ + TQ - 1) / TQ;
   const int ngroups = c.ntg * c.npg * c.nqg;
   if (ngroups > 256) return false;
@@ -427,25 +427,6 @@ int launch_gather(const T* x, const float* wg, const float* bias, const T* mask,
 }
 
 template <typename T>
-int launch_wgrad_tile(const T* P, const T* Q, float* partial, const WGeo& g, int taps, int& slots, cudaStream_t st) {
-  int TT, TP, TQ, grid;
-  WTile c;
-  size_t smem;
-  if (!wtile_config(g, taps, TT, TP, TQ, c, smem, grid)) return -1000;
-  slots = grid * c.lanes;
-#define DD_WT(a, b, q)                                                                                             \
-  if (TT == a && TP == b && TQ == q) {                                                                             \
-    auto k = conv2d_wgrad_tile_kernel<T, a, b, q>;                                                                 \
-    if (int e = dd::set_smem(k, smem, dd::Carveout::kDefault, "conv2d wgrad tile")) return e;                      \
-    k<<<grid, 256, smem, st>>>(P, Q, partial, g, c);                                                               \
-    return dd::check_launch("conv2d_wgrad_tile");                                                                  \
-  }
-  DD_WT(7, 4, 4) DD_WT(7, 4, 1) DD_WT(7, 4, 3) DD_WT(8, 4, 4) DD_WT(4, 4, 4) DD_WT(4, 4, 1) DD_WT(8, 4, 3) DD_WT(8, 4, 1)
-#undef DD_WT
-  return -1000;
-}
-
-template <typename T>
 int launch_wgrad(const T* P, const T* Q, float* partial, const WGeo& g, int taps, int splits, cudaStream_t st) {
   dim3 grid(taps, splits);
   const int tp = (g.cP + 15) / 16, tq = (g.cQ + 15) / 16;
@@ -463,20 +444,44 @@ int launch_wgrad(const T* P, const T* Q, float* partial, const WGeo& g, int taps
 #undef DD_WG
   return dd::check_launch("conv2d_wgrad");
 }
+
+// CUDA-core weight-gradient partials: the all-taps register-tiled form where wtile_config finds a tiling (small channel
+// counts), else one CTA per (tap, pixel range).  slots = partial buffers written, for wgrad_fold_kernel.
+template <typename T>
+int launch_wgrad_cc(const T* P, const T* Q, float* partial, const WGeo& g, int taps, int splits, int& slots, cudaStream_t st) {
+  int TT, TP, TQ, grid;
+  WTile c;
+  size_t smem;
+  if (!wtile_config(g, taps, TT, TP, TQ, c, smem, grid)) {
+    slots = splits;
+    return launch_wgrad(P, Q, partial, g, taps, splits, st);
+  }
+  slots = grid * c.lanes;
+#define DD_WT(a, b, q)                                                                                             \
+  if (TT == a && TP == b && TQ == q) {                                                                             \
+    auto k = conv2d_wgrad_tile_kernel<T, a, b, q>;                                                                 \
+    if (int e = dd::set_smem(k, smem, dd::Carveout::kDefault, "conv2d wgrad tile")) return e;                      \
+    k<<<grid, 256, smem, st>>>(P, Q, partial, g, c);                                                               \
+    return dd::check_launch("conv2d_wgrad_tile");                                                                  \
+  }
+  DD_WT(7, 4, 4) DD_WT(7, 4, 1) DD_WT(7, 4, 3) DD_WT(8, 4, 4) DD_WT(4, 4, 4) DD_WT(4, 4, 1) DD_WT(8, 4, 3) DD_WT(8, 4, 1)
+#undef DD_WT
+  return dd::fail(DD_ERR_UNSUPPORTED, "conv2d wgrad tile: no instantiation for %d taps x %d x %d", TT, TP, TQ);
+}
 }  // namespace
 
-// tcgen05 path for the wide stride-1 (dilated) layers: conv_dil_tc.cu
+// tcgen05 kernels for the stride-1 (dilated) layers: conv_dil_tc.cu, conv_dil_wgrad_tc.cu.  K / N: gathered / produced
+// channels per pixel as launched, of which the first Kreal / Nreal exist in the weights (the rest are zero padding).
 namespace dd {
 bool conv_dil_tc_supported(int K, int N, int KT, int D);
-size_t conv_dil_tc_pack_bytes(int K, int N, int KT);
 int conv_dil_tc(const void* in, const float* w, long long sn, long long sk, int flip, const float* bias, const void* mask, void* out,
                 void* pack_ws, int B, int Hi, int Wi, int Ho, int Wo, int K, int N, int KT, int D, int sign, int off, int relu,
-                cudaStream_t st, int Kreal = 0, int Nreal = 0);
+                cudaStream_t st, int Kreal, int Nreal);
 bool conv_dil_wgrad_tc_supported(int K, int N, int KT, int D);
 size_t conv_dil_wgrad_tc_ws_bytes(int K, int N, int KT);
 int conv_dil_wgrad_tc(const void* in, const void* dout, float* dw, long long sn, long long sk, void* ws, size_t ws_bytes, int B,
-                      int Hi, int Wi, int Ho, int Wo, int K, int N, int KT, int D, int sign, int off, cudaStream_t st, int Kreal = 0,
-                      int Nreal = 0);
+                      int Hi, int Wi, int Ho, int Wo, int K, int N, int KT, int D, int sign, int off, cudaStream_t st, int Kreal,
+                      int Nreal);
 }  // namespace dd
 
 // ---- narrow layers on the tensor-core kernels: 8- / 16-channel pixels zero-padded to the kernels' 32 ------------------------
@@ -511,54 +516,58 @@ __global__ void bias_pad_kernel(const float* __restrict__ b, float* __restrict__
 }
 inline bool narrow(int c) { return c == 8 || c == 16; }
 inline int padded(int c) { return narrow(c) ? 32 : c; }
+size_t pad_slot(long long npix) { return ((size_t)npix * 64 + 1023) / 1024 * 1024; }   // one tensor in 32-channel bf16 pixels
+
+// ---- which engine runs a pass ------------------------------------------------------------------------------------------------
+// A pass (0 forward, 1 input gradient, 2 weight gradient) runs on the tensor cores when the layer is bf16, stride 1, a square
+// filter with one dilation and padding for both axes, and its channel counts, after the padding below, are ones the kernels
+// take.  Everything else, and fp32 (the parity path), runs on the CUDA-core kernels above.
+struct TcPlan {
+  bool ok = false;
+  int K = 0, N = 0;             // gathered / produced channels as launched: x / y, dy / dx, x / dy
+  int Kreal = 0, Nreal = 0;     // as in the layer; K > Kreal or N > Nreal: that tensor goes through a padded copy
+  long long sn = 0, sk = 0;     // strides of the produced / gathered channel index in the torch-layout weights
+  int flip = 0, sign = 0, off = 0;
+  // workspace: [core_ws_bytes | dy's copy, or the forward's 16-channel y | x's copy | padded bias]; offsets past core_ws_bytes
+  size_t x_pad = 0, bias_pad = 0;
+  bool padded() const { return ok && (K != Kreal || N != Nreal); }
+};
+
+TcPlan tc_plan(const dd_conv_desc* d, int dtype, int pass, int act) {
+  TcPlan p;
+  if (dtype != DD_BF16 || d->sh != 1 || d->sw != 1 || d->kh != d->kw || d->dh != d->dw || d->ph != d->pw) return p;
+  if (pass == 0 && act == 2) return p;                  // the kernels' epilogue has bias and ReLU, no sigmoid
+  const bool dgrad = pass == 1;
+  p.Kreal = dgrad ? d->Cout : d->Cin;
+  p.Nreal = dgrad ? d->Cin : d->Cout;
+  p.K = padded(p.Kreal);                                // 8 / 16 gathered channels -> 32 in every pass
+  // produced channels: the weight gradient pads 8 / 16 -> 32 (its kernel takes 32 or 64); the forward pads 8 -> 16 (the
+  // narrowest instantiation) and narrows the result; the input gradient pads none (no layer here needs an 8-channel dx)
+  p.N = pass == 2 ? padded(p.Nreal) : (pass == 0 && p.Nreal == 8 ? 16 : p.Nreal);
+  p.ok = pass == 2 ? dd::conv_dil_wgrad_tc_supported(p.K, p.N, d->kh, d->dh) : dd::conv_dil_tc_supported(p.K, p.N, d->kh, d->dh);
+  // Conv2d weights are [Cout][Cin][t], ConvTranspose2d [Cin][Cout][t].  The ConvT forward and the Conv input gradient gather
+  // from h - D*kh + p (flip 0, sign -1); the Conv forward and the ConvT input gradient from h + D*kh - p (flip 1, sign +1).
+  // The weight gradient takes the forward's strides, sign and offset.
+  const bool convT_gather = d->transposed != dgrad;
+  const long long T = (long long)d->kh * d->kw;
+  p.sn = convT_gather ? T : p.Kreal * T;
+  p.sk = convT_gather ? p.Nreal * T : T;
+  p.flip = !convT_gather;
+  p.sign = convT_gather ? -1 : +1;
+  p.off = convT_gather ? d->ph : -d->ph;
+  const size_t y_slot = narrow(d->Cout) ? pad_slot((long long)d->B * d->Ho * d->Wo) : 0;
+  p.x_pad = y_slot;
+  p.bias_pad = y_slot + (narrow(d->Cin) ? pad_slot((long long)d->B * d->Hi * d->Wi) : 0);
+  return p;
+}
 }  // namespace
 
-static bool tc_wgrad_ok(const dd_conv_desc* d, int dtype) {
-  if (dtype != DD_BF16 || d->sh != 1 || d->sw != 1 || d->kh != d->kw || d->dh != d->dw || d->ph != d->pw) return false;
-  return dd::conv_dil_wgrad_tc_supported(d->Cin, d->Cout, d->kh, d->dh);
-}
-// the same with 8- / 16-channel tensors padded to 32 channels first
-static bool tc_wgrad_padded_ok(const dd_conv_desc* d, int dtype) {
-  if (dtype != DD_BF16 || d->sh != 1 || d->sw != 1 || d->kh != d->kw || d->dh != d->dw || d->ph != d->pw) return false;
-  if (!narrow(d->Cin) && !narrow(d->Cout)) return false;
-  return dd::conv_dil_wgrad_tc_supported(padded(d->Cin), padded(d->Cout), d->kh, d->dh);
-}
-// forward: gathered channels 8 / 16 -> 32; produced channels 8 -> 16 (written to a temporary, then narrowed)
-static bool tc_fwd_padded_ok(const dd_conv_desc* d, int dtype, int act) {
-  if (dtype != DD_BF16 || d->sh != 1 || d->sw != 1 || d->kh != d->kw || d->dh != d->dw || d->ph != d->pw || act == 2) return false;
-  if (!narrow(d->Cin) && d->Cout != 8) return false;
-  return dd::conv_dil_tc_supported(padded(d->Cin), d->Cout == 8 ? 16 : d->Cout, d->kh, d->dh);
-}
-static bool tc_dgrad_padded_ok(const dd_conv_desc* d, int dtype) {
-  if (dtype != DD_BF16 || d->sh != 1 || d->sw != 1 || d->kh != d->kw || d->dh != d->dw || d->ph != d->pw) return false;
-  return narrow(d->Cout) && dd::conv_dil_tc_supported(32, d->Cin, d->kh, d->dh);
-}
-
-// pass: 0 forward, 1 input gradient.  bf16, stride 1, square filter of 3 or 7 taps, one dilation and padding for both axes.
-static bool tc_ok(const dd_conv_desc* d, int dtype, int pass, int act) {
-  if (dtype != DD_BF16 || d->sh != 1 || d->sw != 1 || d->kh != d->kw || d->dh != d->dw || d->ph != d->pw) return false;
-  if (pass == 0 && act == 2) return false;
-  const int K = pass == 0 ? d->Cin : d->Cout, N = pass == 0 ? d->Cout : d->Cin;
-  return dd::conv_dil_tc_supported(K, N, d->kh, d->dh);
-}
-
 extern "C" int dd_conv2d_tc_supported(const dd_conv_desc* d, int dtype, int pass) {
-  if (!d || !desc_ok(d)) return 0;
-  if (pass == 2) return tc_wgrad_ok(d, dtype) || tc_wgrad_padded_ok(d, dtype);
-  return tc_ok(d, dtype, pass, 0) || (pass == 1 ? tc_dgrad_padded_ok(d, dtype) : tc_fwd_padded_ok(d, dtype, 0));
+  return desc_ok(d) && tc_plan(d, dtype, pass, 0).ok;
 }
 
-// everything but the padded copies; they sit behind this (1024-byte aligned)
-static size_t core_ws_bytes(const dd_conv_desc* d);
-static size_t pad_ws_bytes(const dd_conv_desc* d) {
-  if (!tc_wgrad_padded_ok(d, DD_BF16) && !tc_dgrad_padded_ok(d, DD_BF16) && !tc_fwd_padded_ok(d, DD_BF16, 0)) return 0;
-  const size_t np_out = (size_t)d->B * d->Ho * d->Wo, np_in = (size_t)d->B * d->Hi * d->Wi;
-  return (narrow(d->Cout) ? np_out * 64 + 1024 : 0) + (narrow(d->Cin) ? np_in * 64 + 1024 : 0) + 2048;
-}
-extern "C" size_t dd_conv2d_workspace_bytes(const dd_conv_desc* d) {
-  if (!desc_ok(d)) return 256;
-  return core_ws_bytes(d) + pad_ws_bytes(d);
-}
+// CUDA-core weights / weight-gradient partials or the tensor-core weight gradient's partials, then the bias gradient's
+// channel sums; the padded copies sit behind all of it (1024-byte aligned)
 static size_t core_ws_bytes(const dd_conv_desc* d) {
   const long long np_out = (long long)d->B * d->Ho * d->Wo, np_in = (long long)d->B * d->Hi * d->Wi;
   const long long pivot = d->transposed ? np_in : np_out;
@@ -566,10 +575,21 @@ static size_t core_ws_bytes(const dd_conv_desc* d) {
   const size_t chan = (size_t)kChanBlocks * d->Cout * sizeof(double) + 8;
   const size_t tile_partial = (size_t)2 * dd::kSMs * 256 * 128 * sizeof(float);   // all-taps form: slots x taps x cP x cQ <= CTAs x 256 threads x 128 accumulators
   const size_t a = wg_bytes(d), b = (partial > tile_partial ? partial : tile_partial) + chan;
-  const size_t c = tc_wgrad_ok(d, DD_BF16) ? dd::conv_dil_wgrad_tc_ws_bytes(d->Cin, d->Cout, d->kh) + chan
-                   : tc_wgrad_padded_ok(d, DD_BF16) ? dd::conv_dil_wgrad_tc_ws_bytes(padded(d->Cin), padded(d->Cout), d->kh) + chan : 0;
+  const TcPlan wgrad = tc_plan(d, DD_BF16, 2, 0);
+  const size_t c = wgrad.ok ? dd::conv_dil_wgrad_tc_ws_bytes(wgrad.K, wgrad.N, d->kh) + chan : 0;
   const size_t m = a > b ? a : b;
   return ((m > c ? m : c) + 256 + 1023) / 1024 * 1024;
+}
+
+extern "C" size_t dd_conv2d_workspace_bytes(const dd_conv_desc* d) {
+  if (!desc_ok(d)) return 256;
+  size_t pad = 0;
+  if (tc_plan(d, DD_BF16, 0, 0).padded() || tc_plan(d, DD_BF16, 1, 0).padded() || tc_plan(d, DD_BF16, 2, 0).padded()) {
+    // room for the copies at the offsets tc_plan gives
+    const size_t np_out = (size_t)d->B * d->Ho * d->Wo, np_in = (size_t)d->B * d->Hi * d->Wi;
+    pad = (narrow(d->Cout) ? np_out * 64 + 1024 : 0) + (narrow(d->Cin) ? np_in * 64 + 1024 : 0) + 2048;
+  }
+  return core_ws_bytes(d) + pad;
 }
 
 extern "C" int dd_conv2d_fwd(const void* x, const float* w, const float* bias, void* y, const dd_conv_desc* d, int dtype,
@@ -580,52 +600,34 @@ extern "C" int dd_conv2d_fwd(const void* x, const float* w, const float* bias, v
   DD_REQUIRE(ws_bytes >= wg_bytes(d), DD_ERR_WORKSPACE, "dd_conv2d_fwd: workspace %zu < %zu", ws_bytes, wg_bytes(d));
   DD_REQUIRE(act >= 0 && act <= 2, DD_ERR_BAD_ARG, "dd_conv2d_fwd: act %d", act);
   cudaStream_t st = dd::as_stream(stream);
-  const int taps = d->kh * d->kw;
-  if (tc_ok(d, dtype, 0, act)) {
-    // ConvTranspose2d [Cin][Cout][kh][kw]: gathers from h - D*kh + p;  Conv2d [Cout][Cin][kh][kw]: from h + D*kh - p
-    const long long T = taps;
-    if (d->transposed)
-      return dd::conv_dil_tc(x, w, T, (long long)d->Cout * T, 0, bias, nullptr, y, workspace, d->B, d->Hi, d->Wi, d->Ho, d->Wo, d->Cin,
-                             d->Cout, d->kh, d->dh, -1, d->ph, act == 1, st);
-    return dd::conv_dil_tc(x, w, (long long)d->Cin * T, T, 1, bias, nullptr, y, workspace, d->B, d->Hi, d->Wi, d->Ho, d->Wo, d->Cin,
-                           d->Cout, d->kh, d->dh, +1, -d->ph, act == 1, st);
-  }
-  if (tc_fwd_padded_ok(d, dtype, act)) {
-    DD_REQUIRE(ws_bytes >= dd_conv2d_workspace_bytes(d), DD_ERR_WORKSPACE, "dd_conv2d_fwd: workspace %zu < %zu", ws_bytes,
-               dd_conv2d_workspace_bytes(d));
-    const long long np_out = (long long)d->B * d->Ho * d->Wo, np_in = (long long)d->B * d->Hi * d->Wi, T = taps;
-    const int Kp = padded(d->Cin), Np = d->Cout == 8 ? 16 : d->Cout;
-    // behind the core workspace: [padded bias | 16-channel output (if narrowed; it fits the slot sized for 32) | padded input]
-    uint8_t* pb = (uint8_t*)workspace + core_ws_bytes(d);
-    float* bias_p = (float*)pb;
-    pb += 1024;
-    void* yt = y;
-    if (Np != d->Cout) { yt = pb; pb += ((size_t)np_out * 64 + 1023) / 1024 * 1024; }
+  const TcPlan p = tc_plan(d, dtype, 0, act);
+  if (p.ok) {
+    if (p.padded())
+      DD_REQUIRE(ws_bytes >= dd_conv2d_workspace_bytes(d), DD_ERR_WORKSPACE, "dd_conv2d_fwd: workspace %zu < %zu", ws_bytes,
+                 dd_conv2d_workspace_bytes(d));
+    uint8_t* pad = p.padded() ? (uint8_t*)workspace + core_ws_bytes(d) : nullptr;
     const void* xin = x;
-    if (Kp != d->Cin) {
-      if (int e = pad32(x, pb, np_in, d->Cin, st)) return e;
-      xin = pb;
+    if (p.K != p.Kreal) {
+      if (int e = pad32(x, pad + p.x_pad, (long long)d->B * d->Hi * d->Wi, d->Cin, st)) return e;
+      xin = pad + p.x_pad;
     }
+    void* yt = p.N != p.Nreal ? (void*)pad : y;          // 8 produced channels: 16-channel pixels first, narrowed below
     const float* bptr = bias;
-    if (Np != d->Cout && bias) {
-      bias_pad_kernel<<<1, 32, 0, st>>>(bias, bias_p, d->Cout, Np);
+    if (p.N != p.Nreal && bias) {
+      bias_pad_kernel<<<1, 32, 0, st>>>(bias, (float*)(pad + p.bias_pad), d->Cout, p.N);
       if (int e = dd::check_launch("conv2d_bias_pad")) return e;
-      bptr = bias_p;
+      bptr = (const float*)(pad + p.bias_pad);
     }
-    int e = d->transposed
-                ? dd::conv_dil_tc(xin, w, T, (long long)d->Cout * T, 0, bptr, nullptr, yt, workspace, d->B, d->Hi, d->Wi, d->Ho, d->Wo, Kp,
-                                  Np, d->kh, d->dh, -1, d->ph, act == 1, st, d->Cin, d->Cout)
-                : dd::conv_dil_tc(xin, w, (long long)d->Cin * T, T, 1, bptr, nullptr, yt, workspace, d->B, d->Hi, d->Wi, d->Ho, d->Wo, Kp,
-                                  Np, d->kh, d->dh, +1, -d->ph, act == 1, st, d->Cin, d->Cout);
-    if (e) return e;
-    if (Np != d->Cout) {
-      const long long want = (np_out + 255) / 256;
-      chan_unpad16to8_kernel<<<(int)(want < dd::kSMs * 16 ? want : dd::kSMs * 16), 256, 0, st>>>((const __nv_bfloat16*)yt, (__nv_bfloat16*)y, np_out);
-      return dd::check_launch("conv2d_chan_unpad");
-    }
-    return 0;
+    if (int e = dd::conv_dil_tc(xin, w, p.sn, p.sk, p.flip, bptr, nullptr, yt, workspace, d->B, d->Hi, d->Wi, d->Ho, d->Wo, p.K, p.N,
+                                d->kh, d->dh, p.sign, p.off, act == 1, st, p.Kreal, p.Nreal))
+      return e;
+    if (p.N == p.Nreal) return 0;
+    const long long np_out = (long long)d->B * d->Ho * d->Wo, want = (np_out + 255) / 256;
+    chan_unpad16to8_kernel<<<(int)(want < dd::kSMs * 16 ? want : dd::kSMs * 16), 256, 0, st>>>((const __nv_bfloat16*)yt, (__nv_bfloat16*)y, np_out);
+    return dd::check_launch("conv2d_chan_unpad");
   }
   float* wg = (float*)workspace;
+  const int taps = d->kh * d->kw;
   // conv weights are [Cout][Cin][t] (need wg[t][ci][co] = w[co][ci][t]: swap); convT weights are [Cin][Cout][t]
   wprep_kernel<<<64, 256, 0, st>>>(w, wg, d->Cin, d->Cout, taps, d->transposed ? 0 : 1);
   if (int e = dd::check_launch("conv2d_wprep")) return e;
@@ -643,29 +645,21 @@ extern "C" int dd_conv2d_dgrad(const void* dy, const float* w, const void* x_mas
   DD_REQUIRE(dy && w && dx && workspace, DD_ERR_BAD_ARG, "dd_conv2d_dgrad: null pointer");
   DD_REQUIRE(ws_bytes >= wg_bytes(d), DD_ERR_WORKSPACE, "dd_conv2d_dgrad: workspace %zu < %zu", ws_bytes, wg_bytes(d));
   cudaStream_t st = dd::as_stream(stream);
-  const int taps = d->kh * d->kw;
-  if (tc_ok(d, dtype, 1, 0)) {
-    // gathered tensor = dy (Cout channels), produced = dx (Cin channels)
-    const long long T = taps;
-    if (d->transposed)
-      return dd::conv_dil_tc(dy, w, (long long)d->Cout * T, T, 1, nullptr, x_mask, dx, workspace, d->B, d->Ho, d->Wo, d->Hi, d->Wi,
-                             d->Cout, d->Cin, d->kh, d->dh, +1, -d->ph, 0, st);
-    return dd::conv_dil_tc(dy, w, T, (long long)d->Cin * T, 0, nullptr, x_mask, dx, workspace, d->B, d->Ho, d->Wo, d->Hi, d->Wi, d->Cout,
-                           d->Cin, d->kh, d->dh, -1, d->ph, 0, st);
-  }
-  if (tc_dgrad_padded_ok(d, dtype)) {
-    DD_REQUIRE(ws_bytes >= dd_conv2d_workspace_bytes(d), DD_ERR_WORKSPACE, "dd_conv2d_dgrad: workspace %zu < %zu", ws_bytes,
-               dd_conv2d_workspace_bytes(d));
-    uint8_t* dyp = (uint8_t*)workspace + core_ws_bytes(d);
-    if (int e = pad32(dy, dyp, (long long)d->B * d->Ho * d->Wo, d->Cout, st)) return e;
-    const long long T = taps;
-    if (d->transposed)
-      return dd::conv_dil_tc(dyp, w, (long long)d->Cout * T, T, 1, nullptr, x_mask, dx, workspace, d->B, d->Ho, d->Wo, d->Hi, d->Wi,
-                             32, d->Cin, d->kh, d->dh, +1, -d->ph, 0, st, d->Cout);
-    return dd::conv_dil_tc(dyp, w, T, (long long)d->Cin * T, 0, nullptr, x_mask, dx, workspace, d->B, d->Ho, d->Wo, d->Hi, d->Wi, 32,
-                           d->Cin, d->kh, d->dh, -1, d->ph, 0, st, d->Cout);
+  const TcPlan p = tc_plan(d, dtype, 1, 0);
+  if (p.ok) {
+    const void* dyin = dy;
+    if (p.K != p.Kreal) {
+      DD_REQUIRE(ws_bytes >= dd_conv2d_workspace_bytes(d), DD_ERR_WORKSPACE, "dd_conv2d_dgrad: workspace %zu < %zu", ws_bytes,
+                 dd_conv2d_workspace_bytes(d));
+      uint8_t* dyp = (uint8_t*)workspace + core_ws_bytes(d);
+      if (int e = pad32(dy, dyp, (long long)d->B * d->Ho * d->Wo, d->Cout, st)) return e;
+      dyin = dyp;
+    }
+    return dd::conv_dil_tc(dyin, w, p.sn, p.sk, p.flip, nullptr, x_mask, dx, workspace, d->B, d->Ho, d->Wo, d->Hi, d->Wi, p.K, p.N,
+                           d->kh, d->dh, p.sign, p.off, 0, st, p.Kreal, p.Nreal);
   }
   float* wg = (float*)workspace;
+  const int taps = d->kh * d->kw;
   // gathered tensor = dy (Cout channels), produced = dx (Cin channels): wg[t][co][ci]
   wprep_kernel<<<64, 256, 0, st>>>(w, wg, d->Cout, d->Cin, taps, d->transposed ? 1 : 0);
   if (int e = dd::check_launch("conv2d_wprep")) return e;
@@ -687,79 +681,56 @@ extern "C" int dd_conv2d_wgrad(const void* x, const void* dy, float* dw, float* 
   cudaStream_t st = dd::as_stream(stream);
   const int taps = d->kh * d->kw;
   const long long np_out = (long long)d->B * d->Ho * d->Wo, np_in = (long long)d->B * d->Hi * d->Wi;
-  const long long pivot = d->transposed ? np_in : np_out;
-  const bool tc_plain = tc_wgrad_ok(d, dtype), tc_pad = !tc_plain && tc_wgrad_padded_ok(d, dtype);
-  if (tc_plain || tc_pad) {
-    // tensor-core path (csrc/conv_dil_wgrad_tc.cu): partials first, then the bias gradient's channel sums
-    const long long T = taps;
-    const int Kp = padded(d->Cin), Np = padded(d->Cout);
-    const size_t tcb = dd::conv_dil_wgrad_tc_ws_bytes(Kp, Np, d->kh);
+  const TcPlan p = tc_plan(d, dtype, 2, 0);
+  void* chan;                                                // the bias gradient's per-CTA sums, behind the partials
+  if (p.ok) {
+    const size_t tcb = dd::conv_dil_wgrad_tc_ws_bytes(p.K, p.N, d->kh);
+    uint8_t* pad = (uint8_t*)workspace + core_ws_bytes(d);
     const void *xin = x, *dout = dy;
-    if (tc_pad) {                                            // narrow tensors -> 32-channel pixels behind the core workspace
-      uint8_t* pb = (uint8_t*)workspace + core_ws_bytes(d);
-      if (narrow(d->Cout)) {
-        if (int e = pad32(dy, pb, np_out, d->Cout, st)) return e;
-        dout = pb;
-        pb += ((size_t)np_out * 64 + 1023) / 1024 * 1024;
-      }
-      if (narrow(d->Cin)) {
-        if (int e = pad32(x, pb, np_in, d->Cin, st)) return e;
-        xin = pb;
-      }
+    if (p.N != p.Nreal) {
+      if (int e = pad32(dy, pad, np_out, d->Cout, st)) return e;
+      dout = pad;
     }
-    int e = d->transposed
-                ? dd::conv_dil_wgrad_tc(xin, dout, dw, T, (long long)d->Cout * T, workspace, tcb, d->B, d->Hi, d->Wi, d->Ho, d->Wo, Kp,
-                                        Np, d->kh, d->dh, -1, d->ph, st, d->Cin, d->Cout)
-                : dd::conv_dil_wgrad_tc(xin, dout, dw, (long long)d->Cin * T, T, workspace, tcb, d->B, d->Hi, d->Wi, d->Ho, d->Wo, Kp,
-                                        Np, d->kh, d->dh, +1, -d->ph, st, d->Cin, d->Cout);
+    if (p.K != p.Kreal) {
+      if (int e = pad32(x, pad + p.x_pad, np_in, d->Cin, st)) return e;
+      xin = pad + p.x_pad;
+    }
+    if (int e = dd::conv_dil_wgrad_tc(xin, dout, dw, p.sn, p.sk, workspace, tcb, d->B, d->Hi, d->Wi, d->Ho, d->Wo, p.K, p.N, d->kh,
+                                      d->dh, p.sign, p.off, st, p.Kreal, p.Nreal))
+      return e;
+    chan = (uint8_t*)workspace + tcb;
+  } else {
+    const long long pivot = d->transposed ? np_in : np_out;
+    const int splits = wgrad_splits(d, pivot);
+    WGeo g;
+    g.B = d->B;
+    g.kh = d->kh; g.kw = d->kw; g.sh = d->sh; g.sw = d->sw; g.ph = d->ph; g.pw = d->pw; g.dh = d->dh; g.dw = d->dw;
+    g.pix_per_split = ((pivot + splits - 1) / splits + 31) / 32 * 32;
+    const void *Pp, *Qp;
+    if (!d->transposed) { g.cP = d->Cout; g.cQ = d->Cin; g.Hp = d->Ho; g.Wp = d->Wo; g.Hq = d->Hi; g.Wq = d->Wi; Pp = dy; Qp = x; }
+    else { g.cP = d->Cin; g.cQ = d->Cout; g.Hp = d->Hi; g.Wp = d->Wi; g.Hq = d->Ho; g.Wq = d->Wo; Pp = x; Qp = dy; }
+    float* partial = (float*)workspace;
+    int slots;
+    if (dtype != DD_F32 && dtype != DD_BF16) return dd::fail(DD_ERR_UNSUPPORTED, "dd_conv2d_wgrad: dtype %d", dtype);
+    const int e = dtype == DD_F32
+                      ? launch_wgrad_cc<float>((const float*)Pp, (const float*)Qp, partial, g, taps, splits, slots, st)
+                      : launch_wgrad_cc<__nv_bfloat16>((const __nv_bfloat16*)Pp, (const __nv_bfloat16*)Qp, partial, g, taps, splits, slots, st);
     if (e) return e;
-    if (db) {
-      double* cpart = reinterpret_cast<double*>(((uintptr_t)((uint8_t*)workspace + tcb) + 7) & ~(uintptr_t)7);
-      const int lanes = 256 / d->Cout > 0 ? 256 / d->Cout : 1;
-      const long long want = (np_out + lanes - 1) / lanes;
-      const int nblk = (int)(want < kChanBlocks ? want : kChanBlocks);
-      chansum_kernel<__nv_bfloat16><<<nblk, 256, 0, st>>>((const __nv_bfloat16*)dy, np_out, d->Cout, cpart);
-      if (int e3 = dd::check_launch("conv2d_chansum")) return e3;
-      chansum_fold_kernel<<<(d->Cout + 255) / 256, 256, 0, st>>>(cpart, nblk, d->Cout, db);
-      return dd::check_launch("conv2d_chansum_fold");
-    }
-    return 0;
+    const int n = taps * d->Cin * d->Cout;
+    wgrad_fold_kernel<<<(n + 255) / 256 < 1184 ? (n + 255) / 256 : 1184, 256, 0, st>>>(partial, dw, taps, d->Cin * d->Cout, slots);
+    if (int e2 = dd::check_launch("conv2d_wgrad_fold")) return e2;
+    chan = partial + (size_t)slots * n;
   }
-  const int splits = wgrad_splits(d, pivot);
-  WGeo g;
-  g.B = d->B;
-  g.kh = d->kh; g.kw = d->kw; g.sh = d->sh; g.sw = d->sw; g.ph = d->ph; g.pw = d->pw; g.dh = d->dh; g.dw = d->dw;
-  g.pix_per_split = ((pivot + splits - 1) / splits + 31) / 32 * 32;
-  const void *Pp, *Qp;
-  if (!d->transposed) { g.cP = d->Cout; g.cQ = d->Cin; g.Hp = d->Ho; g.Wp = d->Wo; g.Hq = d->Hi; g.Wq = d->Wi; Pp = dy; Qp = x; }
-  else { g.cP = d->Cin; g.cQ = d->Cout; g.Hp = d->Hi; g.Wp = d->Wi; g.Hq = d->Ho; g.Wq = d->Wo; Pp = x; Qp = dy; }
-  float* partial = (float*)workspace;
-  int e, slots = splits;
-  if (dtype != DD_F32 && dtype != DD_BF16) return dd::fail(DD_ERR_UNSUPPORTED, "dd_conv2d_wgrad: dtype %d", dtype);
-  // the all-taps register-tiled form where a tiling exists (small channel counts); else one CTA per (tap, pixel range)
-  e = dtype == DD_F32 ? launch_wgrad_tile<float>((const float*)Pp, (const float*)Qp, partial, g, taps, slots, st)
-                      : launch_wgrad_tile<__nv_bfloat16>((const __nv_bfloat16*)Pp, (const __nv_bfloat16*)Qp, partial, g, taps, slots, st);
-  if (e == -1000) {
-    slots = splits;
-    e = dtype == DD_F32 ? launch_wgrad<float>((const float*)Pp, (const float*)Qp, partial, g, taps, splits, st)
-                        : launch_wgrad<__nv_bfloat16>((const __nv_bfloat16*)Pp, (const __nv_bfloat16*)Qp, partial, g, taps, splits, st);
-  }
-  if (e) return e;
-  const int n = taps * d->Cin * d->Cout;
-  wgrad_fold_kernel<<<(n + 255) / 256 < 1184 ? (n + 255) / 256 : 1184, 256, 0, st>>>(partial, dw, taps, d->Cin * d->Cout, slots);
-  if (int e2 = dd::check_launch("conv2d_wgrad_fold")) return e2;
-  if (db) {
-    double* cpart = reinterpret_cast<double*>(((uintptr_t)(partial + (size_t)slots * n) + 7) & ~(uintptr_t)7);
-    const int lanes = 256 / d->Cout > 0 ? 256 / d->Cout : 1;
-    const long long want = (np_out + lanes - 1) / lanes;
-    const int nblk = (int)(want < kChanBlocks ? want : kChanBlocks);
-    if (dtype == DD_F32) chansum_kernel<float><<<nblk, 256, 0, st>>>((const float*)dy, np_out, d->Cout, cpart);
-    else chansum_kernel<__nv_bfloat16><<<nblk, 256, 0, st>>>((const __nv_bfloat16*)dy, np_out, d->Cout, cpart);
-    if (int e3 = dd::check_launch("conv2d_chansum")) return e3;
-    chansum_fold_kernel<<<(d->Cout + 255) / 256, 256, 0, st>>>(cpart, nblk, d->Cout, db);
-    return dd::check_launch("conv2d_chansum_fold");
-  }
-  return 0;
+  if (!db) return 0;
+  double* cpart = reinterpret_cast<double*>(((uintptr_t)chan + 7) & ~(uintptr_t)7);
+  const int lanes = 256 / d->Cout > 0 ? 256 / d->Cout : 1;
+  const long long want = (np_out + lanes - 1) / lanes;
+  const int nblk = (int)(want < kChanBlocks ? want : kChanBlocks);
+  if (dtype == DD_F32) chansum_kernel<float><<<nblk, 256, 0, st>>>((const float*)dy, np_out, d->Cout, cpart);
+  else chansum_kernel<__nv_bfloat16><<<nblk, 256, 0, st>>>((const __nv_bfloat16*)dy, np_out, d->Cout, cpart);
+  if (int e = dd::check_launch("conv2d_chansum")) return e;
+  chansum_fold_kernel<<<(d->Cout + 255) / 256, 256, 0, st>>>(cpart, nblk, d->Cout, db);
+  return dd::check_launch("conv2d_chansum_fold");
 }
 
 // ================================================================================================

@@ -557,7 +557,6 @@ int conv3x3_c32_fwd_tc(const void* in, const float* w, const float* bias, void* 
                        int stride, int mode, const void* mask, uint32_t* bits, cudaStream_t st);
 int conv3x3_c32_wgrad_tc(const void* x, const void* dy, float* dw, float* db, void* ws, size_t ws_bytes, int B,
                          int H, int W, int stride, cudaStream_t st);
-bool conv_tc_supported(int H, int W, int stride, int mode);
 int conv_c1_fwd_tc(const void* in, int in_flags, const float* w, const float* bias, void* out, uint32_t* bits, int B, int H,
                    int Wm, cudaStream_t st);
 int enc_c1c2_fused_fwd_tc(const void* in, int in_flags, const float* w1, const float* b1, const float* w2, const float* b2,
@@ -577,11 +576,8 @@ extern "C" int dd_conv3x3_c32_fwd(const void* in, const float* w_oihw, const flo
   DD_REQUIRE((uintptr_t)in % 16 == 0 && (uintptr_t)out % 16 == 0, DD_ERR_ALIGNMENT, "dd_conv3x3_c32_fwd: alignment");
   if (B == 0) return 0;
   cudaStream_t st = dd::as_stream(stream);
-  if (dtype == DD_BF16 && impl != DD_IMPL_SIMT) {
-    if (dd::conv_tc_supported(H, W, stride, 0))
-      return dd::conv3x3_c32_fwd_tc(in, w_oihw, bias, out, B, H, W, stride, 0, nullptr, nullptr, st);
-    DD_REQUIRE(impl != DD_IMPL_TCGEN05, DD_ERR_UNSUPPORTED, "dd_conv3x3_c32_fwd: tcgen05 path unsupported for H=%d W=%d stride=%d", H, W, stride);
-  }
+  if (dtype == DD_BF16 && impl != DD_IMPL_SIMT)
+    return dd::conv3x3_c32_fwd_tc(in, w_oihw, bias, out, B, H, W, stride, 0, nullptr, nullptr, st);
   DD_REQUIRE(!(dtype == DD_F32 && impl == DD_IMPL_TCGEN05), DD_ERR_UNSUPPORTED, "tcgen05 conv is bf16 only");
   if (dtype == DD_F32) return conv_fwd_simt<float>((const float*)in, w_oihw, bias, (float*)out, B, H, W, stride, st);
   if (dtype == DD_BF16)
@@ -596,11 +592,8 @@ extern "C" int dd_conv3x3_c32_dgrad(const void* dy, const float* w_oihw, const v
   DD_REQUIRE(stride == 1 || stride == 2, DD_ERR_UNSUPPORTED, "dd_conv3x3_c32_dgrad: stride %d", stride);
   if (B == 0) return 0;
   cudaStream_t st = dd::as_stream(stream);
-  if (dtype == DD_BF16 && impl != DD_IMPL_SIMT) {
-    if (dd::conv_tc_supported(H, W, stride, 1))
-      return dd::conv3x3_c32_fwd_tc(dy, w_oihw, nullptr, dx, B, H, W, stride, 1, x, nullptr, st);
-    DD_REQUIRE(impl != DD_IMPL_TCGEN05, DD_ERR_UNSUPPORTED, "dd_conv3x3_c32_dgrad: tcgen05 path unsupported here");
-  }
+  if (dtype == DD_BF16 && impl != DD_IMPL_SIMT)
+    return dd::conv3x3_c32_fwd_tc(dy, w_oihw, nullptr, dx, B, H, W, stride, 1, x, nullptr, st);
   DD_REQUIRE(!(dtype == DD_F32 && impl == DD_IMPL_TCGEN05), DD_ERR_UNSUPPORTED, "tcgen05 conv is bf16 only");
   if (dtype == DD_F32)
     return conv_dgrad_simt<float>((const float*)dy, w_oihw, (const float*)x, (float*)dx, B, H, W, stride, st);
@@ -616,9 +609,8 @@ extern "C" int dd_conv3x3_c32_fwd_bits(const void* in, const float* w_oihw, cons
   DD_REQUIRE(in && w_oihw && bias && out && bits, DD_ERR_BAD_ARG, "dd_conv3x3_c32_fwd_bits: null pointer");
   DD_REQUIRE(B >= 0 && H > 0 && W > 0, DD_ERR_BAD_ARG, "dd_conv3x3_c32_fwd_bits: bad shape");
   DD_REQUIRE(stride == 1, DD_ERR_UNSUPPORTED, "dd_conv3x3_c32_fwd_bits: stride %d (sign words are kept for stride 1 only)", stride);
-  DD_REQUIRE(dtype == DD_BF16 && impl != DD_IMPL_SIMT && dd::conv_tc_supported(H, W, stride, 0), DD_ERR_UNSUPPORTED,
-             "dd_conv3x3_c32_fwd_bits: sign words come from the bf16 tensor-core kernel only (dtype %d, impl %d, H=%d W=%d)",
-             dtype, impl, H, W);
+  DD_REQUIRE(dtype == DD_BF16 && impl != DD_IMPL_SIMT, DD_ERR_UNSUPPORTED,
+             "dd_conv3x3_c32_fwd_bits: sign words come from the bf16 tensor-core kernel only (dtype %d, impl %d)", dtype, impl);
   if (B == 0) return 0;
   return dd::conv3x3_c32_fwd_tc(in, w_oihw, bias, out, B, H, W, stride, 0, nullptr, bits, dd::as_stream(stream));
 }
@@ -628,9 +620,8 @@ extern "C" int dd_conv3x3_c32_dgrad_bits(const void* dy, const float* w_oihw, co
   DD_REQUIRE(dy && w_oihw && x_bits && dx, DD_ERR_BAD_ARG, "dd_conv3x3_c32_dgrad_bits: null pointer");
   DD_REQUIRE(B >= 0 && H > 0 && W > 0, DD_ERR_BAD_ARG, "dd_conv3x3_c32_dgrad_bits: bad shape");
   DD_REQUIRE(stride == 1 || stride == 2, DD_ERR_UNSUPPORTED, "dd_conv3x3_c32_dgrad_bits: stride %d", stride);
-  DD_REQUIRE(dtype == DD_BF16 && impl != DD_IMPL_SIMT && dd::conv_tc_supported(H, W, stride, 1), DD_ERR_UNSUPPORTED,
-             "dd_conv3x3_c32_dgrad_bits: sign words are read by the bf16 tensor-core kernels only (dtype %d, impl %d, H=%d W=%d)",
-             dtype, impl, H, W);
+  DD_REQUIRE(dtype == DD_BF16 && impl != DD_IMPL_SIMT, DD_ERR_UNSUPPORTED,
+             "dd_conv3x3_c32_dgrad_bits: sign words are read by the bf16 tensor-core kernels only (dtype %d, impl %d)", dtype, impl);
   if (B == 0) return 0;
   return dd::conv3x3_c32_fwd_tc(dy, w_oihw, nullptr, dx, B, H, W, stride, 1, nullptr, const_cast<uint32_t*>(x_bits),
                                 dd::as_stream(stream));
@@ -644,11 +635,8 @@ extern "C" int dd_conv3x3_c32_wgrad(const void* x, const void* dy, float* dw, fl
   DD_REQUIRE(stride == 1 || stride == 2, DD_ERR_UNSUPPORTED, "dd_conv3x3_c32_wgrad: stride %d", stride);
   DD_REQUIRE(ws_bytes >= kWgradWsBytes, DD_ERR_WORKSPACE, "dd_conv3x3_c32_wgrad: workspace %zu < %zu", ws_bytes, kWgradWsBytes);
   cudaStream_t st = dd::as_stream(stream);
-  if (dtype == DD_BF16 && impl != DD_IMPL_SIMT) {
-    if (dd::conv_tc_supported(H, W, stride, 2))
-      return dd::conv3x3_c32_wgrad_tc(x, dy, dw, db, workspace, ws_bytes, B, H, W, stride, st);
-    DD_REQUIRE(impl != DD_IMPL_TCGEN05, DD_ERR_UNSUPPORTED, "dd_conv3x3_c32_wgrad: tcgen05 path unsupported here");
-  }
+  if (dtype == DD_BF16 && impl != DD_IMPL_SIMT)
+    return dd::conv3x3_c32_wgrad_tc(x, dy, dw, db, workspace, ws_bytes, B, H, W, stride, st);
   DD_REQUIRE(!(dtype == DD_F32 && impl == DD_IMPL_TCGEN05), DD_ERR_UNSUPPORTED, "tcgen05 conv is bf16 only");
   if (dtype == DD_F32)
     return conv_wgrad_simt<float>((const float*)x, (const float*)dy, dw, db, (float*)workspace, B, H, W, stride, st);

@@ -1351,13 +1351,6 @@ __global__ void __maxnreg__(80) enc_c1c2_fused_kernel(const TIN* __restrict__ in
 
 namespace dd {
 
-// mode: 0 forward, 1 input gradient, 2 weight gradient
-bool conv_tc_supported(int H, int W, int stride, int mode) {
-  if (H < 1 || W < 1) return false;
-  if (mode == 0) return stride == 1 || stride == 2;
-  return mode >= 0 && mode <= 2 && (stride == 1 || stride == 2);
-}
-
 // bits (may be NULL): the ReLU sign words (see relu_bits), written by mode 0 stride 1, read instead of `mask` by mode 1
 int conv3x3_c32_fwd_tc(const void* in, const float* w, const float* bias, void* out, int B, int H, int W, int stride,
                        int mode, const void* mask, uint32_t* bits, cudaStream_t st) {

@@ -79,7 +79,7 @@ int dd_conv_c1_fwd(const void* in, int in_flags, const float* w_oihw, const floa
 /* ReLU sign words: the ReLU mask of a1 / a2 for the input gradients of c2 / c3, 4 bytes per pixel instead of the
  * 64-byte activation.  One uint32 per pixel [B,H,W] (NHWC pixel order); bit c is 1 exactly when the stored bf16
  * activation of channel c is > 0.  `bits` must be 8-byte aligned.  The *_bits entry points run on the bf16 tensor-core
- * kernels only: fp32, DD_IMPL_SIMT or a shape those kernels do not take return DD_ERR_UNSUPPORTED before anything runs.
+ * kernels only: fp32 or DD_IMPL_SIMT returns DD_ERR_UNSUPPORTED before anything runs.
  * dd_conv_c1_fwd_bits = dd_conv_c1_fwd (same out) that also writes out's sign words. */
 int dd_conv_c1_fwd_bits(const void* in, int in_flags, const float* w_oihw, const float* bias, void* out,
                         uint32_t* bits, int out_dtype, int B, int H, int Wm, int impl, void* stream);
@@ -211,10 +211,13 @@ int dd_conv2d_dgrad(const void* dy, const float* w, const void* x_mask, void* dx
 int dd_conv2d_wgrad(const void* x, const void* dy, float* dw, float* db, const dd_conv_desc* d,
                     int dtype, void* workspace, size_t ws_bytes, void* stream);
 size_t dd_conv2d_workspace_bytes(const dd_conv_desc* d);
-/* 1 when pass (0 forward, 1 input gradient) of this layer runs on the tcgen05 implicit-GEMM kernel (csrc/conv_dil_tc.cu):
- * bf16, stride 1, square filter of 3 or 7 taps with one dilation / padding for both axes, (gathered, produced) channels in
- * {(96,64), (64,32), (32,16), (32,32), (64,96), (32,64)} -- the merging CNN's up_conv_1..3, rm_conv_2, out_conv and the
- * decoder's dc1 / dc2.  Everything else (and fp32: the parity path) runs on the CUDA-core engine. */
+/* 1 when pass (0 forward, 1 input gradient, 2 weight gradient) of this layer runs on the tcgen05 implicit-GEMM kernels
+ * (csrc/conv_dil_tc.cu, conv_dil_wgrad_tc.cu): bf16, stride 1, square filter of 3 or 7 taps with one dilation (1..7) /
+ * padding for both axes, and (gathered, produced) channels in {(96,64), (64,32), (32,16), (32,32), (64,96), (32,64)}
+ * (forward, input gradient) or {32,64,96} x {32,64} (weight gradient) once narrow tensors are zero-padded: 8 / 16
+ * gathered channels to 32, and 8 produced channels to 16 (forward) or 8 / 16 to 32 (weight gradient) -- the merging
+ * CNN's up_conv_1..4, rm_conv_2, out_conv and the decoder's dc1 / dc2.  Everything else (and fp32: the parity path, and
+ * a sigmoid forward) runs on the CUDA-core engine. */
 int dd_conv2d_tc_supported(const dd_conv_desc* d, int dtype, int pass);
 
 /* ---- A15-A17: data movement and loss of the bounding-box model ------------------------------------
