@@ -50,7 +50,9 @@ SIGNATURES = {
     "dd_linear_fwd": (_I, [_P, _I, _P, _P, _P, _P, _Z, _I, _I, _L, _I, _P]),
     "dd_linear_dgrad": (_I, [_P, _P, _P, _I, _P, _Z, _I, _I, _L, _I, _P]),
     "dd_linear_wgrad": (_I, [_P, _P, _I, _P, _P, _I, _I, _L, _I, _P]),
+    "dd_linear_wgrad_acc": (_I, [_P, _P, _I, _P, _P, _I, _I, _L, _I, _I, _P]),
     "dd_linear_bwd_adam": (_I, [_P, _P, _P, _P, _P, _P, _I, _P, _P, _Z, _I, _I, _L, _F, _F, _F, _F, _F, _L, _P]),
+    "dd_linear_bwd_adam_acc": (_I, [_P, _P, _P, _P, _P, _P, _P, _I, _P, _P, _Z, _I, _I, _L, _F, _F, _F, _F, _F, _L, _P]),
     "dd_linear_workspace_bytes": (_Z, [_I, _I, _L]),
     "dd_linear_tc_supported": (_I, [_I, _I, _L]),
     "dd_bce_ts_fwd": (_I, [_P, _P, _I, _P, _P, _P, _P, _P, _Z, _L, _P]),

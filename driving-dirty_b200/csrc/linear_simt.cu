@@ -266,6 +266,67 @@ __global__ void __launch_bounds__(NTHREADS) linear_wgrad_simt(const float* __res
   }
 }
 
+// dd_linear_wgrad_acc: dW[n,k] = dW_old[n,k] + D[n,k], D bit for bit what dd_linear_wgrad writes.  D is the FMA chain of
+// the chunked launches above (rows in order; each 32-row chunk padded with zero rows to its launch's BT, 8 or 32), kept in
+// a register across the chunks, so that the stored gradient is added once, after the last chunk.  KT = 32 k quads x 8
+// n-lanes; x [Bp][128 k] and dy [NCH n][Bp] staged in shared memory (Bp = padded rows, <= 128).
+constexpr int ACC_KT = 32;
+template <typename T>
+__global__ void __launch_bounds__(NTHREADS) linear_wgrad_acc_simt(const float* __restrict__ dy, const T* __restrict__ x,
+                                                                  float* __restrict__ dw, int B, int Bp, int N, long long K,
+                                                                  int nchunk) {
+  constexpr int NS = NTHREADS / ACC_KT;
+  extern __shared__ __align__(16) float smem[];
+  float4* s_x = reinterpret_cast<float4*>(smem);          // [Bp][ACC_KT]
+  float* s_dy = smem + (size_t)Bp * ACC_KT * 4;           // [NCH][Bp]
+  const int tid = threadIdx.x;
+  const int kt = tid % ACC_KT, ns = tid / ACC_KT;
+  const long long kq = (long long)blockIdx.x * ACC_KT + kt;
+  const bool kvalid = kq * 4 < K;
+  for (int i = tid; i < Bp * ACC_KT; i += NTHREADS) {
+    const int b = i / ACC_KT;
+    const long long k = ((long long)blockIdx.x * ACC_KT + i % ACC_KT) * 4;
+    float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (b < B && k < K) {
+      const T* p = x + (size_t)b * K + k;
+      v = make_float4(dd::ld<T>(p), dd::ld<T>(p + 1), dd::ld<T>(p + 2), dd::ld<T>(p + 3));
+    }
+    s_x[i] = v;
+  }
+  const int nbeg = blockIdx.y * nchunk;
+  const int nend = nbeg + nchunk < N ? nbeg + nchunk : N;
+  for (int nb = nbeg; nb < nend; nb += NCH) {
+    const int nc = nend - nb < NCH ? nend - nb : NCH;
+    __syncthreads();
+    for (int i = tid; i < Bp * NCH; i += NTHREADS) {
+      const int b = i / NCH, nl = i - b * NCH;
+      s_dy[nl * Bp + b] = (b < B && nl < nc) ? __ldg(dy + (size_t)b * N + nb + nl) : 0.f;
+    }
+    __syncthreads();
+    if (kvalid) {
+      for (int nl = ns; nl < nc; nl += NS) {
+        float4 o = make_float4(0.f, 0.f, 0.f, 0.f);
+        for (int b4 = 0; b4 < Bp / 4; ++b4) {
+          const float4 d = *reinterpret_cast<const float4*>(s_dy + nl * Bp + 4 * b4);
+          const float dv[4] = {d.x, d.y, d.z, d.w};
+#pragma unroll
+          for (int e = 0; e < 4; ++e) {
+            const float4 xv = s_x[(4 * b4 + e) * ACC_KT + kt];
+            o.x = fmaf(dv[e], xv.x, o.x);
+            o.y = fmaf(dv[e], xv.y, o.y);
+            o.z = fmaf(dv[e], xv.z, o.z);
+            o.w = fmaf(dv[e], xv.w, o.w);
+          }
+        }
+        float4* dst = reinterpret_cast<float4*>(dw + (size_t)(nb + nl) * K) + kq;
+        const float4 old = *dst;
+        o.x = old.x + o.x; o.y = old.y + o.y; o.z = old.z + o.z; o.w = old.w + o.w;
+        __stcs(dst, o);
+      }
+    }
+  }
+}
+
 // db[n] = sum_b dy[b,n]
 __global__ void colsum_kernel(const float* __restrict__ dy, float* __restrict__ db, int B, int N, int accumulate) {
   const int n = blockIdx.x * blockDim.x + threadIdx.x;
@@ -359,6 +420,23 @@ int wgrad_launch(const float* dy, const T* x, float* dw, int B, int N, long long
   return dd::check_launch("linear_wgrad_simt");
 }
 
+template <typename T>
+int wgrad_acc_launch(const float* dy, const T* x, float* dw, int B, int N, long long K, cudaStream_t st) {
+  const int last = B - 32 * ((B - 1) / 32);                      // rows of the last 32-row chunk, padded as its launch pads
+  const int Bp = 32 * ((B - 1) / 32) + (last <= 8 ? 8 : 32);
+  const int kblocks = dd::ceil_div(K / 4, ACC_KT);
+  int want = dd::ceil_div(dd::kSMs * 4, kblocks);
+  int maxsplit = dd::ceil_div(N, NCH);
+  if (want > maxsplit) want = maxsplit;
+  if (want < 1) want = 1;
+  const int nchunk = dd::ceil_div(dd::ceil_div(N, want), NCH) * NCH;
+  const size_t smem = (size_t)Bp * (ACC_KT * 4 + NCH) * sizeof(float);
+  auto k = linear_wgrad_acc_simt<T>;
+  if (int e = dd::set_smem(k, smem, dd::Carveout::kDefault, "linear_wgrad_acc_simt")) return e;
+  k<<<dim3(kblocks, dd::ceil_div(N, nchunk)), NTHREADS, smem, st>>>(dy, x, dw, B, Bp, N, K, nchunk);
+  return dd::check_launch("linear_wgrad_acc_simt");
+}
+
 size_t ws_bytes_for(int B, int N, long long K) {
   const int Bc = B < 32 ? B : 32;
   const FwdPlan f = plan_fwd(N, K);
@@ -378,8 +456,9 @@ int linear_fwd_tc(const float* x, const float* w, const float* bias, float* y, v
 int linear_dgrad_tc(const float* dy, const float* w, void* dx, int dx_dtype, void* ws, size_t ws_bytes, int B, int N,
                     long long K, cudaStream_t st);
 int linear_wgrad_tc(const float* dy, const float* x, float* dw, int B, int N, long long K, int accumulate, cudaStream_t st);
-int linear_bwd_adam_tc(const float* dy, const float* x, float* w, float* m, float* v, void* dx, int dx_dtype, void* ws,
-                       size_t ws_bytes, int B, int N, long long K, const AdamHyper& h, cudaStream_t st);
+int linear_wgrad_acc_multi_tc(const float* dy, const float* x, float* dw, int B, int N, long long K, cudaStream_t st);
+int linear_bwd_adam_tc(const float* dy, const float* x, float* w, float* m, float* v, const float* gpart, void* dx, int dx_dtype,
+                       void* ws, size_t ws_bytes, int B, int N, long long K, const AdamHyper& h, cudaStream_t st);
 }  // namespace dd
 
 // tcgen05 path: only on explicit request (DD_IMPL_TCGEN05) -- fp32 callers under DD_IMPL_AUTO keep the
@@ -464,15 +543,27 @@ extern "C" int dd_linear_dgrad(const float* dy, const float* w, void* dx, int dx
   return 0;
 }
 
+#define DD_WGRAD_COMMON(name)                                                                                          \
+  DD_REQUIRE(dy && x && dw, DD_ERR_BAD_ARG, name ": null pointer");                                                    \
+  DD_REQUIRE(B > 0 && N > 0 && K > 0, DD_ERR_BAD_ARG, name ": bad shape B=%d N=%d K=%lld", B, N, K);                   \
+  DD_REQUIRE(K % 4 == 0, DD_ERR_UNSUPPORTED, name ": K=%lld must be a multiple of 4", K);                              \
+  DD_REQUIRE(x_dtype == DD_F32 || x_dtype == DD_BF16, DD_ERR_UNSUPPORTED, name ": dtype %d", x_dtype);                 \
+  DD_REQUIRE((uintptr_t)dw % 16 == 0, DD_ERR_ALIGNMENT, name ": dw pointer must be 16-byte aligned");                  \
+  DD_REQUIRE(impl != DD_IMPL_TCGEN05 || (x_dtype == DD_F32 && dd::linear_tc_supported(B, N, K)), DD_ERR_UNSUPPORTED, \
+             name ": tcgen05 path needs fp32 x, N %% 4 == K %% 4 == 0 and N*K >= 2^22 (B=%d N=%d K=%lld)", B, N, K);
+
+// db[n] = sum_b dy[b,n], in the 32-row chunks of the weight-gradient launches
+static int colsum_chunked(const float* dy, float* db, int B, int N, cudaStream_t st) {
+  for (int b0 = 0; b0 < B; b0 += 32) {
+    colsum_kernel<<<dd::ceil_div(N, 256), 256, 0, st>>>(dy + (size_t)b0 * N, db, B - b0 < 32 ? B - b0 : 32, N, b0 > 0);
+    if (int e = dd::check_launch("colsum")) return e;
+  }
+  return 0;
+}
+
 extern "C" int dd_linear_wgrad(const float* dy, const void* x, int x_dtype, float* dw, float* db, int B, int N,
                                long long K, int impl, void* stream) {
-  DD_REQUIRE(dy && x && dw, DD_ERR_BAD_ARG, "dd_linear_wgrad: null pointer");
-  DD_REQUIRE(B > 0 && N > 0 && K > 0, DD_ERR_BAD_ARG, "dd_linear_wgrad: bad shape B=%d N=%d K=%lld", B, N, K);
-  DD_REQUIRE(K % 4 == 0, DD_ERR_UNSUPPORTED, "dd_linear_wgrad: K=%lld must be a multiple of 4", K);
-  DD_REQUIRE(x_dtype == DD_F32 || x_dtype == DD_BF16, DD_ERR_UNSUPPORTED, "dd_linear_wgrad: dtype %d", x_dtype);
-  DD_REQUIRE((uintptr_t)dw % 16 == 0, DD_ERR_ALIGNMENT, "dd_linear_wgrad: dw pointer must be 16-byte aligned");
-  DD_REQUIRE(impl != DD_IMPL_TCGEN05 || (x_dtype == DD_F32 && dd::linear_tc_supported(B, N, K)), DD_ERR_UNSUPPORTED,
-             "dd_linear_wgrad: tcgen05 path needs fp32 x, N %% 4 == K %% 4 == 0 and N*K >= 2^22 (B=%d N=%d K=%lld)", B, N, K);
+  DD_WGRAD_COMMON("dd_linear_wgrad");
   cudaStream_t st = dd::as_stream(stream);
   const size_t esz = x_dtype == DD_F32 ? 4 : 2;
   for (int b0 = 0; b0 < B; b0 += 32) {
@@ -497,6 +588,24 @@ extern "C" int dd_linear_wgrad(const float* dy, const void* x, int x_dtype, floa
   return 0;
 }
 
+// dd_linear_wgrad, or with accumulate: dw = dw_old + what dd_linear_wgrad writes, bit for bit (see include/dd_b200.h)
+extern "C" int dd_linear_wgrad_acc(const float* dy, const void* x, int x_dtype, float* dw, float* db, int B, int N,
+                                   long long K, int impl, int accumulate, void* stream) {
+  if (!accumulate) return dd_linear_wgrad(dy, x, x_dtype, dw, db, B, N, K, impl, stream);
+  DD_WGRAD_COMMON("dd_linear_wgrad_acc");
+  DD_REQUIRE(B <= 128, DD_ERR_UNSUPPORTED, "dd_linear_wgrad_acc: accumulating takes at most 128 rows (B=%d)", B);
+  cudaStream_t st = dd::as_stream(stream);
+  int e;
+  if (use_tc(impl, B, N, K))        // one 32-row chunk: the plain kernel's epilogue adds the old value after the MMA sum
+    e = B <= 32 ? dd::linear_wgrad_tc(dy, (const float*)x, dw, B, N, K, 1, st) : dd::linear_wgrad_acc_multi_tc(dy, (const float*)x, dw, B, N, K, st);
+  else if (x_dtype == DD_F32)
+    e = wgrad_acc_launch<float>(dy, (const float*)x, dw, B, N, K, st);
+  else
+    e = wgrad_acc_launch<__nv_bfloat16>(dy, (const __nv_bfloat16*)x, dw, B, N, K, st);
+  if (e) return e;
+  return db ? colsum_chunked(dy, db, B, N, st) : 0;
+}
+
 // Backward pass of a wide linear layer with the Adam update of its weight folded in (world size 1): see include/dd_b200.h.
 // tcgen05 path only (fp32 x, B <= 32, dd_linear_tc_supported); the bias gradient is written as by dd_linear_wgrad.
 extern "C" int dd_linear_bwd_adam(const float* dy, const float* x, float* weight, float* exp_avg, float* exp_avg_sq, void* dx,
@@ -512,7 +621,33 @@ extern "C" int dd_linear_bwd_adam(const float* dy, const float* x, float* weight
              "dd_linear_bwd_adam: workspace %zu < %zu", ws_bytes, dd_linear_workspace_bytes(B, N, K));
   cudaStream_t st = dd::as_stream(stream);
   const dd::AdamHyper h = dd::adam_hyper(lr, beta1, beta2, eps, weight_decay, step, 1.f);
-  if (int e = dd::linear_bwd_adam_tc(dy, x, weight, exp_avg, exp_avg_sq, dx, dx_dtype, workspace, ws_bytes, B, N, K, h, st)) return e;
+  if (int e = dd::linear_bwd_adam_tc(dy, x, weight, exp_avg, exp_avg_sq, nullptr, dx, dx_dtype, workspace, ws_bytes, B, N, K, h, st))
+    return e;
+  if (db) {
+    colsum_kernel<<<dd::ceil_div(N, 256), 256, 0, st>>>(dy, db, B, N, 0);
+    if (int e2 = dd::check_launch("colsum")) return e2;
+  }
+  return 0;
+}
+
+// dd_linear_bwd_adam that steps with this pass's weight gradient plus grad_partial (the earlier passes of the window)
+extern "C" int dd_linear_bwd_adam_acc(const float* dy, const float* x, float* weight, float* exp_avg, float* exp_avg_sq,
+                                      const float* grad_partial, void* dx, int dx_dtype, float* db, void* workspace,
+                                      size_t ws_bytes, int B, int N, long long K, float lr, float beta1, float beta2, float eps,
+                                      float weight_decay, long long step, void* stream) {
+  DD_REQUIRE(dy && x && weight && exp_avg && exp_avg_sq && grad_partial, DD_ERR_BAD_ARG, "dd_linear_bwd_adam_acc: null pointer");
+  DD_REQUIRE(B > 0 && B <= 32 && N > 0 && K > 0 && step >= 1, DD_ERR_BAD_ARG, "dd_linear_bwd_adam_acc: B=%d (<= 32) N=%d K=%lld step=%lld", B, N, K, step);
+  DD_REQUIRE(!dx || dx_dtype == DD_F32 || dx_dtype == DD_BF16, DD_ERR_UNSUPPORTED, "dd_linear_bwd_adam_acc: dtype %d", dx_dtype);
+  DD_REQUIRE(dd::linear_tc_supported(B, N, K), DD_ERR_UNSUPPORTED, "dd_linear_bwd_adam_acc: needs the tcgen05 path (N %% 4 == K %% 4 == 0, N*K >= 2^22)");
+  DD_REQUIRE((((uintptr_t)weight | (uintptr_t)exp_avg | (uintptr_t)exp_avg_sq | (uintptr_t)grad_partial | (uintptr_t)dy | (uintptr_t)x) & 15) == 0,
+             DD_ERR_ALIGNMENT, "dd_linear_bwd_adam_acc: dy / x / weight / moments / grad_partial must be 16-byte aligned");
+  DD_REQUIRE(!dx || (workspace && ws_bytes >= dd_linear_workspace_bytes(B, N, K)), DD_ERR_WORKSPACE,
+             "dd_linear_bwd_adam_acc: workspace %zu < %zu", ws_bytes, dd_linear_workspace_bytes(B, N, K));
+  cudaStream_t st = dd::as_stream(stream);
+  const dd::AdamHyper h = dd::adam_hyper(lr, beta1, beta2, eps, weight_decay, step, 1.f);
+  if (int e = dd::linear_bwd_adam_tc(dy, x, weight, exp_avg, exp_avg_sq, grad_partial, dx, dx_dtype, workspace, ws_bytes, B, N, K,
+                                     h, st))
+    return e;
   if (db) {
     colsum_kernel<<<dd::ceil_div(N, 256), 256, 0, st>>>(dy, db, B, N, 0);
     if (int e2 = dd::check_launch("colsum")) return e2;

@@ -203,6 +203,9 @@ __global__ void split_fold_kernel(const float* __restrict__ partial, const float
 // ------------------------------------------------------------------------------------------------
 // wgrad: dW[n][k] (+)= sum_b dy[b][n] x[b][k]; one 128 x KT output tile per stage (no accumulation across
 // stages), written straight from TMEM to HBM.
+// MULTI (dd_linear_wgrad_acc, B > 32): every 32-row batch chunk of an item gets a stage and a TMEM accumulator of its own;
+// the epilogue sums the chunks in fp32 in the order of the chunked plain launches (D = D_0, then D = D_j + D) and only
+// then adds the stored gradient: dw_old + D, not the (dw_old + D_0) + D_1 of accumulating chunk by chunk.
 // ------------------------------------------------------------------------------------------------
 constexpr int W_STAGES = 3;
 constexpr int W_STAGE_BYTES = 4 * BOX + 8 * BOX;     // dy^T: 4 boxes of 32 n; x: up to 8 boxes of 32 k
@@ -221,8 +224,10 @@ struct WgradGeo {
   long long K;
   int n_tiles, k_tiles, KT;      // KT = 128 or 256 columns per tile
   int accumulate;
+  int bchunks, nbuf;             // MULTI: 32-row batch chunks per item; TMEM accumulators of bchunks * KT columns (1 or 2)
 };
 
+template <bool MULTI>
 __global__ void __launch_bounds__(W_THREADS, 1) linear_wgrad_tc_kernel(const __grid_constant__ CUtensorMap map_dy,
                                                                        const __grid_constant__ CUtensorMap map_x,
                                                                        float* __restrict__ dw, const WgradGeo g) {
@@ -250,15 +255,54 @@ __global__ void __launch_bounds__(W_THREADS, 1) linear_wgrad_tc_kernel(const __g
   if (warp == 0) {
     if (umma::elect_one()) {
       uint32_t c = 0;
-      for (long long it = blockIdx.x; it < items; it += gridDim.x, ++c) {
-        const int ni = (int)(it / g.k_tiles), ki = (int)(it % g.k_tiles);
-        const uint32_t s = c % W_STAGES;
-        umma::mbar_wait(&bars->empty[s], ((c / W_STAGES) & 1) ^ 1);
-        const uint32_t dst = umma::smem_u32(smem + s * W_STAGE_BYTES);
-        umma::mbar_expect_tx(&bars->full[s], stage_tx);
+      if (MULTI) {
+        for (long long it = blockIdx.x; it < items; it += gridDim.x) {
+          const int ni = (int)(it / g.k_tiles), ki = (int)(it % g.k_tiles);
+          for (int bc = 0; bc < g.bchunks; ++bc, ++c) {                 // batch rows [32 bc, 32 bc + 32)
+            const uint32_t s = c % W_STAGES;
+            umma::mbar_wait(&bars->empty[s], ((c / W_STAGES) & 1) ^ 1);
+            const uint32_t dst = umma::smem_u32(smem + s * W_STAGE_BYTES);
+            umma::mbar_expect_tx(&bars->full[s], stage_tx);
 #pragma unroll
-        for (int i = 0; i < 4; ++i) umma::tma_load_2d(dst + i * BOX, &map_dy, ni * 128 + 32 * i, 0, &bars->full[s]);
-        for (int j = 0; j < xboxes; ++j) umma::tma_load_2d(dst + (4 + j) * BOX, &map_x, ki * g.KT + 32 * j, 0, &bars->full[s]);
+            for (int i = 0; i < 4; ++i) umma::tma_load_2d(dst + i * BOX, &map_dy, ni * 128 + 32 * i, 32 * bc, &bars->full[s]);
+            for (int j = 0; j < xboxes; ++j)
+              umma::tma_load_2d(dst + (4 + j) * BOX, &map_x, ki * g.KT + 32 * j, 32 * bc, &bars->full[s]);
+          }
+        }
+      } else {
+        for (long long it = blockIdx.x; it < items; it += gridDim.x, ++c) {
+          const int ni = (int)(it / g.k_tiles), ki = (int)(it % g.k_tiles);
+          const uint32_t s = c % W_STAGES;
+          umma::mbar_wait(&bars->empty[s], ((c / W_STAGES) & 1) ^ 1);
+          const uint32_t dst = umma::smem_u32(smem + s * W_STAGE_BYTES);
+          umma::mbar_expect_tx(&bars->full[s], stage_tx);
+#pragma unroll
+          for (int i = 0; i < 4; ++i) umma::tma_load_2d(dst + i * BOX, &map_dy, ni * 128 + 32 * i, 0, &bars->full[s]);
+          for (int j = 0; j < xboxes; ++j) umma::tma_load_2d(dst + (4 + j) * BOX, &map_x, ki * g.KT + 32 * j, 0, &bars->full[s]);
+        }
+      }
+    }
+  } else if (warp == 1 && MULTI) {
+    const uint32_t idesc = umma::make_idesc_tf32(128, g.KT, true, true);
+    const uint32_t acc_cols = g.bchunks * g.KT;
+    uint32_t c = 0, n_item = 0;
+    for (long long it = blockIdx.x; it < items; it += gridDim.x, ++n_item) {
+      const uint32_t a = n_item % g.nbuf, use = n_item / g.nbuf;
+      umma::mbar_wait(&bars->acc_empty[a], (use & 1) ^ 1);
+      for (int bc = 0; bc < g.bchunks; ++bc, ++c) {
+        const uint32_t s = c % W_STAGES;
+        umma::mbar_wait(&bars->full[s], (c / W_STAGES) & 1);
+        umma::tc_fence_after_sync();
+        const uint32_t base = umma::smem_u32(smem + s * W_STAGE_BYTES);
+        if (umma::elect_one()) {
+#pragma unroll
+          for (int k = 0; k < NB / 8; ++k)
+            umma::mma_tf32_lohi(tmem + a * acc_cols + bc * g.KT, umma::desc_lo(base + k * 1024, BOX), umma::desc_hi_sw128_base32(512),
+                                umma::desc_lo(base + 4 * BOX + k * 1024, BOX), umma::desc_hi_sw128_base32(512), idesc, k > 0 ? 1u : 0u);
+          umma::mma_commit(&bars->empty[s]);
+          if (bc == g.bchunks - 1) umma::mma_commit(&bars->acc_full[a]);
+        }
+        __syncwarp();
       }
     }
   } else if (warp == 1) {
@@ -285,16 +329,29 @@ __global__ void __launch_bounds__(W_THREADS, 1) linear_wgrad_tc_kernel(const __g
     uint32_t c = 0;
     for (long long it = blockIdx.x; it < items; it += gridDim.x, ++c) {
       const int ni = (int)(it / g.k_tiles), ki = (int)(it % g.k_tiles);
-      const uint32_t a = c & 1;
-      umma::mbar_wait_sleep(&bars->acc_full[a], (c >> 1) & 1);
+      const uint32_t a = MULTI ? c % g.nbuf : c & 1;
+      umma::mbar_wait_sleep(&bars->acc_full[a], MULTI ? (c / g.nbuf) & 1 : (c >> 1) & 1);
       umma::tc_fence_after_sync();
       const int n0 = ni * 128 + quarter * 32;
       const long long k0 = (long long)ki * g.KT;
       float* blk = stage_out + (warp - 2) * (32 * W_TPAD);
       for (int cb = 0; cb < g.KT; cb += 32) {
         uint32_t v[32];
-        umma::tmem_ld_32x32(tmem + ((uint32_t)(quarter * 32) << 16) + a * 256 + cb, v);
-        umma::tmem_ld_wait();
+        if (MULTI) {
+          const uint32_t col = tmem + ((uint32_t)(quarter * 32) << 16) + a * g.bchunks * g.KT + cb;
+          umma::tmem_ld_32x32(col, v);
+          umma::tmem_ld_wait();
+          for (int bc = 1; bc < g.bchunks; ++bc) {
+            uint32_t u[32];
+            umma::tmem_ld_32x32(col + bc * g.KT, u);
+            umma::tmem_ld_wait();
+#pragma unroll
+            for (int i = 0; i < 32; ++i) v[i] = __float_as_uint(__uint_as_float(u[i]) + __uint_as_float(v[i]));
+          }
+        } else {
+          umma::tmem_ld_32x32(tmem + ((uint32_t)(quarter * 32) << 16) + a * 256 + cb, v);
+          umma::tmem_ld_wait();
+        }
         // lane = row n0 + lane holds 32 consecutive k: transpose through shared memory so that each store
         // instruction below writes four whole 128-byte row segments instead of 32 scattered 16-byte pieces
         __syncwarp();
@@ -342,12 +399,21 @@ __global__ void __launch_bounds__(W_THREADS, 1) linear_wgrad_tc_kernel(const __g
 // (tools/tma_store_atom32_probe.cu): element (row r, column c) of a 32 x 32 box sits in 32-byte atom (c / 8) ^ (r % 4)
 // of its 128-byte row.
 // ------------------------------------------------------------------------------------------------
-constexpr int BA_STAGES = 3;
-constexpr int BA_TILE = 4 * BOX;                      // W, m or v: [32 n][128 k] as 4 boxes of 32 k
-constexpr int BA_STAGE_BYTES = 3 * BA_TILE + 2 * BOX;  // W, m, v; dy chunk K-major (dgrad) and MN-major (wgrad)
+//
+// Accumulating form (ACC, dd_linear_bwd_adam_acc): the stage also carries the tile of a stored partial gradient G (the
+// earlier backward passes of a gradient-accumulation window), loaded in the same boxes as W, m and v, and the epilogue
+// steps with dW_chunk + G -- 28 bytes per parameter.  A fourth 16 KB tile per stage would need 250 KB at three stages, over
+// the 227 KB of a block: this instantiation runs two stages (178 KB).
+constexpr int BA_STAGES = 3;                          // stages of the plain form (and the size of the barrier arrays)
+constexpr int BA_TILE = 4 * BOX;                      // W, m, v or G: [32 n][128 k] as 4 boxes of 32 k
 constexpr int BA_EPI = 8;
 constexpr int BA_THREADS = 32 * (3 + BA_EPI);
-constexpr int BA_SMEM = BA_STAGES * BA_STAGE_BYTES + 2 * BA_TILE + 2048;   // + x [32 b][128 k], double-buffered per item
+template <bool ACC> struct BaCfg {
+  static constexpr int STAGES = ACC ? 2 : BA_STAGES;
+  static constexpr int DY_OFF = (ACC ? 4 : 3) * BA_TILE;    // W, m, v (, G); then the dy chunk MN-major (wgrad) and K-major (dgrad)
+  static constexpr int STAGE_BYTES = DY_OFF + 2 * BOX;
+  static constexpr int SMEM = STAGES * STAGE_BYTES + 2 * BA_TILE + 2048;   // + x [32 b][128 k], double-buffered per item
+};
 
 struct BwdAdamBars {
   uint64_t full[BA_STAGES], empty[BA_STAGES], tile_ready[BA_STAGES], x_full[2], x_empty[2], g_full[2], g_empty[2], acc_full[2], acc_empty[2];
@@ -362,14 +428,16 @@ __device__ __forceinline__ float lds_f32(uint32_t a) {
 }
 __device__ __forceinline__ void sts_f32(uint32_t a, float v) { asm volatile("st.shared.f32 [%0], %1;" ::"r"(a), "f"(v) : "memory"); }
 // TMEM columns: [0, 64) dgrad accumulator of the item (x 2), [64, 128) G^T of the chunk (x 2)
-template <typename TOUT>
+// map_g (the stored partial gradient, ACC only) comes last, so that the plain instantiation keeps its parameter layout
+template <typename TOUT, bool ACC>
 __global__ void __launch_bounds__(BA_THREADS, 1) linear_bwd_adam_tc_kernel(
     const __grid_constant__ CUtensorMap map_w, const __grid_constant__ CUtensorMap map_m, const __grid_constant__ CUtensorMap map_v,
     const __grid_constant__ CUtensorMap map_dy, const __grid_constant__ CUtensorMap map_dyt, const __grid_constant__ CUtensorMap map_x,
-    TOUT* __restrict__ dx, float* __restrict__ partial, StreamGeo g, const dd::AdamHyper h) {
+    TOUT* __restrict__ dx, float* __restrict__ partial, StreamGeo g, const dd::AdamHyper h, const __grid_constant__ CUtensorMap map_g) {
+  constexpr int STAGES = BaCfg<ACC>::STAGES, STAGE_BYTES = BaCfg<ACC>::STAGE_BYTES, DY_OFF = BaCfg<ACC>::DY_OFF;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = align1024(smem_raw);
-  uint8_t* xbuf = smem + BA_STAGES * BA_STAGE_BYTES;
+  uint8_t* xbuf = smem + STAGES * STAGE_BYTES;
   BwdAdamBars* bars = reinterpret_cast<BwdAdamBars*>(xbuf + 2 * BA_TILE);
   const int tid = threadIdx.x, lane = tid & 31;
   const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);
@@ -377,7 +445,7 @@ __global__ void __launch_bounds__(BA_THREADS, 1) linear_bwd_adam_tc_kernel(
   const bool has_dx = dx != nullptr;
 
   if (tid == 0) {
-    for (int i = 0; i < BA_STAGES; ++i) {
+    for (int i = 0; i < STAGES; ++i) {
       umma::mbar_init(&bars->full[i], 1); umma::mbar_init(&bars->empty[i], 1); umma::mbar_init(&bars->tile_ready[i], BA_EPI);
     }
     for (int i = 0; i < 2; ++i) {
@@ -388,6 +456,7 @@ __global__ void __launch_bounds__(BA_THREADS, 1) linear_bwd_adam_tc_kernel(
     umma::fence_mbar_init();
     umma::tma_prefetch_desc(&map_w); umma::tma_prefetch_desc(&map_m); umma::tma_prefetch_desc(&map_v);
     umma::tma_prefetch_desc(&map_dy); umma::tma_prefetch_desc(&map_dyt); umma::tma_prefetch_desc(&map_x);
+    if (ACC) umma::tma_prefetch_desc(&map_g);
   }
   if (warp == 1) umma::tmem_alloc(&bars->tmem_base, 128);
   const uint32_t tmem = umma::tmem_publish(&bars->tmem_base);
@@ -395,7 +464,7 @@ __global__ void __launch_bounds__(BA_THREADS, 1) linear_bwd_adam_tc_kernel(
   if (warp == 0) {
     // =========================== TMA producer ===================================================
     if (umma::elect_one()) {
-      const uint32_t stage_tx = has_dx ? BA_STAGE_BYTES : BA_STAGE_BYTES - BOX;
+      const uint32_t stage_tx = has_dx ? STAGE_BYTES : STAGE_BYTES - BOX;
       uint32_t c = 0, n_item = 0;
       for (int it = blockIdx.x; it < items; it += gridDim.x, ++n_item) {
         const int ti = it % g.tiles, si = it / g.tiles;
@@ -408,18 +477,19 @@ __global__ void __launch_bounds__(BA_THREADS, 1) linear_bwd_adam_tc_kernel(
         for (int i = 0; i < 4; ++i)                                                           // x[b][k tile], 4 x 32 k
           umma::tma_load_2d(umma::smem_u32(xbuf + xb * BA_TILE + i * BOX), &map_x, ti * 128 + 32 * i, 0, &bars->x_full[xb]);
         for (int ch = c0; ch < c1; ++ch, ++c) {
-          const uint32_t s = c % BA_STAGES;
-          umma::mbar_wait(&bars->empty[s], ((c / BA_STAGES) & 1) ^ 1);
-          const uint32_t dst = umma::smem_u32(smem + s * BA_STAGE_BYTES);
+          const uint32_t s = c % STAGES;
+          umma::mbar_wait(&bars->empty[s], ((c / STAGES) & 1) ^ 1);
+          const uint32_t dst = umma::smem_u32(smem + s * STAGE_BYTES);
           umma::mbar_expect_tx(&bars->full[s], stage_tx);
 #pragma unroll
           for (int i = 0; i < 4; ++i) {                                                       // [n chunk][k tile], 4 x 32 k
             umma::tma_load_2d(dst + i * BOX, &map_w, ti * 128 + 32 * i, ch * kChunk, &bars->full[s]);
             umma::tma_load_2d(dst + BA_TILE + i * BOX, &map_m, ti * 128 + 32 * i, ch * kChunk, &bars->full[s]);
             umma::tma_load_2d(dst + 2 * BA_TILE + i * BOX, &map_v, ti * 128 + 32 * i, ch * kChunk, &bars->full[s]);
+            if (ACC) umma::tma_load_2d(dst + 3 * BA_TILE + i * BOX, &map_g, ti * 128 + 32 * i, ch * kChunk, &bars->full[s]);
           }
-          umma::tma_load_2d(dst + 3 * BA_TILE, &map_dyt, ch * kChunk, 0, &bars->full[s]);             // dy[b][chunk], MN-major
-          if (has_dx) umma::tma_load_2d(dst + 3 * BA_TILE + BOX, &map_dy, ch * kChunk, 0, &bars->full[s]);  // ... K-major
+          umma::tma_load_2d(dst + DY_OFF, &map_dyt, ch * kChunk, 0, &bars->full[s]);             // dy[b][chunk], MN-major
+          if (has_dx) umma::tma_load_2d(dst + DY_OFF + BOX, &map_dy, ch * kChunk, 0, &bars->full[s]);  // ... K-major
         }
       }
     }
@@ -437,23 +507,23 @@ __global__ void __launch_bounds__(BA_THREADS, 1) linear_bwd_adam_tc_kernel(
       umma::mbar_wait(&bars->x_full[a], (n_item >> 1) & 1);
       const uint32_t xbase = umma::smem_u32(xbuf + a * BA_TILE);
       for (int ch = c0; ch < c1; ++ch, ++c) {
-        const uint32_t s = c % BA_STAGES, ga = c & 1;
-        umma::mbar_wait(&bars->full[s], (c / BA_STAGES) & 1);
+        const uint32_t s = c % STAGES, ga = c & 1;
+        umma::mbar_wait(&bars->full[s], (c / STAGES) & 1);
         umma::mbar_wait(&bars->g_empty[ga], ((c >> 1) & 1) ^ 1);
         umma::tc_fence_after_sync();
-        const uint32_t base = umma::smem_u32(smem + s * BA_STAGE_BYTES);
+        const uint32_t base = umma::smem_u32(smem + s * STAGE_BYTES);
         if (umma::elect_one()) {
           if (has_dx) {
 #pragma unroll
             for (int k = 0; k < 4; ++k)
               umma::mma_tf32_lohi(tmem + a * NB, umma::desc_lo(base + k * 1024, BOX), umma::desc_hi_sw128_base32(512),
-                                  umma::desc_lo(base + 3 * BA_TILE + BOX + k * 32, 16), umma::desc_hi_sw128(1024), idesc_d,
+                                  umma::desc_lo(base + DY_OFF + BOX + k * 32, 16), umma::desc_hi_sw128(1024), idesc_d,
                                   (ch > c0 || k > 0) ? 1u : 0u);
           }
 #pragma unroll
           for (int k = 0; k < 4; ++k)
             umma::mma_tf32_lohi(tmem + 2 * NB + ga * NB, umma::desc_lo(xbase + k * 1024, BOX), umma::desc_hi_sw128_base32(512),
-                                umma::desc_lo(base + 3 * BA_TILE + k * 1024, BOX), umma::desc_hi_sw128_base32(512), idesc_g,
+                                umma::desc_lo(base + DY_OFF + k * 1024, BOX), umma::desc_hi_sw128_base32(512), idesc_g,
                                 k > 0 ? 1u : 0u);
           umma::mma_commit(&bars->g_full[ga]);          // also: the dgrad MMAs are done reading the old W tile
           if (ch == c1 - 1) {
@@ -473,9 +543,9 @@ __global__ void __launch_bounds__(BA_THREADS, 1) linear_bwd_adam_tc_kernel(
         const int c0 = si * g.chunks_per_split;
         const int c1 = min(c0 + g.chunks_per_split, g.chunks);
         for (int ch = c0; ch < c1; ++ch, ++c) {
-          const uint32_t s = c % BA_STAGES;
-          umma::mbar_wait_sleep(&bars->tile_ready[s], (c / BA_STAGES) & 1);
-          const uint32_t src = umma::smem_u32(smem + s * BA_STAGE_BYTES);
+          const uint32_t s = c % STAGES;
+          umma::mbar_wait_sleep(&bars->tile_ready[s], (c / STAGES) & 1);
+          const uint32_t src = umma::smem_u32(smem + s * STAGE_BYTES);
 #pragma unroll
           for (int i = 0; i < 4; ++i) {
             umma::tma_store_2d(&map_w, src + i * BOX, ti * 128 + 32 * i, ch * kChunk);
@@ -499,7 +569,7 @@ __global__ void __launch_bounds__(BA_THREADS, 1) linear_bwd_adam_tc_kernel(
       const int c0 = si * g.chunks_per_split;
       const int c1 = min(c0 + g.chunks_per_split, g.chunks);
       for (int ch = c0; ch < c1; ++ch, ++c) {
-        const uint32_t s = c % BA_STAGES, ga = c & 1;
+        const uint32_t s = c % STAGES, ga = c & 1;
         umma::mbar_wait_sleep(&bars->g_full[ga], (c >> 1) & 1);
         umma::tc_fence_after_sync();
         uint32_t gv[16];
@@ -508,13 +578,15 @@ __global__ void __launch_bounds__(BA_THREADS, 1) linear_bwd_adam_tc_kernel(
         umma::tc_fence_before_sync();
         __syncwarp();
         if (lane == 0) umma::mbar_arrive(&bars->g_empty[ga]);
-        const uint32_t wt = umma::smem_u32(smem + s * BA_STAGE_BYTES + quarter * BOX);
+        const uint32_t wt = umma::smem_u32(smem + s * STAGE_BYTES + quarter * BOX);
 #pragma unroll
         for (int j = 0; j < 16; ++j) {
           const int r = sub * 16 + j;
           const uint32_t e = wt + 4 * (r * 32 + ((((lane >> 3) ^ (r & 3)) << 3) | (lane & 7)));
           float m = lds_f32(e + BA_TILE), v = lds_f32(e + 2 * BA_TILE);
-          const float p = dd::adam_one(lds_f32(e), __uint_as_float(gv[j]), m, v, h);
+          float gr = __uint_as_float(gv[j]);
+          if (ACC) gr = gr + lds_f32(e + 3 * BA_TILE);     // dd_linear_wgrad_acc's dW_chunk + G, bit for bit
+          const float p = dd::adam_one(lds_f32(e), gr, m, v, h);
           sts_f32(e, p);
           sts_f32(e + BA_TILE, m);
           sts_f32(e + 2 * BA_TILE, v);
@@ -663,9 +735,20 @@ int linear_dgrad_tc(const float* dy, const float* w, void* dx, int dx_dtype, voi
   return g.splits > 1 ? check_launch("linear_dgrad_fold") : 0;
 }
 
-// dy fp32 [B][N], x fp32 [B][K], W / m / v fp32 [N][K] updated in place; dx [B][K] fp32 or bf16 from the old W, or nullptr
-int linear_bwd_adam_tc(const float* dy, const float* x, float* w, float* m, float* v, void* dx, int dx_dtype, void* ws,
-                       size_t ws_bytes, int B, int N, long long K, const AdamHyper& h, cudaStream_t st) {
+template <bool ACC, typename TOUT>
+int launch_bwd_adam(const CUtensorMap (&maps)[7], TOUT* dx, float* ws, const StreamGeo& g, const AdamHyper& h, cudaStream_t st) {
+  auto k = linear_bwd_adam_tc_kernel<TOUT, ACC>;
+  if (int e = set_smem(k, BaCfg<ACC>::SMEM, Carveout::kMaxShared, "linear_tc")) return e;
+  const int items = g.tiles * g.splits;
+  k<<<items < kSMs ? items : kSMs, BA_THREADS, BaCfg<ACC>::SMEM, st>>>(maps[0], maps[1], maps[2], maps[3], maps[4], maps[5], dx, ws,
+                                                                       g, h, maps[6]);
+  return check_launch("linear_bwd_adam_tc");
+}
+
+// dy fp32 [B][N], x fp32 [B][K], W / m / v fp32 [N][K] updated in place; dx [B][K] fp32 or bf16 from the old W, or nullptr;
+// gpart fp32 [N][K]: the stored partial gradient added to this pass's weight gradient before the step, or nullptr
+int linear_bwd_adam_tc(const float* dy, const float* x, float* w, float* m, float* v, const float* gpart, void* dx, int dx_dtype,
+                       void* ws, size_t ws_bytes, int B, int N, long long K, const AdamHyper& h, cudaStream_t st) {
   StreamGeo g;
   g.B = B; g.LD = (int)K;
   g.tiles = ceil_div(K, 128);
@@ -673,32 +756,29 @@ int linear_bwd_adam_tc(const float* dy, const float* x, float* w, float* m, floa
   plan_stream(g.tiles, g.chunks, g.splits, g.chunks_per_split);
   if (dx && g.splits > 1 && ws_bytes < (size_t)g.splits * B * K * sizeof(float))
     return fail(DD_ERR_WORKSPACE, "linear_bwd_adam_tc: workspace %zu too small for %d splits", ws_bytes, g.splits);
-  CUtensorMap mw, mm, mv, mdy, mdyt, mx;
+  CUtensorMap maps[7] = {};      // W, m, v, dy K-major, dy MN-major, x, G (the plain form passes an unused zero map)
   char msg[256];
-  if (tma_map_2d(&mw, w, 4, N, K, K, 32, 32, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, msg, sizeof msg) ||
-      tma_map_2d(&mm, m, 4, N, K, K, 32, 32, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, msg, sizeof msg) ||
-      tma_map_2d(&mv, v, 4, N, K, K, 32, 32, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, msg, sizeof msg) ||
-      tma_map_2d(&mdy, dy, 4, B, N, N, 32, 32, CU_TENSOR_MAP_SWIZZLE_128B, msg, sizeof msg) ||
-      tma_map_2d(&mdyt, dy, 4, B, N, N, 32, 32, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, msg, sizeof msg) ||
-      tma_map_2d(&mx, x, 4, B, K, K, 32, 32, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, msg, sizeof msg))
+  if (tma_map_2d(&maps[0], w, 4, N, K, K, 32, 32, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, msg, sizeof msg) ||
+      tma_map_2d(&maps[1], m, 4, N, K, K, 32, 32, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, msg, sizeof msg) ||
+      tma_map_2d(&maps[2], v, 4, N, K, K, 32, 32, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, msg, sizeof msg) ||
+      tma_map_2d(&maps[3], dy, 4, B, N, N, 32, 32, CU_TENSOR_MAP_SWIZZLE_128B, msg, sizeof msg) ||
+      tma_map_2d(&maps[4], dy, 4, B, N, N, 32, 32, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, msg, sizeof msg) ||
+      tma_map_2d(&maps[5], x, 4, B, K, K, 32, 32, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, msg, sizeof msg) ||
+      (gpart && tma_map_2d(&maps[6], gpart, 4, N, K, K, 32, 32, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, msg, sizeof msg)))
     return fail(DD_ERR_UNSUPPORTED, "linear_bwd_adam_tc: %s", msg);
-  const int items = g.tiles * g.splits;
-  const int grid = items < kSMs ? items : kSMs;
   const long long n = (long long)B * K;
   if (dx_dtype == DD_BF16 && dx) {
-    auto k = linear_bwd_adam_tc_kernel<__nv_bfloat16>;
-    if (int e = set_smem(k, BA_SMEM, Carveout::kMaxShared, "linear_tc")) return e;
-    k<<<grid, BA_THREADS, BA_SMEM, st>>>(mw, mm, mv, mdy, mdyt, mx, (__nv_bfloat16*)dx, (float*)ws, g, h);
-    if (int e = check_launch("linear_bwd_adam_tc")) return e;
+    auto* d = (__nv_bfloat16*)dx;
+    if (int e = gpart ? launch_bwd_adam<true>(maps, d, (float*)ws, g, h, st) : launch_bwd_adam<false>(maps, d, (float*)ws, g, h, st))
+      return e;
     if (g.splits > 1)
-      split_fold_kernel<__nv_bfloat16><<<ceil_div(n, 256), 256, 0, st>>>((const float*)ws, nullptr, (__nv_bfloat16*)dx, g.splits, n, (int)K);
+      split_fold_kernel<__nv_bfloat16><<<ceil_div(n, 256), 256, 0, st>>>((const float*)ws, nullptr, d, g.splits, n, (int)K);
   } else {
-    auto k = linear_bwd_adam_tc_kernel<float>;
-    if (int e = set_smem(k, BA_SMEM, Carveout::kMaxShared, "linear_tc")) return e;
-    k<<<grid, BA_THREADS, BA_SMEM, st>>>(mw, mm, mv, mdy, mdyt, mx, (float*)dx, (float*)ws, g, h);
-    if (int e = check_launch("linear_bwd_adam_tc")) return e;
+    auto* d = (float*)dx;
+    if (int e = gpart ? launch_bwd_adam<true>(maps, d, (float*)ws, g, h, st) : launch_bwd_adam<false>(maps, d, (float*)ws, g, h, st))
+      return e;
     if (dx && g.splits > 1)
-      split_fold_kernel<float><<<ceil_div(n, 256), 256, 0, st>>>((const float*)ws, nullptr, (float*)dx, g.splits, n, (int)K);
+      split_fold_kernel<float><<<ceil_div(n, 256), 256, 0, st>>>((const float*)ws, nullptr, d, g.splits, n, (int)K);
   }
   return dx && g.splits > 1 ? check_launch("linear_bwd_adam_fold") : 0;
 }
@@ -718,9 +798,35 @@ int linear_wgrad_tc(const float* dy, const float* x, float* dw, int B, int N, lo
     return fail(DD_ERR_UNSUPPORTED, "linear_wgrad_tc: %s", msg);
   const long long items = (long long)g.n_tiles * g.k_tiles;
   const int grid = (int)(items < kSMs ? items : kSMs);
-  if (int e = set_smem(linear_wgrad_tc_kernel, W_SMEM, Carveout::kMaxShared, "linear_tc")) return e;
-  linear_wgrad_tc_kernel<<<grid, W_THREADS, W_SMEM, st>>>(mdy, mx, dw, g);
+  if (int e = set_smem(linear_wgrad_tc_kernel<false>, W_SMEM, Carveout::kMaxShared, "linear_tc")) return e;
+  linear_wgrad_tc_kernel<false><<<grid, W_THREADS, W_SMEM, st>>>(mdy, mx, dw, g);
   return check_launch("linear_wgrad_tc");
+}
+
+// dy fp32 [B][N], x fp32 [B][K], 32 < B <= 128 -> dW fp32 [N][K] += the sum of the 32-row chunks' products, which are added
+// up before the old value (one launch; the batch chunks of an item share its TMEM)
+int linear_wgrad_acc_multi_tc(const float* dy, const float* x, float* dw, int B, int N, long long K, cudaStream_t st) {
+  WgradGeo g = {};
+  g.B = B; g.N = N; g.K = K;
+  g.KT = K >= 256 ? 256 : 128;
+  g.bchunks = ceil_div(B, NB);
+  if (g.bchunks * g.KT > 512) g.KT = 128;
+  if (g.bchunks * g.KT > 512)
+    return fail(DD_ERR_UNSUPPORTED, "linear_wgrad_acc_tc: %d rows exceed the %d TMEM columns (at most %d)", B, 512, 4 * NB);
+  g.nbuf = g.bchunks * g.KT <= 256 ? 2 : 1;
+  g.n_tiles = ceil_div(N, 128);
+  g.k_tiles = ceil_div(K, g.KT);
+  g.accumulate = 1;
+  CUtensorMap mdy, mx;
+  char msg[256];
+  if (tma_map_2d(&mdy, dy, 4, B, N, N, 32, 32, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, msg, sizeof msg) ||
+      tma_map_2d(&mx, x, 4, B, K, K, 32, 32, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, msg, sizeof msg))
+    return fail(DD_ERR_UNSUPPORTED, "linear_wgrad_acc_tc: %s", msg);
+  const long long items = (long long)g.n_tiles * g.k_tiles;
+  const int grid = (int)(items < kSMs ? items : kSMs);
+  if (int e = set_smem(linear_wgrad_tc_kernel<true>, W_SMEM, Carveout::kMaxShared, "linear_tc")) return e;
+  linear_wgrad_tc_kernel<true><<<grid, W_THREADS, W_SMEM, st>>>(mdy, mx, dw, g);
+  return check_launch("linear_wgrad_acc_tc");
 }
 
 }  // namespace dd

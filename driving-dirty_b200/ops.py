@@ -318,9 +318,9 @@ class SkinnyLinear(torch.autograd.Function):
     weight-streaming kernels (x is read as fp32)."""
 
     @staticmethod
-    def forward(ctx, x, w, b, impl, grad_buffer=None, grad_ready=None, fused_update=None):
+    def forward(ctx, x, w, b, impl, grad_buffer=None, grad_ready=None, fused_update=None, grad_begin=None):
         _require_cuda(x, w)
-        ctx.grad_buffer, ctx.grad_ready, ctx.fused_update = grad_buffer, grad_ready, fused_update
+        ctx.grad_buffer, ctx.grad_ready, ctx.fused_update, ctx.grad_begin = grad_buffer, grad_ready, fused_update, grad_begin
         x, wd = _c(x), _c(w.detach())
         if wd.dtype != torch.float32:
             wd = wd.float()
@@ -347,16 +347,17 @@ class SkinnyLinear(torch.autograd.Function):
         dy = _c(dy.float())
         st = stream_ptr()
         dx = dw = db = None
-        if ctx.needs_input_grad[1] and ctx.fused_update is not None and ctx.impl == _lib.IMPL_TCGEN05 and B <= 32 \
-                and x.dtype == torch.float32:
+        fusable = ctx.impl == _lib.IMPL_TCGEN05 and B <= 32 and x.dtype == torch.float32
+        if ctx.needs_input_grad[1] and ctx.fused_update is not None and ctx.fused_update.takes(fusable):
             # optim.FusedAdam (world size 1) folds this weight's Adam step into the backward pass: one kernel computes the
             # input gradient from the old weight and updates the weight and its moments in place; the weight gradient never
-            # exists in HBM (dd_linear_bwd_adam)
+            # exists in HBM (dd_linear_bwd_adam).  With gradient accumulation it takes every pass of a window: the earlier
+            # ones add into its gradient buffer, the last one steps from it (dd_linear_bwd_adam_acc)
             dx = torch.empty(B, K, dtype=ctx.x_dtype, device=x.device) if ctx.needs_input_grad[0] else None
             ws, n = _linear_ws(B, N, K, x.device)
             db = torch.empty(N, dtype=torch.float32, device=x.device) if ctx.has_bias else None
-            ctx.fused_update(dy, x, dx, db, ws, n)
-            return dx, None, db, None, None, None, None
+            ctx.fused_update(dy, x, w, dx, db, ws, n, fusable, ctx.impl)
+            return dx, None, db, None, None, None, None, None
         if ctx.needs_input_grad[0]:
             dx = torch.empty(B, K, dtype=ctx.x_dtype, device=x.device)
             ws, n = _linear_ws(B, N, K, x.device)
@@ -368,15 +369,20 @@ class SkinnyLinear(torch.autograd.Function):
             direct = ctx.grad_buffer is not None
             dw = ctx.grad_buffer if direct else torch.empty_like(w)
             db = torch.empty(N, dtype=torch.float32, device=x.device) if ctx.has_bias else None
-            call("dd_linear_wgrad", dy.data_ptr(), x.data_ptr(), dtype_code(x.dtype), dw.data_ptr(),
-                 db.data_ptr() if db is not None else None, B, N, K, ctx.impl, st)
+            # ... which the passes after the first of a gradient-accumulation window add to (FusedAdam's grad_begin)
+            if direct and ctx.grad_begin is not None and ctx.grad_begin():
+                call("dd_linear_wgrad_acc", dy.data_ptr(), x.data_ptr(), dtype_code(x.dtype), dw.data_ptr(),
+                     db.data_ptr() if db is not None else None, B, N, K, ctx.impl, 1, st)
+            else:
+                call("dd_linear_wgrad", dy.data_ptr(), x.data_ptr(), dtype_code(x.dtype), dw.data_ptr(),
+                     db.data_ptr() if db is not None else None, B, N, K, ctx.impl, st)
             if direct:
                 dw = None
                 if ctx.grad_ready is not None:
                     ctx.grad_ready()
         elif ctx.has_bias and ctx.needs_input_grad[2]:
             db = dy.sum(0)
-        return dx, dw, db, None, None, None, None
+        return dx, dw, db, None, None, None, None, None
 
 
 def linear(x, weight, bias=None, impl=IMPL_AUTO, allow_tf32=False):
@@ -396,7 +402,8 @@ def linear(x, weight, bias=None, impl=IMPL_AUTO, allow_tf32=False):
     if buf is not None and not (buf.shape == weight.shape and buf.dtype == torch.float32 and buf.is_contiguous()):
         raise RuntimeError("linear: weight._dd_grad_buffer does not match the weight")
     return SkinnyLinear.apply(x, weight, bias, impl, buf, getattr(weight, "_dd_grad_ready", None) if buf is not None else None,
-                              getattr(weight, "_dd_fused_update", None) if torch.is_grad_enabled() else None)
+                              getattr(weight, "_dd_fused_update", None) if torch.is_grad_enabled() else None,
+                              getattr(weight, "_dd_grad_begin", None) if buf is not None else None)
 
 
 # --------------------------------------------------------------------------------------------

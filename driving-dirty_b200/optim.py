@@ -26,6 +26,16 @@ the rank that writes a checkpoint (rank 0 under Lightning) assembles the full mo
 collective, and every rank re-slices its own shard on load -- a checkpoint moves between world sizes and to / from
 torch.optim.Adam.
 
+Gradient accumulation (``accumulate_grad_batches=k``, Lightning's flag of the same name): a *window* is the k backward
+passes between two ``step()`` calls.  The wide weights' gradients add up within a window exactly as autograd adds them
+(``dd_linear_wgrad_acc``: the first pass of a window overwrites, later passes add), and their Adam step runs once per
+window -- inside the window's last backward pass where it can: world size N launches the sharded update from pass k,
+world size 1 with ``overlap_backward=True`` runs ``dd_linear_bwd_adam_acc`` (step folded into the backward pass, 28 bytes
+per parameter) on pass k, from a persistent gradient buffer per wide weight that holds passes 1 .. k-1.  A ``step()``
+after fewer than k passes updates from the gradients gathered so far; ``zero_grad()`` discards an unfinished window; a
+(k+1)-th pass without a ``step()`` is refused.  With ``overlap_backward=False`` at world size 1 the wide weights' gradients
+go through autograd, which accumulates them itself.
+
 Semantics are torch.optim.Adam's (amsgrad off, L2 weight decay); ``param_groups[i]['lr']`` is read
 every step, so ``ReduceLROnPlateau`` (roadmap_bce_v2.py:156) works unchanged; tensors whose
 gradient is ``None`` are skipped (a partly frozen flat bucket is updated per tensor on every replica).
@@ -53,6 +63,17 @@ def shard_bounds(numel: int, world: int, rank: int):
     return 4 * lo, 4 * hi
 
 
+def accumulation_factor(accumulate_grad_batches, epoch: int = 0) -> int:
+    """The number of backward passes per optimizer step: an int, or Lightning's ``{epoch: factor}`` schedule (the factor
+    of the largest epoch key <= ``epoch``; 1 before the first key)."""
+    k = accumulate_grad_batches
+    if isinstance(k, dict):
+        k = next((k[e] for e in sorted(k, reverse=True) if epoch >= e), 1)
+    if isinstance(k, bool) or int(k) != k or int(k) < 1:
+        raise ValueError(f"accumulate_grad_batches must be a positive integer, got {k!r}")
+    return int(k)
+
+
 def flat_layout(numels, align: int = _ALIGN):
     """Offsets of tensors packed into one flat region (each start aligned) and the region's length."""
     offs, off = [], 0
@@ -65,10 +86,19 @@ def flat_layout(numels, align: int = _ALIGN):
 class FusedAdam(torch.optim.Optimizer):
     def __init__(self, params, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0, process_group=None,
                  shard_min_numel: int = 1 << 20, multicast: bool | None = None, broadcast_init: bool = True,
-                 overlap_backward: bool = False, fuse_into_backward: bool = False, defer_join: bool = True):
+                 overlap_backward: bool = False, fuse_into_backward: bool = False, defer_join: bool = True,
+                 accumulate_grad_batches=1):
         if lr < 0 or eps < 0 or not (0 <= betas[0] < 1) or not (0 <= betas[1] < 1) or weight_decay < 0:
             raise ValueError("invalid Adam hyper-parameters")
         super().__init__(params, dict(lr=lr, betas=betas, eps=eps, weight_decay=weight_decay))
+        accumulation_factor(accumulate_grad_batches)          # validates an int (a schedule is checked per window)
+        # backward passes per step: an int, or a {epoch: factor} schedule read at the first backward pass of each window
+        # against self.current_epoch() (make_adam: the module's current_epoch); may be changed between steps
+        self.accumulate_grad_batches = accumulate_grad_batches
+        self.current_epoch = lambda: 0
+        self._window_k = None       # factor of the window in progress, resolved at its first backward pass
+        self._passes = {}           # id(wide param) -> backward passes that wrote its gradient in the window in progress
+        self._acc_buf = {}          # world size 1: id(wide param) -> gradient buffer of passes 1 .. k-1 (allocated on first use)
         if len(self.param_groups) > 1 and dist.is_initialized() and dist.get_world_size(process_group) > 1:
             raise NotImplementedError("FusedAdam: the sharded form supports one parameter group")
         self.group = process_group
@@ -169,6 +199,7 @@ class FusedAdam(torch.optim.Optimizer):
             gview = adopt(p, off)
             p.grad = gview
             p._dd_grad_buffer = gview                    # ops.linear's weight-gradient kernel writes here ...
+            p._dd_grad_begin = (lambda q: (lambda: self._begin_grad(q)))(p)          # (overwrite, or accumulate?)
             p._dd_grad_ready = (lambda q: (lambda: self._on_grad_written(q)))(p)     # ... and then calls this
             lo, hi = shard_bounds(p.numel(), self.world, self.rank)
             self._regions[id(p)] = dict(off=off, n=p.numel(), lo=lo, hi=hi, channel=1 + len(self._regions), key=p)
@@ -200,13 +231,56 @@ class FusedAdam(torch.optim.Optimizer):
         memory once: the input gradient is computed from the old weight, the weight gradient is consumed on chip where it is
         produced, and the updated weight and moments are written back -- 24 bytes per parameter instead of the 40 of the
         input-gradient, weight-gradient and Adam kernels, and no gradient buffers (1.3 GB less for RoadMapBCE).  Results are
-        those of the unfused form.  step() then skips these weights.  Like the sharded form's overlap_backward this is for
-        loops that step after every backward (the reference's); ops.linear falls back to a stored gradient whenever the fused
-        kernel does not apply (batch > 32, CUDA-core path), and step() handles that."""
+        those of the unfused form.  step() then skips these weights.  With accumulate_grad_batches = 1 ops.linear falls back
+        to a stored gradient whenever the fused kernel does not apply (batch > 32, CUDA-core path), and step() handles that;
+        with k > 1 every backward pass of these weights comes here (_window_backward)."""
         for g in self.param_groups:
             for p in g["params"]:
                 if p.dim() == 2 and p.numel() >= min_numel and p.is_cuda:
-                    p._dd_fused_update = (lambda q, grp: (lambda dy, x, dx, db, ws, n: self._fused_step(grp, q, dy, x, dx, db, ws, n)))(p, g)
+                    p._dd_fused_update = _BackwardHook(self, g, p)
+
+    def _factor(self):
+        """accumulate_grad_batches of the window in progress (a schedule is resolved at the window's first pass)."""
+        if self._window_k is None:
+            self._window_k = accumulation_factor(self.accumulate_grad_batches, self.current_epoch())
+        return self._window_k
+
+    def _refuse_pass(self, n, what):
+        raise RuntimeError(f"FusedAdam: backward pass {n} without a step() in between reached {what}, but "
+                           f"accumulate_grad_batches={self._window_k} (set it to accumulate more passes per step)")
+
+    @torch.no_grad()
+    def _window_backward(self, g, p, dy, x, w, dx, db, ws, ws_bytes, fusable, impl):
+        """World size 1, accumulate_grad_batches = k > 1: one backward pass of a wide weight.  Passes 1 .. k-1 compute the
+        input gradient and add the weight gradient into the weight's buffer (the first pass overwrites it); pass k runs
+        dd_linear_bwd_adam_acc (the step folded in) where the fused kernel applies, else it adds into the buffer as well and
+        step() steps from there."""
+        key = id(p)
+        k = self._factor()
+        j = self._passes.get(key, 0)
+        if j >= k or key in self._fused:
+            self._refuse_pass(j + 1, "a weight whose window is complete")
+        B, K = x.shape
+        N = p.shape[0]
+        buf = self._acc_buf.get(key)
+        if buf is None:
+            buf = self._acc_buf[key] = torch.empty_like(p)
+        if j + 1 == k and fusable:
+            st = self._state(p, p.numel(), p.device)
+            st["step"] += 1
+            call("dd_linear_bwd_adam_acc", dy.data_ptr(), x.data_ptr(), p.data_ptr(), st["exp_avg"].data_ptr(),
+                 st["exp_avg_sq"].data_ptr(), buf.data_ptr(), dx.data_ptr() if dx is not None else None,
+                 _lib.dtype_code(dx.dtype) if dx is not None else _lib.DD_F32, db.data_ptr() if db is not None else None,
+                 ws.data_ptr(), ws_bytes, B, N, K, float(g["lr"]), float(g["betas"][0]), float(g["betas"][1]),
+                 float(g["eps"]), float(g["weight_decay"]), st["step"], stream_ptr())
+            self._fused[key] = True
+        else:
+            if dx is not None:
+                call("dd_linear_dgrad", dy.data_ptr(), w.data_ptr(), dx.data_ptr(), _lib.dtype_code(dx.dtype), ws.data_ptr(),
+                     ws_bytes, B, N, K, impl, stream_ptr())
+            call("dd_linear_wgrad_acc", dy.data_ptr(), x.data_ptr(), _lib.dtype_code(x.dtype), buf.data_ptr(),
+                 db.data_ptr() if db is not None else None, B, N, K, impl, int(j > 0), stream_ptr())
+        self._passes[key] = j + 1
 
     @torch.no_grad()
     def _fused_step(self, g, p, dy, x, dx, db, ws, ws_bytes):
@@ -228,6 +302,15 @@ class FusedAdam(torch.optim.Optimizer):
 
     # ------------------------------------------------------------------------------------------
     def zero_grad(self, set_to_none: bool = True):
+        # an unfinished accumulation window is discarded (its next pass overwrites the gradient buffer again); a finished
+        # one -- its update already launched or folded into the backward pass -- is left for step()
+        k = self._window_k
+        for key, n in list(self._passes.items()):
+            if n < k and key not in self._fused:
+                del self._passes[key]
+                self._written.discard(key)
+        if not self._passes and not self._written and not self._fused:
+            self._window_k = None
         for g in self.param_groups:
             for p in g["params"]:
                 if id(p) in self._regions:       # persistent view of the symmetric buffer, overwritten by every backward
@@ -268,14 +351,18 @@ class FusedAdam(torch.optim.Optimizer):
         if closure is not None:
             with torch.enable_grad():
                 loss = closure()
+        self._window_k = None
         if self.world == 1:
             for g in self.param_groups:
                 for p in g["params"]:
                     if id(p) in self._fused:              # stepped inside the backward pass
                         continue
-                    if p.grad is not None:
+                    if id(p) in self._passes:             # accumulation buffer: a window without the fused last pass
+                        self._launch_local(g, p, self._acc_buf[id(p)])
+                    elif p.grad is not None:
                         self._launch_local(g, p, p.grad)
             self._fused.clear()
+            self._passes.clear()
             return loss
         if self._symm is None:
             return loss
@@ -328,6 +415,7 @@ class FusedAdam(torch.optim.Optimizer):
                 torch.cuda.current_stream().wait_stream(self._side)
         self._launched.clear()
         self._written.clear()
+        self._passes.clear()
         return loss
 
     def synchronize(self):
@@ -472,18 +560,30 @@ class FusedAdam(torch.optim.Optimizer):
         call("dd_adam_step_sharded", gptrs, wptrs, mcg, mcw, W, self.rank, st["exp_avg"].data_ptr(),
              st["exp_avg_sq"].data_ptr(), lo, hi - lo, lr, b1, b2, eps, wd, st["step"], 1.0 / W, int(ctas_per_sm), stream_ptr())
 
+    def _begin_grad(self, p):
+        """Called by ops.linear's backward before it writes p's gradient replica: 0 = overwrite (first pass of a window),
+        1 = add to it (passes 2 .. k, dd_linear_wgrad_acc)."""
+        n = self._passes.get(id(p), 0)
+        if n >= self._factor():
+            self._refuse_pass(n + 1, "a sharded parameter")
+        return int(n > 0)
+
     @torch.no_grad()
     def _on_grad_written(self, p):
-        """Called by ops.linear's backward right after p's gradient replica is written.  overlap_backward: the reduce
-        + Adam + all-gather kernel is launched here, on a side stream, one 256-thread CTA per SM beside the persistent
-        conv kernels of the rest of the backward pass; step() joins the side stream.  (The weights then change before
-        step() is called: for training loops that step after every backward, like the reference's.)"""
+        """Called by ops.linear's backward right after p's gradient replica is written.  overlap_backward: on the last
+        pass of an accumulation window (every pass when accumulate_grad_batches = 1) the reduce + Adam + all-gather kernel
+        is launched here, on a side stream, one 256-thread CTA per SM beside the persistent conv kernels of the rest of the
+        backward pass; step() joins the side stream.  (The weights then change before step() is called: for training
+        loops that step after every window, like the reference's.)  Earlier passes of a window stay on this rank."""
         key = id(p)
-        if key in self._written:
+        k = self._factor()
+        n = self._passes.get(key, 0) + 1
+        if n > k:
             raise RuntimeError("FusedAdam: two backward passes wrote the gradient of a sharded parameter without a "
-                               "step() in between (its gradient buffer is overwritten, not accumulated)")
+                               f"step() in between (accumulate_grad_batches={k}: a window of {k} passes per step)")
+        self._passes[key] = n
         self._written.add(key)
-        if not self._overlap:
+        if not self._overlap or n < k:
             return
         r = self._regions[key]
         hdl = self._symm["hdl"]
@@ -495,17 +595,48 @@ class FusedAdam(torch.optim.Optimizer):
         self._launched.add(key)
 
 
+def follow_accumulation(opt, module):
+    """Give FusedAdam the module's ``hparams.accumulate_grad_batches`` (1 when absent) and its ``current_epoch`` for an
+    ``{epoch: factor}`` schedule."""
+    hp = getattr(module, "hparams", None)
+    acc = getattr(hp, "accumulate_grad_batches", None) if hp is not None else None
+    accumulation_factor(1 if acc is None else acc)
+    opt.accumulate_grad_batches = 1 if acc is None else acc
+    opt.current_epoch = lambda: int(getattr(module, "current_epoch", 0) or 0)
+
+
+class _BackwardHook:
+    """``weight._dd_fused_update`` at world size 1: ops.linear's backward hands FusedAdam the weight's backward pass when
+    ``takes(fusable)`` -- the fused backward + Adam kernel applies (``fusable``), or an accumulation window is open."""
+
+    def __init__(self, opt, group, p):
+        self.opt, self.group, self.p = opt, group, p
+
+    def takes(self, fusable: bool) -> bool:
+        return fusable or self.opt._factor() > 1
+
+    def __call__(self, dy, x, w, dx, db, ws, ws_bytes, fusable, impl):
+        if self.opt._factor() == 1:
+            self.opt._fused_step(self.group, self.p, dy, x, dx, db, ws, ws_bytes)
+        else:
+            self.opt._window_backward(self.group, self.p, dy, x, w, dx, db, ws, ws_bytes, fusable, impl)
+
+
 def make_adam(module, lr):
     """What the task modules' ``configure_optimizers`` return for ``torch.optim.Adam(self.parameters(), lr)``
     (roadmap_bce_v2.py:155, autoencoder.py:120, spatial_w_rm.py:189).  hparams.optimizer = "fused" (the default when the
     model sits on a CUDA device): ``FusedAdam`` -- the dd_adam_step kernels, and under torch.distributed the sharded
-    reduce + Adam + all-gather exchange, launched from the backward pass; "torch": the reference's optimizer object."""
+    reduce + Adam + all-gather exchange, launched from the backward pass; "torch": the reference's optimizer object.
+    ``hparams.accumulate_grad_batches`` (what Lightning's ``Trainer.add_argparse_args`` puts on the Namespace; an int or an
+    ``{epoch: factor}`` dict, read against ``module.current_epoch`` at the first backward pass of each window) becomes
+    FusedAdam's window of backward passes per step."""
     hp = getattr(module, "hparams", None)
     kind = getattr(hp, "optimizer", "fused") if hp is not None else "fused"
     params = [p for p in module.parameters()]
     on_cuda = bool(params) and all(p.is_cuda for p in params)
     if kind == "fused" and on_cuda:
         opt = FusedAdam(params, lr=lr, overlap_backward=dist.is_initialized() and dist.get_world_size() > 1)
+        follow_accumulation(opt, module)
         # a checkpoint (module.state_dict()) must see the weights of updates that are still in flight on the side stream
         module.register_state_dict_pre_hook(lambda *a, **k: opt.synchronize())
         return opt

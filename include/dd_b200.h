@@ -155,6 +155,14 @@ int dd_linear_dgrad(const float* dy, const float* w, void* dx, int dx_dtype, voi
                     size_t ws_bytes, int B, int N, long long K, int impl, void* stream);
 int dd_linear_wgrad(const float* dy, const void* x, int x_dtype, float* dw, float* db, int B,
                     int N, long long K, int impl, void* stream);
+/* Gradient accumulation over micro-batches (autograd's `.grad +=` on the wide weights between two optimizer steps, e.g.
+ * Lightning's accumulate_grad_batches): accumulate = 0 is dd_linear_wgrad; accumulate = 1 writes dw = dw_old + D, where D is
+ * bit for bit what dd_linear_wgrad writes for the same call -- for B > 32 too, whose 32-row chunks are summed before dw_old
+ * is added, as autograd adds one finished gradient.  db (may be NULL) is always overwritten (the bias goes through autograd).
+ * Errors as dd_linear_wgrad's (null pointer: DD_ERR_BAD_ARG; dw not 16-byte aligned: DD_ERR_ALIGNMENT; tcgen05 without its
+ * shape or with bf16 x: DD_ERR_UNSUPPORTED), and accumulate with B > 128: DD_ERR_UNSUPPORTED. */
+int dd_linear_wgrad_acc(const float* dy, const void* x, int x_dtype, float* dw, float* db, int B,
+                        int N, long long K, int impl, int accumulate, void* stream);
 /* The backward pass of a wide linear layer with torch.optim.Adam's update of W (roadmap_bce_v2.py:155) folded in, for world
  * size 1.  ONE pass over each weight tile: the tile of W, exp_avg and exp_avg_sq is loaded once, the input gradient dx is
  * computed from the OLD W (bit-identical to dd_linear_dgrad), the weight gradient dy^T x is formed on chip and never reaches
@@ -165,6 +173,17 @@ int dd_linear_wgrad(const float* dy, const void* x, int x_dtype, float* dw, floa
 int dd_linear_bwd_adam(const float* dy, const float* x, float* weight, float* exp_avg, float* exp_avg_sq, void* dx,
                        int dx_dtype, float* db, void* workspace, size_t ws_bytes, int B, int N, long long K, float lr,
                        float beta1, float beta2, float eps, float weight_decay, long long step, void* stream);
+/* The last backward pass of a gradient-accumulation window with the step folded in: dd_linear_bwd_adam with the weight
+ * gradient taken as dW + grad_partial, where dW is this pass's dy^T x and grad_partial fp32 [N,K] (16-byte aligned) holds
+ * the sum of the window's earlier passes (dd_linear_wgrad_acc).  Bit for bit dd_linear_dgrad + dd_linear_wgrad_acc into
+ * grad_partial + dd_adam_step from it; grad_partial is only read.  28 bytes per parameter (W, exp_avg, exp_avg_sq read and
+ * written, grad_partial read) instead of the 40 of those three launches.  Errors as dd_linear_bwd_adam's: a null pointer,
+ * B > 32 or step < 1: DD_ERR_BAD_ARG; no tensor-core path for the shape: DD_ERR_UNSUPPORTED; a pointer not 16-byte aligned:
+ * DD_ERR_ALIGNMENT; workspace too small with dx: DD_ERR_WORKSPACE. */
+int dd_linear_bwd_adam_acc(const float* dy, const float* x, float* weight, float* exp_avg, float* exp_avg_sq,
+                           const float* grad_partial, void* dx, int dx_dtype, float* db, void* workspace, size_t ws_bytes,
+                           int B, int N, long long K, float lr, float beta1, float beta2, float eps, float weight_decay,
+                           long long step, void* stream);
 size_t dd_linear_workspace_bytes(int B, int N, long long K);
 /* impl = DD_IMPL_TCGEN05 runs the weight-streaming tensor-core kernels (fp32 operands read as tf32 through
  * TMA; x must be fp32): allowed when this returns 1 (N, K multiples of 4, N*K >= 2^22).  DD_IMPL_AUTO
