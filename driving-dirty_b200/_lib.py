@@ -77,6 +77,9 @@ SIGNATURES = {
     "dd_mse_bwd": (_I, [_P, _P, _P, _P, _L, _P]),
     "dd_adam_step": (_I, [_P, _P, _P, _P, _L, _F, _F, _F, _F, _F, _L, _F, _P]),
     "dd_adam_step_sharded": (_I, [_P, _P, _P, _P, _I, _I, _P, _P, _L, _L, _F, _F, _F, _F, _F, _L, _F, _I, _P]),
+    "dd_grad_sumsq_workspace_bytes": (_Z, []),
+    "dd_grad_sumsq": (_I, [_P, _P, _I, _F, _P, _P, _Z, _P]),
+    "dd_adam_step_clipped": (_I, [_P, _P, _P, _P, _L, _F, _F, _F, _F, _F, _L, _F, _P, _P]),
 }
 
 

@@ -36,6 +36,13 @@ after fewer than k passes updates from the gradients gathered so far; ``zero_gra
 (k+1)-th pass without a ``step()`` is refused.  With ``overlap_backward=False`` at world size 1 the wide weights' gradients
 go through autograd, which accumulates them itself.
 
+Gradient clipping (``gradient_clip_val=c``, Lightning's flag of the same name; world size 1): the step applies
+``torch.nn.utils.clip_grad_norm_(params, c)`` to the gradients it is about to apply -- every group, the window's accumulated
+gradients -- before Adam.  The norm and the coefficient stay on the device (``dd_grad_sumsq``, then ``dd_adam_step_clipped``
+per tensor), so the step has no host sync; ``last_grad_norm`` is the pre-clip total norm, as ``clip_grad_norm_`` returns it.
+Clipping needs every gradient before any update, so under it the wide weights' step does not run inside the backward pass:
+their gradients are written (or accumulated) and step() applies them.
+
 Semantics are torch.optim.Adam's (amsgrad off, L2 weight decay); ``param_groups[i]['lr']`` is read
 every step, so ``ReduceLROnPlateau`` (roadmap_bce_v2.py:156) works unchanged; tensors whose
 gradient is ``None`` are skipped (a partly frozen flat bucket is updated per tensor on every replica).
@@ -43,6 +50,8 @@ gradient is ``None`` are skipped (a partly frozen flat bucket is updated per ten
 from __future__ import annotations
 
 import ctypes
+import math
+import warnings
 
 import torch
 import torch.distributed as dist
@@ -74,6 +83,19 @@ def accumulation_factor(accumulate_grad_batches, epoch: int = 0) -> int:
     return int(k)
 
 
+_NO_SHARDED_CLIP = ("FusedAdam: gradient_clip_val is supported at world size 1; the data-parallel form has no clipping yet "
+                    "(its norm must be that of the rank-averaged gradient)")
+
+
+def gradient_clip_value(c) -> float:
+    """Lightning's ``gradient_clip_val``: the max_norm of clip_grad_norm_, 0.0 (or None) for off."""
+    if c is None:
+        return 0.0
+    if isinstance(c, bool) or not isinstance(c, (int, float)) or not math.isfinite(c) or c < 0:
+        raise ValueError(f"gradient_clip_val must be a finite number >= 0 (0 = off), got {c!r}")
+    return float(c)
+
+
 def flat_layout(numels, align: int = _ALIGN):
     """Offsets of tensors packed into one flat region (each start aligned) and the region's length."""
     offs, off = [], 0
@@ -87,7 +109,7 @@ class FusedAdam(torch.optim.Optimizer):
     def __init__(self, params, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0, process_group=None,
                  shard_min_numel: int = 1 << 20, multicast: bool | None = None, broadcast_init: bool = True,
                  overlap_backward: bool = False, fuse_into_backward: bool = False, defer_join: bool = True,
-                 accumulate_grad_batches=1):
+                 accumulate_grad_batches=1, gradient_clip_val=0.0):
         if lr < 0 or eps < 0 or not (0 <= betas[0] < 1) or not (0 <= betas[1] < 1) or weight_decay < 0:
             raise ValueError("invalid Adam hyper-parameters")
         super().__init__(params, dict(lr=lr, betas=betas, eps=eps, weight_decay=weight_decay))
@@ -96,6 +118,10 @@ class FusedAdam(torch.optim.Optimizer):
         # against self.current_epoch() (make_adam: the module's current_epoch); may be changed between steps
         self.accumulate_grad_batches = accumulate_grad_batches
         self.current_epoch = lambda: 0
+        # last_grad_norm: the last clipped step's total norm, a 0-dim fp32 tensor on the device (None before)
+        self._clip_val = gradient_clip_value(gradient_clip_val)
+        self.last_grad_norm = None
+        self._clip_ws = None        # dd_grad_sumsq's workspace (zeroed once, self-resetting)
         self._window_k = None       # factor of the window in progress, resolved at its first backward pass
         self._passes = {}           # id(wide param) -> backward passes that wrote its gradient in the window in progress
         self._acc_buf = {}          # world size 1: id(wide param) -> gradient buffer of passes 1 .. k-1 (allocated on first use)
@@ -104,6 +130,8 @@ class FusedAdam(torch.optim.Optimizer):
         self.group = process_group
         self.world = dist.get_world_size(process_group) if dist.is_initialized() else 1
         self.rank = dist.get_rank(process_group) if dist.is_initialized() else 0
+        if self._clip_val and self.world > 1:
+            raise NotImplementedError(_NO_SHARDED_CLIP)
         self._regions = {}          # id(param) -> region dict of a wide tensor
         self._flat = None           # region dict of the flat bucket
         self._symm = None
@@ -297,6 +325,23 @@ class FusedAdam(torch.optim.Optimizer):
         self._fused[id(p)] = True
 
     @property
+    def gradient_clip_val(self) -> float:
+        """max_norm of the clip_grad_norm_ every step applies (0 = off).  It decides whether a wide weight's step may run
+        inside the backward pass, so it changes between steps only: not after a backward pass of a window whose step()
+        has not run yet."""
+        return self._clip_val
+
+    @gradient_clip_val.setter
+    def gradient_clip_val(self, c):
+        c = gradient_clip_value(c)
+        if c and self.world > 1:
+            raise NotImplementedError(_NO_SHARDED_CLIP)
+        if c != self._clip_val and (self._passes or self._fused or self._written):
+            raise RuntimeError("FusedAdam: gradient_clip_val cannot change after a backward pass of a window whose step() "
+                               "has not run; change it between steps")
+        self._clip_val = c
+
+    @property
     def uses_multicast(self) -> bool:
         return bool(self._symm and self._symm["mc"])
 
@@ -353,14 +398,23 @@ class FusedAdam(torch.optim.Optimizer):
                 loss = closure()
         self._window_k = None
         if self.world == 1:
+            todo = []
             for g in self.param_groups:
                 for p in g["params"]:
                     if id(p) in self._fused:              # stepped inside the backward pass
                         continue
                     if id(p) in self._passes:             # accumulation buffer: a window without the fused last pass
-                        self._launch_local(g, p, self._acc_buf[id(p)])
+                        todo.append((g, p, self._acc_buf[id(p)]))
                     elif p.grad is not None:
-                        self._launch_local(g, p, p.grad)
+                        todo.append((g, p, p.grad))
+            if self.gradient_clip_val:
+                todo = [(g, p, _f32(grad)) for g, p, grad in todo]
+                coef = self._clip([grad for _, _, grad in todo])
+                for g, p, grad in todo:
+                    self._launch_local(g, p, grad, coef)
+            else:
+                for g, p, grad in todo:
+                    self._launch_local(g, p, grad)
             self._fused.clear()
             self._passes.clear()
             return loss
@@ -537,15 +591,32 @@ class FusedAdam(torch.optim.Optimizer):
             if got:
                 self.state[p] = {"step": got[0], "exp_avg": got[1].clone(), "exp_avg_sq": got[2].clone()}
 
-    def _launch_local(self, g, p, grad):
-        """One dd_adam_step launch: the whole tensor, this replica only."""
-        if not (grad.is_contiguous() and grad.dtype == torch.float32):
-            grad = grad.contiguous().float()
+    def _clip(self, grads):
+        """clip_grad_norm_'s total norm and coefficient over `grads` (contiguous fp32), on the device: one dd_grad_sumsq
+        call.  Sets last_grad_norm; returns the coefficient (a 1-element device tensor)."""
+        dev = self.param_groups[0]["params"][0].device
+        if self._clip_ws is None:
+            self._clip_ws = torch.zeros(int(self._lib.dd_grad_sumsq_workspace_bytes()), dtype=torch.uint8, device=dev)
+        out = torch.empty(4, dtype=torch.float32, device=dev)       # norm, coefficient, fp64 sum of squares
+        n = len(grads)
+        call("dd_grad_sumsq", (ctypes.c_void_p * n)(*[t.data_ptr() for t in grads]),
+             (ctypes.c_longlong * n)(*[t.numel() for t in grads]), n, self.gradient_clip_val, out.data_ptr(),
+             self._clip_ws.data_ptr(), self._clip_ws.numel(), stream_ptr())
+        self.last_grad_norm = out[0]
+        return out[1:]
+
+    def _launch_local(self, g, p, grad, coef=None):
+        """One dd_adam_step launch: the whole tensor, this replica only (dd_adam_step_clipped with a clip coefficient)."""
+        grad = _f32(grad)
         st = self._state(p, p.numel(), p.device)
         st["step"] += 1
-        call("dd_adam_step", p.data_ptr(), grad.data_ptr(), st["exp_avg"].data_ptr(), st["exp_avg_sq"].data_ptr(),
-             p.numel(), float(g["lr"]), float(g["betas"][0]), float(g["betas"][1]), float(g["eps"]),
-             float(g["weight_decay"]), st["step"], 1.0, stream_ptr())
+        args = (p.data_ptr(), grad.data_ptr(), st["exp_avg"].data_ptr(), st["exp_avg_sq"].data_ptr(), p.numel(),
+                float(g["lr"]), float(g["betas"][0]), float(g["betas"][1]), float(g["eps"]), float(g["weight_decay"]),
+                st["step"], 1.0)
+        if coef is None:
+            call("dd_adam_step", *args, stream_ptr())
+        else:
+            call("dd_adam_step_clipped", *args, coef.data_ptr(), stream_ptr())
 
     def _launch_sharded(self, r, ctas_per_sm):
         sy, W = self._symm, self.world
@@ -595,6 +666,10 @@ class FusedAdam(torch.optim.Optimizer):
         self._launched.add(key)
 
 
+def _f32(grad):
+    return grad if grad.is_contiguous() and grad.dtype == torch.float32 else grad.contiguous().float()
+
+
 def follow_accumulation(opt, module):
     """Give FusedAdam the module's ``hparams.accumulate_grad_batches`` (1 when absent) and its ``current_epoch`` for an
     ``{epoch: factor}`` schedule."""
@@ -605,17 +680,32 @@ def follow_accumulation(opt, module):
     opt.current_epoch = lambda: int(getattr(module, "current_epoch", 0) or 0)
 
 
+def follow_clipping(hparams, distributed: bool) -> float:
+    """FusedAdam's gradient_clip_val from the Namespace's (Lightning's flag; 0 when absent).  Under torch.distributed
+    FusedAdam does not clip yet: the flag is then left to the Trainer, as it was before FusedAdam could clip, with a
+    warning."""
+    clip = gradient_clip_value(getattr(hparams, "gradient_clip_val", None))
+    if clip and distributed:
+        warnings.warn("make_adam: FusedAdam does not clip gradients under torch.distributed; gradient_clip_val is left to "
+                      "the Trainer, whose clip misses the wide weights (they step inside the backward pass)")
+        return 0.0
+    return clip
+
+
 class _BackwardHook:
     """``weight._dd_fused_update`` at world size 1: ops.linear's backward hands FusedAdam the weight's backward pass when
-    ``takes(fusable)`` -- the fused backward + Adam kernel applies (``fusable``), or an accumulation window is open."""
+    ``takes(fusable)`` -- the fused backward + Adam kernel applies (``fusable``), or an accumulation window is open.  Under
+    gradient clipping the step cannot run inside the backward pass (the norm needs every gradient first): the pass is never
+    fusable then."""
 
     def __init__(self, opt, group, p):
         self.opt, self.group, self.p = opt, group, p
 
     def takes(self, fusable: bool) -> bool:
-        return fusable or self.opt._factor() > 1
+        return (fusable and not self.opt.gradient_clip_val) or self.opt._factor() > 1
 
     def __call__(self, dy, x, w, dx, db, ws, ws_bytes, fusable, impl):
+        fusable = fusable and not self.opt.gradient_clip_val
         if self.opt._factor() == 1:
             self.opt._fused_step(self.group, self.p, dy, x, dx, db, ws, ws_bytes)
         else:
@@ -629,13 +719,16 @@ def make_adam(module, lr):
     reduce + Adam + all-gather exchange, launched from the backward pass; "torch": the reference's optimizer object.
     ``hparams.accumulate_grad_batches`` (what Lightning's ``Trainer.add_argparse_args`` puts on the Namespace; an int or an
     ``{epoch: factor}`` dict, read against ``module.current_epoch`` at the first backward pass of each window) becomes
-    FusedAdam's window of backward passes per step."""
+    FusedAdam's window of backward passes per step; ``hparams.gradient_clip_val`` (also the Trainer's flag) its clipping at
+    world size 1.  Under torch.distributed FusedAdam does not clip yet: there the flag is left to the Trainer, as before
+    FusedAdam could clip, with a warning."""
     hp = getattr(module, "hparams", None)
     kind = getattr(hp, "optimizer", "fused") if hp is not None else "fused"
     params = [p for p in module.parameters()]
     on_cuda = bool(params) and all(p.is_cuda for p in params)
     if kind == "fused" and on_cuda:
-        opt = FusedAdam(params, lr=lr, overlap_backward=dist.is_initialized() and dist.get_world_size() > 1)
+        distributed = dist.is_initialized() and dist.get_world_size() > 1
+        opt = FusedAdam(params, lr=lr, overlap_backward=distributed, gradient_clip_val=follow_clipping(hp, distributed))
         follow_accumulation(opt, module)
         # a checkpoint (module.state_dict()) must see the weights of updates that are still in flight on the side stream
         module.register_state_dict_pre_hook(lambda *a, **k: opt.synchronize())

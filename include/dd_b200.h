@@ -310,6 +310,27 @@ int dd_adam_step_sharded(const void* const* grad_replicas, void* const* param_re
                          float weight_decay, long long step, float grad_scale, int ctas_per_sm,
                          void* stream);
 
+/* Gradient clipping by the global L2 norm (torch.nn.utils.clip_grad_norm_(params, max_norm), Lightning's
+ * gradient_clip_val), computed and applied on the device: the norm and coefficient never go to the host.
+ * dd_grad_sumsq: the sum of g*g over `count` fp32 tensors given as HOST arrays ptrs[i] / numels[i]
+ * (any length, 0 included, and any 4-byte alignment), in fp64, folded in a fixed order (the same bits
+ * run to run).  Writes out[0] = total_norm = (float)sqrt(sum), out[1] = coef =
+ * clamp(max_norm / (total_norm + 1e-6), max=1) in torch's fp32 arithmetic (NaN passes through the
+ * clamp; an infinite norm gives 0) and the fp64 sum itself at out + 2.  out: device memory, 16 bytes,
+ * 8-byte aligned.  max_norm: finite, >= 0.
+ * workspace: dd_grad_sumsq_workspace_bytes() bytes, zeroed by the caller ONCE (self-resetting); calls
+ * that share a workspace must be ordered (one stream).  Lists longer than 64 tensors take one launch
+ * per 64. */
+size_t dd_grad_sumsq_workspace_bytes(void);
+int dd_grad_sumsq(const void* const* ptrs, const long long* numels, int count, float max_norm,
+                  float* out, void* workspace, size_t ws_bytes, void* stream);
+/* dd_adam_step with the gradient read as (grad * grad_scale) * (*coef), before the L2 weight-decay
+ * term (the order of clip_grad_norm_ followed by torch.optim.Adam).  coef: device pointer to one
+ * float, e.g. dd_grad_sumsq's out + 1.  *coef == 1 gives dd_adam_step's bits. */
+int dd_adam_step_clipped(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, long long n,
+                         float lr, float beta1, float beta2, float eps, float weight_decay, long long step,
+                         float grad_scale, const float* coef, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
