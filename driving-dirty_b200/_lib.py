@@ -53,6 +53,8 @@ SIGNATURES = {
     "dd_linear_wgrad_acc": (_I, [_P, _P, _I, _P, _P, _I, _I, _L, _I, _I, _P]),
     "dd_linear_bwd_adam": (_I, [_P, _P, _P, _P, _P, _P, _I, _P, _P, _Z, _I, _I, _L, _F, _F, _F, _F, _F, _L, _P]),
     "dd_linear_bwd_adam_acc": (_I, [_P, _P, _P, _P, _P, _P, _P, _I, _P, _P, _Z, _I, _I, _L, _F, _F, _F, _F, _F, _L, _P]),
+    "dd_linear_bwd_adam_sumsq": (_I, [_P, _P, _P, _P, _P, _P, _P, _I, _P, _P, _Z, _I, _I, _L, _F, _F, _F, _F, _F, _L, _P, _P,
+                                      _Z, _P]),
     "dd_linear_workspace_bytes": (_Z, [_I, _I, _L]),
     "dd_linear_tc_supported": (_I, [_I, _I, _L]),
     "dd_bce_ts_fwd": (_I, [_P, _P, _I, _P, _P, _P, _P, _P, _Z, _L, _P]),
@@ -80,6 +82,10 @@ SIGNATURES = {
     "dd_grad_sumsq_workspace_bytes": (_Z, []),
     "dd_grad_sumsq": (_I, [_P, _P, _I, _F, _P, _P, _Z, _P]),
     "dd_adam_step_clipped": (_I, [_P, _P, _P, _P, _L, _F, _F, _F, _F, _F, _L, _F, _P, _P]),
+    "dd_adam_step_sharded_sumsq": (_I, [_P, _P, _P, _P, _I, _I, _P, _P, _L, _L, _F, _F, _F, _F, _F, _L, _F, _I, _P, _P, _Z, _P]),
+    "dd_grad_sumsq_each_workspace_bytes": (_Z, []),
+    "dd_grad_sumsq_each": (_I, [_P, _P, _P, _I, _P, _Z, _P]),
+    "dd_grad_sumsq_each_replicas": (_I, [_P, _I, _I, _F, _P, _P, _P, _I, _P, _Z, _P]),
 }
 
 

@@ -7,7 +7,7 @@ import numpy as np
 import torch
 
 from .. import ops
-from ..lightning_compat import LightningModule
+from ..lightning_compat import FusedGradNorm, LightningModule
 from .components import Decoder, Encoder, resolve_dtype
 
 # the reference seeds at import time (autoencoder.py:16-18); kept so that scripts which rely on
@@ -17,7 +17,7 @@ np.random.seed(20200505)
 torch.manual_seed(20200505)
 
 
-class BasicAE(LightningModule):
+class BasicAE(FusedGradNorm, LightningModule):
     def __init__(self, hparams=None):
         super().__init__()
         self.__check_hparams(hparams)

@@ -11,7 +11,7 @@ import torch
 from ... import ops
 from ...autoencoder.autoencoder import BasicAE
 from ...autoencoder.components import resolve_dtype
-from ...lightning_compat import LightningModule
+from ...lightning_compat import FusedGradNorm, LightningModule
 from .components import RoadMapBoxesMergingCNN, SpatialMappingCNN
 
 random.seed(20200505)
@@ -19,7 +19,7 @@ np.random.seed(20200505)
 torch.manual_seed(20200505)
 
 
-class BBSpatialRoadMap(LightningModule):
+class BBSpatialRoadMap(FusedGradNorm, LightningModule):
     def __init__(self, hparams):
         super().__init__()
         self.hparams = hparams

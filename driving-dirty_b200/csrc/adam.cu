@@ -56,13 +56,19 @@ __device__ __forceinline__ void mc_store(float* mc, float4 v) {
 // take 2 x 2560; the input-gradient conv kernel that must run beside the update puts 4 of its 13 warps (88 registers) on one
 // sub-partition, 11264 -- together exactly 16 K.  With 96 registers here that kernel queued behind the whole update
 // (1.8 ms hole in the N = 2 multicast timeline, profiles/r2_step_timeline_n2_multicast_96regs.txt).
-template <int MODE, int UNROLL, bool CLIP = false>
+// NORM (the sharded modes, dd_adam_step_sharded_sumsq): each thread also adds up the squares of the gradient as adam_one
+// consumes it (the replicas' sum in this kernel's order, times grad_scale) in fp64; the CTAs fold them into *sumsq_out
+// through sumsq_ws (dd::sumsq_fold_grid).  Its two parameters come after coef_ptr for the same reason as coef_ptr.
+template <int MODE, int UNROLL, bool CLIP = false, bool NORM = false>
 __global__ void __maxnreg__(MODE == 0 ? 96 : 80) adam_kernel(PeerPtrs pp, const float* __restrict__ mc_grad, float* __restrict__ mc_param,
                                                         float* __restrict__ m, float* __restrict__ v, long long off,
                                                         long long n, int world, int rank, AdamHyper h,
-                                                        const float* __restrict__ coef_ptr = nullptr) {
+                                                        const float* __restrict__ coef_ptr = nullptr,
+                                                        dd::SumsqWorkspace* __restrict__ sumsq_ws = nullptr,
+                                                        double* __restrict__ sumsq_out = nullptr) {
   // element i of the shard is element off + i of the full tensors; n and off are multiples of 4
   const float coef = CLIP ? *coef_ptr : 1.f;
+  double nacc = 0.0;
   const long long n4 = n >> 2;
   const long long stride = (long long)gridDim.x * kThreads;
   const float* __restrict__ g_own = pp.grad[MODE == 0 ? 0 : rank];
@@ -107,6 +113,9 @@ __global__ void __maxnreg__(MODE == 0 ? 96 : 80) adam_kernel(PeerPtrs pp, const 
       const long long i = i0 + u * stride;
       if (i < n4) {
         const long long e = off + 4 * i;
+        if (NORM)
+          nacc += (dd::sq(g[u].x * h.grad_scale) + dd::sq(g[u].y * h.grad_scale)) +
+                  (dd::sq(g[u].z * h.grad_scale) + dd::sq(g[u].w * h.grad_scale));
         if (CLIP) {
           p[u].x = adam_one(p[u].x, g[u].x, mm[u].x, vv[u].x, h, coef);
           p[u].y = adam_one(p[u].y, g[u].y, mm[u].y, vv[u].y, h, coef);
@@ -130,6 +139,18 @@ __global__ void __maxnreg__(MODE == 0 ? 96 : 80) adam_kernel(PeerPtrs pp, const 
       }
     }
   }
+  if constexpr (NORM) {
+    __shared__ double sred[kThreads / 32];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    nacc = dd::warp_sum(nacc);
+    if (lane == 0) sred[warp] = nacc;
+    __syncthreads();
+    if (warp == 0) {
+      double cta = 0.0;
+      for (int w = 0; w < kThreads / 32; ++w) cta += sred[w];
+      dd::sumsq_fold_grid(sumsq_ws, cta, sumsq_out);
+    }
+  }
 }
 
 // tail (n % 4 elements) and unaligned tensors of the local form
@@ -151,22 +172,16 @@ int grid_for(long long n4) {
 }
 
 // ---- dd_grad_sumsq -------------------------------------------------------------------------------------------------------
+using dd::SumsqWorkspace;
+using dd::sq;
 constexpr int kSumsqTensors = 64;              // tensors per launch; a longer list takes several launches
-constexpr int kSumsqBlocks = dd::kSMs * 8;
+constexpr int kSumsqBlocks = dd::kSumsqMaxCtas;
 
 struct TensorList {
   const float* ptr[kSumsqTensors];
   long long n[kSumsqTensors];
   int count;
 };
-
-struct SumsqWorkspace {
-  double partial[kSumsqBlocks];                // CTA b's running sum over the launches of one call
-  unsigned int ticket;
-  unsigned int pad[3];
-};
-
-__device__ __forceinline__ double sq(float x) { return (double)x * (double)x; }   // exact: 24-bit mantissas, 48-bit product
 
 // Grid-stride over each tensor in turn: its unaligned head (< 4 elements) and tail (< 4) by single loads, the rest as
 // UNROLL independent 16-byte streaming loads per thread and iteration.  Each thread sums in fp64, each CTA folds its
@@ -325,23 +340,35 @@ extern "C" int dd_grad_sumsq(const void* const* ptrs, const long long* numels, i
   return 0;
 }
 
-extern "C" int dd_adam_step_sharded(const void* const* grad_replicas, void* const* param_replicas, const void* mc_grad,
-                                    void* mc_param, int world, int rank, float* exp_avg_shard, float* exp_avg_sq_shard,
-                                    long long shard_offset, long long shard_numel, float lr, float beta1, float beta2,
-                                    float eps, float weight_decay, long long step, float grad_scale, int ctas_per_sm, void* stream) {
-  DD_REQUIRE(grad_replicas && param_replicas && exp_avg_shard && exp_avg_sq_shard, DD_ERR_BAD_ARG, "dd_adam_step_sharded: null pointer");
+namespace {
+
+template <bool NORM>
+int adam_step_sharded(const char* what, const void* const* grad_replicas, void* const* param_replicas, const void* mc_grad,
+                      void* mc_param, int world, int rank, float* exp_avg_shard, float* exp_avg_sq_shard, long long shard_offset,
+                      long long shard_numel, float lr, float beta1, float beta2, float eps, float weight_decay, long long step,
+                      float grad_scale, int ctas_per_sm, double* sumsq, void* workspace, size_t ws_bytes, void* stream) {
+  DD_REQUIRE(grad_replicas && param_replicas && exp_avg_shard && exp_avg_sq_shard, DD_ERR_BAD_ARG, "%s: null pointer", what);
   DD_REQUIRE(world >= 1 && world <= kMaxRanks && rank >= 0 && rank < world, DD_ERR_BAD_ARG,
-             "dd_adam_step_sharded: world %d (max %d) rank %d", world, kMaxRanks, rank);
+             "%s: world %d (max %d) rank %d", what, world, kMaxRanks, rank);
   DD_REQUIRE(shard_numel >= 0 && (shard_numel & 3) == 0 && (shard_offset & 3) == 0 && step >= 1, DD_ERR_ALIGNMENT,
-             "dd_adam_step_sharded: shard offset %lld / length %lld must be multiples of 4 elements", shard_offset, shard_numel);
-  if (shard_numel == 0) return 0;
+             "%s: shard offset %lld / length %lld must be multiples of 4 elements", what, shard_offset, shard_numel);
+  if (NORM) {
+    DD_REQUIRE(sumsq && workspace, DD_ERR_BAD_ARG, "%s: null pointer", what);
+    DD_REQUIRE(((uintptr_t)sumsq & 7) == 0, DD_ERR_ALIGNMENT, "%s: sumsq must be 8-byte aligned", what);
+    DD_REQUIRE(ws_bytes >= sizeof(SumsqWorkspace), DD_ERR_WORKSPACE, "%s: workspace %zu < %zu", what, ws_bytes,
+               sizeof(SumsqWorkspace));
+  }
+  if (shard_numel == 0) {                          // an empty shard's sum is 0
+    if (NORM) return (int)cudaMemsetAsync(sumsq, 0, sizeof(double), dd::as_stream(stream));
+    return 0;
+  }
   PeerPtrs pp = {};
   for (int k = 0; k < world; ++k) {
     pp.grad[k] = (const float*)grad_replicas[k];
     pp.param[k] = (float*)param_replicas[k];
-    DD_REQUIRE(pp.grad[k] && pp.param[k], DD_ERR_BAD_ARG, "dd_adam_step_sharded: replica %d is null", k);
+    DD_REQUIRE(pp.grad[k] && pp.param[k], DD_ERR_BAD_ARG, "%s: replica %d is null", what, k);
     DD_REQUIRE(((((uintptr_t)pp.grad[k]) | ((uintptr_t)pp.param[k])) & 15) == 0, DD_ERR_ALIGNMENT,
-               "dd_adam_step_sharded: replica %d is not 16-byte aligned", k);
+               "%s: replica %d is not 16-byte aligned", what, k);
   }
   const AdamHyper h = dd::adam_hyper(lr, beta1, beta2, eps, weight_decay, step, grad_scale);
   cudaStream_t st = dd::as_stream(stream);
@@ -353,16 +380,39 @@ extern "C" int dd_adam_step_sharded(const void* const* grad_replicas, void* cons
   // uses no shared memory) the persistent conv kernels of the backward pass (90-210 KB of shared memory per CTA) could not
   // join an SM that runs an update CTA and queued behind the whole update (1.2 ms gap seen in the step timeline).
   static const bool carveout_set = [] {
-    cudaFuncSetAttribute(adam_kernel<1, 2>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-    cudaFuncSetAttribute(adam_kernel<2, 4>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+    cudaFuncSetAttribute(adam_kernel<1, 2, false, NORM>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+    cudaFuncSetAttribute(adam_kernel<2, 4, false, NORM>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
     return true;
   }();
   (void)carveout_set;
+  SumsqWorkspace* ws = (SumsqWorkspace*)workspace;
   if (mc_grad && mc_param)
-    adam_kernel<2, 4><<<grid, kThreads, 0, st>>>(pp, (const float*)mc_grad, (float*)mc_param, exp_avg_shard, exp_avg_sq_shard,
-                                              shard_offset, shard_numel, world, rank, h);
+    adam_kernel<2, 4, false, NORM><<<grid, kThreads, 0, st>>>(pp, (const float*)mc_grad, (float*)mc_param, exp_avg_shard,
+                                                              exp_avg_sq_shard, shard_offset, shard_numel, world, rank, h,
+                                                              nullptr, ws, sumsq);
   else
-    adam_kernel<1, 2><<<grid, kThreads, 0, st>>>(pp, nullptr, nullptr, exp_avg_shard, exp_avg_sq_shard, shard_offset, shard_numel,
-                                              world, rank, h);
+    adam_kernel<1, 2, false, NORM><<<grid, kThreads, 0, st>>>(pp, nullptr, nullptr, exp_avg_shard, exp_avg_sq_shard, shard_offset,
+                                                              shard_numel, world, rank, h, nullptr, ws, sumsq);
   return dd::check_launch("adam_kernel(sharded)");
+}
+
+}  // namespace
+
+extern "C" int dd_adam_step_sharded(const void* const* grad_replicas, void* const* param_replicas, const void* mc_grad,
+                                    void* mc_param, int world, int rank, float* exp_avg_shard, float* exp_avg_sq_shard,
+                                    long long shard_offset, long long shard_numel, float lr, float beta1, float beta2,
+                                    float eps, float weight_decay, long long step, float grad_scale, int ctas_per_sm, void* stream) {
+  return adam_step_sharded<false>("dd_adam_step_sharded", grad_replicas, param_replicas, mc_grad, mc_param, world, rank,
+                                  exp_avg_shard, exp_avg_sq_shard, shard_offset, shard_numel, lr, beta1, beta2, eps, weight_decay,
+                                  step, grad_scale, ctas_per_sm, nullptr, nullptr, 0, stream);
+}
+
+extern "C" int dd_adam_step_sharded_sumsq(const void* const* grad_replicas, void* const* param_replicas, const void* mc_grad,
+                                          void* mc_param, int world, int rank, float* exp_avg_shard, float* exp_avg_sq_shard,
+                                          long long shard_offset, long long shard_numel, float lr, float beta1, float beta2,
+                                          float eps, float weight_decay, long long step, float grad_scale, int ctas_per_sm,
+                                          double* sumsq, void* workspace, size_t ws_bytes, void* stream) {
+  return adam_step_sharded<true>("dd_adam_step_sharded_sumsq", grad_replicas, param_replicas, mc_grad, mc_param, world, rank,
+                                 exp_avg_shard, exp_avg_sq_shard, shard_offset, shard_numel, lr, beta1, beta2, eps, weight_decay,
+                                 step, grad_scale, ctas_per_sm, sumsq, workspace, ws_bytes, stream);
 }

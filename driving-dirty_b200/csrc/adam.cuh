@@ -4,6 +4,8 @@
 #pragma once
 #include <math.h>
 
+#include "dd_common.cuh"
+
 namespace dd {
 
 struct AdamHyper {
@@ -27,6 +29,40 @@ __device__ __forceinline__ float adam_one(float p, float g, float& m, float& v, 
 // before Adam adds the L2 term).  coef == 1 gives adam_one's bits.
 __device__ __forceinline__ float adam_one(float p, float g, float& m, float& v, const AdamHyper& h, float coef) {
   return adam_apply(p, (g * h.grad_scale) * coef, m, v, h);
+}
+
+// ---- deterministic fp64 sums of squares over a grid (gradient norms) ----------------------------------------------------
+// g*g is exact in fp64 (24-bit mantissas, 48-bit product).  Each CTA folds its threads in a fixed order into partial[its
+// index]; the last CTA to finish (ticket) adds the partials in a fixed order: the same grid gives the same bits on every run,
+// and there are no float atomics.  The workspace is zeroed once by its owner and resets itself; launches that share one
+// must be ordered.
+constexpr int kSumsqMaxCtas = kSMs * 8;
+struct SumsqWorkspace {
+  double partial[kSumsqMaxCtas];
+  unsigned int ticket;
+  unsigned int pad[3];
+};
+
+__device__ __forceinline__ double sq(float x) { return (double)x * (double)x; }
+
+// Called by one whole warp of every CTA of the grid, with the CTA's sum in lane 0; the last CTA writes the grid's sum to *out.
+__device__ __forceinline__ void sumsq_fold_grid(SumsqWorkspace* ws, double cta, double* out) {
+  const int lane = threadIdx.x & 31;
+  unsigned int last = 0;
+  if (lane == 0) {
+    ws->partial[blockIdx.x] = cta;
+    __threadfence();
+    last = atomicAdd(&ws->ticket, 1u) == gridDim.x - 1;
+  }
+  if (!__shfl_sync(0xffffffffu, last, 0)) return;
+  __threadfence();
+  double s = 0.0;
+  for (unsigned int b = lane; b < gridDim.x; b += 32) s += __ldcg(&ws->partial[b]);
+  s = warp_sum(s);
+  if (lane == 0) {
+    *out = s;
+    ws->ticket = 0;
+  }
 }
 
 // bias corrections of step t >= 1, in double

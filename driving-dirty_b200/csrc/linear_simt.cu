@@ -458,7 +458,8 @@ int linear_dgrad_tc(const float* dy, const float* w, void* dx, int dx_dtype, voi
 int linear_wgrad_tc(const float* dy, const float* x, float* dw, int B, int N, long long K, int accumulate, cudaStream_t st);
 int linear_wgrad_acc_multi_tc(const float* dy, const float* x, float* dw, int B, int N, long long K, cudaStream_t st);
 int linear_bwd_adam_tc(const float* dy, const float* x, float* w, float* m, float* v, const float* gpart, void* dx, int dx_dtype,
-                       void* ws, size_t ws_bytes, int B, int N, long long K, const AdamHyper& h, cudaStream_t st);
+                       void* ws, size_t ws_bytes, int B, int N, long long K, const AdamHyper& h, double* sumsq,
+                       SumsqWorkspace* sumsq_ws, cudaStream_t st);
 }  // namespace dd
 
 // tcgen05 path: only on explicit request (DD_IMPL_TCGEN05) -- fp32 callers under DD_IMPL_AUTO keep the
@@ -608,20 +609,25 @@ extern "C" int dd_linear_wgrad_acc(const float* dy, const void* x, int x_dtype, 
 
 // Backward pass of a wide linear layer with the Adam update of its weight folded in (world size 1): see include/dd_b200.h.
 // tcgen05 path only (fp32 x, B <= 32, dd_linear_tc_supported); the bias gradient is written as by dd_linear_wgrad.
-extern "C" int dd_linear_bwd_adam(const float* dy, const float* x, float* weight, float* exp_avg, float* exp_avg_sq, void* dx,
-                                  int dx_dtype, float* db, void* workspace, size_t ws_bytes, int B, int N, long long K, float lr,
-                                  float beta1, float beta2, float eps, float weight_decay, long long step, void* stream) {
-  DD_REQUIRE(dy && x && weight && exp_avg && exp_avg_sq, DD_ERR_BAD_ARG, "dd_linear_bwd_adam: null pointer");
-  DD_REQUIRE(B > 0 && B <= 32 && N > 0 && K > 0 && step >= 1, DD_ERR_BAD_ARG, "dd_linear_bwd_adam: B=%d (<= 32) N=%d K=%lld step=%lld", B, N, K, step);
-  DD_REQUIRE(!dx || dx_dtype == DD_F32 || dx_dtype == DD_BF16, DD_ERR_UNSUPPORTED, "dd_linear_bwd_adam: dtype %d", dx_dtype);
-  DD_REQUIRE(dd::linear_tc_supported(B, N, K), DD_ERR_UNSUPPORTED, "dd_linear_bwd_adam: needs the tcgen05 path (N %% 4 == K %% 4 == 0, N*K >= 2^22)");
-  DD_REQUIRE((((uintptr_t)weight | (uintptr_t)exp_avg | (uintptr_t)exp_avg_sq | (uintptr_t)dy | (uintptr_t)x) & 15) == 0, DD_ERR_ALIGNMENT,
-             "dd_linear_bwd_adam: dy / x / weight / moments must be 16-byte aligned");
+// acc: the step takes this pass's weight gradient plus grad_partial (the earlier passes of the window); sumsq: also the sum
+// of squares of that gradient (nullptr: not computed).
+static int bwd_adam(const char* what, bool acc, const float* dy, const float* x, float* weight, float* exp_avg, float* exp_avg_sq,
+                    const float* grad_partial, void* dx, int dx_dtype, float* db, void* workspace, size_t ws_bytes, int B, int N,
+                    long long K, float lr, float beta1, float beta2, float eps, float weight_decay, long long step, double* sumsq,
+                    void* sumsq_ws, void* stream) {
+  DD_REQUIRE(dy && x && weight && exp_avg && exp_avg_sq && (grad_partial || !acc), DD_ERR_BAD_ARG, "%s: null pointer", what);
+  DD_REQUIRE(B > 0 && B <= 32 && N > 0 && K > 0 && step >= 1, DD_ERR_BAD_ARG, "%s: B=%d (<= 32) N=%d K=%lld step=%lld", what, B, N, K, step);
+  DD_REQUIRE(!dx || dx_dtype == DD_F32 || dx_dtype == DD_BF16, DD_ERR_UNSUPPORTED, "%s: dtype %d", what, dx_dtype);
+  DD_REQUIRE(dd::linear_tc_supported(B, N, K), DD_ERR_UNSUPPORTED, "%s: needs the tcgen05 path (N %% 4 == K %% 4 == 0, N*K >= 2^22)", what);
+  DD_REQUIRE((((uintptr_t)weight | (uintptr_t)exp_avg | (uintptr_t)exp_avg_sq | (uintptr_t)grad_partial | (uintptr_t)dy | (uintptr_t)x) & 15) == 0,
+             DD_ERR_ALIGNMENT, acc ? "%s: dy / x / weight / moments / grad_partial must be 16-byte aligned"
+                                   : "%s: dy / x / weight / moments must be 16-byte aligned", what);
   DD_REQUIRE(!dx || (workspace && ws_bytes >= dd_linear_workspace_bytes(B, N, K)), DD_ERR_WORKSPACE,
-             "dd_linear_bwd_adam: workspace %zu < %zu", ws_bytes, dd_linear_workspace_bytes(B, N, K));
+             "%s: workspace %zu < %zu", what, ws_bytes, dd_linear_workspace_bytes(B, N, K));
   cudaStream_t st = dd::as_stream(stream);
   const dd::AdamHyper h = dd::adam_hyper(lr, beta1, beta2, eps, weight_decay, step, 1.f);
-  if (int e = dd::linear_bwd_adam_tc(dy, x, weight, exp_avg, exp_avg_sq, nullptr, dx, dx_dtype, workspace, ws_bytes, B, N, K, h, st))
+  if (int e = dd::linear_bwd_adam_tc(dy, x, weight, exp_avg, exp_avg_sq, acc ? grad_partial : nullptr, dx, dx_dtype, workspace,
+                                     ws_bytes, B, N, K, h, sumsq, (dd::SumsqWorkspace*)sumsq_ws, st))
     return e;
   if (db) {
     colsum_kernel<<<dd::ceil_div(N, 256), 256, 0, st>>>(dy, db, B, N, 0);
@@ -630,27 +636,30 @@ extern "C" int dd_linear_bwd_adam(const float* dy, const float* x, float* weight
   return 0;
 }
 
-// dd_linear_bwd_adam that steps with this pass's weight gradient plus grad_partial (the earlier passes of the window)
+extern "C" int dd_linear_bwd_adam(const float* dy, const float* x, float* weight, float* exp_avg, float* exp_avg_sq, void* dx,
+                                  int dx_dtype, float* db, void* workspace, size_t ws_bytes, int B, int N, long long K, float lr,
+                                  float beta1, float beta2, float eps, float weight_decay, long long step, void* stream) {
+  return bwd_adam("dd_linear_bwd_adam", false, dy, x, weight, exp_avg, exp_avg_sq, nullptr, dx, dx_dtype, db, workspace, ws_bytes,
+                  B, N, K, lr, beta1, beta2, eps, weight_decay, step, nullptr, nullptr, stream);
+}
+
 extern "C" int dd_linear_bwd_adam_acc(const float* dy, const float* x, float* weight, float* exp_avg, float* exp_avg_sq,
                                       const float* grad_partial, void* dx, int dx_dtype, float* db, void* workspace,
                                       size_t ws_bytes, int B, int N, long long K, float lr, float beta1, float beta2, float eps,
                                       float weight_decay, long long step, void* stream) {
-  DD_REQUIRE(dy && x && weight && exp_avg && exp_avg_sq && grad_partial, DD_ERR_BAD_ARG, "dd_linear_bwd_adam_acc: null pointer");
-  DD_REQUIRE(B > 0 && B <= 32 && N > 0 && K > 0 && step >= 1, DD_ERR_BAD_ARG, "dd_linear_bwd_adam_acc: B=%d (<= 32) N=%d K=%lld step=%lld", B, N, K, step);
-  DD_REQUIRE(!dx || dx_dtype == DD_F32 || dx_dtype == DD_BF16, DD_ERR_UNSUPPORTED, "dd_linear_bwd_adam_acc: dtype %d", dx_dtype);
-  DD_REQUIRE(dd::linear_tc_supported(B, N, K), DD_ERR_UNSUPPORTED, "dd_linear_bwd_adam_acc: needs the tcgen05 path (N %% 4 == K %% 4 == 0, N*K >= 2^22)");
-  DD_REQUIRE((((uintptr_t)weight | (uintptr_t)exp_avg | (uintptr_t)exp_avg_sq | (uintptr_t)grad_partial | (uintptr_t)dy | (uintptr_t)x) & 15) == 0,
-             DD_ERR_ALIGNMENT, "dd_linear_bwd_adam_acc: dy / x / weight / moments / grad_partial must be 16-byte aligned");
-  DD_REQUIRE(!dx || (workspace && ws_bytes >= dd_linear_workspace_bytes(B, N, K)), DD_ERR_WORKSPACE,
-             "dd_linear_bwd_adam_acc: workspace %zu < %zu", ws_bytes, dd_linear_workspace_bytes(B, N, K));
-  cudaStream_t st = dd::as_stream(stream);
-  const dd::AdamHyper h = dd::adam_hyper(lr, beta1, beta2, eps, weight_decay, step, 1.f);
-  if (int e = dd::linear_bwd_adam_tc(dy, x, weight, exp_avg, exp_avg_sq, grad_partial, dx, dx_dtype, workspace, ws_bytes, B, N, K,
-                                     h, st))
-    return e;
-  if (db) {
-    colsum_kernel<<<dd::ceil_div(N, 256), 256, 0, st>>>(dy, db, B, N, 0);
-    if (int e2 = dd::check_launch("colsum")) return e2;
-  }
-  return 0;
+  return bwd_adam("dd_linear_bwd_adam_acc", true, dy, x, weight, exp_avg, exp_avg_sq, grad_partial, dx, dx_dtype, db, workspace,
+                  ws_bytes, B, N, K, lr, beta1, beta2, eps, weight_decay, step, nullptr, nullptr, stream);
+}
+
+extern "C" int dd_linear_bwd_adam_sumsq(const float* dy, const float* x, float* weight, float* exp_avg, float* exp_avg_sq,
+                                        const float* grad_partial, void* dx, int dx_dtype, float* db, void* workspace,
+                                        size_t ws_bytes, int B, int N, long long K, float lr, float beta1, float beta2, float eps,
+                                        float weight_decay, long long step, double* sumsq, void* sumsq_ws, size_t sumsq_ws_bytes,
+                                        void* stream) {
+  DD_REQUIRE(sumsq && sumsq_ws, DD_ERR_BAD_ARG, "dd_linear_bwd_adam_sumsq: null pointer");
+  DD_REQUIRE(((uintptr_t)sumsq & 7) == 0, DD_ERR_ALIGNMENT, "dd_linear_bwd_adam_sumsq: sumsq must be 8-byte aligned");
+  DD_REQUIRE(sumsq_ws_bytes >= sizeof(dd::SumsqWorkspace), DD_ERR_WORKSPACE, "dd_linear_bwd_adam_sumsq: workspace %zu < %zu",
+             sumsq_ws_bytes, sizeof(dd::SumsqWorkspace));
+  return bwd_adam("dd_linear_bwd_adam_sumsq", grad_partial != nullptr, dy, x, weight, exp_avg, exp_avg_sq, grad_partial, dx,
+                  dx_dtype, db, workspace, ws_bytes, B, N, K, lr, beta1, beta2, eps, weight_decay, step, sumsq, sumsq_ws, stream);
 }

@@ -427,13 +427,23 @@ __device__ __forceinline__ float lds_f32(uint32_t a) {
   return v;
 }
 __device__ __forceinline__ void sts_f32(uint32_t a, float v) { asm volatile("st.shared.f32 [%0], %1;" ::"r"(a), "f"(v) : "memory"); }
+// Gradient norm (NORM, dd_linear_bwd_adam_sumsq): each epilogue thread adds the square of every gradient element it hands
+// adam_one, in fp64, for the elements inside the [rows x g.LD] weight only (a ragged edge tile's padding is masked, not
+// assumed zero); the epilogue warps fold their threads in a fixed order and dd::sumsq_fold_grid folds the CTAs into *out.
+struct SumsqSink {
+  dd::SumsqWorkspace* ws;
+  double* out;
+  int rows;                                           // N
+};
 // TMEM columns: [0, 64) dgrad accumulator of the item (x 2), [64, 128) G^T of the chunk (x 2)
-// map_g (the stored partial gradient, ACC only) comes last, so that the plain instantiation keeps its parameter layout
-template <typename TOUT, bool ACC>
+// map_g (the stored partial gradient, ACC only) and then sink (NORM only) come last, so that the plain instantiation keeps its
+// parameter layout
+template <typename TOUT, bool ACC, bool NORM = false>
 __global__ void __launch_bounds__(BA_THREADS, 1) linear_bwd_adam_tc_kernel(
     const __grid_constant__ CUtensorMap map_w, const __grid_constant__ CUtensorMap map_m, const __grid_constant__ CUtensorMap map_v,
     const __grid_constant__ CUtensorMap map_dy, const __grid_constant__ CUtensorMap map_dyt, const __grid_constant__ CUtensorMap map_x,
-    TOUT* __restrict__ dx, float* __restrict__ partial, StreamGeo g, const dd::AdamHyper h, const __grid_constant__ CUtensorMap map_g) {
+    TOUT* __restrict__ dx, float* __restrict__ partial, StreamGeo g, const dd::AdamHyper h, const __grid_constant__ CUtensorMap map_g,
+    SumsqSink sink) {
   constexpr int STAGES = BaCfg<ACC>::STAGES, STAGE_BYTES = BaCfg<ACC>::STAGE_BYTES, DY_OFF = BaCfg<ACC>::DY_OFF;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = align1024(smem_raw);
@@ -564,10 +574,12 @@ __global__ void __launch_bounds__(BA_THREADS, 1) linear_bwd_adam_tc_kernel(
     // thread = k lane (quarter * 32 + lane of the tile: box `quarter`, column `lane`), 16 n rows (half `sub` of the chunk)
     const int quarter = warp & 3, sub = (warp - 2) >> 2;
     uint32_t c = 0, n_item = 0;
+    double nacc = 0.0;
     for (int it = blockIdx.x; it < items; it += gridDim.x, ++n_item) {
       const int ti = it % g.tiles, si = it / g.tiles;
       const int c0 = si * g.chunks_per_split;
       const int c1 = min(c0 + g.chunks_per_split, g.chunks);
+      const bool k_in = ti * 128 + quarter * 32 + lane < g.LD;
       for (int ch = c0; ch < c1; ++ch, ++c) {
         const uint32_t s = c % STAGES, ga = c & 1;
         umma::mbar_wait_sleep(&bars->g_full[ga], (c >> 1) & 1);
@@ -586,6 +598,7 @@ __global__ void __launch_bounds__(BA_THREADS, 1) linear_bwd_adam_tc_kernel(
           float m = lds_f32(e + BA_TILE), v = lds_f32(e + 2 * BA_TILE);
           float gr = __uint_as_float(gv[j]);
           if (ACC) gr = gr + lds_f32(e + 3 * BA_TILE);     // dd_linear_wgrad_acc's dW_chunk + G, bit for bit
+          if (NORM && k_in && ch * kChunk + r < sink.rows) nacc += dd::sq(gr);
           const float p = dd::adam_one(lds_f32(e), gr, m, v, h);
           sts_f32(e, p);
           sts_f32(e + BA_TILE, m);
@@ -619,6 +632,17 @@ __global__ void __launch_bounds__(BA_THREADS, 1) linear_bwd_adam_tc_kernel(
             }
           }
         }
+      }
+    }
+    if constexpr (NORM) {
+      __shared__ double sred[BA_EPI];
+      nacc = dd::warp_sum(nacc);
+      if (lane == 0) sred[warp - 2] = nacc;
+      asm volatile("bar.sync 1, %0;" ::"n"(32 * BA_EPI) : "memory");     // the epilogue warps only
+      if (warp == 2) {
+        double cta = 0.0;
+        for (int w = 0; w < BA_EPI; ++w) cta += sred[w];
+        dd::sumsq_fold_grid(sink.ws, cta, sink.out);
       }
     }
   }
@@ -735,20 +759,31 @@ int linear_dgrad_tc(const float* dy, const float* w, void* dx, int dx_dtype, voi
   return g.splits > 1 ? check_launch("linear_dgrad_fold") : 0;
 }
 
-template <bool ACC, typename TOUT>
-int launch_bwd_adam(const CUtensorMap (&maps)[7], TOUT* dx, float* ws, const StreamGeo& g, const AdamHyper& h, cudaStream_t st) {
-  auto k = linear_bwd_adam_tc_kernel<TOUT, ACC>;
+template <bool ACC, bool NORM, typename TOUT>
+int launch_bwd_adam(const CUtensorMap (&maps)[7], TOUT* dx, float* ws, const StreamGeo& g, const AdamHyper& h, const SumsqSink& sink,
+                    cudaStream_t st) {
+  auto k = linear_bwd_adam_tc_kernel<TOUT, ACC, NORM>;
   if (int e = set_smem(k, BaCfg<ACC>::SMEM, Carveout::kMaxShared, "linear_tc")) return e;
   const int items = g.tiles * g.splits;
   k<<<items < kSMs ? items : kSMs, BA_THREADS, BaCfg<ACC>::SMEM, st>>>(maps[0], maps[1], maps[2], maps[3], maps[4], maps[5], dx, ws,
-                                                                       g, h, maps[6]);
+                                                                       g, h, maps[6], sink);
   return check_launch("linear_bwd_adam_tc");
 }
 
+template <typename TOUT>
+int launch_bwd_adam_any(bool acc, const CUtensorMap (&maps)[7], TOUT* dx, float* ws, const StreamGeo& g, const AdamHyper& h,
+                        const SumsqSink& sink, cudaStream_t st) {
+  if (sink.out)
+    return acc ? launch_bwd_adam<true, true>(maps, dx, ws, g, h, sink, st) : launch_bwd_adam<false, true>(maps, dx, ws, g, h, sink, st);
+  return acc ? launch_bwd_adam<true, false>(maps, dx, ws, g, h, sink, st) : launch_bwd_adam<false, false>(maps, dx, ws, g, h, sink, st);
+}
+
 // dy fp32 [B][N], x fp32 [B][K], W / m / v fp32 [N][K] updated in place; dx [B][K] fp32 or bf16 from the old W, or nullptr;
-// gpart fp32 [N][K]: the stored partial gradient added to this pass's weight gradient before the step, or nullptr
+// gpart fp32 [N][K]: the stored partial gradient added to this pass's weight gradient before the step, or nullptr;
+// sumsq / sumsq_ws: *sumsq = the sum of squares of the gradient the step applies (NORM), or nullptr
 int linear_bwd_adam_tc(const float* dy, const float* x, float* w, float* m, float* v, const float* gpart, void* dx, int dx_dtype,
-                       void* ws, size_t ws_bytes, int B, int N, long long K, const AdamHyper& h, cudaStream_t st) {
+                       void* ws, size_t ws_bytes, int B, int N, long long K, const AdamHyper& h, double* sumsq,
+                       SumsqWorkspace* sumsq_ws, cudaStream_t st) {
   StreamGeo g;
   g.B = B; g.LD = (int)K;
   g.tiles = ceil_div(K, 128);
@@ -767,16 +802,15 @@ int linear_bwd_adam_tc(const float* dy, const float* x, float* w, float* m, floa
       (gpart && tma_map_2d(&maps[6], gpart, 4, N, K, K, 32, 32, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, msg, sizeof msg)))
     return fail(DD_ERR_UNSUPPORTED, "linear_bwd_adam_tc: %s", msg);
   const long long n = (long long)B * K;
+  const SumsqSink sink = {sumsq_ws, sumsq, N};
   if (dx_dtype == DD_BF16 && dx) {
     auto* d = (__nv_bfloat16*)dx;
-    if (int e = gpart ? launch_bwd_adam<true>(maps, d, (float*)ws, g, h, st) : launch_bwd_adam<false>(maps, d, (float*)ws, g, h, st))
-      return e;
+    if (int e = launch_bwd_adam_any(gpart != nullptr, maps, d, (float*)ws, g, h, sink, st)) return e;
     if (g.splits > 1)
       split_fold_kernel<__nv_bfloat16><<<ceil_div(n, 256), 256, 0, st>>>((const float*)ws, nullptr, d, g.splits, n, (int)K);
   } else {
     auto* d = (float*)dx;
-    if (int e = gpart ? launch_bwd_adam<true>(maps, d, (float*)ws, g, h, st) : launch_bwd_adam<false>(maps, d, (float*)ws, g, h, st))
-      return e;
+    if (int e = launch_bwd_adam_any(gpart != nullptr, maps, d, (float*)ws, g, h, sink, st)) return e;
     if (dx && g.splits > 1)
       split_fold_kernel<float><<<ceil_div(n, 256), 256, 0, st>>>((const float*)ws, nullptr, d, g.splits, n, (int)K);
   }

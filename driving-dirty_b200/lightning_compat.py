@@ -37,6 +37,17 @@ class _MinimalLightningModule(nn.Module):
             p.requires_grad = True
         self.train()
 
+    def grad_norm(self, norm_type):
+        """PL 0.7.5's GradInformation.grad_norm: the norm of every parameter's .grad (rounded host floats) and their total."""
+        results, total_norm = {}, 0
+        for name, p in self.named_parameters():
+            if p.requires_grad and p.grad is not None:
+                param_norm = p.grad.data.norm(norm_type)
+                total_norm += param_norm ** norm_type
+                results[f"grad_{norm_type}_norm_{name}"] = round(float(param_norm ** (1 / norm_type)), 3)
+        results[f"grad_{norm_type}_norm_total"] = round(float(total_norm ** (1. / norm_type)), 3)
+        return results
+
     @classmethod
     def load_from_checkpoint(cls, checkpoint_path, map_location=None, **kwargs):
         ckpt = torch.load(checkpoint_path, map_location=map_location or "cpu", weights_only=False)
@@ -49,6 +60,27 @@ class _MinimalLightningModule(nn.Module):
 
 
 LightningModule = _PLModule if HAVE_LIGHTNING else _MinimalLightningModule
+
+
+class FusedGradNorm:
+    """``grad_norm(norm_type)``, the hook behind Lightning's ``track_grad_norm``, for modules whose optimizer
+    (``optim.attach_optimizer``) may be a FusedAdam: the wide weights' gradients never reach ``.grad`` there, and at world
+    size N ``.grad`` is this rank's replica.  With a FusedAdam that tracks this norm the values are its ``grad_norms()``
+    -- the gradients its step applies, the rank mean at world size N -- as device tensors (no rounding, no host copy);
+    otherwise the base class answers, as before."""
+
+    def grad_norm(self, norm_type):
+        from .optim import FusedAdam
+        opt = getattr(self, "_dd_optimizer", None)
+        tracked = (isinstance(opt, FusedAdam) and opt.track_grad_norm == 2 and not isinstance(norm_type, bool)
+                   and isinstance(norm_type, (int, float)) and norm_type == 2)
+        if not tracked:
+            return super().grad_norm(norm_type)
+        norms = opt.grad_norms()
+        by_id = {id(k): v for k, v in norms.items() if not isinstance(k, str)}
+        out = {f"grad_{norm_type}_norm_{name}": by_id[id(p)] for name, p in self.named_parameters() if id(p) in by_id}
+        out[f"grad_{norm_type}_norm_total"] = norms["total"]
+        return out
 
 
 def save_checkpoint(module, path):

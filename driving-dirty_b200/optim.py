@@ -43,6 +43,13 @@ per tensor), so the step has no host sync; ``last_grad_norm`` is the pre-clip to
 Clipping needs every gradient before any update, so under it the wide weights' step does not run inside the backward pass:
 their gradients are written (or accumulated) and step() applies them.
 
+Gradient norms (``track_grad_norm=2``, Lightning's flag of the same name): ``grad_norms()`` returns the L2 norm of every
+gradient the window's step applies -- the accumulated window gradient, the rank mean at world size N, before any clipping --
+as 0-dim fp32 device tensors, and their total, without a host sync.  The wide weights' sums of squares come from the kernels
+that step them (``dd_linear_bwd_adam_sumsq``, ``dd_adam_step_sharded_sumsq``: at world size N each rank sums its shard and
+every rank adds the N shard sums in rank order, so every rank holds the same bits); the stored gradients go through
+``dd_grad_sumsq_each`` (``_replicas`` for the data-parallel flat bucket).  Tracking never changes an update.
+
 Semantics are torch.optim.Adam's (amsgrad off, L2 weight decay); ``param_groups[i]['lr']`` is read
 every step, so ``ReduceLROnPlateau`` (roadmap_bce_v2.py:156) works unchanged; tensors whose
 gradient is ``None`` are skipped (a partly frozen flat bucket is updated per tensor on every replica).
@@ -52,6 +59,7 @@ from __future__ import annotations
 import ctypes
 import math
 import warnings
+import weakref
 
 import torch
 import torch.distributed as dist
@@ -96,6 +104,15 @@ def gradient_clip_value(c) -> float:
     return float(c)
 
 
+def track_grad_norm_value(t) -> bool:
+    """Lightning's ``track_grad_norm``: -1, 0 or None for off; FusedAdam tracks the 2-norm only (2 or 2.0)."""
+    if t is None or (not isinstance(t, bool) and isinstance(t, (int, float)) and t in (-1, 0)):
+        return False
+    if not isinstance(t, bool) and isinstance(t, (int, float)) and t == 2:
+        return True
+    raise ValueError(f"track_grad_norm: FusedAdam tracks the 2-norm only (track_grad_norm=2; -1, 0 or None for off), got {t!r}")
+
+
 def flat_layout(numels, align: int = _ALIGN):
     """Offsets of tensors packed into one flat region (each start aligned) and the region's length."""
     offs, off = [], 0
@@ -109,7 +126,7 @@ class FusedAdam(torch.optim.Optimizer):
     def __init__(self, params, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0, process_group=None,
                  shard_min_numel: int = 1 << 20, multicast: bool | None = None, broadcast_init: bool = True,
                  overlap_backward: bool = False, fuse_into_backward: bool = False, defer_join: bool = True,
-                 accumulate_grad_batches=1, gradient_clip_val=0.0):
+                 accumulate_grad_batches=1, gradient_clip_val=0.0, track_grad_norm=-1):
         if lr < 0 or eps < 0 or not (0 <= betas[0] < 1) or not (0 <= betas[1] < 1) or weight_decay < 0:
             raise ValueError("invalid Adam hyper-parameters")
         super().__init__(params, dict(lr=lr, betas=betas, eps=eps, weight_decay=weight_decay))
@@ -122,6 +139,15 @@ class FusedAdam(torch.optim.Optimizer):
         self._clip_val = gradient_clip_value(gradient_clip_val)
         self.last_grad_norm = None
         self._clip_ws = None        # dd_grad_sumsq's workspace (zeroed once, self-resetting)
+        # gradient norms (grad_norms()): the window's fp64 sums of squares, one slot per parameter (_norm_index), zeros at
+        # the window's start; _present: the parameters whose gradient the window applies; _stored: (parameter id, weak
+        # reference, version) of the stored gradients the window's sums were taken from (world size N: the flat bucket's),
+        # re-taken after step() and zero_grad(), so that a changed stored gradient marks a new window; _after_step: the
+        # window's step() ran, its norms stay readable until the next window's first backward pass
+        self._track = track_grad_norm_value(track_grad_norm)
+        self._sums, self._present, self._stored, self._after_step = None, set(), None, False
+        self._sumsq_ws = {}         # key -> workspace of a kernel that sums one tensor's squares (zeroed once)
+        self._each_ws = None        # dd_grad_sumsq_each's workspace
         self._window_k = None       # factor of the window in progress, resolved at its first backward pass
         self._passes = {}           # id(wide param) -> backward passes that wrote its gradient in the window in progress
         self._acc_buf = {}          # world size 1: id(wide param) -> gradient buffer of passes 1 .. k-1 (allocated on first use)
@@ -141,12 +167,15 @@ class FusedAdam(torch.optim.Optimizer):
         self._written = set()       # ids of wide params whose gradient replica was written since the last step()
         self._launched = set()      # ... and whose update is already running on the side stream
         self._mom, self._mom_of = None, None   # symmetric buffer of this rank's moment shards, accessor for the peers'
+        self._flat_mode = None      # world size N: how this window's flat-bucket norms were taken ("sharded" / "replicated")
         self._flat_replicated = False   # the flat bucket fell back to per-tensor replicated updates (partly frozen model)
         self._lib = _lib.load()     # raises when the CUDA library is missing: no fallback
         for g in self.param_groups:
             for p in g["params"]:
                 self._check_param(p)
         self._fused = {}            # id(param) -> True once its step ran inside the backward pass (world size 1)
+        self._norm_index = {id(p): i for i, p in enumerate(p for g in self.param_groups for p in g["params"])}
+        self._slots = None          # world size N: this rank's fp64 shard sums, [wide regions | flat tensors] (symmetric)
         if self.world > 1:
             self._setup_sharding(shard_min_numel, multicast, broadcast_init)
         elif overlap_backward or fuse_into_backward:
@@ -244,7 +273,12 @@ class FusedAdam(torch.optim.Optimizer):
             cap = -(-max(hi_l - lo_l, r["hi"] - r["lo"], 4) // _ALIGN) * _ALIGN
             r["moff"], r["mcap"] = moff, cap
             moff += 2 * cap
-        self._mom, self._mom_of = self._alloc_moments(moff, dev)
+        # the norm slots (fp64) ride at the end of the same symmetric buffer: one per wide region, then one per flat tensor
+        n_slots = len(self._regions) + len(small)
+        moff += moff & 1
+        self._mom, self._mom_of = self._alloc_moments(moff + 2 * n_slots, dev)
+        self._slots = (moff, n_slots)
+        self._norm_index = {id(p): i for i, p in enumerate([r["key"] for r in self._regions.values()] + small)}
         self._symm = dict(buf=buf, hdl=hdl, total=total, ptrs=ptrs, mc=mc)
         if self._overlap:
             self._side = torch.cuda.Stream(device=dev)
@@ -293,14 +327,20 @@ class FusedAdam(torch.optim.Optimizer):
         buf = self._acc_buf.get(key)
         if buf is None:
             buf = self._acc_buf[key] = torch.empty_like(p)
+        if j == 0:
+            self._window_starts()
         if j + 1 == k and fusable:
             st = self._state(p, p.numel(), p.device)
             st["step"] += 1
-            call("dd_linear_bwd_adam_acc", dy.data_ptr(), x.data_ptr(), p.data_ptr(), st["exp_avg"].data_ptr(),
-                 st["exp_avg_sq"].data_ptr(), buf.data_ptr(), dx.data_ptr() if dx is not None else None,
-                 _lib.dtype_code(dx.dtype) if dx is not None else _lib.DD_F32, db.data_ptr() if db is not None else None,
-                 ws.data_ptr(), ws_bytes, B, N, K, float(g["lr"]), float(g["betas"][0]), float(g["betas"][1]),
-                 float(g["eps"]), float(g["weight_decay"]), st["step"], stream_ptr())
+            args = (dy.data_ptr(), x.data_ptr(), p.data_ptr(), st["exp_avg"].data_ptr(), st["exp_avg_sq"].data_ptr(),
+                    buf.data_ptr(), dx.data_ptr() if dx is not None else None,
+                    _lib.dtype_code(dx.dtype) if dx is not None else _lib.DD_F32, db.data_ptr() if db is not None else None,
+                    ws.data_ptr(), ws_bytes, B, N, K, float(g["lr"]), float(g["betas"][0]), float(g["betas"][1]),
+                    float(g["eps"]), float(g["weight_decay"]), st["step"])
+            if self._track:
+                call("dd_linear_bwd_adam_sumsq", *args, *self._sumsq_slot(p), stream_ptr())
+            else:
+                call("dd_linear_bwd_adam_acc", *args, stream_ptr())
             self._fused[key] = True
         else:
             if dx is not None:
@@ -315,13 +355,18 @@ class FusedAdam(torch.optim.Optimizer):
         if id(p) in self._fused:
             raise RuntimeError("FusedAdam: two backward passes reached a weight whose Adam step is folded into its backward, "
                                "without a step() in between")
+        self._window_starts()
         st = self._state(p, p.numel(), p.device)
         st["step"] += 1
         B, K = x.shape
-        call("dd_linear_bwd_adam", dy.data_ptr(), x.data_ptr(), p.data_ptr(), st["exp_avg"].data_ptr(), st["exp_avg_sq"].data_ptr(),
-             dx.data_ptr() if dx is not None else None, _lib.dtype_code(dx.dtype) if dx is not None else _lib.DD_F32,
-             db.data_ptr() if db is not None else None, ws.data_ptr(), ws_bytes, B, p.shape[0], K, float(g["lr"]),
-             float(g["betas"][0]), float(g["betas"][1]), float(g["eps"]), float(g["weight_decay"]), st["step"], stream_ptr())
+        dxa = (dx.data_ptr() if dx is not None else None, _lib.dtype_code(dx.dtype) if dx is not None else _lib.DD_F32)
+        args = (db.data_ptr() if db is not None else None, ws.data_ptr(), ws_bytes, B, p.shape[0], K, float(g["lr"]),
+                float(g["betas"][0]), float(g["betas"][1]), float(g["eps"]), float(g["weight_decay"]), st["step"])
+        head = (dy.data_ptr(), x.data_ptr(), p.data_ptr(), st["exp_avg"].data_ptr(), st["exp_avg_sq"].data_ptr())
+        if self._track:
+            call("dd_linear_bwd_adam_sumsq", *head, None, *dxa, *args, *self._sumsq_slot(p), stream_ptr())
+        else:
+            call("dd_linear_bwd_adam", *head, *dxa, *args, stream_ptr())
         self._fused[id(p)] = True
 
     @property
@@ -340,6 +385,20 @@ class FusedAdam(torch.optim.Optimizer):
             raise RuntimeError("FusedAdam: gradient_clip_val cannot change after a backward pass of a window whose step() "
                                "has not run; change it between steps")
         self._clip_val = c
+
+    @property
+    def track_grad_norm(self):
+        """2 when grad_norms() tracks the 2-norm, else -1 (off).  It decides which kernels the backward pass launches, so it
+        changes between steps only."""
+        return 2 if self._track else -1
+
+    @track_grad_norm.setter
+    def track_grad_norm(self, t):
+        on = track_grad_norm_value(t)
+        if on != self._track and (self._passes or self._fused or self._written):
+            raise RuntimeError("FusedAdam: track_grad_norm cannot change after a backward pass of a window whose step() "
+                               "has not run; change it between steps")
+        self._track = on
 
     @property
     def uses_multicast(self) -> bool:
@@ -367,6 +426,8 @@ class FusedAdam(torch.optim.Optimizer):
                 else:
                     p.grad.detach_()
                     p.grad.zero_()
+        if self._after_step:                     # clearing the gradients starts no window: only a backward pass does
+            self._stored = self._fingerprint(self._stored_todo())
 
     def _state(self, key, numel, device):
         st = self.state[key]
@@ -398,15 +459,11 @@ class FusedAdam(torch.optim.Optimizer):
                 loss = closure()
         self._window_k = None
         if self.world == 1:
-            todo = []
-            for g in self.param_groups:
-                for p in g["params"]:
-                    if id(p) in self._fused:              # stepped inside the backward pass
-                        continue
-                    if id(p) in self._passes:             # accumulation buffer: a window without the fused last pass
-                        todo.append((g, p, self._acc_buf[id(p)]))
-                    elif p.grad is not None:
-                        todo.append((g, p, p.grad))
+            todo = self._local_todo()
+            if self._track:
+                if self._after_step:                      # no backward pass reached a wide weight since the last step
+                    self._window_starts()
+                self._stored_sums(todo)
             if self.gradient_clip_val:
                 todo = [(g, p, _f32(grad)) for g, p, grad in todo]
                 coef = self._clip([grad for _, _, grad in todo])
@@ -417,12 +474,15 @@ class FusedAdam(torch.optim.Optimizer):
                     self._launch_local(g, p, grad)
             self._fused.clear()
             self._passes.clear()
+            self._stepped()
             return loss
         if self._symm is None:
             return loss
+        if self._track and self._after_step:             # no backward pass reached a wide weight since the last step
+            self._window_starts()
         hdl = self._symm["hdl"]
         todo = [r for key, r in self._regions.items() if key in self._written and key not in self._launched]
-        fl = self._flat
+        fl, restage = self._flat, False
         if fl is not None:
             have = [p.grad is not None for p in fl["params"]]
             if any(have) and (self._flat_replicated or not all(have)):
@@ -435,6 +495,8 @@ class FusedAdam(torch.optim.Optimizer):
                     raise NotImplementedError("FusedAdam (world > 1): the flat bucket was already stepped in its sharded form; "
                                               "freeze parameters before the first step, not after")
                 self._flat_replicated = True
+                # grad_norms() took its sums from an all-reduced copy; from the averaged p.grad if they changed since
+                renorm = self._track and self._flat_stale()
                 nccl = dist.get_backend(self.group) == "nccl"
                 g = self.param_groups[0]
                 for p in fl["params"]:
@@ -444,13 +506,19 @@ class FusedAdam(torch.optim.Optimizer):
                     if not nccl:
                         p.grad.div_(self.world)
                     self._launch_local(g, p, p.grad)
+                if renorm:
+                    self._flat_norms_replicated([p.grad for p in fl["params"] if p.grad is not None])
             elif all(have):
-                torch._foreach_copy_(fl["grad_views"], [p.grad for p in fl["params"]])
+                restage = self._flat_mode != "sharded" or self._flat_stale()
+                if restage:                            # else grad_norms() staged these very gradients
+                    torch._foreach_copy_(fl["grad_views"], [p.grad for p in fl["params"]])
                 todo.append(fl)
         if todo:
             hdl.barrier()                                  # every rank has written its gradient replicas
+            if self._track and fl is not None and todo[-1] is fl and restage:
+                self._flat_norms_sharded()                 # read before the closing barrier: no replica changes under it
             for r in todo:
-                self._launch_sharded(r, ctas_per_sm=8)
+                self._launch_region(r, ctas_per_sm=8)
             hdl.barrier()                                  # every replica holds the new weights
         if self._launched:
             # The updates launched from the backward pass run on the side stream and end with a cross-rank barrier (new
@@ -470,6 +538,7 @@ class FusedAdam(torch.optim.Optimizer):
         self._launched.clear()
         self._written.clear()
         self._passes.clear()
+        self._stepped()
         return loss
 
     def synchronize(self):
@@ -618,7 +687,16 @@ class FusedAdam(torch.optim.Optimizer):
         else:
             call("dd_adam_step_clipped", *args, coef.data_ptr(), stream_ptr())
 
-    def _launch_sharded(self, r, ctas_per_sm):
+    def _launch_region(self, r, ctas_per_sm):
+        """The sharded update of a region; with tracking, a wide region's also writes this rank's shard sum of squares into
+        the region's norm slot (the flat bucket's per-tensor sums come from _flat_norms_*)."""
+        if self._track and r is not self._flat:
+            self._present.add(id(r["key"]))
+            self._launch_sharded(r, ctas_per_sm=ctas_per_sm, norm=True)
+        else:
+            self._launch_sharded(r, ctas_per_sm=ctas_per_sm)
+
+    def _launch_sharded(self, r, ctas_per_sm, norm=False):
         sy, W = self._symm, self.world
         lo, hi, total = r["lo"], r["hi"], sy["total"]
         st = self._shard_state(r)
@@ -628,8 +706,238 @@ class FusedAdam(torch.optim.Optimizer):
         mcg = ctypes.c_void_p(sy["mc"] + 4 * r["off"]) if sy["mc"] else None
         mcw = ctypes.c_void_p(sy["mc"] + 4 * (total + r["off"])) if sy["mc"] else None
         lr, b1, b2, eps, wd = self._hyper()
-        call("dd_adam_step_sharded", gptrs, wptrs, mcg, mcw, W, self.rank, st["exp_avg"].data_ptr(),
-             st["exp_avg_sq"].data_ptr(), lo, hi - lo, lr, b1, b2, eps, wd, st["step"], 1.0 / W, int(ctas_per_sm), stream_ptr())
+        args = (gptrs, wptrs, mcg, mcw, W, self.rank, st["exp_avg"].data_ptr(), st["exp_avg_sq"].data_ptr(), lo, hi - lo, lr, b1,
+                b2, eps, wd, st["step"], 1.0 / W, int(ctas_per_sm))
+        if norm:
+            ws = self._sumsq_workspace(r["channel"])
+            call("dd_adam_step_sharded_sumsq", *args, self._slot_ptr(self._norm_index[id(r["key"])]), ws.data_ptr(), ws.numel(),
+                 stream_ptr())
+        else:
+            call("dd_adam_step_sharded", *args, stream_ptr())
+
+    # ------------------------------------------------------------------------------------------
+    # gradient norms (track_grad_norm)
+    # ------------------------------------------------------------------------------------------
+    def grad_norms(self):
+        """{param: L2 norm of the gradient the window's step applies, a 0-dim fp32 device tensor} for every parameter with a
+        gradient in the window, plus ``"total"``, the norm of all of them together.  The gradient is the window's (summed
+        over accumulate_grad_batches passes), the rank mean at world size N, before any clipping.  No host sync.  Valid
+        from the window's last backward pass (before or after step()) until the next window's first backward pass; outside
+        that range it raises.  At world size N every rank must call it (it may exchange the flat bucket's gradients), and
+        every rank gets the same bits; with overlap_backward=False the wide weights update inside step(), so their norms
+        exist only after it."""
+        if not self._track:
+            raise RuntimeError("FusedAdam.grad_norms: track_grad_norm is off (set track_grad_norm=2)")
+        if self.world == 1:
+            if self._after_step and self._changed(self._stored, self._local_todo()):
+                # a backward pass wrote stored gradients since step() (zero_grad() alone does not count)
+                if any(hasattr(p, "_dd_fused_update") for g in self.param_groups for p in g["params"]):
+                    raise RuntimeError("FusedAdam.grad_norms: the next window's backward pass has begun; its norms are "
+                                       "valid once the window's last backward pass has run")
+                self._window_starts()                    # stored gradients only: a new window's gradients
+            if not self._after_step:
+                self._check_window_complete()
+                self._stored_sums(self._local_todo())
+        else:
+            self._dist_sums()
+        return self._result()
+
+    def _window_starts(self):
+        """The first backward pass of a window after a step(): the previous window's norms are gone."""
+        if self._after_step:
+            self._sums, self._present, self._stored, self._after_step = None, set(), None, False
+            self._flat_mode = None
+
+    def _window_sums(self):
+        if self._sums is None:
+            dev = self.param_groups[0]["params"][0].device
+            self._sums = torch.zeros(len(self._norm_index), dtype=torch.float64, device=dev)
+        return self._sums
+
+    def _sumsq_workspace(self, key):
+        ws = self._sumsq_ws.get(key)
+        if ws is None:
+            dev = self.param_groups[0]["params"][0].device
+            ws = self._sumsq_ws[key] = torch.zeros(int(self._lib.dd_grad_sumsq_workspace_bytes()), dtype=torch.uint8, device=dev)
+        return ws
+
+    def _sumsq_slot(self, p):
+        """(sum pointer, workspace pointer, workspace bytes) for the fused kernel stepping p at world size 1."""
+        self._present.add(id(p))
+        ws = self._sumsq_workspace(id(p))
+        return self._window_sums()[self._norm_index[id(p)]].data_ptr(), ws.data_ptr(), ws.numel()
+
+    def _slot_ptr(self, i):
+        """Device address of this rank's norm slot i (world size N)."""
+        return self._mom.data_ptr() + 4 * self._slots[0] + 8 * i
+
+    def _local_todo(self):
+        """World size 1: (group, param, gradient) of every tensor step() applies from a stored gradient."""
+        todo = []
+        for g in self.param_groups:
+            for p in g["params"]:
+                if id(p) in self._fused:              # stepped inside the backward pass
+                    continue
+                if id(p) in self._passes:             # accumulation buffer: a window without the fused last pass
+                    todo.append((g, p, self._acc_buf[id(p)]))
+                elif p.grad is not None:
+                    todo.append((g, p, p.grad))
+        return todo
+
+    @staticmethod
+    def _fingerprint(todo):
+        return [(id(p), weakref.ref(grad), grad._version) for _, p, grad in todo]
+
+    @staticmethod
+    def _changed(fp, todo):
+        """`todo` (group, param, gradient) is not the set of tensors, at the versions, that fingerprint `fp` recorded."""
+        return fp is None or len(todo) != len(fp) or any(
+            key != id(p) or ref() is not grad or grad._version != v for (_, p, grad), (key, ref, v) in zip(todo, fp))
+
+    def _stored_todo(self):
+        """The stored gradients whose sums grad_norms() takes itself: world size 1 what step() applies from a stored
+        gradient, world size N the flat bucket's."""
+        if self.world == 1:
+            return self._local_todo()
+        return [(None, p, p.grad) for p in (self._flat["params"] if self._flat is not None else []) if p.grad is not None]
+
+    def _flat_stale(self):
+        return self._flat_mode is None or self._changed(self._stored, self._stored_todo())
+
+    def _stepped(self):
+        """End of step(): the window's norms stay readable, against the stored gradients as step() leaves them."""
+        self._after_step = self._track
+        if self._track:
+            self._stored = self._fingerprint(self._stored_todo())
+
+    def _stored_sums(self, todo):
+        """World size 1: the sums of squares of the stored gradients `todo` (once per window; again if they changed)."""
+        if not self._changed(self._stored, todo):
+            return
+        sums = self._window_sums()
+        self._sumsq_each([_f32(grad) for _, _, grad in todo], [sums[self._norm_index[id(p)]] for _, p, _ in todo])
+        self._present.update(id(p) for _, p, _ in todo)
+        self._stored = self._fingerprint(todo)
+
+    def _check_window_complete(self):
+        k = self._window_k
+        for key, n in self._passes.items():
+            if key not in self._fused and key not in self._launched and k is not None and n < k:
+                raise RuntimeError(f"FusedAdam.grad_norms: the window has run {n} of its {k} backward passes "
+                                   "(accumulate_grad_batches); its norms exist after its last backward pass")
+
+    def _mean_copies(self):
+        """World size N, replicated flat form, before step(): the rank mean of each present gradient, by the all-reduce
+        step() runs, on a copy -- p.grad stays this rank's, for whatever the training loop does before step()."""
+        nccl = dist.get_backend(self.group) == "nccl"
+        out = []
+        for p in self._flat["params"]:
+            if p.grad is None:
+                continue
+            t = p.grad.clone()
+            dist.all_reduce(t, op=dist.ReduceOp.AVG if nccl else dist.ReduceOp.SUM, group=self.group)
+            out.append(t if nccl else t.div_(self.world))
+        return out
+
+    def _flat_norms_replicated(self, means):
+        """Per-tensor sums of the rank means `means` of the flat bucket's present gradients (the same bits on every
+        rank)."""
+        fl, sums = self._flat, self._window_sums()
+        ps = [p for p in fl["params"] if p.grad is not None]
+        self._sumsq_each(means, [sums[self._norm_index[id(p)]] for p in ps])
+        self._present.update(id(p) for p in ps)
+        self._flat_mode = "replicated"
+        self._stored = self._fingerprint(self._stored_todo())
+
+    def _flat_norms_sharded(self):
+        """This rank's part of the flat bucket's per-tensor sums: its shard of each tensor, the rank mean as the sharded
+        update consumes it, into the tensor's norm slot.  Between a barrier after every replica is written and one before
+        any is written again."""
+        fl = self._flat
+        offs, numels, outs = [], [], []
+        for p, o in zip(fl["params"], fl["offs"]):
+            a, b = max(o, fl["lo"]), min(o + p.numel(), fl["hi"])
+            offs.append(fl["off"] + (a if b > a else fl["lo"]))
+            numels.append(max(b - a, 0))
+            outs.append(self._norm_index[id(p)])
+        self._sumsq_each_replicas(offs, numels, outs)
+        self._present.update(id(p) for p in fl["params"])
+        self._flat_mode = "sharded"
+        self._stored = self._fingerprint(self._stored_todo())
+
+    def _dist_sums(self):
+        """World size N: the window's sums -- each wide region's and (sharded form) each flat tensor's from the N ranks'
+        slots, added in rank order, so every rank holds the same bits."""
+        if self._side is not None:
+            torch.cuda.current_stream().wait_stream(self._side)     # its launches end with the cross-rank barrier
+        if self._after_step and self._changed(self._stored, self._stored_todo()):
+            self._window_starts()        # a backward pass wrote the flat gradients since step(): no wide weight started it
+        if not self._after_step:
+            for key in self._written:
+                if key not in self._launched:
+                    if not self._overlap:
+                        raise RuntimeError("FusedAdam.grad_norms: with overlap_backward=False the data-parallel form updates "
+                                           "the wide weights inside step(), so their norms exist only after step()")
+                    self._check_window_complete()
+            fl = self._flat
+            if fl is not None and self._flat_stale():
+                have = [p.grad is not None for p in fl["params"]]
+                if any(have) and (self._flat_replicated or not all(have)):
+                    self._flat_norms_replicated(self._mean_copies())
+                elif all(have):
+                    # staged into the replica here; step() copies again only if p.grad changed since (e.g. a clip)
+                    torch._foreach_copy_(fl["grad_views"], [p.grad for p in fl["params"]])
+                    hdl = self._symm["hdl"]
+                    hdl.barrier()                              # every rank has written its flat gradient replica
+                    self._flat_norms_sharded()
+                    hdl.barrier()                              # every rank's flat slots are written
+        base, n = self._slots
+        acc = None
+        for rk in range(self.world):                           # rank order: the same bits on every rank
+            t = self._mom_of(rk)[base: base + 2 * n].view(torch.float64)
+            acc = t.clone() if acc is None else acc.add_(t)
+        sums = self._window_sums()
+        regions = list(self._regions.values())
+        R = len(regions)
+        sums[:R].copy_(acc[:R])
+        for i, r in enumerate(regions):
+            if id(r["key"]) not in self._present:
+                sums[i].zero_()
+        if self._flat_mode == "sharded":
+            sums[R:].copy_(acc[R:])
+
+    def _result(self):
+        if not self._present:
+            raise RuntimeError("FusedAdam.grad_norms: no gradient in this window yet; its norms exist after its last "
+                               "backward pass")
+        sums = self._sums
+        norms = sums.sqrt().float()
+        out = {p: norms[self._norm_index[id(p)]] for g in self.param_groups for p in g["params"] if id(p) in self._present}
+        out["total"] = sums.sum().sqrt().float()
+        return out
+
+    # the device calls of the stored-gradient sums (tests/test_grad_norm_cpu.py emulates them)
+    def _sumsq_each(self, grads, outs):
+        if not grads:
+            return
+        dev = grads[0].device
+        if self._each_ws is None:
+            self._each_ws = torch.zeros(int(self._lib.dd_grad_sumsq_each_workspace_bytes()), dtype=torch.uint8, device=dev)
+        n = len(grads)
+        call("dd_grad_sumsq_each", (ctypes.c_void_p * n)(*[t.data_ptr() for t in grads]),
+             (ctypes.c_longlong * n)(*[t.numel() for t in grads]), (ctypes.c_void_p * n)(*[o.data_ptr() for o in outs]), n,
+             self._each_ws.data_ptr(), self._each_ws.numel(), stream_ptr())
+
+    def _sumsq_each_replicas(self, offs, numels, slots):
+        """Per-tensor sums of the flat bucket's rank mean over this rank's shard, into this rank's norm slots `slots`."""
+        sy, n = self._symm, len(offs)
+        outs = [self._slot_ptr(i) for i in slots]
+        if self._each_ws is None:
+            self._each_ws = torch.zeros(int(self._lib.dd_grad_sumsq_each_workspace_bytes()), dtype=torch.uint8,
+                                        device=self._mom.device)
+        call("dd_grad_sumsq_each_replicas", (ctypes.c_void_p * self.world)(*sy["ptrs"]), self.world, self.rank,
+             1.0 / self.world, (ctypes.c_longlong * n)(*offs), (ctypes.c_longlong * n)(*numels), (ctypes.c_void_p * n)(*outs),
+             n, self._each_ws.data_ptr(), self._each_ws.numel(), stream_ptr())
 
     def _begin_grad(self, p):
         """Called by ops.linear's backward before it writes p's gradient replica: 0 = overwrite (first pass of a window),
@@ -637,6 +945,8 @@ class FusedAdam(torch.optim.Optimizer):
         n = self._passes.get(id(p), 0)
         if n >= self._factor():
             self._refuse_pass(n + 1, "a sharded parameter")
+        if n == 0:
+            self._window_starts()
         return int(n > 0)
 
     @torch.no_grad()
@@ -661,9 +971,30 @@ class FusedAdam(torch.optim.Optimizer):
         self._side.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(self._side):
             hdl.barrier(channel=r["channel"])
-            self._launch_sharded(r, ctas_per_sm=1)
+            self._launch_region(r, ctas_per_sm=1)
             hdl.barrier(channel=r["channel"])
         self._launched.add(key)
+
+
+def follow_norm_tracking(hparams) -> int:
+    """FusedAdam's track_grad_norm from the Namespace's (Lightning's flag; off when absent).  A norm FusedAdam cannot track
+    is left to Lightning, with a warning."""
+    t = getattr(hparams, "track_grad_norm", None) if hparams is not None else None
+    try:
+        return 2 if track_grad_norm_value(t) else -1
+    except ValueError:
+        warnings.warn(f"make_adam: FusedAdam cannot track the {t!r}-norm of the gradients (only the 2-norm); "
+                      "track_grad_norm is left to Lightning, whose numbers miss the wide weights (their step runs inside "
+                      "a kernel and they keep no .grad) and, under torch.distributed, are this rank's own gradients")
+        return -1
+
+
+def attach_optimizer(module, opt):
+    """Record `opt` as the optimizer of `module` (its grad_norm() reads FusedAdam.grad_norms() from it), and let a
+    checkpoint (module.state_dict()) see the weights of updates still in flight on the side stream."""
+    module._dd_optimizer = opt
+    if isinstance(opt, FusedAdam):
+        module.register_state_dict_pre_hook(lambda *a, **k: opt.synchronize())
 
 
 def _f32(grad):
@@ -721,16 +1052,19 @@ def make_adam(module, lr):
     ``{epoch: factor}`` dict, read against ``module.current_epoch`` at the first backward pass of each window) becomes
     FusedAdam's window of backward passes per step; ``hparams.gradient_clip_val`` (also the Trainer's flag) its clipping at
     world size 1.  Under torch.distributed FusedAdam does not clip yet: there the flag is left to the Trainer, as before
-    FusedAdam could clip, with a warning."""
+    FusedAdam could clip, with a warning.  ``hparams.track_grad_norm`` = 2 (the Trainer's flag too) turns on FusedAdam's
+    gradient norms, which the module's grad_norm() returns; another norm is left to Lightning, with a warning."""
     hp = getattr(module, "hparams", None)
     kind = getattr(hp, "optimizer", "fused") if hp is not None else "fused"
     params = [p for p in module.parameters()]
     on_cuda = bool(params) and all(p.is_cuda for p in params)
     if kind == "fused" and on_cuda:
         distributed = dist.is_initialized() and dist.get_world_size() > 1
-        opt = FusedAdam(params, lr=lr, overlap_backward=distributed, gradient_clip_val=follow_clipping(hp, distributed))
+        opt = FusedAdam(params, lr=lr, overlap_backward=distributed, gradient_clip_val=follow_clipping(hp, distributed),
+                        track_grad_norm=follow_norm_tracking(hp))
         follow_accumulation(opt, module)
-        # a checkpoint (module.state_dict()) must see the weights of updates that are still in flight on the side stream
-        module.register_state_dict_pre_hook(lambda *a, **k: opt.synchronize())
+        attach_optimizer(module, opt)
         return opt
-    return torch.optim.Adam(params, lr=lr)
+    opt = torch.optim.Adam(params, lr=lr)
+    attach_optimizer(module, opt)
+    return opt

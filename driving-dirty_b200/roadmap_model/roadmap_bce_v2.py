@@ -12,7 +12,7 @@ from .. import ops
 from .._lib import IMPL_AUTO
 from ..autoencoder.autoencoder import BasicAE
 from ..autoencoder.components import resolve_dtype
-from ..lightning_compat import LightningModule
+from ..lightning_compat import FusedGradNorm, LightningModule
 from ..utils.helper import compute_ts_road_map  # noqa: F401  (re-exported like the reference)
 
 random.seed(20200505)
@@ -20,7 +20,7 @@ np.random.seed(20200505)
 torch.manual_seed(20200505)
 
 
-class RoadMapBCE(LightningModule):
+class RoadMapBCE(FusedGradNorm, LightningModule):
     def __init__(self, hparams):
         super().__init__()
         self.hparams = hparams

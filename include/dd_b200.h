@@ -184,6 +184,18 @@ int dd_linear_bwd_adam_acc(const float* dy, const float* x, float* weight, float
                            const float* grad_partial, void* dx, int dx_dtype, float* db, void* workspace, size_t ws_bytes,
                            int B, int N, long long K, float lr, float beta1, float beta2, float eps, float weight_decay,
                            long long step, void* stream);
+/* The fused step that also reports the gradient's norm (FusedAdam's track_grad_norm): grad_partial NULL is
+ * dd_linear_bwd_adam, non-NULL dd_linear_bwd_adam_acc, with the same results bit for bit (W, moments, dx, db), and in
+ * addition *sumsq = the fp64 sum of g*g over the [N,K] gradient g that the step applies (dy^T x, or dy^T x + grad_partial),
+ * each square exact in fp64 and the sum folded in a fixed order: the same bits on every run.  Only real elements count
+ * (ragged N and K included).  sumsq: device, 8-byte aligned.  sumsq_ws: dd_grad_sumsq_workspace_bytes() bytes (passed as
+ * sumsq_ws_bytes), zeroed by the caller ONCE (self-resetting); calls that share one must be ordered (one stream).  Errors as
+ * dd_linear_bwd_adam's, plus a null sumsq / sumsq_ws: DD_ERR_BAD_ARG; sumsq misaligned: DD_ERR_ALIGNMENT; sumsq_ws too
+ * small: DD_ERR_WORKSPACE. */
+int dd_linear_bwd_adam_sumsq(const float* dy, const float* x, float* weight, float* exp_avg, float* exp_avg_sq,
+                             const float* grad_partial, void* dx, int dx_dtype, float* db, void* workspace, size_t ws_bytes,
+                             int B, int N, long long K, float lr, float beta1, float beta2, float eps, float weight_decay,
+                             long long step, double* sumsq, void* sumsq_ws, size_t sumsq_ws_bytes, void* stream);
 size_t dd_linear_workspace_bytes(int B, int N, long long K);
 /* impl = DD_IMPL_TCGEN05 runs the weight-streaming tensor-core kernels (fp32 operands read as tf32 through
  * TMA; x must be fp32): allowed when this returns 1 (N, K multiples of 4, N*K >= 2^22).  DD_IMPL_AUTO
@@ -330,6 +342,40 @@ int dd_grad_sumsq(const void* const* ptrs, const long long* numels, int count, f
 int dd_adam_step_clipped(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, long long n,
                          float lr, float beta1, float beta2, float eps, float weight_decay, long long step,
                          float grad_scale, const float* coef, void* stream);
+
+/* Gradient norms per parameter (FusedAdam's track_grad_norm, Lightning's grad_norm), without a host round trip.
+ * dd_adam_step_sharded_sumsq: dd_adam_step_sharded with the same results bit for bit, that also writes *sumsq = the fp64
+ * sum of g*g over this rank's shard, g being the gradient exactly as the update consumes it (the sum of the replicas
+ * in the kernel's order, times grad_scale); 0 for an empty shard.  Folded in a fixed order: the same bits on every run.
+ * sumsq: device, 8-byte aligned (e.g. this rank's slot of a symmetric buffer, which the caller's closing barrier publishes
+ * to the peers).  workspace: dd_grad_sumsq_workspace_bytes() bytes, zeroed ONCE (self-resetting); launches that share one
+ * must be ordered.  Errors as dd_adam_step_sharded's, plus a null sumsq / workspace: DD_ERR_BAD_ARG; sumsq misaligned:
+ * DD_ERR_ALIGNMENT; workspace too small: DD_ERR_WORKSPACE. */
+int dd_adam_step_sharded_sumsq(const void* const* grad_replicas, void* const* param_replicas,
+                               const void* mc_grad, void* mc_param, int world, int rank,
+                               float* exp_avg_shard, float* exp_avg_sq_shard, long long shard_offset,
+                               long long shard_numel, float lr, float beta1, float beta2, float eps,
+                               float weight_decay, long long step, float grad_scale, int ctas_per_sm,
+                               double* sumsq, void* workspace, size_t ws_bytes, void* stream);
+/* dd_grad_sumsq_each: one fp64 sum of g*g per tensor, *outs[i] for tensor ptrs[i] / numels[i] (HOST arrays; fp32 tensors
+ * of any length and any 4-byte alignment; outs[i]: device, 8-byte aligned).  Each sum is folded in a fixed order: the same
+ * bits on every run.  Lists longer than 64 tensors take one launch per 64.
+ * dd_grad_sumsq_each_replicas: the same for tensors of a data-parallel flat gradient bucket, whose `world` replicas are
+ * peer-mapped at grad_replicas[k] (HOST array, index = rank, 16-byte aligned): tensor i is elements
+ * [offsets[i], offsets[i] + numels[i]) of the bucket (offsets[i] a multiple of 4), and its gradient is the replicas' sum in
+ * dd_adam_step_sharded's order for an element this rank owns (this rank's replica first, then rank+1, rank+2, ...), times
+ * grad_scale -- so over this rank's shard it is exactly the gradient that rank's sharded update consumes.  The caller puts a
+ * cross-rank barrier before (gradients complete) and keeps the replicas unchanged until every rank's call has finished.
+ * workspace: dd_grad_sumsq_each_workspace_bytes() bytes, zeroed by the caller ONCE (self-resetting); calls that share a
+ * workspace must be ordered.  Errors: a null pointer or negative length: DD_ERR_BAD_ARG; a tensor not 4-byte aligned, an
+ * out not 8-byte aligned, an offset not a multiple of 4 or a replica not 16-byte aligned: DD_ERR_ALIGNMENT; world outside
+ * 1..16 or rank outside the world: DD_ERR_BAD_ARG; workspace too small: DD_ERR_WORKSPACE. */
+size_t dd_grad_sumsq_each_workspace_bytes(void);
+int dd_grad_sumsq_each(const void* const* ptrs, const long long* numels, double* const* outs, int count,
+                       void* workspace, size_t ws_bytes, void* stream);
+int dd_grad_sumsq_each_replicas(const void* const* grad_replicas, int world, int rank, float grad_scale,
+                                const long long* offsets, const long long* numels, double* const* outs, int count,
+                                void* workspace, size_t ws_bytes, void* stream);
 
 #ifdef __cplusplus
 }
